@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — 6DOF env-steps/s of the batched CUDA env step on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one Rocket6DOF env-step for every env of the batch (workload: BASELINE.json configs[2],
 2^20 envs per GPU, uniform random actions, auto-reset on).  Rank 0 prints ONE JSON line:
@@ -15,8 +15,11 @@ A "step" is one Rocket6DOF env-step for every env of the batch (workload: BASELI
   cpu_baseline  the CPU oracle (C restatement, all host threads) on a bounded sample of the workload
 --impl reference times the UNMODIFIED reference env (baseline/_ref) under a SubprocVecEnv-protocol harness on the
 host cores (the Python/SciPy port's and the C oracle's numbers are reported beside it).
+--dump-outputs DIR writes what the last timed step returned (rank 0's envs) as DIR/<name>.npy, so that two builds run
+with the same arguments (same seeds, same inputs) can be compared output for output.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -27,11 +30,13 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 METRIC = "6dof_env_steps_per_sec"
 UNIT = "env-steps/s"
 F_FIX, F_ATT = 985.0, 1850.0          # algorithmic FP64 flops per env-step: 985 + 1850 * attempts (SURVEY §8d)
 BYTES_PER_STEP = 336.0                # algorithmic HBM bytes per env-step (SURVEY §8d)
+DUMP_ENVS = 1 << 19                   # --dump-outputs: 80 B per env (obs, reward, done, flags, index), 42 MB at most
 
 
 def parse():
@@ -55,7 +60,16 @@ def parse():
                     help="cpu_baseline leg of the default run: VecEnv.step calls of the reference env per worker")
     ap.add_argument("--config4-envs", type=int, default=1 << 23,
                     help="envs per GPU of the BASELINE.json configs[3] leg (runs when WORLD_SIZE == 8; 0 = off)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write obs / reward / done / flags of the last timed step for a fixed, "
+                         "seeded sample of at most %d envs (all envs below that), and their indices, as DIR/<name>.npy"
+                         % DUMP_ENVS)
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------
@@ -95,6 +109,11 @@ class ClockSampler:
                                       stderr=subprocess.DEVNULL)
         except Exception:
             self.p = None
+        atexit.register(self._kill)          # a run that fails before stop() leaves no sampler behind
+
+    def _kill(self):
+        if self.p is not None and self.p.poll() is None:
+            self.p.kill()
 
     def stop(self):
         out = {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
@@ -125,6 +144,25 @@ class ClockSampler:
         if sm:
             out.update(sm_mhz=statistics.median(sm), sm_max_mhz=max(mx), reasons=sorted(reasons), samples=len(sm))
         return out
+
+
+def dump_outputs(out_dir, obs, reward, done, flags):
+    """What one Rocket6DOFBatch.step returned (obs [14, N] float32, reward [N] float64, done / flags [N] uint8), for a
+    fixed sample of the envs drawn with a fixed seed, as float32 / float64 .npy files: env_index [m] (float64),
+    obs [m, 14] (float32), reward [m] (float64), done [m] and flags [m] (float32; flags keeps the bit field's value)."""
+    import numpy as np
+    import torch
+    n = reward.shape[0]
+    idx = np.arange(n) if n <= DUMP_ENVS else np.sort(np.random.default_rng(0).choice(n, DUMP_ENVS, replace=False))
+    sel = torch.from_numpy(idx).to(reward.device)
+    arrays = {"env_index": idx.astype(np.float64),
+              "obs": obs[:, sel].t().cpu().numpy(),
+              "reward": reward[sel].cpu().numpy(),
+              "done": done[sel].to(torch.float32).cpu().numpy(),
+              "flags": flags[sel].to(torch.float32).cpu().numpy()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def cpu_oracle_throughput(n_envs, n_steps, threads):
@@ -294,6 +332,8 @@ def run_b200(args):
     e1.record(stream)
     torch.cuda.synchronize()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env.obs, env.reward, env.done, env.flags)
     barrier()
     ms_step = ms_total / K
     value = world * n * K / (ms_total * 1e-3)

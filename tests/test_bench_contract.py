@@ -1,5 +1,6 @@
-"""bench.py contract, CPU side: the reference arm runs without a GPU, prints ONE JSON line with the keys the driver
-reads, and the b200 arm refuses to run without a CUDA device (no CPU fallback)."""
+"""bench.py contract: the reference arm runs without a GPU and prints ONE JSON line with the keys a consumer of the
+line reads, the b200 arm refuses to run without a CUDA device (no CPU fallback), and on the GPU --dump-outputs writes
+the same outputs on every run with the same arguments."""
 import json
 import os
 import subprocess
@@ -35,3 +36,30 @@ def test_b200_arm_needs_a_gpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1"],
                          capture_output=True, text=True, timeout=200)
     assert out.returncode != 0 and "no CPU fallback" in (out.stderr + out.stdout)
+
+
+@pytest.mark.gpu
+@pytest.mark.timeout(900)
+def test_dump_outputs_repeat_exactly(tmp_path):
+    """--dump-outputs writes obs / reward / done / flags of the last timed step as float32 / float64 .npy files, and two
+    runs with the same arguments (seeded inputs) write the same values, so that two builds can be compared output for
+    output."""
+    import numpy as np
+    n, dumps = 4096, []
+    for r in range(2):
+        d = tmp_path / f"run{r}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "1",
+                              "--envs", str(n), "--preroll", "200", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=800)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == 3
+        dumps.append({p.stem: np.load(p) for p in d.glob("*.npy")})
+    a, b = dumps
+    assert sorted(a) == ["done", "env_index", "flags", "obs", "reward"]
+    assert a["obs"].shape == (n, 14) and a["obs"].dtype == np.float32 and a["reward"].dtype == np.float64
+    assert np.array_equal(a["env_index"], np.arange(n))
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64) and a[k].shape[0] == n, k
+        assert np.array_equal(a[k], b[k]), k
+    assert np.isfinite(a["obs"]).all() and a["done"].any()
