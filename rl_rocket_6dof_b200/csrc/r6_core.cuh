@@ -1582,8 +1582,30 @@ R6_HD void mlp_policy(const float *W, const float *x, float &a0, float &a1, floa
     a2 = fminf(fmaxf(out[2], -1.0f), 1.0f);
 }
 
+// sin(pi x), cos(pi x): exact argument reduction, 1 ulp (CUDA math library); the host build in double precision
+R6_HD void sincospi_f32(float x, float &s, float &c)
+{
+#if defined(__CUDA_ARCH__)
+    sincospif(x, &s, &c);
+#else
+    s = (float)sin(3.141592653589793 * (double)x);
+    c = (float)cos(3.141592653589793 * (double)x);
+#endif
+}
+R6_HD float cospi_f32(float x)
+{
+#if defined(__CUDA_ARCH__)
+    return cospif(x);
+#else
+    return (float)cos(3.141592653589793 * (double)x);
+#endif
+}
+
 // Gaussian policy head (SB3 DiagGaussianDistribution with a state-independent log_std): sample and log-probability.
-// eps from one Philox block keyed (seed, global env, step) through Box-Muller.
+// eps from one Philox block keyed (seed, global env, step) through Box-Muller, with the accurate logf (1 ulp) and
+// sincospif / cospif (1 ulp) on both builds: z is good to 3 ulp everywhere.  Not the MUFU forms __logf / __sincosf:
+// their error is absolute, as large as ln u itself where u -> 1 (the radius off by a fifth), and above their
+// documented accuracy elsewhere (tests/test_gpu_policy_ref.py measures the noise against a float64 statement).
 constexpr uint32_t kStreamPolicy = 0x50414354u;   // 'PACT'
 R6_HD void gaussian_head(const float (&mean)[4], const float *log_std, bool stochastic, uint64_t seed, uint64_t genv,
                          uint64_t step, float (&raw)[3], float &logp)
@@ -1595,20 +1617,14 @@ R6_HD void gaussian_head(const float (&mean)[4], const float *log_std, bool stoc
         const float s = 1.0f / 4294967296.0f;
         const float u1 = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)r.y * s;
         const float u3 = ((float)(r.z >> 8) + 0.5f) * (1.0f / 16777216.0f), u4 = (float)r.w * s;
-#if defined(__CUDA_ARCH__)
-        // MUFU log / sin / cos: the arguments are in [0, 2 pi) and (0, 1], where the fast units are good to ~1e-6
-        const float ra = sqrtf(-2.0f * __logf(u1)), rb = sqrtf(-2.0f * __logf(u3));
+        // u1, u3 in (0, 1] (1.0 for the top grid value: k + 0.5 rounds to even): logf <= 0, so the roots are real.
+        // The angles 2 pi u2, 2 pi u4 are formed exactly as pi * (2 u).
+        const float ra = sqrtf(-2.0f * logf(u1)), rb = sqrtf(-2.0f * logf(u3));
         float sn, cs;
-        __sincosf(6.283185307179586f * u2, &sn, &cs);
+        sincospi_f32(2.0f * u2, sn, cs);
         z[0] = ra * cs;
         z[1] = ra * sn;
-        z[2] = rb * __cosf(6.283185307179586f * u4);
-#else
-        const float ra = sqrtf(-2.0f * logf(u1)), rb = sqrtf(-2.0f * logf(u3));
-        z[0] = ra * cosf(6.283185307179586f * u2);
-        z[1] = ra * sinf(6.283185307179586f * u2);
-        z[2] = rb * cosf(6.283185307179586f * u4);
-#endif
+        z[2] = rb * cospi_f32(2.0f * u4);
     }
     logp = 0.0f;
 #pragma unroll

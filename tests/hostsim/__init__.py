@@ -51,6 +51,9 @@ def lib():
         L.hs_philox_action.argtypes = [C.c_uint64] * 3 + [C.c_void_p]
         L.hs_mlp_pack.argtypes = [C.c_void_p, C.c_void_p]
         L.hs_mlp.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+        L.hs_mlp_forward.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+        L.hs_gaussian_head.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_uint64, C.c_void_p, C.c_void_p, C.c_int64,
+                                       C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -81,16 +84,46 @@ class HostSimBatch:
         return self.outs
 
 
-def mlp_actions(weights, obs13):
-    """Fused-policy network of the kernels (host build) on packed weights: obs [n,13] f32 -> actions [n,3]."""
-    from rl_rocket_6dof_b200._lib import R6Mlp
+def _packed(weights):
+    from rl_rocket_6dof_b200._lib import make_mlp
     L = lib()
     w = {k: np.ascontiguousarray(v, np.float32) for k, v in weights.items()}
-    from rl_rocket_6dof_b200._lib import make_mlp
     m = make_mlp(w)
     W = np.zeros(L.hs_mlp_floats(), np.float32)
     L.hs_mlp_pack(C.byref(m), W.ctypes.data)
+    return W
+
+
+def mlp_actions(weights, obs13):
+    """Fused-policy network of the kernels (host build) on packed weights: obs [n,13] f32 -> actions [n,3]."""
+    W = _packed(weights)
     x = np.ascontiguousarray(obs13, np.float32).reshape(-1, 13)
     out = np.zeros((len(x), 3), np.float32)
-    L.hs_mlp(W.ctypes.data, x.ctypes.data, len(x), out.ctypes.data)
+    lib().hs_mlp(W.ctypes.data, x.ctypes.data, len(x), out.ctypes.data)
     return out
+
+
+def mlp_forward(weights, obs13):
+    """Raw outputs of the same network: (unclipped mean [n,3], value [n]; 0 without a critic head)."""
+    W = _packed(weights)
+    x = np.ascontiguousarray(obs13, np.float32).reshape(-1, 13)
+    out = np.zeros((len(x), 4), np.float32)
+    lib().hs_mlp_forward(W.ctypes.data, x.ctypes.data, len(x), out.ctypes.data)
+    return out[:, :3], out[:, 3]
+
+
+def gaussian_head(mean, log_std, stochastic, seed, genv, step):
+    """Host build of the kernels' Gaussian policy head: (raw action [n,3], log-prob [n]) for mean [n,3] and per-row
+    global env ids / step indices (uint64)."""
+    mean = np.asarray(mean, np.float32).reshape(-1, 3)
+    n = len(mean)
+    m4 = np.zeros((n, 4), np.float32)
+    m4[:, :3] = mean
+    g = np.ascontiguousarray(np.broadcast_to(np.asarray(genv, np.uint64), (n,)))
+    s = np.ascontiguousarray(np.broadcast_to(np.asarray(step, np.uint64), (n,)))
+    ls = None if log_std is None else np.ascontiguousarray(log_std, np.float32)
+    raw = np.zeros((n, 3), np.float32)
+    logp = np.zeros(n, np.float32)
+    lib().hs_gaussian_head(m4.ctypes.data, None if ls is None else ls.ctypes.data, int(bool(stochastic)), int(seed),
+                           g.ctypes.data, s.ctypes.data, n, raw.ctypes.data, logp.ctypes.data)
+    return raw, logp

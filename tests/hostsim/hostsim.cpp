@@ -133,6 +133,28 @@ void hs_mlp(const float *W, const float *obs13, int64_t n, float *actions)
     for (int64_t i = 0; i < n; i++) mlp_policy(W, obs13 + 13 * i, actions[3 * i], actions[3 * i + 1], actions[3 * i + 2]);
 }
 
+// raw network outputs (out[4 i .. 4 i + 3] = unclipped mean, value) of the float32 FMA network
+void hs_mlp_forward(const float *W, const float *obs13, int64_t n, float *out4)
+{
+    for (int64_t i = 0; i < n; i++) {
+        float o[4];
+        mlp_forward(W, obs13 + 13 * i, o);
+        for (int c = 0; c < 4; c++) out4[4 * i + c] = o[c];
+    }
+}
+
+// Gaussian policy head per row: mean4 [n][4] (value column ignored), genv / step [n], log_std [3] or NULL
+void hs_gaussian_head(const float *mean4, const float *log_std, int32_t stochastic, uint64_t seed, const uint64_t *genv,
+                      const uint64_t *step, int64_t n, float *raw3, float *logp)
+{
+    for (int64_t i = 0; i < n; i++) {
+        const float m[4] = {mean4[4 * i], mean4[4 * i + 1], mean4[4 * i + 2], mean4[4 * i + 3]};
+        float raw[3];
+        gaussian_head(m, log_std, stochastic != 0, seed, genv[i], step[i], raw, logp[i]);
+        for (int c = 0; c < 3; c++) raw3[3 * i + c] = raw[c];
+    }
+}
+
 void hs_philox_action(uint64_t seed, uint64_t genv, uint64_t step, float a[3]) { philox_action(seed, genv, step, a[0], a[1], a[2]); }
 
 }  // extern "C"

@@ -436,16 +436,17 @@ def test_collect_rollout_in_place_trajectory_equals_step_by_step(lanes, auto_res
     b = Rocket6DOFBatch(n, **kw)
     a.reset(); b.reset()
     ro = a.collect_rollout(k, wd, stochastic=True)
-    obs, rew, dn, val, act = [], [], [], [], []
+    obs, rew, dn, val, act, lps = [], [], [], [], [], []
     for j in range(k):
         obs.append(b.obs[:13].t().clone())
         ae, raw, v, lp = b.policy_forward(wd, stochastic=True, tensor_cores=3)
         b.step(ae)
-        act.append(raw.clone()); val.append(v.clone()); rew.append(b.reward_f32.clone()); dn.append(b.done.clone())
+        act.append(raw.clone()); val.append(v.clone()); lps.append(lp.clone())
+        rew.append(b.reward_f32.clone()); dn.append(b.done.clone())
     torch.cuda.synchronize()
     assert torch.equal(ro["obs"], torch.stack(obs)) and torch.equal(ro["actions"], torch.stack(act))
     assert torch.equal(ro["values"], torch.stack(val)) and torch.equal(ro["rewards"], torch.stack(rew))
-    assert torch.equal(ro["dones"], torch.stack(dn))
+    assert torch.equal(ro["dones"], torch.stack(dn)) and torch.equal(ro["log_probs"], torch.stack(lps))
     assert torch.equal(a.obs, b.obs) and torch.equal(a.reward_f32, b.reward_f32) and torch.equal(a.done, b.done)
     assert torch.equal(a.state, b.state) and torch.equal(a.stats, b.stats)
     if not auto_reset:
