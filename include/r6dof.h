@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 16
+#define R6_ABI_VERSION 17
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -298,6 +298,76 @@ int r6_policy_range(const R6Mlp *mlp, const float *obs, int64_t n, int64_t first
  */
 int r6_gae(const float *rew, const float *values, const uint8_t *done, const float *last_values, int32_t T, int64_t n,
            double gamma, double gae_lambda, float *adv, float *ret, void *stream);
+
+/*
+ * PPO update (stable-baselines3 1.6.0 `PPO.train`, the optimiser of main_6DOF.py:136).
+ *
+ * Flat parameter vector of the actor-critic, R6_PPO_NPARAMS float32 in SB3 [out][in] order:
+ *     w0 [128][13] @0, b0 [128] @1664, w1 [64][128] @1792, b1 [64] @9984, w2 [3][64] @10048, b2 [3] @10240,
+ *     wv [64] @10243, bv [1] @10307, log_std [3] @10308
+ * (w1 starts at float 1792 so that an R6Mlp pointing into a 16-byte aligned buffer keeps w1 16-byte aligned, as
+ * r6_policy tensor_cores = 2 / 3 need).
+ */
+#define R6_PPO_NPARAMS 10311
+#define R6_PPO_NTERMS 5
+/* terms[] slots of r6_ppo_grad (float64 sums over the minibatch) */
+enum { R6_PPO_T_PG = 0, R6_PPO_T_VLOSS, R6_PPO_T_CLIPPED, R6_PPO_T_APPROX_KL, R6_PPO_T_BAD_INDEX };
+
+/* The [T][n] trajectory of a collected rollout; sample s = t * n + i. */
+typedef struct R6PpoRollout {
+    const float *obs;        /* observation component c of (t, i) at obs[t * obs_stride_step + c * obs_stride_comp +
+                                i * obs_stride_env] (element strides): the strided [T, n, 13] view of the in-place
+                                [T + 1][14][n] collection buffer and a dense [T][n][13] array are both accepted */
+    int64_t obs_stride_step, obs_stride_comp, obs_stride_env;
+    const float *actions;    /* [T][n][3] raw (unclipped) Gaussian samples */
+    const float *log_probs;  /* [T][n] log-probabilities at collection */
+    const float *advantages; /* [T][n] */
+    const float *returns;    /* [T][n] */
+    int64_t T, n;
+} R6PpoRollout;
+
+typedef struct R6PpoCoef {
+    double clip_range, vf_coef, ent_coef;
+    const double *adv_stats; /* DEVICE [2] = (mean, 1 / (std + 1e-8)) of the minibatch's advantages, or NULL = no
+                                normalisation.  A device pointer, so that no minibatch has to synchronise */
+} R6PpoCoef;
+
+typedef struct R6AdamCoef {
+    double lr, beta1, beta2, eps;
+    double max_grad_norm;    /* clip_grad_norm_(max_grad_norm) on the scaled gradient; <= 0: no clipping */
+    double scale;            /* g = scale * grad_sum (1 / minibatch size turns r6_ppo_grad's sum into the mean) */
+} R6AdamCoef;
+
+int r6_ppo_rollout_size(void);
+int r6_ppo_coef_size(void);
+int r6_adam_coef_size(void);
+
+/* Size of r6_ppo_grad's work buffer for a minibatch of B samples (DEVICE bytes, no initialisation needed). */
+int64_t r6_ppo_work_bytes(int64_t B);
+
+/*
+ * Sum over the minibatch idx[0..B) (int64 sample indices s = t * n + i, any order, duplicates allowed) of the
+ * per-sample gradient of SB3 1.6's PPO loss
+ *     -min(A' ratio, A' clip(ratio, 1 - clip_range, 1 + clip_range)) + vf_coef (R - V)^2 - ent_coef entropy,
+ * ratio = exp(logp(actions) - log_probs), A' the (optionally normalised) advantage, into grad_sum [R6_PPO_NPARAMS]
+ * (flat layout above), and the loss-term sums into terms [R6_PPO_NTERMS] float64: policy-gradient loss, value loss
+ * (R - V)^2, the number of samples with |ratio - 1| > clip_range, (ratio - 1) - log ratio, and the number of indices
+ * outside [0, T n) (those samples are skipped).  mlp must carry wv, bv and log_std.  Sums, not means: the caller scales.
+ * The launch shape depends on B only, so the result is bit-reproducible on any device.
+ */
+int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *idx, int64_t B, const R6PpoCoef *coef,
+                float *grad_sum, double *terms, void *work, void *stream);
+
+/*
+ * One torch.optim.Adam step (no weight decay, no amsgrad) on the flat parameters, after clip_grad_norm_:
+ *     g = scale * grad_sum;  norm = ||g||_2 (accumulated in float64);  g *= min(1, max_grad_norm / (norm + 1e-6));
+ *     m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g^2;
+ *     p -= lr / (1 - beta1^step) * m / (sqrt(v) / sqrt(1 - beta2^step) + eps)
+ * params, grad_sum, m, v: float32 [P] DEVICE; step >= 1 counts the updates including this one; grad_norm_out
+ * (nullable DEVICE double) receives the norm before clipping.
+ */
+int r6_adam_step(float *params, const float *grad_sum, float *m, float *v, int64_t P, const R6AdamCoef *coef,
+                 int64_t step, double *grad_norm_out, void *stream);
 
 /* Zeroes stats[8] (asynchronously, on the stream). */
 int r6_stats_reset(double *stats, void *stream);

@@ -9,11 +9,14 @@ GPU raises — there is no CPU path):
     Rocket6DOF                          single-env gym contract of the reference
     make_env / make_vec_env             what main_6DOF.py:44-53 builds, batched
     TrajectoryRecorder                  [T, N] record of states / actions / times (SIM.states, .actions, .times)
+    ActorCriticParams, PPOConfig,       PPO training on the device (SB3 1.6 PPO.train / learn): flat actor-critic
+    PPOTrainer                          parameters, hyper-parameters, collect + update loop
 """
 from .params import EnvParams, derive_params, load_config  # noqa: F401
 
 __all__ = ["EnvParams", "derive_params", "load_config", "Rocket6DOFBatch", "Rocket6DOFVecEnv", "Rocket6DOF",
-           "make_env", "make_vec_env", "make_annealed_env", "make_annealed_vec_env", "TrajectoryRecorder"]
+           "make_env", "make_vec_env", "make_annealed_env", "make_annealed_vec_env", "TrajectoryRecorder",
+           "ActorCriticParams", "PPOConfig", "PPOTrainer"]
 
 
 def __getattr__(name):  # lazy: params are usable without torch / CUDA
@@ -29,6 +32,9 @@ def __getattr__(name):  # lazy: params are usable without torch / CUDA
     if name == "TrajectoryRecorder":
         from .recorder import TrajectoryRecorder
         return TrajectoryRecorder
+    if name in ("ActorCriticParams", "PPOConfig", "PPOTrainer"):
+        from . import ppo
+        return getattr(ppo, name)
     if name in ("make_env", "make_vec_env", "make_annealed_env", "make_annealed_vec_env"):
         from . import factory
         return getattr(factory, name)

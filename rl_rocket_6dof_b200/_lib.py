@@ -12,7 +12,7 @@ from .params import R6Params
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libr6dof.so")
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 u8p = C.c_void_p
 
@@ -41,6 +41,25 @@ class R6Mlp(C.Structure):
                 ("wv", C.c_void_p), ("bv", C.c_void_p), ("log_std", C.c_void_p)]     # nullable: critic head, Gaussian log-std
 
 
+class R6PpoRollout(C.Structure):
+    _fields_ = [("obs", C.c_void_p), ("obs_stride_step", C.c_int64), ("obs_stride_comp", C.c_int64),
+                ("obs_stride_env", C.c_int64), ("actions", C.c_void_p), ("log_probs", C.c_void_p),
+                ("advantages", C.c_void_p), ("returns", C.c_void_p), ("T", C.c_int64), ("n", C.c_int64)]
+
+
+class R6PpoCoef(C.Structure):
+    _fields_ = [("clip_range", C.c_double), ("vf_coef", C.c_double), ("ent_coef", C.c_double), ("adv_stats", C.c_void_p)]
+
+
+class R6AdamCoef(C.Structure):
+    _fields_ = [("lr", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double),
+                ("max_grad_norm", C.c_double), ("scale", C.c_double)]
+
+
+PPO_NPARAMS = 10311
+PPO_NTERMS = 5
+
+
 def make_mlp(weights: dict) -> "R6Mlp":
     """R6Mlp from a dict of tensors / arrays exposing data_ptr() or ctypes.data (optional keys: wv, bv, log_std)."""
     def ptr(x):
@@ -53,7 +72,8 @@ def make_mlp(weights: dict) -> "R6Mlp":
 
 
 EXPORTS = ["r6_abi_version", "r6_last_error", "r6_params_size", "r6_buffers_size", "r6_reset", "r6_step",
-           "r6_rollout", "r6_sim_step_raw", "r6_tgo", "r6_stats_reset", "r6_peak_fma", "r6_gae", "r6_policy", "r6_policy_ex", "r6_step_random", "r6_step_range", "r6_policy_range", "r6_work_bytes"]
+           "r6_rollout", "r6_sim_step_raw", "r6_tgo", "r6_stats_reset", "r6_peak_fma", "r6_gae", "r6_policy", "r6_policy_ex", "r6_step_random", "r6_step_range", "r6_policy_range", "r6_work_bytes",
+           "r6_ppo_rollout_size", "r6_ppo_coef_size", "r6_adam_coef_size", "r6_ppo_work_bytes", "r6_ppo_grad", "r6_adam_step"]
 
 
 class R6Error(RuntimeError):
@@ -87,6 +107,9 @@ def load(path: str | None = None):
         raise R6Error(f"R6Params layout mismatch: C {L.r6_params_size()} vs ctypes {C.sizeof(R6Params)}")
     if L.r6_buffers_size() != C.sizeof(R6Buffers):
         raise R6Error(f"R6Buffers layout mismatch: C {L.r6_buffers_size()} vs ctypes {C.sizeof(R6Buffers)}")
+    for name, st in (("r6_ppo_rollout_size", R6PpoRollout), ("r6_ppo_coef_size", R6PpoCoef), ("r6_adam_coef_size", R6AdamCoef)):
+        if getattr(L, name)() != C.sizeof(st):
+            raise R6Error(f"{st.__name__} layout mismatch: C {getattr(L, name)()} vs ctypes {C.sizeof(st)}")
     pp, bp = C.POINTER(R6Params), C.POINTER(R6Buffers)
     L.r6_reset.argtypes = [pp, bp, C.c_int64, C.c_int64, C.c_void_p, C.c_uint64, C.c_void_p]
     L.r6_step.argtypes = [pp, bp, C.c_int64, C.c_int64, C.c_void_p, C.c_uint64, C.c_void_p]
@@ -108,6 +131,12 @@ def load(path: str | None = None):
     L.r6_policy.argtypes = [C.POINTER(R6Mlp), C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
     L.r6_gae.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_double, C.c_double,
                          C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_ppo_work_bytes.argtypes = [C.c_int64]
+    L.r6_ppo_work_bytes.restype = C.c_int64
+    L.r6_ppo_grad.argtypes = [C.POINTER(R6Mlp), C.POINTER(R6PpoRollout), C.c_void_p, C.c_int64, C.POINTER(R6PpoCoef),
+                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_adam_step.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(R6AdamCoef), C.c_int64,
+                               C.c_void_p, C.c_void_p]
     L.r6_peak_fma.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
     _lib = L
     return L

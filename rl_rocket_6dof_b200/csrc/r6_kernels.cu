@@ -10,6 +10,7 @@
 //   rollout_kernel, rollout_tc_kernel  k steps per launch with the state in registers (Philox / buffer / policy)
 //   policy_kernel, policy_tc5_kernel   the policy MLP alone: float32 FMAs, mma.sync 3xTF32 tiles, or tcgen05.mma with
 //                                    accumulators and activations in TMEM (r6_mlp_tc.cuh, r6_mlp_tcgen05.cuh)
+//   ppo_grad_kernel | ppo_reduce_kernel, adam_kernel   the PPO update: minibatch loss gradient, Adam step
 //   reset_kernel, sim_raw_kernel, tgo_kernel, gae_kernel, peak_fma_kernel
 //
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo (see build.py).
@@ -25,6 +26,7 @@
 #include "r6_core.cuh"
 #include "r6_mlp_tc.cuh"
 #include "r6_mlp_tcgen05.cuh"
+#include "r6_ppo.cuh"
 
 namespace {
 
@@ -897,6 +899,239 @@ gae_kernel(const float *__restrict__ rew, const float *__restrict__ values, cons
     }
 }
 
+// PPO minibatch gradient (r6_ppo_grad).  A grid of ppo_ctas(B) CTAs (a function of B only, so the summation order and
+// the result do not depend on the device) walks tiles of 128 samples.  Each thread runs the forward pass, loss head
+// and deltas of its sample (r6_ppo.cuh) and stages its inputs, activations and deltas in shared memory unit-major,
+// [unit][sample]; the CTA then accumulates the weight gradients cooperatively into register accumulators that live
+// across all its tiles: dW1 (64 x 128) as an 8 x 8 block per thread, dW0 with db0 (128 x 14) one row per thread, the
+// heads (dW2, dwv, db1) on threads 0..63 and the scalar sums on 64..75.  Every accumulator adds its samples in tile
+// order, one fma per sample.  The dW1 block is parked in shared memory between tiles (registers would spill).  Each CTA writes one partial [P] and its float64 term sums into the work buffer, and
+// ppo_reduce_kernel adds the partials in CTA order.
+constexpr int kPpoTS = kThreads + 4;   // row stride of the [unit][sample] tiles: 16-byte rows, conflict-free float4 reads
+constexpr int kPpoRowH0 = 0, kPpoRowH1 = 128, kPpoRowD1 = 192, kPpoRowX = 256, kPpoRowG = 272, kPpoRowT = 280;
+constexpr int kPpoRows = 284;          // h0 (then delta0) 128, h1 64, delta1 64, x 16, head gradients + bad-index flag 8,
+                                       // loss terms 4
+constexpr int kPpoAccW1 = kMlpH1 * kMlpH0;     // dW1 accumulators, [r * 8 + c][thread]
+constexpr int kSmemPpo = (kMlpFloats + kPpoRows * kPpoTS + kPpoAccW1) * (int)sizeof(float);   // 224,976 B: 1 CTA per SM
+constexpr int kPpoMaxCtas = 148;
+static_assert(kThreads == 128 && kMlpFloats % 4 == 0 && kPpoRowG + 8 == kPpoRowT, "PPO tile layout");
+int64_t ppo_ctas(int64_t B)
+{
+    const int64_t tiles = (B + kThreads - 1) / kThreads;
+    return tiles < kPpoMaxCtas ? tiles : kPpoMaxCtas;
+}
+
+__global__ void __launch_bounds__(kThreads, 1)
+ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restrict__ idx, int64_t B, float clip, float vf,
+                float ent, const double *__restrict__ adv_stats, double *__restrict__ part_terms, float *__restrict__ part)
+{
+    extern __shared__ __align__(16) double r6_smem[];
+    float *Ws = reinterpret_cast<float *>(r6_smem);
+    float *S = Ws + kMlpFloats;
+    float *A1 = S + kPpoRows * kPpoTS;
+    const int tid = threadIdx.x, kq = tid & 7, jq = tid >> 3;
+    for (int i = tid; i < kMlpFloats; i += kThreads) Ws[i] = mlp_pack_element(mlp, i);
+    for (int i = tid; i < kPpoAccW1; i += kThreads) A1[i] = 0.0f;
+    const int64_t nsamp = ro.T * ro.n;
+    float aW0[14], aHd[5];                   // dW0[tid][0..12], db0[tid]; dW2[0..2][tid], dwv, db1
+    double aS = 0.0;                         // thread 64 + r: sum of row kPpoRowG + r
+#pragma unroll
+    for (int c = 0; c < 14; c++) aW0[c] = 0.0f;
+#pragma unroll
+    for (int c = 0; c < 5; c++) aHd[c] = 0.0f;
+    __syncthreads();
+    const int64_t tiles = (B + kThreads - 1) / kThreads;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        {   // this thread's sample: forward, loss head, delta1 (a slot past B or with a bad index contributes zeros)
+            const int64_t s = tile * kThreads + tid;
+            const int64_t q = s < B ? idx[s] : -1;
+            const bool ok = q >= 0 && q < nsamp;
+            float x[kMlpIn], out[4];
+            if (ok) {
+                const int64_t t = q / ro.n, i = q - t * ro.n;
+                const float *o = ro.obs + t * ro.obs_stride_step + i * ro.obs_stride_env;
+#pragma unroll
+                for (int c = 0; c < kMlpIn; c++) x[c] = o[c * ro.obs_stride_comp];
+            } else {
+#pragma unroll
+                for (int c = 0; c < kMlpIn; c++) x[c] = 0.0f;
+            }
+#pragma unroll
+            for (int c = 0; c < kMlpIn; c++) S[(kPpoRowX + c) * kPpoTS + tid] = x[c];
+            ppo_forward(Ws, x, S + kPpoRowH0 * kPpoTS + tid, S + kPpoRowH1 * kPpoTS + tid, kPpoTS, out);
+            PpoHead hd = {};
+            if (ok) {
+                const float a[3] = {ro.actions[3 * q], ro.actions[3 * q + 1], ro.actions[3 * q + 2]};
+                ppo_head(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], mlp.log_std, clip, vf,
+                         ent, hd);
+            }
+            ppo_delta1(Ws, hd, S + kPpoRowH1 * kPpoTS + tid, S + kPpoRowD1 * kPpoTS + tid, kPpoTS);
+#pragma unroll
+            for (int r = 0; r < 7; r++) S[(kPpoRowG + r) * kPpoTS + tid] = hd.g[r];
+            S[(kPpoRowG + 7) * kPpoTS + tid] = (s < B && !ok) ? 1.0f : 0.0f;
+            S[(kPpoRowT + 0) * kPpoTS + tid] = hd.pg;
+            S[(kPpoRowT + 1) * kPpoTS + tid] = hd.vloss;
+            S[(kPpoRowT + 2) * kPpoTS + tid] = hd.clipped;
+            S[(kPpoRowT + 3) * kPpoTS + tid] = hd.kl;
+        }
+        __syncthreads();
+        // dW1 += delta1^T h0 (every thread: dW1[kq + 8 r][jq + 16 c], in two halves of r), heads and scalar sums
+#pragma unroll 1
+        for (int r0 = 0; r0 < 8; r0 += 4) {
+            float aW1[4][8];
+#pragma unroll
+            for (int r = 0; r < 4; r++)
+#pragma unroll
+                for (int c = 0; c < 8; c++) aW1[r][c] = A1[((r0 + r) * 8 + c) * kThreads + tid];
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                F4 h[8];
+#pragma unroll
+                for (int c = 0; c < 8; c++) h[c] = ld4(S + (kPpoRowH0 + jq + 16 * c) * kPpoTS + s4);
+#pragma unroll
+                for (int r = 0; r < 4; r++) {
+                    const F4 d = ld4(S + (kPpoRowD1 + kq + 8 * (r0 + r)) * kPpoTS + s4);
+#pragma unroll
+                    for (int c = 0; c < 8; c++) {
+                        float a = aW1[r][c];
+                        a = __fmaf_rn(d.x, h[c].x, a); a = __fmaf_rn(d.y, h[c].y, a);
+                        a = __fmaf_rn(d.z, h[c].z, a); a = __fmaf_rn(d.w, h[c].w, a);
+                        aW1[r][c] = a;
+                    }
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < 4; r++)
+#pragma unroll
+                for (int c = 0; c < 8; c++) A1[((r0 + r) * 8 + c) * kThreads + tid] = aW1[r][c];
+        }
+        if (tid < kMlpH1) {
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                const F4 hv = ld4(S + (kPpoRowH1 + tid) * kPpoTS + s4), dv = ld4(S + (kPpoRowD1 + tid) * kPpoTS + s4);
+#pragma unroll
+                for (int c = 0; c < 4; c++) {
+                    const F4 g = ld4(S + (kPpoRowG + c) * kPpoTS + s4);
+                    float a = aHd[c];
+                    a = __fmaf_rn(g.x, hv.x, a); a = __fmaf_rn(g.y, hv.y, a);
+                    a = __fmaf_rn(g.z, hv.z, a); a = __fmaf_rn(g.w, hv.w, a);
+                    aHd[c] = a;
+                }
+                aHd[4] = (((aHd[4] + dv.x) + dv.y) + dv.z) + dv.w;
+            }
+        } else if (tid < kMlpH1 + 12) {
+            const float *row = S + (kPpoRowG + tid - kMlpH1) * kPpoTS;
+#pragma unroll 4
+            for (int s = 0; s < kThreads; s++) aS += (double)row[s];
+        }
+        __syncthreads();
+        {   // delta0 over h0, in place: this thread's column only
+            float d1[kMlpH1];
+#pragma unroll
+            for (int k = 0; k < kMlpH1; k++) d1[k] = S[(kPpoRowD1 + k) * kPpoTS + tid];
+#pragma unroll 1
+            for (int j = 0; j < kMlpH0; j++) {
+                float *p = S + (kPpoRowH0 + j) * kPpoTS + tid;
+                *p = ppo_delta0(Ws, j, d1, *p);
+            }
+        }
+        __syncthreads();
+        // dW0[tid] += delta0_tid [x, 1]
+#pragma unroll 1
+        for (int s4 = 0; s4 < kThreads; s4 += 4) {
+            const F4 d = ld4(S + (kPpoRowH0 + tid) * kPpoTS + s4);
+#pragma unroll
+            for (int c = 0; c < kMlpIn; c++) {
+                const F4 xv = ld4(S + (kPpoRowX + c) * kPpoTS + s4);
+                float a = aW0[c];
+                a = __fmaf_rn(d.x, xv.x, a); a = __fmaf_rn(d.y, xv.y, a);
+                a = __fmaf_rn(d.z, xv.z, a); a = __fmaf_rn(d.w, xv.w, a);
+                aW0[c] = a;
+            }
+            aW0[13] = (((aW0[13] + d.x) + d.y) + d.z) + d.w;
+        }
+        __syncthreads();
+    }
+    float *P = part + (int64_t)blockIdx.x * kPpoParams;
+#pragma unroll
+    for (int r = 0; r < 8; r++)
+#pragma unroll
+        for (int c = 0; c < 8; c++) P[kPpoOffW1 + (kq + 8 * r) * kMlpH0 + jq + 16 * c] = A1[(r * 8 + c) * kThreads + tid];
+#pragma unroll
+    for (int c = 0; c < kMlpIn; c++) P[kPpoOffW0 + tid * kMlpIn + c] = aW0[c];
+    P[kPpoOffB0 + tid] = aW0[13];
+    if (tid < kMlpH1) {
+#pragma unroll
+        for (int c = 0; c < 3; c++) P[kPpoOffW2 + c * kMlpH1 + tid] = aHd[c];
+        P[kPpoOffWv + tid] = aHd[3];
+        P[kPpoOffB1 + tid] = aHd[4];
+    } else if (tid < kMlpH1 + 12) {
+        const int r = tid - kMlpH1;          // rows: g0..g2 (db2), g3 (dbv), g4..g6 (dlog_std), bad index, 4 loss terms
+        double *T = part_terms + (int64_t)blockIdx.x * R6_PPO_NTERMS;
+        if (r < 3) P[kPpoOffB2 + r] = (float)aS;
+        else if (r == 3) P[kPpoOffBv] = (float)aS;
+        else if (r < 7) P[kPpoOffLogStd + r - 4] = (float)aS;
+        else if (r == 7) T[R6_PPO_T_BAD_INDEX] = aS;
+        else T[r - 8] = aS;
+    }
+}
+
+// grad[p] = sum of the CTA partials in CTA order (float64, rounded once); terms likewise
+__global__ void __launch_bounds__(256)
+ppo_reduce_kernel(const double *__restrict__ part_terms, const float *__restrict__ part, int G, float *__restrict__ grad,
+                  double *__restrict__ terms)
+{
+    const int p = blockIdx.x * 256 + threadIdx.x;
+    if (p < kPpoParams) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += (double)part[(int64_t)g * kPpoParams + p];
+        grad[p] = (float)s;
+    }
+    if (blockIdx.x == 0 && threadIdx.x < R6_PPO_NTERMS) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += part_terms[g * R6_PPO_NTERMS + threadIdx.x];
+        terms[threadIdx.x] = s;
+    }
+}
+
+// r6_adam_step: one CTA (P is ~10^4).  The squared norm is summed in float64 in a fixed order (strided per thread,
+// then a fixed warp-shuffle tree, then the 32 warp sums in order), so the step is deterministic.
+constexpr int kAdamThreads = 1024;
+struct AdamArgs {
+    float scale, c[6];
+    double max_norm;
+};
+__global__ void __launch_bounds__(kAdamThreads, 1)
+adam_kernel(float *__restrict__ p, const float *__restrict__ gs, float *__restrict__ m, float *__restrict__ v, int P,
+            const AdamArgs a, double *__restrict__ norm_out)
+{
+    __shared__ double red[kAdamThreads / 32];
+    __shared__ float coef_s;
+    double s = 0.0;
+    for (int i = threadIdx.x; i < P; i += kAdamThreads) {
+        const double g = (double)(a.scale * gs[i]);
+        s = fma(g, g, s);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int w = 0; w < kAdamThreads / 32; w++) t += red[w];
+        const double norm = sqrt(t);
+        coef_s = clip_coef(a.max_norm, norm);
+        if (norm_out) *norm_out = norm;
+    }
+    __syncthreads();
+    const float coef = coef_s;
+    for (int i = threadIdx.x; i < P; i += kAdamThreads) {
+        float pi = p[i], mi = m[i], vi = v[i];
+        adam_element(pi, mi, vi, __fmul_rn(a.scale * gs[i], coef), a.c);
+        p[i] = pi; m[i] = mi; v[i] = vi;
+    }
+}
+
 // FMA-pipe micro-benchmark: 8 independent chains per thread
 template <typename T>
 __global__ void __launch_bounds__(256) peak_fma_kernel(int iters, double *sink)
@@ -957,6 +1192,7 @@ int ensure_attributes()
     rc |= enable_smem(policy_kernel<false>, kSmemPolicy);
     rc |= enable_smem(policy_tc5_kernel<true>, tc5::kSmemBytes);
     rc |= enable_smem(policy_tc5_kernel<false>, tc5::kSmemBytes);
+    rc |= enable_smem(ppo_grad_kernel, kSmemPpo);
     rc |= enable_smem(sim_raw_kernel<false>);
     rc |= enable_smem(sim_raw_kernel<true>);
     if (rc) return R6_ECUDA;
@@ -1240,6 +1476,60 @@ int r6_gae(const float *rew, const float *values, const uint8_t *done, const flo
     gae_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rew, values, done, last_values, T, n, (float)gamma,
                                                                           (float)(gamma * gae_lambda), adv, ret);
     return check_launch("r6_gae");
+}
+
+int r6_ppo_rollout_size(void) { return (int)sizeof(R6PpoRollout); }
+int r6_ppo_coef_size(void) { return (int)sizeof(R6PpoCoef); }
+int r6_adam_coef_size(void) { return (int)sizeof(R6AdamCoef); }
+
+int64_t r6_ppo_work_bytes(int64_t B)
+{
+    return B > 0 ? ppo_ctas(B) * (int64_t)(R6_PPO_NTERMS * sizeof(double) + kPpoParams * sizeof(float)) : 0;
+}
+
+int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *idx, int64_t B, const R6PpoCoef *coef,
+                float *grad_sum, double *terms, void *work, void *stream)
+{
+    if (!mlp || !mlp->w0 || !mlp->b0 || !mlp->w1 || !mlp->b1 || !mlp->w2 || !mlp->b2)
+        return fail(R6_EINVAL, "policy weights are null%s");
+    if (!mlp->wv || !mlp->bv || !mlp->log_std) return fail(R6_EINVAL, "r6_ppo_grad needs the critic head and log_std%s");
+    if (!rollout || !rollout->obs || !rollout->actions || !rollout->log_probs || !rollout->advantages || !rollout->returns)
+        return fail(R6_EINVAL, "null rollout buffer%s");
+    if (rollout->T < 0 || rollout->n < 0 || B < 0) return fail(R6_EINVAL, "negative size%s");
+    if (!coef || !grad_sum || !terms || (B > 0 && (!idx || !work))) return fail(R6_EINVAL, "null pointer%s");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (B == 0) {
+        cudaError_t e = cudaMemsetAsync(grad_sum, 0, sizeof(float) * kPpoParams, s);
+        if (e == cudaSuccess) e = cudaMemsetAsync(terms, 0, sizeof(double) * R6_PPO_NTERMS, s);
+        if (e != cudaSuccess) return fail(R6_ECUDA, "cudaMemsetAsync: %s", cudaGetErrorString(e));
+        return R6_OK;
+    }
+    int rc = ensure_attributes();
+    if (rc) return rc;
+    const int G = (int)ppo_ctas(B);
+    double *pt = static_cast<double *>(work);
+    float *pp = reinterpret_cast<float *>(pt + (int64_t)G * R6_PPO_NTERMS);
+    ppo_grad_kernel<<<G, kThreads, kSmemPpo, s>>>(*mlp, *rollout, idx, B, (float)coef->clip_range, (float)coef->vf_coef,
+                                                  (float)coef->ent_coef, coef->adv_stats, pt, pp);
+    rc = check_launch("r6_ppo_grad");
+    if (rc) return rc;
+    ppo_reduce_kernel<<<(kPpoParams + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
+    return check_launch("r6_ppo_grad (reduce)");
+}
+
+int r6_adam_step(float *params, const float *grad_sum, float *m, float *v, int64_t P, const R6AdamCoef *coef,
+                 int64_t step, double *grad_norm_out, void *stream)
+{
+    if (!params || !grad_sum || !m || !v || !coef) return fail(R6_EINVAL, "null pointer%s");
+    if (P < 0 || P > (int64_t)1 << 30) return fail(R6_EINVAL, "P out of range%s");
+    if (step < 1) return fail(R6_EINVAL, "step must be >= 1%s");
+    if (P == 0) return R6_OK;
+    AdamArgs a;
+    a.scale = (float)coef->scale;
+    a.max_norm = coef->max_grad_norm;
+    adam_coefs(*coef, step, a.c);
+    adam_kernel<<<1, kAdamThreads, 0, (cudaStream_t)stream>>>(params, grad_sum, m, v, (int)P, a, grad_norm_out);
+    return check_launch("r6_adam_step");
 }
 
 int r6_stats_reset(double *stats, void *stream)
