@@ -23,6 +23,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "r6_core.cuh"
 #include "r6_mlp_tc.cuh"
 #include "r6_mlp_tcgen05.cuh"
@@ -77,6 +79,7 @@ template <class R> constexpr int int_ctas() { return sizeof(R) == 4 ? R6_INT_CTA
 template <class R> constexpr int first_ctas() { return sizeof(R) == 4 ? R6_INT_CTAS_F32 : R6_FIRST_CTAS_F64; }
 // stage storage per CTA: 55,296 B (float64) / 27,648 B (float32); + packed policy weights (42,000 B) for R6_ACT_MLP
 template <class R> constexpr int smem_bytes() { return 6 * r6::kNK * kThreads * (int)sizeof(R); }
+template <class R> constexpr int smem_int_bytes() { return smem_bytes<R>() * kIntThreads / kThreads; }   // one-warp CTAs
 template <class R> constexpr int smem_mlp_bytes() { return smem_bytes<R>() + r6::kMlpFloats * (int)sizeof(float); }
 // tensor-core policy: fragment-ordered weights (43,792 B) + one [16][33] float staging tile per warp
 template <class R> constexpr int smem_tc_bytes()
@@ -86,13 +89,13 @@ template <class R> constexpr int smem_tc_bytes()
 constexpr int kSmemBytes = smem_bytes<double>();
 
 using namespace r6;
-template <class R> using KStore = KShared<R, kThreads>;
 
-template <class R>
-__device__ __forceinline__ KStore<R> make_kstore()
+// the RK stage storage of this thread in a CTA of kWidth threads (dynamic shared memory)
+template <class R, int kWidth = kThreads>
+__device__ __forceinline__ KShared<R, kWidth> make_kstore()
 {
     extern __shared__ __align__(16) double r6_smem[];
-    KStore<R> K;
+    KShared<R, kWidth> K;
     K.base = reinterpret_cast<R *>(r6_smem) + 2 * threadIdx.x;
     return K;
 }
@@ -173,6 +176,37 @@ __device__ __forceinline__ void write_obs(float *obs, int64_t n, int64_t i, cons
         if (c < rows) obs[(int64_t)c * n + i] = obs_component(p, dv, y, c);   // rocket_env.py:503-504
 }
 
+// The outputs of an env-step.  reward_terms is written by the one-step kernels only (step_kernel, post_body): in a
+// rollout it would keep the terms live across the step loop.
+__device__ __forceinline__ void write_step_out(const R6Buffers &b, int64_t i, const StepOut &o)
+{
+    if (b.reward) b.reward[i] = o.reward;
+    if (b.reward_f32) b.reward_f32[i] = (float)o.reward;
+    b.done[i] = o.finished ? 1 : 0;
+    b.flags[i] = (uint8_t)o.flags;
+    if (b.nattempts) b.nattempts[i] = (uint8_t)o.natt;
+    if (b.status) b.status[i] = (int8_t)o.status;
+}
+
+// (return, length) of the episode that just ended
+template <class R>
+__device__ __forceinline__ void write_ep_info(const R6Buffers &b, int64_t n, int64_t i, const EnvT<R> &e)
+{
+    if (b.ep_info) { b.ep_info[i] = e.ep_return; b.ep_info[n + i] = (double)e.k; }
+}
+
+// End of an episode with the post-step state in registers: batch statistics, terminal observation / state
+// (DummyVecEnv's terminal_observation, montecarlo_script.py:35) and (return, length)
+template <class R>
+__device__ __forceinline__ void end_episode(const R6Params &p, const R6Buffers &b, const Derived &dv, int64_t n, int64_t i,
+                                            const EnvT<R> &e, uint32_t flags)
+{
+    if (b.stats) stats_episode<R>(b.stats, flags, e.ep_return, e.k);
+    write_obs(b.terminal_obs, n, i, p, dv, e.y);
+    write_terminal_state(b, n, i, e.y);
+    write_ep_info(b, n, i, e);
+}
+
 // ---------------------------------------------------------------------------------------------
 template <class R>
 __global__ void __launch_bounds__(kThreads)
@@ -227,7 +261,7 @@ step_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t n, in
             const float *__restrict__ actions, uint64_t seed)
 {
     const int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x;
-    KStore<R> K = make_kstore<R>();
+    auto K = make_kstore<R>();
     float ob[14];
     // one-episode semantics (auto_reset = 0): a finished env stays frozen until r6_reset (obs_row_major implies auto_reset)
     const bool live = i < n && (p.auto_reset || b.done[i] == 0);
@@ -237,24 +271,14 @@ step_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t n, in
         const float a0 = actions[3 * i], a1 = actions[3 * i + 1], a2 = actions[3 * i + 2];
         StepOut o;
         env_step<kExact>(p, dv, b.t_table, e, a0, a1, a2, o, K);
-        if (b.reward) b.reward[i] = o.reward;
-        if (b.reward_f32) b.reward_f32[i] = (float)o.reward;
-        b.done[i] = o.finished ? 1 : 0;
-        b.flags[i] = (uint8_t)o.flags;
-        if (b.nattempts) b.nattempts[i] = (uint8_t)o.natt;
-        if (b.status) b.status[i] = (int8_t)o.status;
+        write_step_out(b, i, o);
         if (b.reward_terms) {
 #pragma unroll
             for (int k = 0; k < R6_NTERMS; k++) b.reward_terms[(int64_t)k * n + i] = o.post.terms[k];
         }
         if (o.finished) {
-            if (b.stats) stats_episode<R>(b.stats, o.flags, e.ep_return, e.k);
-            if (b.ep_info) { b.ep_info[i] = e.ep_return; b.ep_info[n + i] = (double)e.k; }
-            // keep the terminal observation / state (DummyVecEnv's terminal_observation, montecarlo_script.py:35);
-            // with auto_reset hand back the reset obs
-            write_obs(b.terminal_obs, n, i, p, dv, e.y);
-            write_terminal_state(b, n, i, e.y);
-            if (p.auto_reset) env_reset(p, b, seed, env_offset + i, e);
+            end_episode(p, b, dv, n, i, e, o.flags);
+            if (p.auto_reset) env_reset(p, b, seed, env_offset + i, e);      // with auto_reset hand back the reset obs
         }
         if (p.obs_row_major) {
 #pragma unroll
@@ -269,6 +293,42 @@ step_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t n, in
     if (b.stats) stats_steps(b.stats, live ? 1 : 0);
 }
 
+// the action of env i in the kernel pair: from the [n][3] buffer, or from Philox without one (r6_step_random)
+__device__ __forceinline__ void step_action(const float *__restrict__ actions, uint64_t seed, int64_t env_offset,
+                                            int64_t step_index, int64_t i, float &a0, float &a1, float &a2)
+{
+    if (actions != nullptr) { a0 = actions[3 * i]; a1 = actions[3 * i + 1]; a2 = actions[3 * i + 2]; }
+    else philox_action(seed, (uint64_t)(env_offset + i), (uint64_t)step_index, a0, a1, a2);
+}
+
+// Integrator pass kPass of env i on the state in `state`: 0 = the whole step (env_integrate), 1 = probe + the first
+// px.budget attempts, 2 = resumed from px.  Returns true while the env is unfinished (kPass != 0); a finished env's
+// status and attempt count go to `scratch` for post_kernel.
+template <bool kExact, int kPass, class R, class KS>
+__device__ __forceinline__ bool integrate_env(const R6Params &p, const R6Buffers &b, int64_t n, int64_t i,
+                                              const float *__restrict__ actions, uint64_t seed, int64_t env_offset,
+                                              int64_t step_index, KS &K, PassCtx<R> &px)
+{
+    R *state = reinterpret_cast<R *>(b.state);
+    R y[14];
+#pragma unroll
+    for (int c = 0; c < 14; c++) y[c] = state[(int64_t)c * n + i];
+    float a0, a1, a2;
+    step_action(actions, seed, env_offset, step_index, i, a0, a1, a2);
+    int status, natt;
+    if constexpr (kPass == 0) env_integrate<kExact>(p, b.t_table, y, b.m0[i], b.step_count[i], a0, a1, a2, K, status, natt);
+    else status = env_integrate_pass<kExact, kPass>(p, b.t_table, y, b.m0[i], kPass == 1 ? b.step_count[i] : 0, a0, a1, a2, K,
+                                                    px, natt);
+#pragma unroll
+    for (int c = 0; c < 14; c++) state[(int64_t)c * n + i] = y[c];
+    const bool unfinished = kPass != 0 && status == -2;
+    if (!unfinished) {
+        b.scratch[i] = (uint8_t)(int8_t)status;
+        b.scratch[n + i] = (uint8_t)natt;
+    }
+    return unfinished;
+}
+
 // The same env-step as two kernels (used by r6_step when R6Buffers.scratch is given): the divergent, register- and
 // shared-memory-hungry integrator on its own, with a hot instruction footprint that fits the instruction cache, and
 // a uniform post-step kernel (reward, flags, wrappers, statistics, auto-reset, observation) without stage storage
@@ -279,25 +339,12 @@ integrate_kernel(const R6Params p, const R6Buffers b, int64_t n, const float *__
                  uint64_t seed, int64_t step_index, int64_t i0, int64_t i1)
 {
     const int64_t i = i0 + (int64_t)blockIdx.x * kIntThreads + threadIdx.x;     // this launch steps envs [i0, i1)
-    extern __shared__ __align__(16) double r6_smem[];
-    KShared<R, kIntThreads> K;
-    K.base = reinterpret_cast<R *>(r6_smem) + 2 * threadIdx.x;
+    auto K = make_kstore<R, kIntThreads>();
     grid_dependency_wait();
     if (i >= i1) return;
     if (!p.auto_reset && b.done[i] != 0) return;      // one-episode semantics: a finished env stays frozen until r6_reset
-    R *state = reinterpret_cast<R *>(b.state);
-    R y[14];
-#pragma unroll
-    for (int c = 0; c < 14; c++) y[c] = state[(int64_t)c * n + i];
-    float a0, a1, a2;
-    if (actions != nullptr) { a0 = actions[3 * i]; a1 = actions[3 * i + 1]; a2 = actions[3 * i + 2]; }
-    else philox_action(seed, (uint64_t)(env_offset + i), (uint64_t)step_index, a0, a1, a2);   // r6_step_random
-    int status, natt;
-    env_integrate<kExact>(p, b.t_table, y, b.m0[i], b.step_count[i], a0, a1, a2, K, status, natt);
-#pragma unroll
-    for (int c = 0; c < 14; c++) state[(int64_t)c * n + i] = y[c];
-    b.scratch[i] = (uint8_t)(int8_t)status;
-    b.scratch[n + i] = (uint8_t)natt;
+    PassCtx<R> px;
+    integrate_env<kExact, 0>(p, b, n, i, actions, seed, env_offset, step_index, K, px);
 }
 
 // ---- multi-pass integration (R6Buffers.work given): the integrator cut at RK-attempt boundaries -------------------
@@ -354,30 +401,13 @@ integrate_first_kernel(const R6Params p, const R6Buffers b, int64_t n, const flo
                        uint64_t seed, int64_t step_index, int64_t i0, int64_t i1, int lane)
 {
     const int64_t i = i0 + (int64_t)blockIdx.x * kIntThreads + threadIdx.x;
-    extern __shared__ __align__(16) double r6_smem[];
-    KShared<R, kIntThreads> K;
-    K.base = reinterpret_cast<R *>(r6_smem) + 2 * threadIdx.x;
+    auto K = make_kstore<R, kIntThreads>();
     PassCtx<R> px;
     bool unfinished = false;
     grid_dependency_wait();
     if (i < i1 && (p.auto_reset || b.done[i] == 0)) {       // one-episode semantics: finished envs stay frozen
-        R *state = reinterpret_cast<R *>(b.state);
-        R y[14];
-#pragma unroll
-        for (int c = 0; c < 14; c++) y[c] = state[(int64_t)c * n + i];
-        float a0, a1, a2;
-        if (actions != nullptr) { a0 = actions[3 * i]; a1 = actions[3 * i + 1]; a2 = actions[3 * i + 2]; }
-        else philox_action(seed, (uint64_t)(env_offset + i), (uint64_t)step_index, a0, a1, a2);
-        int natt;
         px.budget = 1;
-        const int status = env_integrate_pass<kExact, 1>(p, b.t_table, y, b.m0[i], b.step_count[i], a0, a1, a2, K, px, natt);
-#pragma unroll
-        for (int c = 0; c < 14; c++) state[(int64_t)c * n + i] = y[c];
-        unfinished = status == -2;
-        if (!unfinished) {
-            b.scratch[i] = (uint8_t)(int8_t)status;
-            b.scratch[n + i] = (uint8_t)natt;
-        }
+        unfinished = integrate_env<kExact, 1>(p, b, n, i, actions, seed, env_offset, step_index, K, px);
     }
     work_append<R>(work_view(b.work, n), n, 0, lane, i0, unfinished, i, px);
 }
@@ -390,13 +420,10 @@ integrate_resume_kernel(const R6Params p, const R6Buffers b, int64_t n, const fl
 {
     constexpr int src = kLast ? 1 : 0;
     constexpr int budget = kLast ? (1 << 30) : 1;
-    extern __shared__ __align__(16) double r6_smem[];
-    KShared<R, kIntThreads> K;
-    K.base = reinterpret_cast<R *>(r6_smem) + 2 * threadIdx.x;
+    auto K = make_kstore<R, kIntThreads>();
     const WorkView W = work_view(b.work, n);
     grid_dependency_wait();
     const int64_t cnt = W.count[2 * lane + src];
-    R *state = reinterpret_cast<R *>(b.state);
     for (int64_t s0 = (int64_t)blockIdx.x * kIntThreads; s0 < cnt; s0 += (int64_t)gridDim.x * kIntThreads) {
         const int64_t slot = s0 + threadIdx.x;
         PassCtx<R> px;
@@ -409,21 +436,7 @@ integrate_resume_kernel(const R6Params p, const R6Buffers b, int64_t n, const fl
             px.t = (R)c[i0 + slot]; px.h_abs = (R)c[n + i0 + slot]; px.h_ref = (R)c[2 * n + i0 + slot];
             px.t_bound = (R)c[3 * n + i0 + slot];
             px.natt = meta & 255; px.rejected = (meta & 256) != 0; px.budget = budget;
-            R y[14];
-#pragma unroll
-            for (int cc = 0; cc < 14; cc++) y[cc] = state[(int64_t)cc * n + i];
-            float a0, a1, a2;
-            if (actions != nullptr) { a0 = actions[3 * i]; a1 = actions[3 * i + 1]; a2 = actions[3 * i + 2]; }
-            else philox_action(seed, (uint64_t)(env_offset + i), (uint64_t)step_index, a0, a1, a2);
-            int natt;
-            const int status = env_integrate_pass<kExact, 2>(p, b.t_table, y, b.m0[i], 0, a0, a1, a2, K, px, natt);
-#pragma unroll
-            for (int cc = 0; cc < 14; cc++) state[(int64_t)cc * n + i] = y[cc];
-            unfinished = status == -2;
-            if (!unfinished) {
-                b.scratch[i] = (uint8_t)(int8_t)status;
-                b.scratch[n + i] = (uint8_t)natt;
-            }
+            unfinished = integrate_env<kExact, 2>(p, b, n, i, actions, seed, env_offset, step_index, K, px);
         }
         if constexpr (!kLast) work_append<R>(W, n, 1, lane, i0, unfinished, i, px);
     }
@@ -447,12 +460,7 @@ __device__ __forceinline__ void post_body(const R6Params &p, const R6Buffers &b,
     write_obs(b.obs, n, i, p, dv, e.y);          // first thing: the float64 state is then dead but for q and the casts
     StepOut o;
     env_post(p, dv, e, a0, a1, a2, status, natt, o);
-    if (b.reward) b.reward[i] = o.reward;
-    if (b.reward_f32) b.reward_f32[i] = (float)o.reward;
-    b.done[i] = o.finished ? 1 : 0;
-    b.flags[i] = (uint8_t)o.flags;
-    if (b.nattempts) b.nattempts[i] = (uint8_t)o.natt;
-    if (b.status) b.status[i] = (int8_t)o.status;
+    write_step_out(b, i, o);
     if (b.reward_terms) {
 #pragma unroll
         for (int k = 0; k < R6_NTERMS; k++) b.reward_terms[(int64_t)k * n + i] = o.post.terms[k];
@@ -462,7 +470,7 @@ __device__ __forceinline__ void post_body(const R6Params &p, const R6Buffers &b,
         // the integrator) so that the 14 doubles are not kept alive through the reward code for this path's sake.
         // (Moving this path out of line into a __noinline__ function cost 5-8 us: measured, rejected.)
         if (b.stats) stats_episode<R>(b.stats, o.flags, e.ep_return, e.k);
-        if (b.ep_info) { b.ep_info[i] = e.ep_return; b.ep_info[n + i] = (double)e.k; }
+        write_ep_info(b, n, i, e);
         const R *state = reinterpret_cast<const R *>(b.state);
         if (p.auto_reset) {
             R yt[14];
@@ -503,12 +511,58 @@ post_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t n, in
         EnvT<R> e;
         env_load(b, n, i, e);
         float a0, a1, a2;
-        if (actions != nullptr) { a0 = actions[3 * i]; a1 = actions[3 * i + 1]; a2 = actions[3 * i + 2]; }
-        else philox_action(seed, (uint64_t)(env_offset + i), (uint64_t)step_index, a0, a1, a2);
+        step_action(actions, seed, env_offset, step_index, i, a0, a1, a2);
         const int status = (int)(int8_t)b.scratch[i], natt = (int)b.scratch[n + i];
         post_body(p, b, dv, n, i, env_offset, seed, e, a0, a1, a2, status, natt);
     }
     if (b.stats) stats_steps(b.stats, live ? 1 : 0);
+}
+
+// The trajectory record of a rollout (each pointer nullable): obs [k][13][n], actions [k][n][3], rewards and done [k][n]
+struct Traj {
+    float *obs, *act, *rew;
+    uint8_t *done;
+};
+
+// Step j of a rollout on the registers of `e`: record the observation and action, step, record reward and done, count
+// the step; at the end of an episode reset the env (auto_reset) or freeze it and pad the rest of the record (reward 0,
+// done = 2).  Returns true when the env froze.
+template <bool kExact, class R, class KS>
+__device__ __forceinline__ bool rollout_step(const R6Params &p, const R6Buffers &b, const Derived &dv, int64_t n, int64_t i,
+                                             int64_t env_offset, uint64_t seed, const Traj &tr, int j, int k_steps, float a0,
+                                             float a1, float a2, EnvT<R> &e, StepOut &o, KS &K, int &steps)
+{
+    if (tr.obs) {
+#pragma unroll
+        for (int c = 0; c < 13; c++) tr.obs[((int64_t)j * 13 + c) * n + i] = obs_component(p, dv, e.y, c);
+    }
+    if (tr.act) { float *a = tr.act + ((int64_t)j * n + i) * 3; a[0] = a0; a[1] = a1; a[2] = a2; }
+    env_step<kExact>(p, dv, b.t_table, e, a0, a1, a2, o, K);
+    if (tr.rew) tr.rew[(int64_t)j * n + i] = (float)o.reward;
+    if (tr.done) tr.done[(int64_t)j * n + i] = o.finished ? 1 : 0;
+    steps++;
+    if (o.finished) {
+        end_episode(p, b, dv, n, i, e, o.flags);
+        if (!p.auto_reset) {
+            for (int jj = j + 1; jj < k_steps; jj++) {
+                if (tr.rew) tr.rew[(int64_t)jj * n + i] = 0.0f;
+                if (tr.done) tr.done[(int64_t)jj * n + i] = 2;
+            }
+            return true;
+        }
+        env_reset(p, b, seed, env_offset + i, e);
+    }
+    return false;
+}
+
+// the end of a rollout: the last step's outputs, the observation and the env registers
+template <class R>
+__device__ __forceinline__ void rollout_store(const R6Params &p, const R6Buffers &b, const Derived &dv, int64_t n, int64_t i,
+                                              const EnvT<R> &e, const StepOut &o)
+{
+    write_step_out(b, i, o);
+    write_obs(b.obs, n, i, p, dv, e.y);
+    env_store(b, n, i, e);
 }
 
 // k fused steps, state in registers; actions from Philox, a [k][n][3] buffer or the fused policy MLP.
@@ -521,8 +575,9 @@ rollout_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t n,
                const float *__restrict__ act_buf, const R6Mlp mlp, uint64_t seed, int64_t step_base, float *traj_obs,
                float *traj_act, float *traj_rew, uint8_t *traj_done)
 {
+    const Traj tr = {traj_obs, traj_act, traj_rew, traj_done};
     const int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x;
-    KStore<R> K = make_kstore<R>();
+    auto K = make_kstore<R>();
     const float *W = nullptr;
     if (kMode == R6_ACT_MLP) {
         // pack the policy weights into shared memory once per CTA (transposes W1, pads W0 rows)
@@ -551,39 +606,9 @@ rollout_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t n,
                 const float *a = act_buf + ((int64_t)j * n + i) * 3;
                 a0 = a[0]; a1 = a[1]; a2 = a[2];
             }
-            if (traj_obs) {
-#pragma unroll
-                for (int c = 0; c < 13; c++) traj_obs[((int64_t)j * 13 + c) * n + i] = obs_component(p, dv, e.y, c);
-            }
-            if (traj_act) { float *a = traj_act + ((int64_t)j * n + i) * 3; a[0] = a0; a[1] = a1; a[2] = a2; }
-            env_step<kExact>(p, dv, b.t_table, e, a0, a1, a2, o, K);
-            if (traj_rew) traj_rew[(int64_t)j * n + i] = (float)o.reward;
-            if (traj_done) traj_done[(int64_t)j * n + i] = o.finished ? 1 : 0;
-            my_steps++;
-            if (o.finished) {
-                if (b.stats) stats_episode<R>(b.stats, o.flags, e.ep_return, e.k);
-                write_obs(b.terminal_obs, n, i, p, dv, e.y);
-                write_terminal_state(b, n, i, e.y);
-                if (b.ep_info) { b.ep_info[i] = e.ep_return; b.ep_info[n + i] = (double)e.k; }
-                if (!p.auto_reset) {
-                    // frozen: the rest of the trajectory record (if any) is padding
-                    for (int jj = j + 1; jj < k_steps; jj++) {
-                        if (traj_rew) traj_rew[(int64_t)jj * n + i] = 0.0f;
-                        if (traj_done) traj_done[(int64_t)jj * n + i] = 2;
-                    }
-                    break;
-                }
-                env_reset(p, b, seed, env_offset + i, e);
-            }
+            if (rollout_step<kExact>(p, b, dv, n, i, env_offset, seed, tr, j, k_steps, a0, a1, a2, e, o, K, my_steps)) break;
         }
-        if (b.reward) b.reward[i] = o.reward;
-        if (b.reward_f32) b.reward_f32[i] = (float)o.reward;
-        b.done[i] = o.finished ? 1 : 0;
-        b.flags[i] = (uint8_t)o.flags;
-        if (b.nattempts) b.nattempts[i] = (uint8_t)o.natt;
-        if (b.status) b.status[i] = (int8_t)o.status;
-        write_obs(b.obs, n, i, p, dv, e.y);
-        env_store(b, n, i, e);
+        rollout_store(p, b, dv, n, i, e, o);
     }
     if (b.stats) stats_steps(b.stats, my_steps);
 }
@@ -596,8 +621,9 @@ __global__ void __launch_bounds__(kThreads, 2)
 rollout_tc_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t n, int64_t env_offset, int k_steps,
                   const R6Mlp mlp, uint64_t seed, float *traj_obs, float *traj_act, float *traj_rew, uint8_t *traj_done)
 {
+    const Traj tr = {traj_obs, traj_act, traj_rew, traj_done};
     const int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x;
-    KStore<R> K = make_kstore<R>();
+    auto K = make_kstore<R>();
     extern __shared__ __align__(16) double r6_smem[];
     float *Ws = reinterpret_cast<float *>(reinterpret_cast<char *>(r6_smem) + smem_bytes<R>());
     for (int idx = threadIdx.x; idx < kMlpTcFloats; idx += kThreads) Ws[idx] = mlp_tc_pack_element(mlp, idx);
@@ -622,42 +648,10 @@ rollout_tc_kernel(const R6Params p, const R6Buffers b, const Derived dv, int64_t
 #pragma unroll
         for (int c = 0; c < kMlpIn; c++) x[c] = obs_component(p, dv, e.y, c);
         mlp_policy_tc(Ws, scratch, x, a0, a1, a2);
-        if (live) {
-            if (traj_obs) {
-#pragma unroll
-                for (int c = 0; c < 13; c++) traj_obs[((int64_t)j * 13 + c) * n + i] = x[c];
-            }
-            if (traj_act) { float *a = traj_act + ((int64_t)j * n + i) * 3; a[0] = a0; a[1] = a1; a[2] = a2; }
-            env_step<false>(p, dv, b.t_table, e, a0, a1, a2, o, K);
-            if (traj_rew) traj_rew[(int64_t)j * n + i] = (float)o.reward;
-            if (traj_done) traj_done[(int64_t)j * n + i] = o.finished ? 1 : 0;
-            my_steps++;
-            if (o.finished) {
-                if (b.stats) stats_episode<R>(b.stats, o.flags, e.ep_return, e.k);
-                write_obs(b.terminal_obs, n, i, p, dv, e.y);
-                write_terminal_state(b, n, i, e.y);
-                if (b.ep_info) { b.ep_info[i] = e.ep_return; b.ep_info[n + i] = (double)e.k; }
-                if (!p.auto_reset) {
-                    for (int jj = j + 1; jj < k_steps; jj++) {
-                        if (traj_rew) traj_rew[(int64_t)jj * n + i] = 0.0f;
-                        if (traj_done) traj_done[(int64_t)jj * n + i] = 2;
-                    }
-                    live = false;
-                } else
-                    env_reset(p, b, seed, env_offset + i, e);
-            }
-        }
+        if (live && rollout_step<false>(p, b, dv, n, i, env_offset, seed, tr, j, k_steps, a0, a1, a2, e, o, K, my_steps))
+            live = false;
     }
-    if (loaded) {
-        if (b.reward) b.reward[i] = o.reward;
-        if (b.reward_f32) b.reward_f32[i] = (float)o.reward;
-        b.done[i] = o.finished ? 1 : 0;
-        b.flags[i] = (uint8_t)o.flags;
-        if (b.nattempts) b.nattempts[i] = (uint8_t)o.natt;
-        if (b.status) b.status[i] = (int8_t)o.status;
-        write_obs(b.obs, n, i, p, dv, e.y);
-        env_store(b, n, i, e);
-    }
+    if (loaded) rollout_store(p, b, dv, n, i, e, o);
     if (b.stats) stats_steps(b.stats, my_steps);
 }
 
@@ -668,7 +662,7 @@ sim_raw_kernel(double *state, const double *u, const double *m0, const double *t
                int8_t *status, uint8_t *nattempts)
 {
     const int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x;
-    KStore<double> K = make_kstore<double>();
+    auto K = make_kstore<double>();
     if (i >= n) return;
     double y[14];
 #pragma unroll
@@ -1158,28 +1152,21 @@ int enable_smem(F kernel, int bytes = kSmemBytes)
     if (e != cudaSuccess) return fail(R6_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     return R6_OK;
 }
+template <class R, bool kExact>
+int enable_density()
+{
+    constexpr int si = smem_int_bytes<R>();
+    return enable_smem(step_kernel<R, kExact>, smem_bytes<R>()) | enable_smem(integrate_kernel<R, kExact>, si) |
+           enable_smem(integrate_first_kernel<R, kExact>, si) | enable_smem(integrate_resume_kernel<R, kExact, false>, si) |
+           enable_smem(integrate_resume_kernel<R, kExact, true>, si) |
+           enable_smem(rollout_kernel<R, R6_ACT_PHILOX, kExact>, smem_bytes<R>()) |
+           enable_smem(rollout_kernel<R, R6_ACT_BUFFER, kExact>, smem_bytes<R>()) |
+           enable_smem(rollout_kernel<R, R6_ACT_MLP, kExact>, smem_mlp_bytes<R>());
+}
 template <class R>
 int enable_all()
 {
-    int rc = 0;
-    rc |= enable_smem(step_kernel<R, false>, smem_bytes<R>());
-    rc |= enable_smem(step_kernel<R, true>, smem_bytes<R>());
-    rc |= enable_smem(integrate_kernel<R, false>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(integrate_kernel<R, true>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(integrate_first_kernel<R, false>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(integrate_first_kernel<R, true>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(integrate_resume_kernel<R, false, false>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(integrate_resume_kernel<R, true, false>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(integrate_resume_kernel<R, false, true>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(integrate_resume_kernel<R, true, true>, smem_bytes<R>() * kIntThreads / kThreads);
-    rc |= enable_smem(rollout_kernel<R, R6_ACT_PHILOX, false>, smem_bytes<R>());
-    rc |= enable_smem(rollout_kernel<R, R6_ACT_PHILOX, true>, smem_bytes<R>());
-    rc |= enable_smem(rollout_kernel<R, R6_ACT_BUFFER, false>, smem_bytes<R>());
-    rc |= enable_smem(rollout_kernel<R, R6_ACT_BUFFER, true>, smem_bytes<R>());
-    rc |= enable_smem(rollout_kernel<R, R6_ACT_MLP, false>, smem_mlp_bytes<R>());
-    rc |= enable_smem(rollout_kernel<R, R6_ACT_MLP, true>, smem_mlp_bytes<R>());
-    rc |= enable_smem(rollout_tc_kernel<R>, smem_tc_bytes<R>());
-    return rc;
+    return enable_density<R, false>() | enable_density<R, true>() | enable_smem(rollout_tc_kernel<R>, smem_tc_bytes<R>());
 }
 int ensure_attributes()
 {
@@ -1236,71 +1223,75 @@ void launch_pdl(void (*kern)(KArgs...), unsigned grid, unsigned block, size_t sm
     cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 
-template <class R>
+// f(R(), std::bool_constant<kExact>()) with the density form dt needs: the series up to kMaxDtSeries, exact beyond
+template <class R, class F>
+auto dispatch_density(double dt, F &&f)
+{
+    return dt <= kMaxDtSeries ? f(R(), std::false_type()) : f(R(), std::true_type());
+}
+// ... and with R the working precision of p
+template <class F>
+auto dispatch(const R6Params *p, F &&f)
+{
+    return p->precision == R6_PREC_F32 ? dispatch_density<float>(p->dt, f) : dispatch_density<double>(p->dt, f);
+}
+
+int check_mlp(const R6Mlp *mlp)
+{
+    if (!mlp || !mlp->w0 || !mlp->b0 || !mlp->w1 || !mlp->b1 || !mlp->w2 || !mlp->b2)
+        return fail(R6_EINVAL, "policy weights are null%s");
+    return R6_OK;
+}
+
+template <class R, bool kExact>
 void launch_step(const R6Params *p, const R6Buffers *b, const Derived &dv, int64_t n, int64_t env_offset,
                  const float *actions, uint64_t seed, cudaStream_t s, int64_t step_index = 0, int64_t first = 0,
                  int64_t count = -1, int lane = 0)
 {
-    if (b->scratch != nullptr) {                 // kernel pair over the env sub-range [first, first + count)
-        if (count < 0) count = n;
-        const int64_t last = first + count;
-        const unsigned gi = (unsigned)((count + kIntThreads - 1) / kIntThreads);
-        constexpr int smem_i = smem_bytes<R>() * kIntThreads / kThreads;
-        const bool series = p->dt <= kMaxDtSeries;
-        if (b->work != nullptr) {                // integrator cut at attempt boundaries (see integrate_first_kernel)
-            // list 0 holds ~2/3 of the range, list 1 ~1 %; the resume kernels walk longer lists with a grid stride
-            const unsigned g1 = gi - gi / 4, g2 = gi / 16 + 1;
-            const unsigned gp = (unsigned)((count + kPostThreads - 1) / kPostThreads);
-            if (series) {
-                launch_pdl(integrate_first_kernel<R, false>, gi, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, last, lane);
-                launch_pdl(integrate_resume_kernel<R, false, false>, g1, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, lane);
-                launch_pdl(integrate_resume_kernel<R, false, true>, g2, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, lane);
-            } else {
-                launch_pdl(integrate_first_kernel<R, true>, gi, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, last, lane);
-                launch_pdl(integrate_resume_kernel<R, true, false>, g1, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, lane);
-                launch_pdl(integrate_resume_kernel<R, true, true>, g2, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, lane);
-            }
-            launch_pdl(post_kernel<R>, gp, kPostThreads, 0, s, *p, *b, dv, n, env_offset, actions, seed, step_index, first, last, lane);
-            return;
-        } else if (series)
-            launch_pdl(integrate_kernel<R, false>, gi, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, last);
-        else
-            launch_pdl(integrate_kernel<R, true>, gi, kIntThreads, smem_i, s, *p, *b, n, actions, env_offset, seed, step_index, first, last);
-        launch_pdl(post_kernel<R>, (unsigned)((count + kPostThreads - 1) / kPostThreads), kPostThreads, 0, s, *p, *b, dv, n, env_offset, actions, seed, step_index, first, last, lane);
+    if (b->scratch == nullptr) {
+        step_kernel<R, kExact><<<(unsigned)blocks_for(n), kThreads, smem_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, actions, seed);
         return;
     }
-    const unsigned g = (unsigned)blocks_for(n);
-    if (p->dt <= kMaxDtSeries) step_kernel<R, false><<<g, kThreads, smem_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, actions, seed);
-    else step_kernel<R, true><<<g, kThreads, smem_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, actions, seed);
+    // kernel pair over the env sub-range [first, first + count)
+    if (count < 0) count = n;
+    const int64_t last = first + count;
+    const unsigned gi = (unsigned)((count + kIntThreads - 1) / kIntThreads);
+    constexpr int si = smem_int_bytes<R>();
+    if (b->work != nullptr) {                    // integrator cut at attempt boundaries (see integrate_first_kernel)
+        // list 0 holds ~2/3 of the range, list 1 ~1 %; the resume kernels walk longer lists with a grid stride
+        const unsigned g1 = gi - gi / 4, g2 = gi / 16 + 1;
+        launch_pdl(integrate_first_kernel<R, kExact>, gi, kIntThreads, si, s, *p, *b, n, actions, env_offset, seed, step_index, first, last, lane);
+        launch_pdl(integrate_resume_kernel<R, kExact, false>, g1, kIntThreads, si, s, *p, *b, n, actions, env_offset, seed, step_index, first, lane);
+        launch_pdl(integrate_resume_kernel<R, kExact, true>, g2, kIntThreads, si, s, *p, *b, n, actions, env_offset, seed, step_index, first, lane);
+    } else
+        launch_pdl(integrate_kernel<R, kExact>, gi, kIntThreads, si, s, *p, *b, n, actions, env_offset, seed, step_index, first, last);
+    launch_pdl(post_kernel<R>, (unsigned)((count + kPostThreads - 1) / kPostThreads), kPostThreads, 0, s, *p, *b, dv, n, env_offset, actions, seed, step_index, first, last, lane);
 }
 
-template <class R>
+template <class R, bool kExact>
 int launch_rollout(const R6Params *p, const R6Buffers *b, const Derived &dv, int64_t n, int64_t env_offset, int32_t k,
-                   int32_t mode, const R6Mlp *mlp, const float *act_buf, uint64_t seed, int64_t step_base,
-                   float *traj_obs, float *traj_act, float *traj_rew, uint8_t *traj_done, cudaStream_t s)
+                   int32_t mode, const R6Mlp *mlp, const float *act_buf, uint64_t seed, int64_t step_base, const Traj &tr,
+                   cudaStream_t s)
 {
     const unsigned g = (unsigned)blocks_for(n);
-    const bool exact = !(p->dt <= kMaxDtSeries);
-    R6Mlp m{};
-#define R6_LAUNCH_ROLLOUT(MODE, EXACT, BUF, SMEM)                                                                   \
-    rollout_kernel<R, MODE, EXACT><<<g, kThreads, SMEM, s>>>(*p, *b, dv, n, env_offset, k, BUF, m, seed, step_base, \
-                                                             traj_obs, traj_act, traj_rew, traj_done)
-    if (mode == R6_ACT_PHILOX) {
-        if (exact) R6_LAUNCH_ROLLOUT(R6_ACT_PHILOX, true, nullptr, smem_bytes<R>()); else R6_LAUNCH_ROLLOUT(R6_ACT_PHILOX, false, nullptr, smem_bytes<R>());
-    } else if (mode == R6_ACT_BUFFER) {
+    if (mode == R6_ACT_PHILOX)
+        rollout_kernel<R, R6_ACT_PHILOX, kExact><<<g, kThreads, smem_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, k, nullptr, R6Mlp{}, seed,
+                                                                                     step_base, tr.obs, tr.act, tr.rew, tr.done);
+    else if (mode == R6_ACT_BUFFER) {
         if (!act_buf) return fail(R6_EINVAL, "act_buf is null%s");
-        if (exact) R6_LAUNCH_ROLLOUT(R6_ACT_BUFFER, true, act_buf, smem_bytes<R>()); else R6_LAUNCH_ROLLOUT(R6_ACT_BUFFER, false, act_buf, smem_bytes<R>());
+        rollout_kernel<R, R6_ACT_BUFFER, kExact><<<g, kThreads, smem_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, k, act_buf, R6Mlp{}, seed,
+                                                                                     step_base, tr.obs, tr.act, tr.rew, tr.done);
     } else if (mode == R6_ACT_MLP || mode == R6_ACT_MLP_TC) {
-        if (!mlp || !mlp->w0 || !mlp->b0 || !mlp->w1 || !mlp->b1 || !mlp->w2 || !mlp->b2)
-            return fail(R6_EINVAL, "policy weights are null%s");
-        m = *mlp;
-        if (mode == R6_ACT_MLP_TC && !exact)
-            rollout_tc_kernel<R><<<g, kThreads, smem_tc_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, k, m, seed, traj_obs,
-                                                                       traj_act, traj_rew, traj_done);
-        else if (exact) R6_LAUNCH_ROLLOUT(R6_ACT_MLP, true, nullptr, smem_mlp_bytes<R>()); else R6_LAUNCH_ROLLOUT(R6_ACT_MLP, false, nullptr, smem_mlp_bytes<R>());
+        if (int rc = check_mlp(mlp)) return rc;
+        // rollout_tc_kernel has the series density only: at dt > kMaxDtSeries the float32 network runs instead
+        if (mode == R6_ACT_MLP_TC && !kExact)
+            rollout_tc_kernel<R><<<g, kThreads, smem_tc_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, k, *mlp, seed, tr.obs, tr.act,
+                                                                       tr.rew, tr.done);
+        else
+            rollout_kernel<R, R6_ACT_MLP, kExact><<<g, kThreads, smem_mlp_bytes<R>(), s>>>(*p, *b, dv, n, env_offset, k, nullptr, *mlp, seed,
+                                                                                         step_base, tr.obs, tr.act, tr.rew, tr.done);
     } else
         return fail(R6_EINVAL, "unsupported action mode%s");
-#undef R6_LAUNCH_ROLLOUT
     return R6_OK;
 }
 
@@ -1336,8 +1327,7 @@ int r6_step(const R6Params *p, const R6Buffers *b, int64_t n, int64_t env_offset
     if (n == 0) return R6_OK;
     if ((rc = ensure_attributes())) return rc;
     const Derived dv = make_derived(*p);
-    if (p->precision == R6_PREC_F32) launch_step<float>(p, b, dv, n, env_offset, actions, seed, (cudaStream_t)stream);
-    else launch_step<double>(p, b, dv, n, env_offset, actions, seed, (cudaStream_t)stream);
+    dispatch(p, [&](auto r, auto exact) { launch_step<decltype(r), exact>(p, b, dv, n, env_offset, actions, seed, (cudaStream_t)stream); });
     return check_launch("r6_step");
 }
 
@@ -1350,8 +1340,9 @@ int r6_step_random(const R6Params *p, const R6Buffers *b, int64_t n, int64_t env
     if (n == 0) return R6_OK;
     if ((rc = ensure_attributes())) return rc;
     const Derived dv = make_derived(*p);
-    if (p->precision == R6_PREC_F32) launch_step<float>(p, b, dv, n, env_offset, nullptr, seed, (cudaStream_t)stream, step_index);
-    else launch_step<double>(p, b, dv, n, env_offset, nullptr, seed, (cudaStream_t)stream, step_index);
+    dispatch(p, [&](auto r, auto exact) {
+        launch_step<decltype(r), exact>(p, b, dv, n, env_offset, nullptr, seed, (cudaStream_t)stream, step_index);
+    });
     return check_launch("r6_step_random");
 }
 
@@ -1368,10 +1359,9 @@ int r6_step_range(const R6Params *p, const R6Buffers *b, int64_t n, int64_t firs
     if (count == 0) return R6_OK;
     if ((rc = ensure_attributes())) return rc;
     const Derived dv = make_derived(*p);
-    if (p->precision == R6_PREC_F32)
-        launch_step<float>(p, b, dv, n, env_offset, actions, seed, (cudaStream_t)stream, step_index, first, count, lane);
-    else
-        launch_step<double>(p, b, dv, n, env_offset, actions, seed, (cudaStream_t)stream, step_index, first, count, lane);
+    dispatch(p, [&](auto r, auto exact) {
+        launch_step<decltype(r), exact>(p, b, dv, n, env_offset, actions, seed, (cudaStream_t)stream, step_index, first, count, lane);
+    });
     return check_launch("r6_step_range");
 }
 
@@ -1385,12 +1375,11 @@ int r6_rollout(const R6Params *p, const R6Buffers *b, int64_t n, int64_t env_off
     if (n == 0 || k == 0) return R6_OK;
     if ((rc = ensure_attributes())) return rc;
     const Derived dv = make_derived(*p);
-    if (p->precision == R6_PREC_F32)
-        rc = launch_rollout<float>(p, b, dv, n, env_offset, k, mode, mlp, act_buf, seed, step_base, traj_obs, traj_act,
-                                   traj_rew, traj_done, (cudaStream_t)stream);
-    else
-        rc = launch_rollout<double>(p, b, dv, n, env_offset, k, mode, mlp, act_buf, seed, step_base, traj_obs, traj_act,
-                                    traj_rew, traj_done, (cudaStream_t)stream);
+    const Traj tr = {traj_obs, traj_act, traj_rew, traj_done};
+    rc = dispatch(p, [&](auto r, auto exact) {
+        return launch_rollout<decltype(r), exact>(p, b, dv, n, env_offset, k, mode, mlp, act_buf, seed, step_base, tr,
+                                                  (cudaStream_t)stream);
+    });
     if (rc) return rc;
     return check_launch("r6_rollout");
 }
@@ -1403,9 +1392,10 @@ int r6_sim_step_raw(double *state, const double *u, const double *m0, const doub
     if (n == 0) return R6_OK;
     int rc = ensure_attributes();
     if (rc) return rc;
-    const unsigned g = (unsigned)blocks_for(n);
-    if (dt <= kMaxDtSeries) sim_raw_kernel<false><<<g, kThreads, kSmemBytes, (cudaStream_t)stream>>>(state, u, m0, t, dt, n, status, nattempts);
-    else sim_raw_kernel<true><<<g, kThreads, kSmemBytes, (cudaStream_t)stream>>>(state, u, m0, t, dt, n, status, nattempts);
+    dispatch_density<double>(dt, [&](double, auto exact) {
+        sim_raw_kernel<exact><<<(unsigned)blocks_for(n), kThreads, kSmemBytes, (cudaStream_t)stream>>>(state, u, m0, t, dt, n, status,
+                                                                                                      nattempts);
+    });
     return check_launch("r6_sim_step_raw");
 }
 
@@ -1422,8 +1412,7 @@ int r6_policy_range(const R6Mlp *mlp, const float *obs, int64_t n, int64_t first
                     int32_t stochastic, uint64_t seed, int64_t env_offset, int64_t step_index, float *actions,
                     float *actions_raw, float *values, float *log_prob, void *stream)
 {
-    if (!mlp || !mlp->w0 || !mlp->b0 || !mlp->w1 || !mlp->b1 || !mlp->w2 || !mlp->b2)
-        return fail(R6_EINVAL, "policy weights are null%s");
+    if (int rc = check_mlp(mlp)) return rc;
     if (!obs || !actions) return fail(R6_EINVAL, "null pointer%s");
     if (n < 0) return fail(R6_EINVAL, "n < 0%s");
     if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
@@ -1490,8 +1479,7 @@ int64_t r6_ppo_work_bytes(int64_t B)
 int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *idx, int64_t B, const R6PpoCoef *coef,
                 float *grad_sum, double *terms, void *work, void *stream)
 {
-    if (!mlp || !mlp->w0 || !mlp->b0 || !mlp->w1 || !mlp->b1 || !mlp->w2 || !mlp->b2)
-        return fail(R6_EINVAL, "policy weights are null%s");
+    if (int rc = check_mlp(mlp)) return rc;
     if (!mlp->wv || !mlp->bv || !mlp->log_std) return fail(R6_EINVAL, "r6_ppo_grad needs the critic head and log_std%s");
     if (!rollout || !rollout->obs || !rollout->actions || !rollout->log_probs || !rollout->advantages || !rollout->returns)
         return fail(R6_EINVAL, "null rollout buffer%s");
