@@ -21,7 +21,6 @@ for rep in range(2):
         n0 = int(n * frac) // 1024 * 1024
         env.join()
         env._lane_ranges = [(0, n0), (n0, n - n0)]
-        env._lane_jobs = [(rg, env._lane_streams[r]) for r, rg in enumerate(env._lane_ranges)]
         for _ in range(20):
             env.step_random(1)
         torch.cuda.synchronize()

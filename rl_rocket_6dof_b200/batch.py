@@ -37,8 +37,7 @@ class Rocket6DOFBatch:
                  num_envs_global: Optional[int] = None, debug_buffers: bool = False, record_attempts: bool = False,
                  ic_table: Optional[np.ndarray] = None, params: Optional[EnvParams] = None,
                  precision: str = "fp64", reward_annealing: bool = False, vertical_attitude_reward=None,
-                 split_step: Optional[bool] = None, lanes: int = 1, multipass: Optional[bool] = None,
-                 chunks: Optional[int] = None):
+                 split_step: Optional[bool] = None, lanes: int = 1, multipass: Optional[bool] = None):
         if not torch.cuda.is_available():
             raise RuntimeError("Rocket6DOFBatch needs a CUDA device (no CPU fallback)")
         self.lib = _lib.load()
@@ -97,16 +96,9 @@ class Rocket6DOFBatch:
                     raise ValueError("lanes must be <= min(num_envs, 32)")
                 split_step = True
                 self._lane_streams = [torch.cuda.Stream(device=dev) for _ in range(self.lanes)]
-                # `chunks` >= lanes contiguous env sub-ranges, dealt round-robin to the lane streams: a sub-range's
-                # kernels (integrator passes, post-step) follow each other on one stream while its state, work lists
-                # and outputs are still in L2 when the sub-range is small enough
-                self.chunks = self.lanes if chunks is None else int(chunks)
-                if self.chunks < self.lanes or self.chunks > 32 or self.chunks > n:
-                    raise ValueError("chunks must be in [lanes, min(num_envs, 32)]")
-                base, rem = divmod(n, self.chunks)
-                self._lane_ranges = [(r * base + min(r, rem), base + (1 if r < rem else 0)) for r in range(self.chunks)]
-                self._lane_jobs = [(rg, self._lane_streams[r % self.lanes]) for r, rg in enumerate(self._lane_ranges)]
                 self._lane_fork = torch.cuda.Event()
+            base, rem = divmod(n, self.lanes)           # one contiguous env sub-range (first, count) per lane
+            self._lane_ranges = [(r * base + min(r, rem), base + (1 if r < rem else 0)) for r in range(self.lanes)]
             self._lanes_pending = False
             self.scratch = torch.zeros(2, n, dtype=torch.uint8, device=dev) if split_step else None
             # multi-pass integrator (R6Buffers.work): one RK attempt per pass, unfinished envs compacted into work
@@ -159,31 +151,57 @@ class Rocket6DOFBatch:
         return torch.cuda.current_stream(self.device).cuda_stream
 
     # ------------------------------------------------------------------ stream lanes
-    def _step_lanes(self, actions: Optional[torch.Tensor], k: int, join: bool):
-        """k env-steps over the lanes: every lane stream first waits for what the caller's stream has enqueued so far
-        (the producer of `actions`, the previous joined step), then runs its sub-range's kernel pairs back to back."""
-        cur = torch.cuda.current_stream(self.device)
-        self._lane_fork.record(cur)
-        ap = 0 if actions is None else actions.data_ptr()
-        with torch.cuda.device(self.device):
-            for st in self._lane_streams:
+    def _fork(self, actions: Optional[torch.Tensor] = None, mlp: Optional[dict] = None) -> list:
+        """(lane, first, count, stream) for every lane; with one lane the whole batch on the caller's stream.  With lanes,
+        every lane stream first waits for what the caller's stream has enqueued so far (the producer of `actions`, the
+        previous joined step), and the caller's tensors the lanes read (`actions`, the weights in `mlp`) are recorded on
+        every lane stream, so that the allocator does not hand their memory out again before the lanes are done with it
+        (the caller may drop them before `join()`)."""
+        streams = [torch.cuda.current_stream(self.device)]
+        if self.lanes > 1:
+            self._lane_fork.record(streams[0])
+            streams = self._lane_streams
+            reads = [t for t in [actions, *(mlp or {}).values()] if isinstance(t, torch.Tensor)]
+            for st in streams:
                 st.wait_event(self._lane_fork)
-                if actions is not None:
-                    actions.record_stream(st)
-            for j in range(int(k)):
-                for ln, ((first, count), st) in enumerate(self._lane_jobs):
-                    _lib.check(self.lib.r6_step_range(C.byref(self._p), C.byref(self._b), self.num_envs, first, count, ln,
-                                                      self.env_offset, ap, self.seed_value, self.steps_done + j,
-                                                      st.cuda_stream), self.lib)
-        self.steps_done += int(k)
-        self._lanes_pending = True
-        if join:
-            self.join()
+                for t in reads:
+                    t.record_stream(st)
+        return [(ln, first, count, st) for ln, ((first, count), st) in enumerate(zip(self._lane_ranges, streams))]
+
+    def _advance(self, k: int, join: bool = True):
+        """Counts k env-steps issued by `_fork`'s schedule; with lanes they are pending until `join()`."""
+        self.steps_done += k
+        if self.lanes > 1:
+            self._lanes_pending = True
+            if join:
+                self.join()
+
+    def _env_step(self, lane: int, first: int, count: int, actions: int, step_index: int, stream: torch.cuda.Stream):
+        """One env-step of envs [first, first + count) on `stream`; `actions` is a device pointer, 0 for in-kernel Philox
+        actions of step `step_index`.  With lanes, the kernel pair on the lane's sub-range; on one stream, r6_step (which
+        picks the fused kernel, the kernel pair or the multi-pass integrator) or the random-action kernel pair."""
+        L, p, b, s = self.lib, C.byref(self._p), C.byref(self._b), stream.cuda_stream
+        if self.lanes > 1:
+            rc = L.r6_step_range(p, b, self.num_envs, first, count, lane, self.env_offset, actions, self.seed_value,
+                                 step_index, s)
+        elif actions:
+            rc = L.r6_step(p, b, self.num_envs, self.env_offset, actions, self.seed_value, s)
+        else:
+            rc = L.r6_step_random(p, b, self.num_envs, self.env_offset, self.seed_value, step_index, s)
+        _lib.check(rc, L)
+
+    def _policy(self, m: R6Mlp, obs: int, first: int, count: int, tensor_cores, stochastic: bool, step_index: int,
+                act: int, raw: Optional[int], val: Optional[int], logp: Optional[int], stream: torch.cuda.Stream):
+        """The policy network over envs [first, first + count) of the component-major observations at device pointer
+        `obs` (r6_policy_range); the output pointers raw / val / logp may be None (not written)."""
+        _lib.check(self.lib.r6_policy_range(C.byref(m), obs, self.num_envs, first, count, int(tensor_cores),
+                                            int(bool(stochastic)), self.seed_value, self.env_offset, step_index, act, raw,
+                                            val, logp, stream.cuda_stream), self.lib)
 
     def join(self):
         """Orders everything the lanes have been given before whatever the caller's current stream does next.  A no-op
-        without lanes or when nothing is pending; every method other than `step(..., join=False)` /
-        `step_random(..., join=False)` joins by itself."""
+        without lanes or when nothing is pending; every method other than `step(..., join=False)`,
+        `step_random(..., join=False)` and `step_policy(..., join=False)` joins by itself."""
         if self._lanes_pending:
             cur = torch.cuda.current_stream(self.device)
             for st in self._lane_streams:
@@ -215,13 +233,10 @@ class Rocket6DOFBatch:
         if actions.dtype != torch.float32 or not actions.is_cuda or actions.shape != (self.num_envs, 3):
             raise ValueError("actions must be a float32 CUDA tensor of shape [num_envs, 3]")
         actions = actions.contiguous()
-        if self.lanes > 1:
-            self._step_lanes(actions, 1, join)
-            return self.obs, self.reward, self.done, self.flags
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.r6_step(C.byref(self._p), C.byref(self._b), self.num_envs, self.env_offset,
-                                        actions.data_ptr(), self.seed_value, self._stream()), self.lib)
-        self.steps_done += 1
+            for ln, first, count, st in self._fork(actions):
+                self._env_step(ln, first, count, actions.data_ptr(), self.steps_done, st)
+        self._advance(1, join)
         return self.obs, self.reward, self.done, self.flags
 
     def rollout(self, k: int, mode: int = ACT_PHILOX, *, actions: Optional[torch.Tensor] = None,
@@ -273,32 +288,30 @@ class Rocket6DOFBatch:
         if self.scratch is None:                       # the random-action step exists only as the kernel pair
             self.scratch = torch.zeros(2, self.num_envs, dtype=torch.uint8, device=self.device)
             self._b.scratch = self.scratch.data_ptr()
-        if self.lanes > 1:
-            self._step_lanes(None, k, join)
-            return self.obs, self.reward, self.done, self.flags
+        k = int(k)
         with torch.cuda.device(self.device):
-            for _ in range(int(k)):
-                _lib.check(self.lib.r6_step_random(C.byref(self._p), C.byref(self._b), self.num_envs, self.env_offset,
-                                                   self.seed_value, self.steps_done, self._stream()), self.lib)
-                self.steps_done += 1
+            lanes = self._fork()
+            for j in range(k):
+                for ln, first, count, st in lanes:
+                    self._env_step(ln, first, count, 0, self.steps_done + j, st)
+        self._advance(k, join)
         return self.obs, self.reward, self.done, self.flags
 
     def policy_actions(self, mlp: dict, *, tensor_cores=False, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Deterministic policy actions [N, 3] for the current observations (one r6_policy launch).
+        """Deterministic policy actions [N, 3] for the current observations (one policy launch).
         tensor_cores: False / 0 = float32 FMA network; True / 1 = mma.sync 3xTF32 tiles (faithful to 2e-6);
         2 = tcgen05 + TMEM single-pass TF32 (fast mode, ~1e-3); 3 = tcgen05 + TMEM 3xTF32 (faithful to 3e-6)."""
         self.join()
         if out is None:
             out = torch.empty(self.num_envs, 3, dtype=torch.float32, device=self.device)
-        m = _lib.make_mlp(mlp)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.r6_policy(C.byref(m), self.obs.data_ptr(), self.num_envs, int(tensor_cores),
-                                          out.data_ptr(), self._stream()), self.lib)
+            self._policy(_lib.make_mlp(mlp), self.obs.data_ptr(), 0, self.num_envs, tensor_cores, False, self.steps_done,
+                         out.data_ptr(), None, None, None, torch.cuda.current_stream(self.device))
         return out
 
     def policy_forward(self, mlp: dict, *, stochastic: bool = False, tensor_cores=False, step_index: Optional[int] = None,
                        out: Optional[tuple] = None):
-        """SB3 `ActorCriticPolicy.forward` for the current observations in one launch (`r6_policy_ex`): returns
+        """SB3 `ActorCriticPolicy.forward` for the current observations in one launch: returns
         (env_actions [N,3] clipped, raw_actions [N,3], values [N], log_prob [N]).  `mlp` may carry the critic head
         ("wv", "bv") and the Gaussian "log_std"; stochastic=True samples mean + exp(log_std) eps with Philox noise
         keyed by (seed, global env id, step_index) — reproducible and independent of the shard count."""
@@ -311,12 +324,10 @@ class Rocket6DOFBatch:
             raw = torch.empty(n, 3, dtype=torch.float32, device=dev)
             val = torch.empty(n, dtype=torch.float32, device=dev)
             logp = torch.empty(n, dtype=torch.float32, device=dev)
-        m = _lib.make_mlp(mlp)
         step = self.steps_done if step_index is None else int(step_index)
         with torch.cuda.device(dev):
-            _lib.check(self.lib.r6_policy_ex(C.byref(m), self.obs.data_ptr(), n, int(tensor_cores), int(bool(stochastic)),
-                                             self.seed_value, self.env_offset, step, act.data_ptr(), raw.data_ptr(),
-                                             val.data_ptr(), logp.data_ptr(), self._stream()), self.lib)
+            self._policy(_lib.make_mlp(mlp), self.obs.data_ptr(), 0, n, tensor_cores, stochastic, step, act.data_ptr(),
+                         raw.data_ptr(), val.data_ptr(), logp.data_ptr(), torch.cuda.current_stream(dev))
         return act, raw, val, logp
 
     def collect_rollout(self, k: int, mlp: dict, *, gamma: float = 0.99, gae_lambda: float = 0.95,
@@ -345,48 +356,31 @@ class Rocket6DOFBatch:
         dones = torch.empty(k, n, dtype=torch.uint8, device=dev)
         a_env = torch.empty(n, 3, dtype=torch.float32, device=dev)
         m = _lib.make_mlp(mlp)
-        L = self.lib
         # Without auto-reset a finished env is frozen: the step reads its done flag and writes NOTHING for it, so its
         # obs / reward / done must carry over from the previous step — that mode keeps the per-step copies.
         in_place = bool(self.auto_reset)
         saved = (self._b.obs, self._b.reward_f32, self._b.done)
-        if self.lanes > 1:                           # every lane runs [policy, env step] x k over its env range on its stream
-            jobs = list(enumerate(self._lane_jobs))
-            self._lane_fork.record(torch.cuda.current_stream(dev))
-            for st in self._lane_streams:
-                st.wait_event(self._lane_fork)
-        else:
-            jobs = [(0, ((0, n), torch.cuda.current_stream(dev)))]
+        lanes = self._fork(mlp=mlp)                  # every lane runs [policy, env step] x k over its env range on its stream
         try:
             with torch.cuda.device(dev):
                 for j in range(k):
                     if in_place:
                         self._b.obs, self._b.reward_f32, self._b.done = (obs_cm[j + 1].data_ptr(), rews[j].data_ptr(),
                                                                         dones[j].data_ptr())
-                    for ln, ((first, count), st) in jobs:
+                    for ln, first, count, st in lanes:
                         if not in_place and j > 0:
                             with torch.cuda.stream(st):
                                 obs_cm[j, :, first:first + count] = self.obs[:, first:first + count]
-                        _lib.check(L.r6_policy_range(C.byref(m), obs_cm[j].data_ptr(), n, first, count, int(tensor_cores),
-                                                     int(bool(stochastic)), self.seed_value, self.env_offset,
-                                                     self.steps_done + j, a_env.data_ptr(), acts[j].data_ptr(),
-                                                     vals[j].data_ptr(), logp[j].data_ptr(), st.cuda_stream), L)
-                        if self.lanes > 1:
-                            _lib.check(L.r6_step_range(C.byref(self._p), C.byref(self._b), n, first, count, ln, self.env_offset,
-                                                       a_env.data_ptr(), self.seed_value, self.steps_done + j, st.cuda_stream), L)
-                        else:                        # whole batch on the caller's stream: r6_step picks fused / split / multi-pass
-                            _lib.check(L.r6_step(C.byref(self._p), C.byref(self._b), n, self.env_offset, a_env.data_ptr(),
-                                                 self.seed_value, st.cuda_stream), L)
+                        self._policy(m, obs_cm[j].data_ptr(), first, count, tensor_cores, stochastic, self.steps_done + j,
+                                     a_env.data_ptr(), acts[j].data_ptr(), vals[j].data_ptr(), logp[j].data_ptr(), st)
+                        self._env_step(ln, first, count, a_env.data_ptr(), self.steps_done + j, st)
                         if not in_place:
                             with torch.cuda.stream(st):
                                 rews[j, first:first + count] = self.reward_f32[first:first + count]
                                 dones[j, first:first + count] = self.done[first:first + count]
         finally:
             self._b.obs, self._b.reward_f32, self._b.done = saved
-        self.steps_done += k
-        if self.lanes > 1:
-            self._lanes_pending = True
-            self.join()
+        self._advance(k)
         if k > 0 and in_place:                       # the batch's own output tensors end up as after k calls of step()
             self.obs.copy_(obs_cm[k])
             self.reward_f32.copy_(rews[k - 1])
@@ -401,33 +395,19 @@ class Rocket6DOFBatch:
         the actions, the step kernel consumes them — VecEnv semantics (auto-reset as configured).  Faster than the
         single fused rollout kernel for large batches; `rollout(k, ACT_MLP)` remains for one-episode semantics.
         With stream lanes every lane runs its own policy -> step chain (r6_policy_range, r6_step_range) for the k
-        steps and the lanes are joined at the end."""
+        steps and the lanes are joined at the end (join=False leaves them running, as in `step`)."""
         act = getattr(self, "_policy_act", None)
         if act is None:
             act = self._policy_act = torch.empty(self.num_envs, 3, dtype=torch.float32, device=self.device)
-        if self.lanes > 1:
-            m = _lib.make_mlp(mlp)
-            cur = torch.cuda.current_stream(self.device)
-            self._lane_fork.record(cur)
-            n, L = self.num_envs, self.lib
-            with torch.cuda.device(self.device):
-                for st in self._lane_streams:
-                    st.wait_event(self._lane_fork)
-                for j in range(int(k)):
-                    for ln, ((first, count), st) in enumerate(self._lane_jobs):
-                        _lib.check(L.r6_policy_range(C.byref(m), self.obs.data_ptr(), n, first, count, int(tensor_cores), 0,
-                                                     self.seed_value, self.env_offset, self.steps_done + j, act.data_ptr(),
-                                                     None, None, None, st.cuda_stream), L)
-                        _lib.check(L.r6_step_range(C.byref(self._p), C.byref(self._b), n, first, count, ln, self.env_offset,
-                                                   act.data_ptr(), self.seed_value, self.steps_done + j, st.cuda_stream), L)
-            self.steps_done += int(k)
-            self._lanes_pending = True
-            if join:
-                self.join()
-            return self.obs, self.reward, self.done, self.flags
-        for _ in range(int(k)):
-            self.policy_actions(mlp, tensor_cores=tensor_cores, out=act)
-            self.step(act)
+        k, m = int(k), _lib.make_mlp(mlp)
+        with torch.cuda.device(self.device):
+            lanes = self._fork(mlp=mlp)
+            for j in range(k):
+                for ln, first, count, st in lanes:
+                    self._policy(m, self.obs.data_ptr(), first, count, tensor_cores, False, self.steps_done + j,
+                                 act.data_ptr(), None, None, None, st)
+                    self._env_step(ln, first, count, act.data_ptr(), self.steps_done + j, st)
+        self._advance(k, join)
         return self.obs, self.reward, self.done, self.flags
 
     # ------------------------------------------------------------------ state injection / inspection

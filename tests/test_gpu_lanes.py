@@ -50,6 +50,10 @@ def test_lanes_equal_single_stream(lanes, n):
     one.step_random(40)
     many.step_random(40)
     _same(one, many)
+    one.step_random(30)
+    many.step_random(30, join=False)
+    many.join()
+    _same(one, many)
     assert one.steps_done == many.steps_done
 
 
@@ -114,6 +118,14 @@ def test_closed_loop_on_lanes(tc):
     import torch
     assert torch.equal(one._policy_act, many._policy_act)
     assert float(one.stats[0]) > 0
+    # free-running, then joined, with the weights dropped by the caller right after the call: the lanes still read them,
+    # so their memory must not come back from the allocator (here as zeroed tensors of the same sizes) before the join
+    one.step_policy(40, wd, tensor_cores=tc)
+    many.step_policy(40, pol.to_device(w, many.device), tensor_cores=tc, join=False)
+    zeros = [torch.zeros_like(t) for t in wd.values()]          # noqa: F841 (held until after the join)
+    many.join()
+    _same(one, many)
+    assert torch.equal(one._policy_act, many._policy_act)
 
 
 def test_collect_rollout_on_lanes():

@@ -420,7 +420,7 @@ def test_collect_rollout_on_device():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("lanes,auto_reset", [(1, True), (2, True), (1, False)])
+@pytest.mark.parametrize("lanes,auto_reset", [(1, True), (2, True), (1, False), (2, False)])
 def test_collect_rollout_in_place_trajectory_equals_step_by_step(lanes, auto_reset):
     """collect_rollout writes the trajectory in place (the env step's obs / reward / done pointers are redirected into the
     [k, ...] buffers, the policy reads the previous slice): bit-identical to policy_forward + step + copies per step, on one

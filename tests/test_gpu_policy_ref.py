@@ -57,6 +57,31 @@ def launch(wd, obs, mode, stochastic=False, seed=0, env_offset=0, step=0, first=
     return tuple(t.cpu().numpy() for t in (act, raw, val, lp))
 
 
+def test_whole_batch_entry_points_equal_policy_range():
+    """r6_policy (deterministic actions) and r6_policy_ex (actions, raw actions, values, log-probs) give the bits of
+    r6_policy_range over (0, n)."""
+    import torch
+    _l, L = _lib()
+    n = 4097
+    wd = _dev(ref.weights("golden"))
+    x = _obs_cm(ref.obs_sets(n, seed=7)["normal5"])
+    m = _l.make_mlp(wd)
+    st = torch.cuda.current_stream().cuda_stream
+    for mode in (0, 3):
+        a = torch.empty(n, 3, device="cuda")
+        _l.check(L.r6_policy(C.byref(m), x.data_ptr(), n, mode, a.data_ptr(), st), L)
+        torch.cuda.synchronize()
+        assert np.array_equal(a.cpu().numpy(), launch(wd, x, mode, nulls=True)[0]), mode
+        for stochastic in (False, True):
+            outs = (torch.empty(n, 3, device="cuda"), torch.empty(n, 3, device="cuda"), torch.empty(n, device="cuda"),
+                    torch.empty(n, device="cuda"))
+            _l.check(L.r6_policy_ex(C.byref(m), x.data_ptr(), n, mode, int(stochastic), 5, 100, 3,
+                                    *(t.data_ptr() for t in outs), st), L)
+            torch.cuda.synchronize()
+            for got, want in zip(outs, launch(wd, x, mode, stochastic, 5, 100, 3)):
+                assert np.array_equal(got.cpu().numpy(), want), (mode, stochastic)
+
+
 def noise_bar(seed, genv, step):
     """(z_ref [n,3], bar [n,3]) for the device noise of (seed, genv, step): philox_ref.policy_noise_bar (3 ulp)."""
     z = pr.policy_noise(seed, genv, step)
