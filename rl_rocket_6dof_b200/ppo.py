@@ -96,7 +96,8 @@ class PPOConfig:
     would mean 2^27-sample rollouts in 2^21 minibatches of 64.  Here a rollout is `n_steps` (default 32) steps of every
     env, and `batch_size` defaults to a quarter of it (4 minibatches per epoch).  As in SB3 the last minibatch of an
     epoch may be short.  A minibatch of one sample is not normalised (its std is undefined: SB3 1.6 yields NaN there
-    [memory]; later SB3 releases add the same guard)."""
+    [memory]; later SB3 releases add the same guard).  A callable learning_rate is SB3's schedule: it is called once per
+    update with progress_remaining (see `PPOTrainer.learn`)."""
     learning_rate: Union[float, Callable[[float], float]] = 3e-4
     n_steps: int = 32
     batch_size: Optional[int] = None
@@ -213,7 +214,12 @@ class PPOTrainer:
         return int(self.cfg.batch_size) if self.cfg.batch_size else max(1, -(-total // 4))
 
     def train(self, rollout: dict) -> dict:
-        """n_epochs passes over the rollout in minibatches of a seeded on-device permutation; returns SB3's train/ logs."""
+        """n_epochs passes over the rollout in minibatches of a seeded on-device permutation; returns SB3's train/ logs.
+
+        As SB3 1.6 logs them [memory]: policy_gradient_loss, value_loss, clip_fraction and entropy_loss are means over
+        every minibatch that ran (the one `target_kl` stops at included), approx_kl is the mean over the minibatches of
+        the last epoch that ran, entropy_loss and loss use each minibatch's log_std before its Adam step, and loss is the
+        last minibatch's.  The learning rate is `learning_rate(progress_remaining)`."""
         cfg, dev = self.cfg, self.params.flat.device
         T, n = rollout["advantages"].shape
         total = T * n
@@ -221,6 +227,7 @@ class PPOTrainer:
         lr = _progress_lr(cfg.learning_rate, self.progress_remaining)
         nmb = -(-total // bs)
         terms = torch.zeros(cfg.n_epochs * nmb, _lib.PPO_NTERMS, dtype=torch.float64, device=dev)
+        log_std_sums = torch.zeros(cfg.n_epochs * nmb, dtype=torch.float64, device=dev)
         sizes = []
         L = _lib.load()
         need = int(L.r6_ppo_work_bytes(min(bs, total)))
@@ -229,12 +236,14 @@ class PPOTrainer:
         done = False
         for epoch in range(cfg.n_epochs):
             perm = torch.randperm(total, generator=self.gen, device=dev)
+            epoch_start = len(sizes)
             for start in range(0, total, bs):
                 idx = perm[start:start + bs]
                 k = len(sizes)
                 loss_and_grad(self.params, rollout, idx, clip_range=cfg.clip_range, vf_coef=cfg.vf_coef,
                               ent_coef=cfg.ent_coef, normalize_advantage=cfg.normalize_advantage, grad_sum=self._grad,
                               terms=terms[k], work=self._work)
+                log_std_sums[k] = self.params.log_std.sum(dtype=torch.float64)    # this minibatch's entropy (no sync)
                 sizes.append(idx.numel())
                 if cfg.target_kl is not None:
                     kl = float(terms[k, _lib.PPO_NTERMS - 2]) / idx.numel()      # the one host read per minibatch
@@ -251,31 +260,33 @@ class PPOTrainer:
         if t[:, 4].sum() != 0:
             raise ValueError("a minibatch index was outside the rollout")
         means = t[:, :4] / np.asarray(sizes, np.float64)[:, None]
+        entropy = log_std_sums[:len(sizes)].cpu().numpy() + 3 * (0.5 + _LOG_SQRT_2PI)     # per minibatch
         log_std = self.params.log_std.detach().double().cpu().numpy()
-        entropy = float(np.sum(log_std + 0.5 + _LOG_SQRT_2PI))
         v, r = rollout["values"].reshape(-1).double(), rollout["returns"].reshape(-1).double()
         var_r = float(r.var())
         ev = float("nan") if var_r == 0 else 1.0 - float((r - v).var()) / var_r
         return {"train/policy_gradient_loss": float(means[:, 0].mean()), "train/value_loss": float(means[:, 1].mean()),
-                "train/entropy_loss": -entropy, "train/approx_kl": float(means[:, 3].mean()),
+                "train/entropy_loss": float(-entropy.mean()), "train/approx_kl": float(means[epoch_start:, 3].mean()),
                 "train/clip_fraction": float(means[:, 2].mean()),
-                "train/loss": float(means[-1, 0] - cfg.ent_coef * entropy + cfg.vf_coef * means[-1, 1]),
+                "train/loss": float(means[-1, 0] - cfg.ent_coef * entropy[-1] + cfg.vf_coef * means[-1, 1]),
                 "train/explained_variance": ev, "train/std": float(np.exp(log_std).mean()),
                 "train/n_updates": self.n_updates, "train/learning_rate": lr, "train/clip_range": cfg.clip_range}
 
     def learn(self, total_timesteps: int, callback: Optional[Callable[[dict], None]] = None) -> list:
         """Alternates collect_rollout (n_steps of every env) and train until total_timesteps env-steps; returns one log
-        dict per iteration (train/ logs plus the env's episode statistics of that collection under rollout/)."""
+        dict per iteration (train/ logs plus the env's episode statistics of that collection under rollout/).  As in
+        SB3, progress_remaining is updated after the collection, so update i of a run from 0 uses
+        1 - i n_steps N / total_timesteps (the last one 0 when total_timesteps is a multiple of n_steps N)."""
         b, cfg = self.batch, self.cfg
         if self.num_timesteps == 0:
             b.reset()
         logs = []
         while self.num_timesteps < total_timesteps:
-            self.progress_remaining = 1.0 - self.num_timesteps / total_timesteps
             b.reset_stats()
             ro = b.collect_rollout(cfg.n_steps, self.params.mlp(), gamma=cfg.gamma, gae_lambda=cfg.gae_lambda,
                                    tensor_cores=cfg.tensor_cores)
             self.num_timesteps += cfg.n_steps * b.num_envs
+            self.progress_remaining = 1.0 - self.num_timesteps / total_timesteps
             log = {"rollout/" + k: v for k, v in b.stats_dict().items()}
             log.update(self.train(ro))
             log["time/total_timesteps"] = self.num_timesteps

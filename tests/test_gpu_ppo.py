@@ -68,6 +68,43 @@ def test_grad_within_bound(family, B):
         g_dense = g
 
 
+def test_grad_at_training_minibatch_sizes():
+    """B = 2^18 + 129, the size class of the trainer's minibatches (2^16 envs x 32 steps / 4 = 2^19): every CTA
+    accumulates 14 tiles with dW1 parked in shared memory between them, where the SIZES above reach about 2.  Drawn
+    without replacement from a T = 32 rollout; dense and strided obs.  Not in the SIZES cross-product: the reference
+    costs about 35 s of CPU here.  It is summed in chunks (grad_sum and bound are sums over samples, with the global
+    samples_per_cta), so host memory stays near 1 GB."""
+    from rl_rocket_6dof_b200 import ppo
+    w = pr.weights("golden")
+    B, T, n = 2 ** 18 + 129, 32, 8400
+    x = pr.obs_sets(T * n, seed=11)["golden"]
+    a, old, adv, ret = rf.minibatch(w, x, seed=11)
+    idx = np.random.default_rng(11).choice(T * n, B, replace=False)
+    st = rf.adv_stats(adv[idx])
+    spc = rf.samples_per_cta(B)
+    assert spc == 14 * 128
+    g64, t64, bnd, tb = 0.0, 0.0, 0.0, 0.0
+    for s in range(0, B, 1 << 15):
+        j = idx[s:s + (1 << 15)]
+        q = rf.per_sample(w, x[j], a[j], old[j], (adv[j].astype(np.float64) - st[0]) * st[1], ret[j])
+        g_c, t_c = rf.grad_sum(q)
+        b_c, tb_c = rf.bound(q, samples_per_cta=spc)
+        g64, t64, bnd, tb = g64 + g_c, t64 + t_c, bnd + b_c, tb + tb_c
+    for strided in (False, True):
+        ro = _rollout(x, a, old, adv, ret, T, strided)
+        g, terms = ppo.loss_and_grad(_params(w), ro, torch.from_numpy(idx).to(DEV))
+        g, terms = g.cpu().numpy().astype(np.float64), terms.cpu().numpy()
+        r = np.abs(g - g64) / bnd
+        print(f"B {B} strided {strided}: max |kernel - ref| / bound {r.max():.3g}, median bound / |g| "
+              f"{np.median(bnd / np.maximum(np.abs(g64), 1e-30)):.3g}")
+        assert np.all(r <= rf.C_BAR), (strided, float(r.max()), int(r.argmax()))
+        assert terms[2] == t64[2] and terms[4] == 0
+        assert np.all(np.abs(terms[[0, 1, 3]] - t64[[0, 1, 3]]) <= rf.C_BAR * tb[[0, 1, 3]])
+        if strided:
+            assert np.array_equal(g, g_dense)
+        g_dense = g
+
+
 def test_bound_has_teeth_and_runs_are_reproducible():
     from rl_rocket_6dof_b200 import ppo
     w = pr.weights("golden")

@@ -11,22 +11,15 @@ import torch
 import ppo_hostsim
 import policy_ref as pr
 import ppo_ref as rf
+import ppo_train_ref as tr
 
 
 def autograd_sum(w, x, a, old, adv_n, ret, clip, vf_coef, ent_coef):
-    """Sum over samples of the gradient of pg + vf_coef (R - v)^2 - ent_coef entropy, torch float64 autograd."""
+    """Sum over samples of the gradient of pg + vf_coef (R - v)^2 - ent_coef entropy: len(x) times the gradient of
+    SB3's minibatch-mean loss (ppo_train_ref.sb3_loss), torch float64 autograd."""
     P = {k: torch.tensor(np.asarray(v, np.float32).astype(np.float64), requires_grad=True) for k, v in w.items()}
-    X = torch.tensor(np.asarray(x, np.float32).astype(np.float64))
-    h = torch.tanh(torch.tanh(X @ P["w0"].T + P["b0"]) @ P["w1"].T + P["b1"])
-    mean, v = h @ P["w2"].T + P["b2"], h @ P["wv"].reshape(64) + P["bv"][0]
-    dist = torch.distributions.Normal(mean, torch.exp(P["log_std"]))
-    logp = dist.log_prob(torch.tensor(np.asarray(a, np.float32).astype(np.float64))).sum(1)
-    ratio = torch.exp(logp - torch.tensor(np.asarray(old, np.float32).astype(np.float64)))
-    A = torch.tensor(adv_n)
-    pg = -torch.min(A * ratio, A * torch.clamp(ratio, 1 - clip, 1 + clip))
-    vl = (torch.tensor(np.asarray(ret, np.float32).astype(np.float64)) - v) ** 2
-    ent = dist.entropy().sum(1)
-    (pg + vf_coef * vl - ent_coef * ent).sum().backward()
+    loss, _ = tr.sb3_loss(P, x, a, old, adv_n, ret, clip, vf_coef, ent_coef)
+    (len(x) * loss).backward()
     return np.concatenate([P[k].grad.numpy().reshape(-1) for k, _ in rf.LAYOUT])
 
 
@@ -95,6 +88,45 @@ def test_adam_step_matches_torch(max_norm):
         assert np.all(np.abs(p32 - ref) <= 4 * 2.0 ** -24 * np.abs(ref) + 1e-3 * 3e-4 * step)
     if max_norm == 0.5:
         assert norm > max_norm          # the clip was active
+
+
+@pytest.mark.parametrize("family,max_norm", [("saturating", 0.5), ("sb3_init", 1e6)])
+def test_sb3_train_step_matches_grad_sum_and_bounds_the_host_step(family, max_norm):
+    """ppo_train_ref's SB3 statement (autograd of the minibatch-mean loss, clip_grad_norm_, Adam) on one ppo_ref
+    minibatch: its gradient is grad_sum / B to float64 round-off and its logged terms the term sums / B; the host build
+    of r6_adam_step fed the host build's gradient sum lands within C_BAR x the per-step bound, and the bound fails for a
+    step scaled by 1 / batch_size instead of 1 / len(idx) (clip off) and for the clip factor omitted (clip on)."""
+    from rl_rocket_6dof_b200.ppo import NPARAMS, PPOConfig
+    w = pr.weights(family)
+    n, B, step, lr, ent = 400, 300, 3, 3e-4, 0.01
+    x = pr.obs_sets(n, seed=4)["uniform"]
+    a, old, adv, ret = rf.minibatch(w, x, seed=5)
+    ro = dict(obs=x, actions=a, log_probs=old, advantages=adv, returns=ret)
+    idx = np.random.default_rng(6).permutation(n)[:B]
+    cfg = PPOConfig(ent_coef=ent, max_grad_norm=max_norm)
+    rng = np.random.default_rng(7)
+    p = rf.flat(w)
+    m = (rng.standard_normal(NPARAMS) * 1e-2).astype(np.float32)
+    v = (rng.standard_normal(NPARAMS) ** 2 * 1e-4).astype(np.float32)
+    m[::7], v[::7] = 0, 0                                      # moments that start at zero, as after sb3_init
+    ref = tr.reference_step(p, m, v, step, ro, idx, lr, cfg)
+    st = rf.adv_stats(adv[idx])
+    q = rf.per_sample(w, x[idx], a[idx], old[idx], (adv[idx].astype(np.float64) - st[0]) * st[1], ret[idx], ent_coef=ent)
+    g64, t64 = rf.grad_sum(q)
+    assert np.allclose(B * ref["grad"], g64, rtol=1e-10, atol=1e-10 * np.abs(g64).max())
+    for k, j in (("pg", 0), ("value_loss", 1), ("clip_fraction", 2), ("approx_kl", 3)):
+        assert math.isclose(B * ref["logs"][k], t64[j], rel_tol=1e-10, abs_tol=1e-12), k
+    assert (ref["clip"] < 1) == (max_norm == 0.5)
+    gs = ppo_hostsim.ppo_sample_grad(p, x[idx], a[idx], old[idx], adv[idx], ret[idx], adv_stats=st, ent_coef=ent)[0]
+    gs = gs.astype(np.float64).sum(0).astype(np.float32)
+    p32, m32, v32 = p.copy(), m.copy(), v.copy()
+    norm = ppo_hostsim.adam_step(p32, gs, m32, v32, adam_coef(lr, max_norm, 1.0 / B), step)
+    assert abs(norm - ref["norm"]) <= 1e-3 * ref["norm"]
+    r = np.abs(p32 - ref["p"]) / ref["bound"]
+    assert np.all(r <= rf.C_BAR), (float(r.max()), int(r.argmax()))
+    wrong = (tr.reference_step(p, m, v, step, ro, idx, lr, cfg, scale=1.0 / (B + 100)) if max_norm > 1 else
+             tr.reference_step(p, m, v, step, ro, idx, lr, PPOConfig(ent_coef=ent, max_grad_norm=1e30)))
+    assert np.any(np.abs(p32 - wrong["p"]) > rf.C_BAR * wrong["bound"])
 
 
 def adam_coef(lr, max_norm, scale):
