@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 17
+#define R6_ABI_VERSION 18
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -298,6 +298,30 @@ int r6_policy_range(const R6Mlp *mlp, const float *obs, int64_t n, int64_t first
  */
 int r6_gae(const float *rew, const float *values, const uint8_t *done, const float *last_values, int32_t T, int64_t n,
            double gamma, double gae_lambda, float *adv, float *ret, void *stream);
+
+/*
+ * Bootstrapping of TimeLimit truncations with the critic, as stable-baselines3 1.6.0
+ * `OnPolicyAlgorithm.collect_rollouts` does while collecting (SB3 issue #633):
+ *     if done and infos[i]["terminal_observation"] is not None and infos[i]["TimeLimit.truncated"]:
+ *         rewards[i] += gamma * predict_values(terminal_observation)
+ * in three passes that need no host synchronise:
+ *  1. r6_trunc_record after each env step of the rollout (step = its index in [0, T)), on the stream and env sub-range of
+ *     that step: every env of [first, first + count) with R6_F_TRUNCATED in flags[i] takes the first slot s with
+ *     slot_step[s][i] < 0, sets slot_step[s][i] = step and copies rows 0..12 of terminal_obs[:, i] into slot_obs[s][:, i].
+ *     A truncation that finds no free slot is dropped (nothing is written past slot slots - 1); one env truncates at most
+ *     ceil(T / max_episode_steps) times in T steps, so that many slots always suffice.  Launched as a programmatic
+ *     dependent like the env-step kernels.  slot_step: int32 [slots][n], all -1 before the first step of the rollout;
+ *     slot_obs: float32 [slots][13][n] (component-major, the observation layout r6_policy_range reads).
+ *  2. r6_policy_range over each slot layer slot_obs[s] (all n columns; columns of free slots hold anything and their
+ *     values are not read), with the collection's tensor_cores mode, writing V into slot_values[s].
+ *  3. r6_trunc_bootstrap: rew[t][i] = f32(rew[t][i] + f32(f32(gamma) * slot_values[s][i])) for every slot with
+ *     t = slot_step[s][i] in [0, T) — SB3's float32 arithmetic, two roundings, no FMA.  rew: float32 [T][n] (the rewards
+ *     of the rollout, before r6_gae); slot_values: float32 [slots][n].
+ */
+int r6_trunc_record(const uint8_t *flags, const float *terminal_obs, int64_t n, int64_t first, int64_t count, int32_t step,
+                    int32_t slots, int32_t *slot_step, float *slot_obs, void *stream);
+int r6_trunc_bootstrap(float *rew, int32_t T, int64_t n, int32_t slots, const int32_t *slot_step, const float *slot_values,
+                       double gamma, void *stream);
 
 /*
  * PPO update (stable-baselines3 1.6.0 `PPO.train`, the optimiser of main_6DOF.py:136).

@@ -12,7 +12,7 @@ from .params import R6Params
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libr6dof.so")
-ABI_VERSION = 17
+ABI_VERSION = 18
 
 u8p = C.c_void_p
 
@@ -73,7 +73,8 @@ def make_mlp(weights: dict) -> "R6Mlp":
 
 EXPORTS = ["r6_abi_version", "r6_last_error", "r6_params_size", "r6_buffers_size", "r6_reset", "r6_step",
            "r6_rollout", "r6_sim_step_raw", "r6_tgo", "r6_stats_reset", "r6_peak_fma", "r6_gae", "r6_policy", "r6_policy_ex", "r6_step_random", "r6_step_range", "r6_policy_range", "r6_work_bytes",
-           "r6_ppo_rollout_size", "r6_ppo_coef_size", "r6_adam_coef_size", "r6_ppo_work_bytes", "r6_ppo_grad", "r6_adam_step"]
+           "r6_ppo_rollout_size", "r6_ppo_coef_size", "r6_adam_coef_size", "r6_ppo_work_bytes", "r6_ppo_grad", "r6_adam_step",
+           "r6_trunc_record", "r6_trunc_bootstrap"]
 
 
 class R6Error(RuntimeError):
@@ -131,6 +132,10 @@ def load(path: str | None = None):
     L.r6_policy.argtypes = [C.POINTER(R6Mlp), C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
     L.r6_gae.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_double, C.c_double,
                          C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_trunc_record.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
+                                  C.c_void_p, C.c_void_p]
+    L.r6_trunc_bootstrap.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_double,
+                                     C.c_void_p]
     L.r6_ppo_work_bytes.argtypes = [C.c_int64]
     L.r6_ppo_work_bytes.restype = C.c_int64
     L.r6_ppo_grad.argtypes = [C.POINTER(R6Mlp), C.POINTER(R6PpoRollout), C.c_void_p, C.c_int64, C.POINTER(R6PpoCoef),

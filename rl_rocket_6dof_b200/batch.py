@@ -331,12 +331,18 @@ class Rocket6DOFBatch:
         return act, raw, val, logp
 
     def collect_rollout(self, k: int, mlp: dict, *, gamma: float = 0.99, gae_lambda: float = 0.95,
-                        stochastic: bool = True, tensor_cores=3) -> dict:
+                        stochastic: bool = True, tensor_cores=3, bootstrap_truncated: bool = False) -> dict:
         """What SB3's `PPO.collect_rollouts` + `RolloutBuffer.compute_returns_and_advantage` produce for k steps of
         this VecEnv, entirely on the device: per step one policy launch (action, value, log-prob; by default the
         faithful tcgen05 3xTF32 kernel, tensor_cores=3) and one env step, then the GAE scan.  Returns tensors shaped
         [k, N, ...]: obs (13), actions (raw Gaussian samples), values, log_probs, rewards, dones, advantages, returns.
-        (Bootstrapping time-limit truncations with the critic is left to the caller, as in `gae.compute_gae`.)
+
+        bootstrap_truncated=True adds SB3's timeout handling: the reward of a step that ended its episode by the TimeLimit
+        (flag F_TRUNCATED) becomes fl32(r + fl32(gamma * V(terminal observation))), V from the same policy kernel and
+        `tensor_cores` mode as `values`, before the GAE scan; `dones` stays as it is.  Each truncation is filed after its
+        step (`r6_trunc_record`), the critic runs once per slot layer after the rollout and `r6_trunc_bootstrap` adds the
+        values, all without a host synchronise.  Needs auto-reset (ValueError otherwise).  The default False leaves the
+        rewards as the env returned them.
 
         The trajectory is written in place: the env step of step j writes its observations straight into slice j + 1 of
         a component-major buffer [k + 1, 14, N] (the layout the kernels read and write), its reward and done flags into
@@ -346,7 +352,15 @@ class Rocket6DOFBatch:
         from .gae import compute_gae
         k = int(k)
         n, dev = self.num_envs, self.device
+        if bootstrap_truncated and not self.auto_reset:
+            raise ValueError("bootstrap_truncated needs auto_reset=True (a frozen one-episode env keeps its flags)")
         self.join()
+        # one slot per truncation an env can have in k steps: two of them are at least max_episode_steps apart
+        limit = int(self._p.max_episode_steps)
+        slots = -(-k // limit) if bootstrap_truncated and limit > 0 else 0
+        if slots:                                    # filled before the lanes fork, so that they see the -1
+            slot_step = torch.full((slots, n), -1, dtype=torch.int32, device=dev)
+            slot_obs = torch.empty(slots, 13, n, dtype=torch.float32, device=dev)
         obs_cm = torch.empty(k + 1, 14, n, dtype=torch.float32, device=dev)
         obs_cm[0].copy_(self.obs)
         acts = torch.empty(k, n, 3, dtype=torch.float32, device=dev)
@@ -374,6 +388,10 @@ class Rocket6DOFBatch:
                         self._policy(m, obs_cm[j].data_ptr(), first, count, tensor_cores, stochastic, self.steps_done + j,
                                      a_env.data_ptr(), acts[j].data_ptr(), vals[j].data_ptr(), logp[j].data_ptr(), st)
                         self._env_step(ln, first, count, a_env.data_ptr(), self.steps_done + j, st)
+                        if slots:
+                            _lib.check(self.lib.r6_trunc_record(self.flags.data_ptr(), self.terminal_obs.data_ptr(), n, first,
+                                                                count, j, slots, slot_step.data_ptr(), slot_obs.data_ptr(),
+                                                                st.cuda_stream), self.lib)
                         if not in_place:
                             with torch.cuda.stream(st):
                                 rews[j, first:first + count] = self.reward_f32[first:first + count]
@@ -386,6 +404,15 @@ class Rocket6DOFBatch:
             self.reward_f32.copy_(rews[k - 1])
             self.done.copy_(dones[k - 1])
         _, _, last_v, _ = self.policy_forward(mlp, stochastic=False, tensor_cores=tensor_cores)
+        if slots:
+            cur = torch.cuda.current_stream(dev)
+            slot_v = torch.empty(slots, n, dtype=torch.float32, device=dev)
+            with torch.cuda.device(dev):
+                for s in range(slots):
+                    self._policy(m, slot_obs[s].data_ptr(), 0, n, tensor_cores, False, 0, a_env.data_ptr(), None,
+                                 slot_v[s].data_ptr(), None, cur)
+                _lib.check(self.lib.r6_trunc_bootstrap(rews.data_ptr(), k, n, slots, slot_step.data_ptr(), slot_v.data_ptr(),
+                                                       float(gamma), cur.cuda_stream), self.lib)
         adv, ret = compute_gae(rews, vals, dones, last_v, gamma, gae_lambda)
         return dict(obs=obs_cm[:k, :13].permute(0, 2, 1), actions=acts, values=vals, log_probs=logp, rewards=rews, dones=dones,
                     advantages=adv, returns=ret, last_values=last_v)

@@ -11,6 +11,7 @@
 //   policy_kernel, policy_tc5_kernel   the policy MLP alone: float32 FMAs, mma.sync 3xTF32 tiles, or tcgen05.mma with
 //                                    accumulators and activations in TMEM (r6_mlp_tc.cuh, r6_mlp_tcgen05.cuh)
 //   ppo_grad_kernel | ppo_reduce_kernel, adam_kernel   the PPO update: minibatch loss gradient, Adam step
+//   trunc_record_kernel, trunc_bootstrap_kernel   time-limit truncations filed per step, bootstrapped with the critic
 //   reset_kernel, sim_raw_kernel, tgo_kernel, gae_kernel, peak_fma_kernel
 //
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo (see build.py).
@@ -893,6 +894,46 @@ gae_kernel(const float *__restrict__ rew, const float *__restrict__ values, cons
     }
 }
 
+// Time-limit bootstrap of a collected rollout (SB3 1.6 OnPolicyAlgorithm.collect_rollouts: rewards[idx] += gamma *
+// V(terminal_observation) where TimeLimit.truncated).  After each env step, every env whose step was a truncation files
+// the step index and the 13 observation rows of its terminal observation into its first free slot (slot_step < 0); an env
+// that did not truncate reads its one flags byte and nothing else.  Every thread waits for the env step first, so that
+// this grid never completes ahead of it and a programmatic dependent launched after this one still sees the step's output.
+__global__ void __launch_bounds__(256)
+trunc_record_kernel(const uint8_t *__restrict__ flags, const float *__restrict__ terminal_obs, int64_t n, int64_t i0, int64_t i1,
+                    int step, int slots, int32_t *__restrict__ slot_step, float *__restrict__ slot_obs)
+{
+    const int64_t i = i0 + (int64_t)blockIdx.x * 256 + threadIdx.x;
+    grid_dependency_wait();
+    if (i >= i1 || !(flags[i] & R6_F_TRUNCATED)) return;
+    for (int s = 0; s < slots; s++) {                    // never past slot slots - 1: a further truncation is dropped
+        int32_t *st = slot_step + (int64_t)s * n + i;
+        if (*st >= 0) continue;
+        *st = step;
+        float *o = slot_obs + (int64_t)s * 13 * n + i;
+#pragma unroll
+        for (int c = 0; c < 13; c++) o[(int64_t)c * n] = terminal_obs[(int64_t)c * n + i];
+        return;
+    }
+}
+
+// rew[t][i] = fl32(rew[t][i] + fl32(gamma * V[s][i])) for every filed slot (s, i) with t = slot_step[s][i] in [0, T):
+// float32 reward buffer, float32 value, python-float gamma, two roundings and no FMA, as SB3 computes it.  Two slots of one
+// env never hold the same step, so every (t, i) is touched at most once.
+__global__ void __launch_bounds__(256)
+trunc_bootstrap_kernel(float *__restrict__ rew, int T, int64_t n, int slots, const int32_t *__restrict__ slot_step,
+                       const float *__restrict__ slot_values, float gamma)
+{
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    for (int s = 0; s < slots; s++) {
+        const int t = slot_step[(int64_t)s * n + i];
+        if (t < 0 || t >= T) continue;
+        float *r = rew + (int64_t)t * n + i;
+        *r = __fadd_rn(*r, __fmul_rn(gamma, slot_values[(int64_t)s * n + i]));
+    }
+}
+
 // PPO minibatch gradient (r6_ppo_grad).  A grid of ppo_ctas(B) CTAs (a function of B only, so the summation order and
 // the result do not depend on the device) walks tiles of 128 samples.  Each thread runs the forward pass, loss head
 // and deltas of its sample (r6_ppo.cuh) and stages its inputs, activations and deltas in shared memory unit-major,
@@ -1465,6 +1506,30 @@ int r6_gae(const float *rew, const float *values, const uint8_t *done, const flo
     gae_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rew, values, done, last_values, T, n, (float)gamma,
                                                                           (float)(gamma * gae_lambda), adv, ret);
     return check_launch("r6_gae");
+}
+
+int r6_trunc_record(const uint8_t *flags, const float *terminal_obs, int64_t n, int64_t first, int64_t count, int32_t step,
+                    int32_t slots, int32_t *slot_step, float *slot_obs, void *stream)
+{
+    if (!flags || !terminal_obs || !slot_step || !slot_obs) return fail(R6_EINVAL, "null pointer%s");
+    if (n < 0) return fail(R6_EINVAL, "n < 0%s");
+    if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
+    if (step < 0 || slots < 0) return fail(R6_EINVAL, "step and slots must be >= 0%s");
+    if (count == 0 || slots == 0) return R6_OK;
+    launch_pdl(trunc_record_kernel, (unsigned)((count + 255) / 256), 256, 0, (cudaStream_t)stream, flags, terminal_obs, n, first,
+               first + count, step, slots, slot_step, slot_obs);
+    return check_launch("r6_trunc_record");
+}
+
+int r6_trunc_bootstrap(float *rew, int32_t T, int64_t n, int32_t slots, const int32_t *slot_step, const float *slot_values,
+                       double gamma, void *stream)
+{
+    if (!rew || !slot_step || !slot_values) return fail(R6_EINVAL, "null pointer%s");
+    if (T < 0 || n < 0 || slots < 0) return fail(R6_EINVAL, "negative size%s");
+    if (T == 0 || n == 0 || slots == 0) return R6_OK;
+    trunc_bootstrap_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rew, T, n, slots, slot_step, slot_values,
+                                                                                       (float)gamma);
+    return check_launch("r6_trunc_bootstrap");
 }
 
 int r6_ppo_rollout_size(void) { return (int)sizeof(R6PpoRollout); }

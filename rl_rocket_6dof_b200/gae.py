@@ -3,8 +3,11 @@
 The consumer of the env step in the reference is SB3's PPO (`model.learn`, main_6DOF.py:136), whose
 `RolloutBuffer.compute_returns_and_advantage` runs on the host.  `compute_gae` is the same recurrence as one CUDA
 kernel over the `[T, N]` trajectory tensors the rollout kernel already wrote, so a training loop never has to
-leave the GPU.  (Bootstrapping of time-limit truncations with the critic, which SB3 does while collecting, stays
-with the caller: it needs the value network.)
+leave the GPU.  Bootstrapping of time-limit truncations with the critic, which SB3 does while collecting, happens
+before this scan: `Rocket6DOFBatch.collect_rollout(..., bootstrap_truncated=True)` files each truncation's terminal
+observation as it is stepped and adds gamma * V to its reward (`r6_trunc_record` / `r6_trunc_bootstrap`).  The fused
+`rollout(k, record=True)` keeps the env state in registers for all k steps and does not file them: there the
+bootstrapping is left to the caller.
 """
 from __future__ import annotations
 

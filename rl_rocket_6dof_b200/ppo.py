@@ -1,6 +1,8 @@
 """PPO training on the device: the update of stable-baselines3 1.6's `PPO.train` (the `model.learn` of main_6DOF.py:136)
 over rollouts collected by `Rocket6DOFBatch.collect_rollout`, with the loss gradient (`r6_ppo_grad`) and the Adam step
-(`r6_adam_step`) as CUDA kernels.  Nothing leaves the GPU during an update unless `target_kl` is set.
+(`r6_adam_step`) as CUDA kernels.  Nothing leaves the GPU during an update unless `target_kl` is set.  As SB3's
+`collect_rollouts` does, the collection bootstraps episodes cut by the TimeLimit with the critic
+(`collect_rollout(..., bootstrap_truncated=True)`), so the batch must auto-reset.
 
     params = ActorCriticParams.sb3_init(seed=0, device="cuda:0")
     trainer = PPOTrainer(batch, params, PPOConfig(), seed=0)
@@ -284,7 +286,7 @@ class PPOTrainer:
         while self.num_timesteps < total_timesteps:
             b.reset_stats()
             ro = b.collect_rollout(cfg.n_steps, self.params.mlp(), gamma=cfg.gamma, gae_lambda=cfg.gae_lambda,
-                                   tensor_cores=cfg.tensor_cores)
+                                   tensor_cores=cfg.tensor_cores, bootstrap_truncated=True)
             self.num_timesteps += cfg.n_steps * b.num_envs
             self.progress_remaining = 1.0 - self.num_timesteps / total_timesteps
             log = {"rollout/" + k: v for k, v in b.stats_dict().items()}
