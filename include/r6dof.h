@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 18
+#define R6_ABI_VERSION 19
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -287,6 +287,43 @@ int r6_policy_range(const R6Mlp *mlp, const float *obs, int64_t n, int64_t first
                     float *actions_raw, float *values, float *log_prob, void *stream);
 
 /*
+ * Generalised state-dependent exploration (stable-baselines3 1.6.0 `PPO(..., use_sde=True)`: StateDependentNoiseDistribution
+ * with full_std=True, use_expln=False, learn_features=False, epsilon=1e-6; the latent is the 64-unit trunk output h):
+ *     E_i = exp(log_std) * xi_i   (xi_i ~ N(0, 1) [64][3], one matrix per env, drawn by policy.reset_noise(n_envs))
+ *     raw = mean + h E_i,   std_a = sqrt(sum_k h_k^2 exp(2 log_std[k][a]) + 1e-6)
+ * log_prob and entropy are those of N(mean, std), summed over the 3 actions, with h detached.
+ */
+#define R6_SDE_LATENT 64
+#define R6_SDE_NXI 192        /* xi components per env: [64][3], component c = 3 k + a */
+typedef struct R6Sde {
+    const float *log_std;     /* [64][3] */
+    const float *xi;          /* [192][n] component-major standard normals (r6_sde_noise); nullable for r6_ppo_grad_sde */
+} R6Sde;
+int r6_sde_size(void);
+
+/*
+ * StateDependentNoiseDistribution.sample_weights / policy.reset_noise(n_envs) for the envs [first, first + count) of a
+ * batch of n: xi[c][i] for the 192 components, standard normals from Philox4x32-10 keyed (seed, env_offset + i,
+ * step_index) through Box-Muller.  The result depends on the global env id and the draw step only, not on the shard, lane
+ * or sub-range that draws it.  The exploration matrix is E = exp(log_std) * xi, formed by the policy kernel with the
+ * current log_std (log_std does not change during a collection, so that is SB3's draw-time product).
+ */
+int r6_sde_noise(int64_t n, int64_t first, int64_t count, uint64_t seed, int64_t env_offset, int64_t step_index, float *xi,
+                 void *stream);
+
+/*
+ * r6_policy_range with the gSDE head (SB3 ActorCriticPolicy.forward with use_sde=True): mean and value as
+ * r6_policy_range; stochastic != 0: actions_raw = mean + h (exp(log_std) * xi) with the env's xi column; log_prob of
+ * actions_raw under N(mean, std) above; stochastic == 0: the mean and its log_prob.  mlp->log_std is not read.  Deterministic
+ * actions and the values are bit-identical to r6_policy_range's.  tensor_cores = 0 (float32 FMAs), 2 or 3 (tcgen05,
+ * the h E and h^2 sigma^2 sums formed in the layer-1 epilogue from the TF32 hi + lo parts); 1 (mma.sync) is not
+ * available for gSDE (R6_EINVAL).
+ */
+int r6_policy_sde_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, int64_t n, int64_t first, int64_t count,
+                        int32_t tensor_cores, int32_t stochastic, float *actions, float *actions_raw, float *values,
+                        float *log_prob, void *stream);
+
+/*
  * Generalised advantage estimation over a recorded rollout, on the device, so that the PPO update of
  * main_6DOF.py:136 (`model.learn`) can consume r6_rollout's trajectory buffers without a host round trip.
  * Restates stable-baselines3 1.6.0 `RolloutBuffer.compute_returns_and_advantage` (common/buffers.py; SB3 is a
@@ -383,11 +420,27 @@ int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *id
                 float *grad_sum, double *terms, void *work, void *stream);
 
 /*
+ * r6_ppo_grad for a gSDE policy (PPO(use_sde=True).train; SB3 1.6 also calls reset_noise(batch_size) per minibatch, which
+ * does not enter the loss).  Flat layout R6_PPO_NPARAMS_SDE: the prefix of R6_PPO_NPARAMS through bv, then
+ * log_std [64][3] @10308.  Per sample, std_a, log_prob and entropy of N(mean, std) as r6_policy_sde_range; the entropy
+ * bonus uses that per-sample entropy, and
+ *     d loss / d log_std[k][a] = exp(2 log_std[k][a]) sum_s h_{s,k}^2 (w_s (z_{s,a}^2 - 1) - ent_coef) / std_a(s)^2,
+ * w = d pg / d logp, z = (a - mean) / std.  terms [R6_PPO_NTERMS_SDE]: those of r6_ppo_grad plus the sum of the per-sample
+ * entropies (R6_PPO_T_ENTROPY).  sde->log_std is the [64][3] matrix (sde->xi is not read; mlp->log_std is not read).
+ */
+#define R6_PPO_NPARAMS_SDE 10500
+#define R6_PPO_NTERMS_SDE 6
+#define R6_PPO_T_ENTROPY 5
+int64_t r6_ppo_sde_work_bytes(int64_t B);
+int r6_ppo_grad_sde(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
+                    const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream);
+
+/*
  * One torch.optim.Adam step (no weight decay, no amsgrad) on the flat parameters, after clip_grad_norm_:
  *     g = scale * grad_sum;  norm = ||g||_2 (accumulated in float64);  g *= min(1, max_grad_norm / (norm + 1e-6));
  *     m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g^2;
  *     p -= lr / (1 - beta1^step) * m / (sqrt(v) / sqrt(1 - beta2^step) + eps)
- * params, grad_sum, m, v: float32 [P] DEVICE; step >= 1 counts the updates including this one; grad_norm_out
+ * params, grad_sum, m, v: float32 [P] DEVICE (any P: R6_PPO_NPARAMS, R6_PPO_NPARAMS_SDE); step >= 1 counts the updates including this one; grad_norm_out
  * (nullable DEVICE double) receives the norm before clipping.
  */
 int r6_adam_step(float *params, const float *grad_sum, float *m, float *v, int64_t P, const R6AdamCoef *coef,

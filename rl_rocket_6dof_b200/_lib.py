@@ -12,7 +12,7 @@ from .params import R6Params
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libr6dof.so")
-ABI_VERSION = 18
+ABI_VERSION = 19
 
 u8p = C.c_void_p
 
@@ -56,8 +56,15 @@ class R6AdamCoef(C.Structure):
                 ("max_grad_norm", C.c_double), ("scale", C.c_double)]
 
 
+class R6Sde(C.Structure):
+    _fields_ = [("log_std", C.c_void_p), ("xi", C.c_void_p)]     # gSDE log_std [64][3], noise [192][n]
+
+
 PPO_NPARAMS = 10311
 PPO_NTERMS = 5
+PPO_NPARAMS_SDE = 10500
+PPO_NTERMS_SDE = 6
+SDE_NXI = 192
 
 
 def make_mlp(weights: dict) -> "R6Mlp":
@@ -67,14 +74,18 @@ def make_mlp(weights: dict) -> "R6Mlp":
             return None
         return x.data_ptr() if hasattr(x, "data_ptr") else x.ctypes.data
     m = R6Mlp(*[ptr(weights[k]) for k in ("w0", "b0", "w1", "b1", "w2", "b2")])
-    m.wv, m.bv, m.log_std = ptr(weights.get("wv")), ptr(weights.get("bv")), ptr(weights.get("log_std"))
+    ls = weights.get("log_std")
+    if ls is not None and len(ls.shape) == 2:          # gSDE [64, 3]: passed through R6Sde, never as the Gaussian [3]
+        ls = None
+    m.wv, m.bv, m.log_std = ptr(weights.get("wv")), ptr(weights.get("bv")), ptr(ls)
     return m
 
 
 EXPORTS = ["r6_abi_version", "r6_last_error", "r6_params_size", "r6_buffers_size", "r6_reset", "r6_step",
            "r6_rollout", "r6_sim_step_raw", "r6_tgo", "r6_stats_reset", "r6_peak_fma", "r6_gae", "r6_policy", "r6_policy_ex", "r6_step_random", "r6_step_range", "r6_policy_range", "r6_work_bytes",
            "r6_ppo_rollout_size", "r6_ppo_coef_size", "r6_adam_coef_size", "r6_ppo_work_bytes", "r6_ppo_grad", "r6_adam_step",
-           "r6_trunc_record", "r6_trunc_bootstrap"]
+           "r6_trunc_record", "r6_trunc_bootstrap", "r6_sde_size", "r6_sde_noise", "r6_policy_sde_range",
+           "r6_ppo_sde_work_bytes", "r6_ppo_grad_sde"]
 
 
 class R6Error(RuntimeError):
@@ -108,7 +119,8 @@ def load(path: str | None = None):
         raise R6Error(f"R6Params layout mismatch: C {L.r6_params_size()} vs ctypes {C.sizeof(R6Params)}")
     if L.r6_buffers_size() != C.sizeof(R6Buffers):
         raise R6Error(f"R6Buffers layout mismatch: C {L.r6_buffers_size()} vs ctypes {C.sizeof(R6Buffers)}")
-    for name, st in (("r6_ppo_rollout_size", R6PpoRollout), ("r6_ppo_coef_size", R6PpoCoef), ("r6_adam_coef_size", R6AdamCoef)):
+    for name, st in (("r6_ppo_rollout_size", R6PpoRollout), ("r6_ppo_coef_size", R6PpoCoef), ("r6_adam_coef_size", R6AdamCoef),
+                     ("r6_sde_size", R6Sde)):
         if getattr(L, name)() != C.sizeof(st):
             raise R6Error(f"{st.__name__} layout mismatch: C {getattr(L, name)()} vs ctypes {C.sizeof(st)}")
     pp, bp = C.POINTER(R6Params), C.POINTER(R6Buffers)
@@ -142,6 +154,13 @@ def load(path: str | None = None):
                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.r6_adam_step.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(R6AdamCoef), C.c_int64,
                                C.c_void_p, C.c_void_p]
+    L.r6_sde_noise.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]
+    L.r6_policy_sde_range.argtypes = [C.POINTER(R6Mlp), C.POINTER(R6Sde), C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32,
+                                      C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_ppo_sde_work_bytes.argtypes = [C.c_int64]
+    L.r6_ppo_sde_work_bytes.restype = C.c_int64
+    L.r6_ppo_grad_sde.argtypes = [C.POINTER(R6Mlp), C.POINTER(R6Sde), C.POINTER(R6PpoRollout), C.c_void_p, C.c_int64,
+                                  C.POINTER(R6PpoCoef), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.r6_peak_fma.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
     _lib = L
     return L

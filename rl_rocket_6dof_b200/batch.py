@@ -124,6 +124,10 @@ class Rocket6DOFBatch:
                 self.ic_table = torch.from_numpy(np.ascontiguousarray(ic_table, np.float32).reshape(-1, 14)).to(dev)
         self._b = self._make_buffers()
         self.steps_done = 0          # global step counter (Philox action stream)
+        # gSDE noise xi [192, N] (r6_sde_noise), allocated by the first reset_noise: 768 B per env, 805 MB at 2^20 envs.
+        # Redrawing xi inside the policy kernel instead would save that memory but roughly double the kernel's XU work
+        # against ~0.1 ms of HBM reads per 2^20-env step (both estimates, not measured).
+        self.sde_xi = None
 
     # ------------------------------------------------------------------ plumbing
     def _make_buffers(self) -> R6Buffers:
@@ -191,12 +195,44 @@ class Rocket6DOFBatch:
         _lib.check(rc, L)
 
     def _policy(self, m: R6Mlp, obs: int, first: int, count: int, tensor_cores, stochastic: bool, step_index: int,
-                act: int, raw: Optional[int], val: Optional[int], logp: Optional[int], stream: torch.cuda.Stream):
+                act: int, raw: Optional[int], val: Optional[int], logp: Optional[int], stream: torch.cuda.Stream,
+                sde: Optional[_lib.R6Sde] = None):
         """The policy network over envs [first, first + count) of the component-major observations at device pointer
-        `obs` (r6_policy_range); the output pointers raw / val / logp may be None (not written)."""
+        `obs` (r6_policy_range, or r6_policy_sde_range with gSDE inputs `sde`); the output pointers raw / val / logp may be
+        None (not written)."""
+        if sde is not None:
+            _lib.check(self.lib.r6_policy_sde_range(C.byref(m), C.byref(sde), obs, self.num_envs, first, count, int(tensor_cores),
+                                                    int(bool(stochastic)), act, raw, val, logp, stream.cuda_stream), self.lib)
+            return
         _lib.check(self.lib.r6_policy_range(C.byref(m), obs, self.num_envs, first, count, int(tensor_cores),
                                             int(bool(stochastic)), self.seed_value, self.env_offset, step_index, act, raw,
                                             val, logp, stream.cuda_stream), self.lib)
+
+    def _sde(self, mlp: dict) -> Optional[_lib.R6Sde]:
+        """The gSDE inputs when `mlp` carries a [64, 3] log_std (drawing the noise first if none was drawn), else None."""
+        ls = mlp.get("log_std")
+        if ls is None or ls.dim() != 2:
+            return None
+        if tuple(ls.shape) != (64, 3) or ls.dtype != torch.float32 or not ls.is_contiguous():
+            raise ValueError("a gSDE log_std must be a contiguous float32 [64, 3] tensor")
+        if self.sde_xi is None:
+            self.reset_noise()
+        return _lib.R6Sde(ls.data_ptr(), self.sde_xi.data_ptr())
+
+    def _noise(self, first: int, count: int, step_index: int, stream: torch.cuda.Stream):
+        _lib.check(self.lib.r6_sde_noise(self.num_envs, first, count, self.seed_value, self.env_offset, int(step_index),
+                                         self.sde_xi.data_ptr(), stream.cuda_stream), self.lib)
+
+    def reset_noise(self, step_index: Optional[int] = None):
+        """SB3's `policy.reset_noise(n_envs)` for a gSDE policy: draws a new standard-normal xi [64, 3] for every env,
+        keyed by (seed, global env id, step_index; default `steps_done`).  The exploration matrix is exp(log_std) * xi,
+        formed by the policy kernel with the log_std it is given."""
+        self.join()
+        with torch.cuda.device(self.device):
+            if self.sde_xi is None:
+                self.sde_xi = torch.empty(_lib.SDE_NXI, self.num_envs, dtype=torch.float32, device=self.device)
+            self._noise(0, self.num_envs, self.steps_done if step_index is None else step_index,
+                        torch.cuda.current_stream(self.device))
 
     def join(self):
         """Orders everything the lanes have been given before whatever the caller's current stream does next.  A no-op
@@ -314,7 +350,8 @@ class Rocket6DOFBatch:
         """SB3 `ActorCriticPolicy.forward` for the current observations in one launch: returns
         (env_actions [N,3] clipped, raw_actions [N,3], values [N], log_prob [N]).  `mlp` may carry the critic head
         ("wv", "bv") and the Gaussian "log_std"; stochastic=True samples mean + exp(log_std) eps with Philox noise
-        keyed by (seed, global env id, step_index) — reproducible and independent of the shard count."""
+        keyed by (seed, global env id, step_index) — reproducible and independent of the shard count.  A [64, 3]
+        log_std selects gSDE: mean + h (exp(log_std) * xi) with the noise of the last `reset_noise` (step_index unused)."""
         self.join()
         n, dev = self.num_envs, self.device
         if out is not None:                      # (act, raw, val, logp) contiguous float32 CUDA tensors to write into
@@ -327,11 +364,12 @@ class Rocket6DOFBatch:
         step = self.steps_done if step_index is None else int(step_index)
         with torch.cuda.device(dev):
             self._policy(_lib.make_mlp(mlp), self.obs.data_ptr(), 0, n, tensor_cores, stochastic, step, act.data_ptr(),
-                         raw.data_ptr(), val.data_ptr(), logp.data_ptr(), torch.cuda.current_stream(dev))
+                         raw.data_ptr(), val.data_ptr(), logp.data_ptr(), torch.cuda.current_stream(dev), self._sde(mlp))
         return act, raw, val, logp
 
     def collect_rollout(self, k: int, mlp: dict, *, gamma: float = 0.99, gae_lambda: float = 0.95,
-                        stochastic: bool = True, tensor_cores=3, bootstrap_truncated: bool = False) -> dict:
+                        stochastic: bool = True, tensor_cores=3, bootstrap_truncated: bool = False,
+                        sde_sample_freq: int = -1) -> dict:
         """What SB3's `PPO.collect_rollouts` + `RolloutBuffer.compute_returns_and_advantage` produce for k steps of
         this VecEnv, entirely on the device: per step one policy launch (action, value, log-prob; by default the
         faithful tcgen05 3xTF32 kernel, tensor_cores=3) and one env step, then the GAE scan.  Returns tensors shaped
@@ -343,6 +381,10 @@ class Rocket6DOFBatch:
         step (`r6_trunc_record`), the critic runs once per slot layer after the rollout and `r6_trunc_bootstrap` adds the
         values, all without a host synchronise.  Needs auto-reset (ValueError otherwise).  The default False leaves the
         rewards as the env returned them.
+
+        A [64, 3] log_std in `mlp` collects with gSDE, as SB3's collect_rollouts with use_sde=True: `reset_noise` at the
+        start of the rollout, and with sde_sample_freq > 0 every lane redraws the noise of its env range before step j
+        whenever j % sde_sample_freq == 0, keyed by steps_done + j (step 0 reuses the start draw, which has that key).
 
         The trajectory is written in place: the env step of step j writes its observations straight into slice j + 1 of
         a component-major buffer [k + 1, 14, N] (the layout the kernels read and write), its reward and done flags into
@@ -370,6 +412,9 @@ class Rocket6DOFBatch:
         dones = torch.empty(k, n, dtype=torch.uint8, device=dev)
         a_env = torch.empty(n, 3, dtype=torch.float32, device=dev)
         m = _lib.make_mlp(mlp)
+        sde = self._sde(mlp)
+        if sde is not None:
+            self.reset_noise()
         # Without auto-reset a finished env is frozen: the step reads its done flag and writes NOTHING for it, so its
         # obs / reward / done must carry over from the previous step — that mode keeps the per-step copies.
         in_place = bool(self.auto_reset)
@@ -385,8 +430,10 @@ class Rocket6DOFBatch:
                         if not in_place and j > 0:
                             with torch.cuda.stream(st):
                                 obs_cm[j, :, first:first + count] = self.obs[:, first:first + count]
+                        if sde is not None and sde_sample_freq > 0 and j > 0 and j % sde_sample_freq == 0:
+                            self._noise(first, count, self.steps_done + j, st)
                         self._policy(m, obs_cm[j].data_ptr(), first, count, tensor_cores, stochastic, self.steps_done + j,
-                                     a_env.data_ptr(), acts[j].data_ptr(), vals[j].data_ptr(), logp[j].data_ptr(), st)
+                                     a_env.data_ptr(), acts[j].data_ptr(), vals[j].data_ptr(), logp[j].data_ptr(), st, sde)
                         self._env_step(ln, first, count, a_env.data_ptr(), self.steps_done + j, st)
                         if slots:
                             _lib.check(self.lib.r6_trunc_record(self.flags.data_ptr(), self.terminal_obs.data_ptr(), n, first,

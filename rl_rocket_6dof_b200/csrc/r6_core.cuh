@@ -1535,8 +1535,10 @@ R6_HD float mlp_pack_element(const R6Mlp &m, int idx)
     return mlp_b2_row(m, idx - kMlpOffB2);
 }
 
-// raw outputs: out[0..2] = Gaussian mean (unclipped), out[3] = value
-R6_HD void mlp_forward(const float *W, const float *x, float (&out)[4])
+// raw outputs: out[0..2] = Gaussian mean (unclipped), out[3] = value.  latent(k, h) is called with every unit h of
+// the last hidden layer (the gSDE head reads it; the plain forward passes a no-op).
+template <class Latent>
+R6_HD void mlp_forward_latent(const float *W, const float *x, float (&out)[4], Latent &&latent)
 {
     float acc[kMlpH1];
 #pragma unroll
@@ -1562,6 +1564,7 @@ R6_HD void mlp_forward(const float *W, const float *x, float (&out)[4])
 #pragma unroll
     for (int k = 0; k < kMlpH1; k++) {
         const float h = tanhf(acc[k] + W[kMlpOffB1 + k]);
+        latent(k, h);
         o0 = f32_fma(W[kMlpOffW2 + k], h, o0);
         o1 = f32_fma(W[kMlpOffW2 + kMlpH1 + k], h, o1);
         o2 = f32_fma(W[kMlpOffW2 + 2 * kMlpH1 + k], h, o2);
@@ -1571,6 +1574,10 @@ R6_HD void mlp_forward(const float *W, const float *x, float (&out)[4])
     out[1] = o1 + W[kMlpOffB2 + 1];
     out[2] = o2 + W[kMlpOffB2 + 2];
     out[3] = o3 + W[kMlpOffB2 + 3];
+}
+R6_HD void mlp_forward(const float *W, const float *x, float (&out)[4])
+{
+    mlp_forward_latent(W, x, out, [](int, float) {});
 }
 // deterministic action of evaluate_policy / predict: the mean clipped to the action space
 R6_HD void mlp_policy(const float *W, const float *x, float &a0, float &a1, float &a2)
@@ -1635,7 +1642,47 @@ R6_HD void gaussian_head(const float (&mean)[4], const float *log_std, bool stoc
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Generalised state-dependent exploration (SB3 1.6 StateDependentNoiseDistribution, full_std, no expln, latent_sde =
+// the 64-unit trunk output h, detached) [memory]:
+//     E_i = sigma (.) xi_i,  sigma = exp(log_std) [64][3],  xi_i ~ N(0, 1) drawn per env by reset_noise
+//     raw = mean + h E_i,    std_a = sqrt(sum_k h_k^2 sigma_ka^2 + 1e-6),   log_prob / entropy of N(mean, std)
+// xi is a component-major [192][n] buffer, component c = 3 k + a (SB3's [64][3] order).  Component block b (c = 4b ..
+// 4b + 3) of an env is one Philox block keyed (seed, global env id, draw step), so the buffer does not depend on the
+// shard, lane or sub-range that drew it; Box-Muller with the accurate logf / sincospif of gaussian_head (see there).
+constexpr int kSdeLatent = 64, kSdeXi = kSdeLatent * kMlpOut, kSdeBlocks = kSdeXi / 4;
+constexpr uint32_t kStreamSde = 0x47534445u;      // 'GSDE' ^ (step hi << 8) ^ block
+R6_HD void sde_noise_block(uint64_t seed, uint64_t genv, uint64_t step, int b, float (&z)[4])
+{
+    U4 ctr = {(uint32_t)genv, (uint32_t)(genv >> 32), (uint32_t)step, kStreamSde ^ ((uint32_t)(step >> 32) << 8) ^ (uint32_t)b};
+    const U4 r = philox4x32_10(ctr, (uint32_t)seed, (uint32_t)(seed >> 32));
+    const float s = 1.0f / 4294967296.0f;
+    const float u1 = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)r.y * s;
+    const float u3 = ((float)(r.z >> 8) + 0.5f) * (1.0f / 16777216.0f), u4 = (float)r.w * s;
+    const float ra = sqrtf(-2.0f * logf(u1)), rb = sqrtf(-2.0f * logf(u3));
+    float sn, cs;
+    sincospi_f32(2.0f * u2, sn, cs);
+    z[0] = ra * cs;
+    z[1] = ra * sn;
+    sincospi_f32(2.0f * u4, sn, cs);
+    z[2] = rb * cs;
+    z[3] = rb * sn;
+}
 
+// The gSDE policy head of one env from the partial sums of the latent: nz[a] = sum_k h_k E_ka (the noise),
+// var[a] = sum_k h_k^2 sigma_ka^2.  stochastic: raw = mean + nz, else the mean; logp of raw under N(mean, std).
+R6_HD void sde_head(const float (&mean)[4], const float (&nz)[3], const float (&var)[3], bool stochastic, float (&raw)[3],
+                    float &logp)
+{
+    logp = 0.0f;
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+        const float v = var[a] + 1e-6f;                   // std^2 (SB3: sqrt(variance + epsilon), squared back by Normal)
+        raw[a] = stochastic ? mean[a] + nz[a] : mean[a];
+        const float d = raw[a] - mean[a];
+        logp += -(d * d) / (2.0f * v) - logf(sqrtf(v)) - 0.9189385332046727f;
+    }
+}
 
 // ------------------------------------------------------------------------------------------------
 // Registers carried by the thread that owns an environment, and the glue of one env step

@@ -694,17 +694,55 @@ struct PolicyOut {
     int64_t env_offset, step;
     int64_t i0, i1;                           // env sub-range of this launch (r6_policy_range); n stays the obs stride
 };
-__device__ __forceinline__ void policy_epilogue(const PolicyOut &po, const float *log_std, int64_t i, const float (&out)[4])
+__device__ __forceinline__ void policy_store(const PolicyOut &po, int64_t i, const float (&raw)[3], float logp, float value)
 {
-    float raw[3], logp;
-    gaussian_head(out, log_std, po.stochastic != 0, po.seed, (uint64_t)(po.env_offset + i), (uint64_t)po.step, raw, logp);
 #pragma unroll
     for (int c = 0; c < 3; c++) {
         po.actions[3 * i + c] = fminf(fmaxf(raw[c], -1.0f), 1.0f);
         if (po.raw) po.raw[3 * i + c] = raw[c];
     }
-    if (po.values) po.values[i] = out[3];
+    if (po.values) po.values[i] = value;
     if (po.logp) po.logp[i] = logp;
+}
+__device__ __forceinline__ void policy_epilogue(const PolicyOut &po, const float *log_std, int64_t i, const float (&out)[4])
+{
+    float raw[3], logp;
+    gaussian_head(out, log_std, po.stochastic != 0, po.seed, (uint64_t)(po.env_offset + i), (uint64_t)po.step, raw, logp);
+    policy_store(po, i, raw, logp, out[3]);
+}
+// the gSDE head from the latent sums nz (h E) and var (h^2 sigma^2) of env i
+__device__ __forceinline__ void sde_epilogue(const PolicyOut &po, int64_t i, const float (&out)[4], const float (&nz)[3],
+                                             const float (&var)[3])
+{
+    float raw[3], logp;
+    sde_head(out, nz, var, po.stochastic != 0, raw, logp);
+    policy_store(po, i, raw, logp, out[3]);
+}
+// gSDE inputs of a policy launch: log_std [64][3] and the xi [192][n] buffer of r6_sde_noise
+struct SdeIn {
+    const float *log_std, *xi;
+};
+// sigma = exp(log_std) and sigma^2 (one float32 product, as SB3's std ** 2) into shared memory
+__device__ __forceinline__ void sde_stage(const float *log_std, float *sig, float *sig2, int tid, int nthreads)
+{
+    for (int c = tid; c < kSdeXi; c += nthreads) {
+        const float sg = expf(log_std[c]);
+        sig[c] = sg;
+        sig2[c] = sg * sg;
+    }
+}
+
+// StateDependentNoiseDistribution.sample_weights (r6_sde_noise): one thread per (env, Philox block); blockIdx.y = block
+__global__ void __launch_bounds__(256)
+sde_noise_kernel(uint64_t seed, int64_t env_offset, int64_t step, int64_t n, int64_t i0, int64_t i1, float *__restrict__ xi)
+{
+    const int64_t i = i0 + (int64_t)blockIdx.x * 256 + threadIdx.x;
+    const int b = blockIdx.y;
+    if (i >= i1) return;
+    float z[4];
+    sde_noise_block(seed, (uint64_t)(env_offset + i), (uint64_t)step, b, z);
+#pragma unroll
+    for (int q = 0; q < 4; q++) xi[(int64_t)(4 * b + q) * n + i] = z[q];
 }
 
 // The policy as its own kernel (r6_policy / r6_policy_ex): uniform work, no integrator state => small code, high
@@ -733,6 +771,39 @@ policy_kernel(const R6Mlp mlp, const float *__restrict__ obs, int64_t n, const P
 }
 constexpr int kSmemPolicyTc = (r6::kMlpTcFloats + (kThreads / 32) * 16 * 33) * (int)sizeof(float);
 constexpr int kSmemPolicy = r6::kMlpFloats * (int)sizeof(float);
+
+// The policy with the gSDE head on float32 FMAs (r6_policy_sde_range tensor_cores = 0): policy_kernel<false> plus, per
+// unit k of the last hidden layer, nz_a += h_k (sigma_ka xi_ka) and var_a += h_k^2 sigma_ka^2 (xi read coalesced over envs)
+__global__ void __launch_bounds__(kThreads, 4)
+policy_sde_kernel(const R6Mlp mlp, const SdeIn sde, const float *__restrict__ obs, int64_t n, const PolicyOut po)
+{
+    extern __shared__ __align__(16) double r6_smem[];
+    float *Ws = reinterpret_cast<float *>(r6_smem);
+    float *sig = Ws + kMlpFloats, *sig2 = sig + kSdeXi;
+    for (int idx = threadIdx.x; idx < kMlpFloats; idx += kThreads) Ws[idx] = mlp_pack_element(mlp, idx);
+    sde_stage(sde.log_std, sig, sig2, threadIdx.x, kThreads);
+    __syncthreads();
+    const int64_t i1 = po.i1;
+    const int64_t tiles = (i1 - po.i0 + kThreads - 1) / kThreads;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        const int64_t i = po.i0 + tile * kThreads + threadIdx.x;
+        const bool in = i < i1, draw = in && po.stochastic != 0;
+        float x[kMlpIn], out[4], nz[3] = {0.0f, 0.0f, 0.0f}, var[3] = {0.0f, 0.0f, 0.0f};
+#pragma unroll
+        for (int c = 0; c < kMlpIn; c++) x[c] = in ? obs[(int64_t)c * n + i] : 0.0f;
+        mlp_forward_latent(Ws, x, out, [&](int k, float h) {
+            const float hh = h * h;
+#pragma unroll
+            for (int a = 0; a < 3; a++) {
+                const int c = 3 * k + a;
+                if (draw) nz[a] = f32_fma(h, sig[c] * __ldg(sde.xi + (int64_t)c * n + i), nz[a]);
+                var[a] = f32_fma(hh, sig2[c], var[a]);
+            }
+        });
+        if (in) sde_epilogue(po, i, out, nz, var);
+    }
+}
+constexpr int kSmemPolicySde = kSmemPolicy + 2 * kSdeXi * (int)sizeof(float);
 
 // The policy on tcgen05 with accumulators and activations in tensor memory (r6_policy tensor_cores = 3: 3xTF32, float32
 // accuracy; tensor_cores = 2: single-pass TF32).  Layout, schedule and measurements: r6_mlp_tcgen05.cuh.
@@ -872,6 +943,160 @@ policy_tc5_kernel(const R6Mlp mlp, const float *__restrict__ obs, int64_t n, con
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
 }
 
+// policy_tc5_kernel with the gSDE head (r6_policy_sde_range tensor_cores = 2 / 3): the sums h E and h^2 sigma^2 are
+// formed in the last hidden layer's epilogue (epilogue_in_tmem_sde), where each of the two threads of an env row holds
+// 32 of the 64 activations; the second half hands its sums to the first through shared memory (kOffSdePart), and the
+// first writes the env's outputs.  A copy of policy_tc5_kernel rather than a template flag of it, so that the plain
+// kernel keeps its register allocation.
+template <bool kFaithful>
+__global__ void __launch_bounds__(tc5::kThreads, 1)
+policy_tc5_sde_kernel(const R6Mlp mlp, const SdeIn sde, const float *__restrict__ obs, int64_t n, const PolicyOut po)
+{
+    using namespace tc5;
+    extern __shared__ __align__(16) double r6_smem[];
+    char *S = reinterpret_cast<char *>(r6_smem);
+    const int tid = threadIdx.x, group = tid >> 8, lt = tid & 127, half = (tid >> 7) & 1, warp = tid >> 5;
+    // programmatic dependent launch: the previous kernel on the stream may have produced the observations — or the weights
+    // (an optimiser step), so the wait comes before the weight staging, not after it
+    grid_dependency_wait();
+    // ---- one-time per CTA: weights split into TF32 hi / lo parts in canonical K-major tiles, biases, barriers, TMEM ----
+    for (int idx = tid; idx < 128 * 16; idx += tc5::kThreads) {
+        const int r = idx >> 4, k = idx & 15;
+        float hi, lo;
+        split_tf32(k < kMlpIn ? mlp.w0[r * kMlpIn + k] : 0.0f, hi, lo);
+        *reinterpret_cast<float *>(S + kOffW0h + tile_off(r, k, 16)) = hi;
+        *reinterpret_cast<float *>(S + kOffW0l + tile_off(r, k, 16)) = lo;
+    }
+    // W1 / W2 rows are 16-byte aligned runs of 4 consecutive k = one 16-byte chunk of the canonical tile: vector copies
+    // (the staging is a fixed cost per CTA and launch: 11 264 weights)
+    for (int idx = tid; idx < 64 * 32; idx += tc5::kThreads) {
+        const int r = idx >> 5, k = (idx & 31) * 4;
+        const float4 w = *reinterpret_cast<const float4 *>(mlp.w1 + r * kMlpH0 + k);
+        float4 h, l;
+        split_tf32(w.x, h.x, l.x); split_tf32(w.y, h.y, l.y); split_tf32(w.z, h.z, l.z); split_tf32(w.w, h.w, l.w);
+        *reinterpret_cast<float4 *>(S + kOffW1h + tile_off(r, k, 128)) = h;
+        *reinterpret_cast<float4 *>(S + kOffW1l + tile_off(r, k, 128)) = l;
+    }
+    for (int idx = tid; idx < 16 * 16; idx += tc5::kThreads) {
+        const int r = idx >> 4, k = (idx & 15) * 4;
+        float4 h, l;
+        split_tf32(r < kMlpRows ? mlp_w2_row(mlp, r, k) : 0.0f, h.x, l.x);
+        split_tf32(r < kMlpRows ? mlp_w2_row(mlp, r, k + 1) : 0.0f, h.y, l.y);
+        split_tf32(r < kMlpRows ? mlp_w2_row(mlp, r, k + 2) : 0.0f, h.z, l.z);
+        split_tf32(r < kMlpRows ? mlp_w2_row(mlp, r, k + 3) : 0.0f, h.w, l.w);
+        *reinterpret_cast<float4 *>(S + kOffW2h + tile_off(r, k, 64)) = h;
+        *reinterpret_cast<float4 *>(S + kOffW2l + tile_off(r, k, 64)) = l;
+    }
+    float *bias = reinterpret_cast<float *>(S + kOffBias);
+    const float bscale = kFaithful ? kTwoLog2e : 1.0f;      // faithful mode: hidden-layer biases pre-scaled for the exp2 form of tanh
+    if (tid < 128) bias[tid] = bscale * mlp.b0[tid];
+    if (tid < 64) bias[128 + tid] = bscale * mlp.b1[tid];
+    if (tid < 4) bias[192 + tid] = mlp_b2_row(mlp, tid);
+    sde_stage(sde.log_std, reinterpret_cast<float *>(S + kOffSde), reinterpret_cast<float *>(S + kOffSde) + kSdeXi, tid,
+              tc5::kThreads);
+    if (tid == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(S + kOffBar)) : "memory");
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(S + kOffBar + 8)) : "memory");
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(S + kOffTmemPtr)), "n"(kTmemCols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    fence_async_smem();                      // the weight tiles are read by the async proxy (B operand of the MMAs)
+    fence_before();
+    __syncthreads();
+    fence_after();
+    // warp-uniform copies (a shuffle result is uniform to the compiler) of everything the MMA-issuing warp computes with
+    const int warp_u = __shfl_sync(0xffffffffu, warp, 0);
+    const uint32_t tmem_base = __shfl_sync(0xffffffffu, *reinterpret_cast<volatile uint32_t *>(S + kOffTmemPtr), 0);
+    const uint32_t tmem_g = tmem_base + (uint32_t)(warp_u >> 3) * kGroupCols;              // this group's columns, lane 0
+    const uint32_t tmem_row = tmem_g + ((uint32_t)((warp & 3) * 32) << 16);                // this warp's 32 TMEM lanes
+    const uint32_t sbase = __shfl_sync(0xffffffffu, smem_u32(S), 0);
+    const uint32_t aW0h = sbase + kOffW0h, aW0l = sbase + kOffW0l, aW1h = sbase + kOffW1h;
+    const uint32_t aW1l = sbase + kOffW1l, aW2h = sbase + kOffW2h, aW2l = sbase + kOffW2l;
+    const uint32_t bar = sbase + kOffBar + 8 * (uint32_t)(warp_u >> 3);
+    const bool issuer = (warp_u & 7) == 0;          // the first warp of each group issues its MMAs (one elected lane each)
+    uint32_t phase = 0;
+    const int64_t i1 = po.i1;
+    const int64_t tiles = (i1 - po.i0 + kTile - 1) / kTile;
+    // Both groups run the SAME number of tile slots (a slot past the end is all masked rows) so that the epilogue token
+    // is handed over a matching number of times.
+    const int64_t slots = (tiles + 2 * (int64_t)gridDim.x - 1) / (2 * (int64_t)gridDim.x);
+    // this thread's 8 observation components of one tile, as loaded (split and stored one slot later)
+    float xo[8];
+    auto load_obs = [&](int64_t tile) {
+        const int64_t i = po.i0 + tile * kTile + lt;
+#pragma unroll
+        for (int q = 0; q < 8; q++) {
+            const int k = 8 * half + q;
+            xo[q] = (k < kMlpIn && i < i1) ? __ldg(obs + (int64_t)k * n + i) : 0.0f;
+        }
+    };
+    load_obs(2 * (int64_t)blockIdx.x + group);
+    float outv[4] = {0.0f, 0.0f, 0.0f, 0.0f};      // the output layer of the previous tile, written out one slot later
+    float nzv[3] = {0.0f, 0.0f, 0.0f}, varv[3] = {0.0f, 0.0f, 0.0f};   // and its latent sums
+    int64_t out_i = i1;
+    if (group == 1) token_pass(0);                 // group 0 takes the first epilogue turn
+    for (int64_t slot = 0; slot < slots; slot++) {
+        const int64_t tile = 2 * ((int64_t)blockIdx.x + slot * gridDim.x) + group;
+        const int64_t i = po.i0 + tile * kTile + lt;
+        // ---- observations of this thread's env, split -> row `lt` of the input tile: 8 of its 16 K columns per thread ----
+        {
+            float h[8], l[8];
+#pragma unroll
+            for (int q = 0; q < 8; q++) split_tf32(xo[q], h[q], l[q]);
+            tmem_st8(tmem_row + kColD1 + 8 * half, h);
+            if (kFaithful) tmem_st8(tmem_row + kColL + 8 * half, l);
+            tmem_st_wait();
+        }
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD0, tmem_g + kColD1, tmem_g + kColL, aW0h, aW0l, 512, 2, 128, false); if (elect_one()) mma_commit(bar); }
+        load_obs(tile + 2 * (int64_t)gridDim.x);       // next slot's observations: in flight under this tile's three layers
+        if (half == 0 && out_i < i1) sde_epilogue(po, out_i, outv, nzv, varv);        // the previous tile's outputs, under MMA0
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- hidden layer 0, first half of the units -> layer 1 partial product ----
+        epilogue_in_tmem<kFaithful>(tmem_row, kColD0, bias, half, group);
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD1, tmem_g + kColD0, tmem_g + kColL, aW1h, aW1l, 4096, 8, 64, false); if (elect_one()) mma_commit(bar); }
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- second half ----
+        epilogue_in_tmem<kFaithful>(tmem_row, kColD0 + 64, bias + 64, half, group);
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD1, tmem_g + kColD0 + 64, tmem_g + kColL, aW1h + 2048, aW1l + 2048, 4096, 8, 64, true); if (elect_one()) mma_commit(bar); }
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- hidden layer 1 -> output layer (its 16 accumulator columns reuse the head of the dead D0) ----
+        float pnz[3], pvar[3];
+        float *const sig = reinterpret_cast<float *>(S + kOffSde), *const sig2 = sig + kSdeXi;
+        float *const part = reinterpret_cast<float *>(S + kOffSdePart) + (group * kTile + lt) * 6;   // this row's exchange slot
+        epilogue_in_tmem_sde<kFaithful>(tmem_row, kColD1, bias + 128, half, group, sig, sig2, sde.xi, n, i,
+                                        po.stochastic != 0 && i < i1, pnz, pvar);
+        if (half == 1) {                 // read by the row's first half after the group barrier below
+#pragma unroll
+            for (int a = 0; a < 3; a++) { part[a] = pnz[a]; part[3 + a] = pvar[a]; }
+        }
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD0, tmem_g + kColD1, tmem_g + kColL, aW2h, aW2l, 2048, 8, 16, false); if (elect_one()) mma_commit(bar); }
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        out_i = i1;
+        if (half == 0) {
+            tmem_ld4(tmem_row + kColD0, outv);
+#pragma unroll
+            for (int q = 0; q < 4; q++) outv[q] += bias[192 + q];
+#pragma unroll
+            for (int a = 0; a < 3; a++) { nzv[a] = pnz[a] + part[a]; varv[a] = pvar[a] + part[3 + a]; }
+            out_i = i;
+        }
+        // no barrier here: the next slot's input stores go to D1 / L (their reader, this tile's last MMA, has completed),
+        // and the next MMA0, which overwrites the columns just read, is issued behind the group barrier that follows them
+    }
+    if (half == 0 && out_i < i1) sde_epilogue(po, out_i, outv, nzv, varv);
+    if (group == 0) token_take(0);                 // consume group 1's last hand-over: no barrier is left half-arrived at exit
+    fence_before();
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
+}
+
 // GAE scan: one thread per env walks its column of the [T][n] trajectory backwards (every access coalesced over
 // envs).  HBM-bound: 17 B per (t, env).  No FMA contraction: the float32 roundings are NumPy's.
 __global__ void __launch_bounds__(256)
@@ -950,23 +1175,40 @@ constexpr int kPpoAccW1 = kMlpH1 * kMlpH0;     // dW1 accumulators, [r * 8 + c][
 constexpr int kSmemPpo = (kMlpFloats + kPpoRows * kPpoTS + kPpoAccW1) * (int)sizeof(float);   // 224,976 B: 1 CTA per SM
 constexpr int kPpoMaxCtas = 148;
 static_assert(kThreads == 128 && kMlpFloats % 4 == 0 && kPpoRowG + 8 == kPpoRowT, "PPO tile layout");
+// gSDE (ppo_grad_sde_kernel): rows G + 4 .. G + 6 carry r_a instead of the log_std gradient, one more row holds the
+// per-sample entropy, and sigma^2 [64][3] follows the dW1 accumulators: 226,272 B
+constexpr int kPpoRowE = kPpoRowT + 4, kPpoRowsSde = kPpoRows + 1;
+constexpr int kSmemPpoSde = (kMlpFloats + kPpoRowsSde * kPpoTS + kPpoAccW1 + kSdeXi) * (int)sizeof(float);
+static_assert(kSmemPpoSde <= 232448, "PPO gSDE tile layout");
 int64_t ppo_ctas(int64_t B)
 {
     const int64_t tiles = (B + kThreads - 1) / kThreads;
     return tiles < kPpoMaxCtas ? tiles : kPpoMaxCtas;
 }
 
-__global__ void __launch_bounds__(kThreads, 1)
-ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restrict__ idx, int64_t B, float clip, float vf,
-                float ent, const double *__restrict__ adv_stats, double *__restrict__ part_terms, float *__restrict__ part)
+template <bool kSde>
+__device__ __forceinline__ void ppo_grad_body(const R6Mlp mlp, const float *sde_log_std, const R6PpoRollout ro,
+                                              const int64_t *__restrict__ idx, int64_t B, float clip, float vf, float ent,
+                                              const double *__restrict__ adv_stats, double *__restrict__ part_terms,
+                                              float *__restrict__ part)
 {
+    constexpr int kP = kSde ? kPpoParamsSde : kPpoParams, kNT = kSde ? R6_PPO_NTERMS_SDE : R6_PPO_NTERMS;
+    constexpr int kRows = kSde ? kPpoRowsSde : kPpoRows;
     extern __shared__ __align__(16) double r6_smem[];
     float *Ws = reinterpret_cast<float *>(r6_smem);
     float *S = Ws + kMlpFloats;
-    float *A1 = S + kPpoRows * kPpoTS;
+    float *A1 = S + kRows * kPpoTS;
+    float *sig2 = A1 + kPpoAccW1;            // gSDE only
     const int tid = threadIdx.x, kq = tid & 7, jq = tid >> 3;
     for (int i = tid; i < kMlpFloats; i += kThreads) Ws[i] = mlp_pack_element(mlp, i);
     for (int i = tid; i < kPpoAccW1; i += kThreads) A1[i] = 0.0f;
+    if constexpr (kSde) {
+        for (int c = tid; c < kSdeXi; c += kThreads) {
+            const float sg = expf(sde_log_std[c]);
+            sig2[c] = sg * sg;
+        }
+    }
+    float aLs[3] = {0.0f, 0.0f, 0.0f};       // gSDE: sum_s r_a h_tid^2 (threads 0..63)
     const int64_t nsamp = ro.T * ro.n;
     float aW0[14], aHd[5];                   // dW0[tid][0..12], db0[tid]; dW2[0..2][tid], dwv, db1
     double aS = 0.0;                         // thread 64 + r: sum of row kPpoRowG + r
@@ -994,11 +1236,17 @@ ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restric
 #pragma unroll
             for (int c = 0; c < kMlpIn; c++) S[(kPpoRowX + c) * kPpoTS + tid] = x[c];
             ppo_forward(Ws, x, S + kPpoRowH0 * kPpoTS + tid, S + kPpoRowH1 * kPpoTS + tid, kPpoTS, out);
-            PpoHead hd = {};
+            std::conditional_t<kSde, PpoHeadSde, PpoHead> hd = {};
             if (ok) {
                 const float a[3] = {ro.actions[3 * q], ro.actions[3 * q + 1], ro.actions[3 * q + 2]};
-                ppo_head(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], mlp.log_std, clip, vf,
-                         ent, hd);
+                if constexpr (kSde) {
+                    float var[3];
+                    sde_latent_var(S + kPpoRowH1 * kPpoTS + tid, kPpoTS, sig2, var);
+                    ppo_head_sde(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], var, clip,
+                                 vf, ent, hd);
+                } else
+                    ppo_head(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], mlp.log_std,
+                             clip, vf, ent, hd);
             }
             ppo_delta1(Ws, hd, S + kPpoRowH1 * kPpoTS + tid, S + kPpoRowD1 * kPpoTS + tid, kPpoTS);
 #pragma unroll
@@ -1008,6 +1256,7 @@ ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restric
             S[(kPpoRowT + 1) * kPpoTS + tid] = hd.vloss;
             S[(kPpoRowT + 2) * kPpoTS + tid] = hd.clipped;
             S[(kPpoRowT + 3) * kPpoTS + tid] = hd.kl;
+            if constexpr (kSde) S[kPpoRowE * kPpoTS + tid] = hd.ent;
         }
         __syncthreads();
         // dW1 += delta1^T h0 (every thread: dW1[kq + 8 r][jq + 16 c], in two halves of r), heads and scalar sums
@@ -1053,8 +1302,19 @@ ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restric
                     aHd[c] = a;
                 }
                 aHd[4] = (((aHd[4] + dv.x) + dv.y) + dv.z) + dv.w;
+                if constexpr (kSde) {
+                    const F4 hh = {hv.x * hv.x, hv.y * hv.y, hv.z * hv.z, hv.w * hv.w};
+#pragma unroll
+                    for (int c = 0; c < 3; c++) {
+                        const F4 r = ld4(S + (kPpoRowG + 4 + c) * kPpoTS + s4);
+                        float a = aLs[c];
+                        a = __fmaf_rn(r.x, hh.x, a); a = __fmaf_rn(r.y, hh.y, a);
+                        a = __fmaf_rn(r.z, hh.z, a); a = __fmaf_rn(r.w, hh.w, a);
+                        aLs[c] = a;
+                    }
+                }
             }
-        } else if (tid < kMlpH1 + 12) {
+        } else if (tid < kMlpH1 + (kSde ? 13 : 12)) {
             const float *row = S + (kPpoRowG + tid - kMlpH1) * kPpoTS;
 #pragma unroll 4
             for (int s = 0; s < kThreads; s++) aS += (double)row[s];
@@ -1087,7 +1347,7 @@ ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restric
         }
         __syncthreads();
     }
-    float *P = part + (int64_t)blockIdx.x * kPpoParams;
+    float *P = part + (int64_t)blockIdx.x * kP;
 #pragma unroll
     for (int r = 0; r < 8; r++)
 #pragma unroll
@@ -1100,15 +1360,33 @@ ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restric
         for (int c = 0; c < 3; c++) P[kPpoOffW2 + c * kMlpH1 + tid] = aHd[c];
         P[kPpoOffWv + tid] = aHd[3];
         P[kPpoOffB1 + tid] = aHd[4];
-    } else if (tid < kMlpH1 + 12) {
+        if constexpr (kSde) {
+#pragma unroll
+            for (int c = 0; c < 3; c++) P[kPpoOffLogStd + 3 * tid + c] = aLs[c] * sig2[3 * tid + c];
+        }
+    } else if (tid < kMlpH1 + (kSde ? 13 : 12)) {
         const int r = tid - kMlpH1;          // rows: g0..g2 (db2), g3 (dbv), g4..g6 (dlog_std), bad index, 4 loss terms
-        double *T = part_terms + (int64_t)blockIdx.x * R6_PPO_NTERMS;
+        double *T = part_terms + (int64_t)blockIdx.x * kNT;   // (gSDE: r_a sums unused, entropy last)
         if (r < 3) P[kPpoOffB2 + r] = (float)aS;
         else if (r == 3) P[kPpoOffBv] = (float)aS;
-        else if (r < 7) P[kPpoOffLogStd + r - 4] = (float)aS;
+        else if (r < 7) { if (!kSde) P[kPpoOffLogStd + r - 4] = (float)aS; }
         else if (r == 7) T[R6_PPO_T_BAD_INDEX] = aS;
-        else T[r - 8] = aS;
+        else if (r < 12) T[r - 8] = aS;
+        else T[R6_PPO_T_ENTROPY] = aS;
     }
+}
+__global__ void __launch_bounds__(kThreads, 1)
+ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restrict__ idx, int64_t B, float clip, float vf,
+                float ent, const double *__restrict__ adv_stats, double *__restrict__ part_terms, float *__restrict__ part)
+{
+    ppo_grad_body<false>(mlp, nullptr, ro, idx, B, clip, vf, ent, adv_stats, part_terms, part);
+}
+__global__ void __launch_bounds__(kThreads, 1)
+ppo_grad_sde_kernel(const R6Mlp mlp, const float *__restrict__ log_std, const R6PpoRollout ro, const int64_t *__restrict__ idx,
+                    int64_t B, float clip, float vf, float ent, const double *__restrict__ adv_stats,
+                    double *__restrict__ part_terms, float *__restrict__ part)
+{
+    ppo_grad_body<true>(mlp, log_std, ro, idx, B, clip, vf, ent, adv_stats, part_terms, part);
 }
 
 // grad[p] = sum of the CTA partials in CTA order (float64, rounded once); terms likewise
@@ -1128,6 +1406,25 @@ ppo_reduce_kernel(const double *__restrict__ part_terms, const float *__restrict
         terms[threadIdx.x] = s;
     }
 }
+
+// ppo_reduce_kernel over the gSDE layout
+__global__ void __launch_bounds__(256)
+ppo_reduce_sde_kernel(const double *__restrict__ part_terms, const float *__restrict__ part, int G, float *__restrict__ grad,
+                      double *__restrict__ terms)
+{
+    const int p = blockIdx.x * 256 + threadIdx.x;
+    if (p < kPpoParamsSde) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += (double)part[(int64_t)g * kPpoParamsSde + p];
+        grad[p] = (float)s;
+    }
+    if (blockIdx.x == 0 && threadIdx.x < R6_PPO_NTERMS_SDE) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += part_terms[g * R6_PPO_NTERMS_SDE + threadIdx.x];
+        terms[threadIdx.x] = s;
+    }
+}
+
 
 // r6_adam_step: one CTA (P is ~10^4).  The squared norm is summed in float64 in a fixed order (strided per thread,
 // then a fixed warp-shuffle tree, then the 32 warp sums in order), so the step is deterministic.
@@ -1221,6 +1518,10 @@ int ensure_attributes()
     rc |= enable_smem(policy_tc5_kernel<true>, tc5::kSmemBytes);
     rc |= enable_smem(policy_tc5_kernel<false>, tc5::kSmemBytes);
     rc |= enable_smem(ppo_grad_kernel, kSmemPpo);
+    rc |= enable_smem(ppo_grad_sde_kernel, kSmemPpoSde);
+    rc |= enable_smem(policy_sde_kernel, kSmemPolicySde);
+    rc |= enable_smem(policy_tc5_sde_kernel<true>, tc5::kSmemBytesSde);
+    rc |= enable_smem(policy_tc5_sde_kernel<false>, tc5::kSmemBytesSde);
     rc |= enable_smem(sim_raw_kernel<false>);
     rc |= enable_smem(sim_raw_kernel<true>);
     if (rc) return R6_ECUDA;
@@ -1483,6 +1784,53 @@ int r6_policy_range(const R6Mlp *mlp, const float *obs, int64_t n, int64_t first
     return check_launch("r6_policy");
 }
 
+int r6_sde_size(void) { return (int)sizeof(R6Sde); }
+
+int r6_sde_noise(int64_t n, int64_t first, int64_t count, uint64_t seed, int64_t env_offset, int64_t step_index, float *xi,
+                 void *stream)
+{
+    if (!xi) return fail(R6_EINVAL, "null pointer%s");
+    if (n < 0) return fail(R6_EINVAL, "n < 0%s");
+    if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
+    if (count == 0) return R6_OK;
+    sde_noise_kernel<<<dim3((unsigned)((count + 255) / 256), kSdeBlocks), 256, 0, (cudaStream_t)stream>>>(
+        seed, env_offset, step_index, n, first, first + count, xi);
+    return check_launch("r6_sde_noise");
+}
+
+int r6_policy_sde_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, int64_t n, int64_t first, int64_t count,
+                        int32_t tensor_cores, int32_t stochastic, float *actions, float *actions_raw, float *values,
+                        float *log_prob, void *stream)
+{
+    if (int rc = check_mlp(mlp)) return rc;
+    if (!sde || !sde->log_std || !sde->xi || !obs || !actions) return fail(R6_EINVAL, "null pointer%s");
+    if (n < 0) return fail(R6_EINVAL, "n < 0%s");
+    if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
+    if (tensor_cores == 1) return fail(R6_EINVAL, "gSDE has no mma.sync policy kernel (tensor_cores = 1): use 0, 2 or 3%s");
+    if (tensor_cores < 0 || tensor_cores > 3) return fail(R6_EINVAL, "tensor_cores must be 0, 2 or 3%s");
+    if (count == 0) return R6_OK;
+    int rc = ensure_attributes();
+    if (rc) return rc;
+    int dev = 0, sm_count = 0;
+    cudaGetDevice(&dev);
+    if (cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sm_count <= 0) sm_count = 148;
+    const PolicyOut po = {actions, actions_raw, values, log_prob, stochastic, 0, 0, 0, first, first + count};
+    const SdeIn si = {sde->log_std, sde->xi};
+    cudaStream_t s = (cudaStream_t)stream;
+    if (tensor_cores >= 2) {
+        if ((reinterpret_cast<uintptr_t>(mlp->w1) & 15u) != 0) return fail(R6_EINVAL, "tensor_cores = 2 / 3 need w1 16-byte aligned%s");
+        const int64_t pairs = (blocks_for(count) + 1) / 2;
+        const unsigned g5 = (unsigned)(pairs < sm_count ? pairs : sm_count);
+        if (tensor_cores == 3) launch_pdl(policy_tc5_sde_kernel<true>, g5, tc5::kThreads, tc5::kSmemBytesSde, s, *mlp, si, obs, n, po);
+        else launch_pdl(policy_tc5_sde_kernel<false>, g5, tc5::kThreads, tc5::kSmemBytesSde, s, *mlp, si, obs, n, po);
+    } else {
+        const int64_t wave = (int64_t)sm_count * 4;
+        const unsigned g = (unsigned)(blocks_for(count) < wave ? blocks_for(count) : wave);
+        policy_sde_kernel<<<g, kThreads, kSmemPolicySde, s>>>(*mlp, si, obs, n, po);
+    }
+    return check_launch("r6_policy_sde_range");
+}
+
 int r6_policy_ex(const R6Mlp *mlp, const float *obs, int64_t n, int32_t tensor_cores, int32_t stochastic, uint64_t seed,
                  int64_t env_offset, int64_t step_index, float *actions, float *actions_raw, float *values,
                  float *log_prob, void *stream)
@@ -1541,19 +1889,23 @@ int64_t r6_ppo_work_bytes(int64_t B)
     return B > 0 ? ppo_ctas(B) * (int64_t)(R6_PPO_NTERMS * sizeof(double) + kPpoParams * sizeof(float)) : 0;
 }
 
-int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *idx, int64_t B, const R6PpoCoef *coef,
-                float *grad_sum, double *terms, void *work, void *stream)
+}  // extern "C"
+
+namespace {
+// r6_ppo_grad / r6_ppo_grad_sde (sde_log_std != NULL): the gradient kernel, then the reduction of its CTA partials
+template <bool kSde>
+int ppo_grad_launch(const R6Mlp *mlp, const float *sde_log_std, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
+                    const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream)
 {
-    if (int rc = check_mlp(mlp)) return rc;
-    if (!mlp->wv || !mlp->bv || !mlp->log_std) return fail(R6_EINVAL, "r6_ppo_grad needs the critic head and log_std%s");
+    constexpr int kP = kSde ? kPpoParamsSde : kPpoParams, kNT = kSde ? R6_PPO_NTERMS_SDE : R6_PPO_NTERMS;
     if (!rollout || !rollout->obs || !rollout->actions || !rollout->log_probs || !rollout->advantages || !rollout->returns)
         return fail(R6_EINVAL, "null rollout buffer%s");
     if (rollout->T < 0 || rollout->n < 0 || B < 0) return fail(R6_EINVAL, "negative size%s");
     if (!coef || !grad_sum || !terms || (B > 0 && (!idx || !work))) return fail(R6_EINVAL, "null pointer%s");
     cudaStream_t s = (cudaStream_t)stream;
     if (B == 0) {
-        cudaError_t e = cudaMemsetAsync(grad_sum, 0, sizeof(float) * kPpoParams, s);
-        if (e == cudaSuccess) e = cudaMemsetAsync(terms, 0, sizeof(double) * R6_PPO_NTERMS, s);
+        cudaError_t e = cudaMemsetAsync(grad_sum, 0, sizeof(float) * kP, s);
+        if (e == cudaSuccess) e = cudaMemsetAsync(terms, 0, sizeof(double) * kNT, s);
         if (e != cudaSuccess) return fail(R6_ECUDA, "cudaMemsetAsync: %s", cudaGetErrorString(e));
         return R6_OK;
     }
@@ -1561,13 +1913,45 @@ int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *id
     if (rc) return rc;
     const int G = (int)ppo_ctas(B);
     double *pt = static_cast<double *>(work);
-    float *pp = reinterpret_cast<float *>(pt + (int64_t)G * R6_PPO_NTERMS);
-    ppo_grad_kernel<<<G, kThreads, kSmemPpo, s>>>(*mlp, *rollout, idx, B, (float)coef->clip_range, (float)coef->vf_coef,
-                                                  (float)coef->ent_coef, coef->adv_stats, pt, pp);
-    rc = check_launch("r6_ppo_grad");
-    if (rc) return rc;
-    ppo_reduce_kernel<<<(kPpoParams + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
-    return check_launch("r6_ppo_grad (reduce)");
+    float *pp = reinterpret_cast<float *>(pt + (int64_t)G * kNT);
+    const float clip = (float)coef->clip_range, vf = (float)coef->vf_coef, ent = (float)coef->ent_coef;
+    if constexpr (kSde) {
+        ppo_grad_sde_kernel<<<G, kThreads, kSmemPpoSde, s>>>(*mlp, sde_log_std, *rollout, idx, B, clip, vf, ent, coef->adv_stats, pt, pp);
+        rc = check_launch("r6_ppo_grad_sde");
+        if (rc) return rc;
+        ppo_reduce_sde_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
+        return check_launch("r6_ppo_grad_sde (reduce)");
+    } else {
+        ppo_grad_kernel<<<G, kThreads, kSmemPpo, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, coef->adv_stats, pt, pp);
+        rc = check_launch("r6_ppo_grad");
+        if (rc) return rc;
+        ppo_reduce_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
+        return check_launch("r6_ppo_grad (reduce)");
+    }
+}
+}  // namespace
+
+extern "C" {
+
+int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *idx, int64_t B, const R6PpoCoef *coef,
+                float *grad_sum, double *terms, void *work, void *stream)
+{
+    if (int rc = check_mlp(mlp)) return rc;
+    if (!mlp->wv || !mlp->bv || !mlp->log_std) return fail(R6_EINVAL, "r6_ppo_grad needs the critic head and log_std%s");
+    return ppo_grad_launch<false>(mlp, nullptr, rollout, idx, B, coef, grad_sum, terms, work, stream);
+}
+
+int64_t r6_ppo_sde_work_bytes(int64_t B)
+{
+    return B > 0 ? ppo_ctas(B) * (int64_t)(R6_PPO_NTERMS_SDE * sizeof(double) + kPpoParamsSde * sizeof(float)) : 0;
+}
+
+int r6_ppo_grad_sde(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
+                    const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream)
+{
+    if (int rc = check_mlp(mlp)) return rc;
+    if (!mlp->wv || !mlp->bv || !sde || !sde->log_std) return fail(R6_EINVAL, "r6_ppo_grad_sde needs the critic head and log_std%s");
+    return ppo_grad_launch<true>(mlp, sde->log_std, rollout, idx, B, coef, grad_sum, terms, work, stream);
 }
 
 int r6_adam_step(float *params, const float *grad_sum, float *m, float *v, int64_t P, const R6AdamCoef *coef,

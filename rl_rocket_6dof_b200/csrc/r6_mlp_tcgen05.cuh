@@ -59,6 +59,9 @@ constexpr int kOffBias = 88 << 10;                                   // b0[128] 
 constexpr int kOffBar = kOffBias + (128 + 64 + 4) * 4;               // one mbarrier per group
 constexpr int kOffTmemPtr = kOffBar + 16;
 constexpr int kSmemBytes = kOffTmemPtr + 16;
+// gSDE kernels only: sigma [192], sigma^2 [192], and per group the second column half's partial sums [128 rows][6]
+constexpr int kOffSde = kSmemBytes, kOffSdePart = kOffSde + 2 * 192 * 4;
+constexpr int kSmemBytesSde = kOffSdePart + 2 * kTile * 6 * 4;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ int tile_off(int r, int k, int ktot) { return (r & 7) * 16 + (r >> 3) * (ktot * 32) + (k >> 2) * 128 + (k & 3) * 4; }
@@ -214,6 +217,52 @@ __device__ __forceinline__ void epilogue_in_tmem(uint32_t tmem_row, uint32_t src
         for (int q = 0; q < 32; q++) v[q] = round_tf32(tanh_fast(v[q] + bias[cc + q]));
         token_pass(group ^ 1);
         tmem_st32(tmem_row + src + cc, v);
+    }
+    tmem_st_wait();
+}
+
+// epilogue_in_tmem of the last hidden layer with the gSDE sums over this thread's 32 units k = cc .. cc + 31 of its env row
+// i: nz_a = sum_k h_k (sigma_ka xi_ka) (when draw) and var_a = sum_k h_k^2 sigma_ka^2, h the activation the next MMA
+// consumes (hi + lo in faithful mode, hi in fast mode).  Formed after the token is handed over (under the other group's
+// arithmetic), from xi read coalesced over the rows and sigma, sigma^2 in shared memory.
+template <bool kFaithful>
+__device__ __forceinline__ void epilogue_in_tmem_sde(uint32_t tmem_row, uint32_t src, const float *bias, int half, int group,
+                                                     const float *sig, const float *sig2, const float *__restrict__ xi,
+                                                     int64_t n, int64_t i, bool draw, float (&nz)[3], float (&var)[3])
+{
+    const int cc = 32 * half;
+    float v[32], l[32];
+    tmem_ld32(tmem_row + src + cc, v);
+    token_take(group);
+    if constexpr (kFaithful) {
+#pragma unroll
+        for (int q = 0; q < 32; q++) split_tf32(tanh_exact_scaled(fmaf(v[q], kTwoLog2e, bias[cc + q])), v[q], l[q]);
+        token_pass(group ^ 1);
+        tmem_st32(tmem_row + src + cc, v);
+        tmem_st32(tmem_row + kColL + cc, l);
+    } else {
+#pragma unroll
+        for (int q = 0; q < 32; q++) v[q] = round_tf32(tanh_fast(v[q] + bias[cc + q]));
+        token_pass(group ^ 1);
+        tmem_st32(tmem_row + src + cc, v);
+    }
+#pragma unroll
+    for (int a = 0; a < 3; a++) nz[a] = var[a] = 0.0f;
+    // xi walked by one pointer bumped n floats per component: precomputed per-component 64-bit offsets (loop invariants
+    // across tiles) would not fit the 128 registers of a 512-thread CTA
+    const float *px = xi + (int64_t)(3 * cc) * n + i;
+    const int64_t stride = n;
+#pragma unroll
+    for (int q = 0; q < 32; q++) {
+        const float h = kFaithful ? v[q] + l[q] : v[q], hh = h * h;
+#pragma unroll
+        for (int a = 0; a < 3; a++) {
+            const int c = 3 * (cc + q) + a;
+            if (draw) nz[a] = fmaf(h, sig[c] * __ldg(px), nz[a]);
+            var[a] = fmaf(hh, sig2[c], var[a]);
+            px += stride;
+            asm volatile("" : "+l"(px));
+        }
     }
     tmem_st_wait();
 }

@@ -23,6 +23,9 @@ namespace r6 {
 constexpr int kPpoOffW0 = 0, kPpoOffB0 = 1664, kPpoOffW1 = 1792, kPpoOffB1 = 9984, kPpoOffW2 = 10048,
               kPpoOffB2 = 10240, kPpoOffWv = 10243, kPpoOffBv = 10307, kPpoOffLogStd = 10308, kPpoParams = 10311;
 static_assert(kPpoParams == R6_PPO_NPARAMS, "flat layout");
+// the gSDE layout: the same prefix through bv, then log_std [64][3] (SB3 order)
+constexpr int kPpoParamsSde = kPpoOffLogStd + kSdeXi;
+static_assert(kPpoParamsSde == R6_PPO_NPARAMS_SDE, "flat layout (gSDE)");
 static_assert(kPpoOffB0 == kMlpH0 * kMlpIn && kPpoOffW1 == kPpoOffB0 + kMlpH0 && kPpoOffB1 == kPpoOffW1 + kMlpH1 * kMlpH0 &&
               kPpoOffW2 == kPpoOffB1 + kMlpH1 && kPpoOffB2 == kPpoOffW2 + 3 * kMlpH1 && kPpoOffWv == kPpoOffB2 + 3 &&
               kPpoOffBv == kPpoOffWv + kMlpH1 && kPpoOffLogStd == kPpoOffBv + 1 && kPpoOffW1 % 4 == 0, "flat layout");
@@ -113,6 +116,68 @@ R6_HD void ppo_head(const float (&out)[4], const float *a, float old_logp, float
     h.vloss = e * e;
     h.clipped = fabsf(ratio - 1.0f) > clip ? 1.0f : 0.0f;
     h.kl = (ratio - 1.0f) - lr;
+}
+
+// 1 / sqrt(v), rounded once (the device form has no slow path, unlike a division)
+R6_HD float f32_rsqrt(float v)
+{
+#if defined(__CUDA_ARCH__)
+    return __frsqrt_rn(v);
+#else
+    return (float)(1.0 / sqrt((double)v));
+#endif
+}
+
+// The gSDE head (SB3 StateDependentNoiseDistribution, see sde_head in r6_core.cuh) [memory]: per-sample
+// std_a^2 = var_a + 1e-6 with var_a = sum_k h_k^2 sigma_ka^2 (h detached), logp and entropy of N(mean, std) summed over
+// the actions.  g[0..3] as ppo_head; g[4 + a] = r_a = (w (z_a^2 - 1) - ent_coef) / std_a^2, so that
+// d loss / d log_std[k][a] = sigma_ka^2 sum_s r_{s,a} h_{s,k}^2; ent = the sample's entropy.
+struct PpoHeadSde : PpoHead {
+    float ent;
+};
+R6_HD void ppo_head_sde(const float (&out)[4], const float *a, float old_logp, float adv, float ret, const float (&var)[3],
+                        float clip, float vf_coef, float ent_coef, PpoHeadSde &h)
+{
+    float z[3], isg[3], logp = 0.0f, ent = 0.0f;
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+        const float v = var[j] + 1e-6f;
+        isg[j] = f32_rsqrt(v);
+        const float ls = 0.5f * logf(v);                 // log std
+        z[j] = (a[j] - out[j]) * isg[j];
+        logp += -0.5f * (z[j] * z[j]) - ls - 0.9189385332046727f;
+        ent += (0.5f + 0.9189385332046727f) + ls;
+    }
+    const float lr = logp - old_logp;
+    const float ratio = expf(lr);
+    const float rc = fminf(fmaxf(ratio, 1.0f - clip), 1.0f + clip);
+    const float s1 = adv * ratio, s2 = adv * rc;
+    h.pg = -fminf(s1, s2);
+    const float w = s1 <= s2 ? -s1 : 0.0f;
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+        h.g[j] = w * (z[j] * isg[j]);
+        h.g[4 + j] = (w * f32_fma(z[j], z[j], -1.0f) - ent_coef) * (isg[j] * isg[j]);
+    }
+    const float e = out[3] - ret;
+    h.g[3] = 2.0f * vf_coef * e;
+    h.vloss = e * e;
+    h.clipped = fabsf(ratio - 1.0f) > clip ? 1.0f : 0.0f;
+    h.kl = (ratio - 1.0f) - lr;
+    h.ent = ent;
+}
+
+// var_a = sum_k h1[k * st]^2 sig2[3 k + a] in k order (sig2 = sigma^2 [64][3])
+R6_HD void sde_latent_var(const float *h1, int st, const float *sig2, float (&var)[3])
+{
+    var[0] = var[1] = var[2] = 0.0f;
+#pragma unroll 4
+    for (int k = 0; k < kMlpH1; k++) {
+        const float h = h1[k * st], hh = h * h;
+        var[0] = f32_fma(hh, sig2[3 * k], var[0]);
+        var[1] = f32_fma(hh, sig2[3 * k + 1], var[1]);
+        var[2] = f32_fma(hh, sig2[3 * k + 2], var[2]);
+    }
 }
 
 // delta1_k = (sum_c W2[c][k] g_c + wv_k g_v) (1 - h1_k^2), from h1[k * st] into d1[k * st]

@@ -16,8 +16,10 @@ import numpy as np
 import torch
 
 SHAPES = {"w0": (128, 13), "b0": (128,), "w1": (64, 128), "b1": (64,), "w2": (3, 64), "b2": (3,)}
-# optional: the critic head on the same latent and the Gaussian log-std (needed only to COLLECT training rollouts)
+# optional: the critic head on the same latent and the Gaussian log-std (needed only to COLLECT training rollouts);
+# log_std is [3] (diagonal Gaussian) or, for a gSDE policy (use_sde=True), [64, 3]
 OPTIONAL_SHAPES = {"wv": (64,), "bv": (1,), "log_std": (3,)}
+SDE_LOG_STD_SHAPE = (64, 3)
 _SB3_OPTIONAL = {"wv": "value_net.weight", "bv": "value_net.bias", "log_std": "log_std"}
 _SB3_KEYS = {
     "w0": "mlp_extractor.shared_net.0.weight", "b0": "mlp_extractor.shared_net.0.bias",
@@ -39,8 +41,13 @@ def _check(w: Dict[str, np.ndarray]) -> Dict[str, np.ndarray]:
         out[k] = a
     for k, shp in OPTIONAL_SHAPES.items():
         if k in w and w[k] is not None:
-            a = np.ascontiguousarray(np.asarray(w[k], dtype=np.float32)).reshape(shp)
-            out[k] = a
+            a = np.ascontiguousarray(np.asarray(w[k], dtype=np.float32))
+            if k == "log_std" and a.size == 64 * 3:
+                shp = SDE_LOG_STD_SHAPE
+            if a.size != int(np.prod(shp)):
+                raise ValueError(f"policy tensor {k} has shape {a.shape}, expected {shp}"
+                                 + (f" or {SDE_LOG_STD_SHAPE} (gSDE)" if k == "log_std" else ""))
+            out[k] = a.reshape(shp)
     return out
 
 

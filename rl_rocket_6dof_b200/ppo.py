@@ -9,7 +9,9 @@ over rollouts collected by `Rocket6DOFBatch.collect_rollout`, with the loss grad
     logs = trainer.learn(total_timesteps=10_000_000)
 
 The network is SB3's default `MlpPolicy` of SB3 1.6: a shared tanh trunk 13 -> 128 -> 64, `action_net` 64 -> 3,
-`value_net` 64 -> 1 and a state-independent `log_std` (no gSDE, no `clip_range_vf`).
+`value_net` 64 -> 1 and a state-independent `log_std` [3], or with `PPOConfig(use_sde=True)` SB3's generalised
+state-dependent exploration (gSDE: log_std [64, 3], noise h (exp(log_std) * xi) held between `reset_noise` draws;
+params from `ActorCriticParams.sb3_init(use_sde=True)`).  No `clip_range_vf`.
 """
 from __future__ import annotations
 
@@ -27,28 +29,36 @@ from . import _lib
 LAYOUT = (("w0", (128, 13)), ("b0", (128,)), ("w1", (64, 128)), ("b1", (64,)), ("w2", (3, 64)), ("b2", (3,)),
           ("wv", (64,)), ("bv", (1,)), ("log_std", (3,)))
 NPARAMS = _lib.PPO_NPARAMS
+# the gSDE layout (R6_PPO_NPARAMS_SDE): the same prefix, log_std [64][3]
+LAYOUT_SDE = LAYOUT[:-1] + (("log_std", (64, 3)),)
+NPARAMS_SDE = _lib.PPO_NPARAMS_SDE
 _LOG_SQRT_2PI = 0.5 * math.log(2.0 * math.pi)
 
 
 class ActorCriticParams:
-    """The actor-critic as one flat float32 CUDA tensor `flat` [R6_PPO_NPARAMS] with views w0 ... log_std into it."""
+    """The actor-critic as one flat float32 CUDA tensor `flat` with views w0 ... log_std into it: [R6_PPO_NPARAMS]
+    with log_std [3], or [R6_PPO_NPARAMS_SDE] with the gSDE log_std [64, 3] (`use_sde`)."""
 
     def __init__(self, flat: torch.Tensor):
-        if flat.dtype != torch.float32 or not flat.is_cuda or flat.shape != (NPARAMS,) or not flat.is_contiguous():
-            raise ValueError(f"flat parameters must be a contiguous float32 CUDA tensor of {NPARAMS} elements")
+        if (flat.dtype != torch.float32 or not flat.is_cuda or flat.shape not in ((NPARAMS,), (NPARAMS_SDE,))
+                or not flat.is_contiguous()):
+            raise ValueError(f"flat parameters must be a contiguous float32 CUDA tensor of {NPARAMS} or {NPARAMS_SDE} "
+                             "(gSDE) elements")
         self.flat = flat
+        self.use_sde = flat.numel() == NPARAMS_SDE
+        self.layout = LAYOUT_SDE if self.use_sde else LAYOUT
         o = 0
-        for name, shape in LAYOUT:
+        for name, shape in self.layout:
             size = int(np.prod(shape))
             setattr(self, name, flat[o:o + size].view(shape))
             o += size
-        assert o == NPARAMS
+        assert o == flat.numel()
 
     @classmethod
-    def sb3_init(cls, seed: int = 0, device="cuda") -> "ActorCriticParams":
+    def sb3_init(cls, seed: int = 0, device="cuda", use_sde: bool = False) -> "ActorCriticParams":
         """SB3's construction-time weights (ortho_init): `torch.nn.init.orthogonal_` with gain sqrt(2) on the trunk,
-        0.01 on action_net and 1 on value_net, zero biases, log_std 0.  Drawn on the CPU with a generator seeded by
-        `seed`, so they do not depend on the device."""
+        0.01 on action_net and 1 on value_net, zero biases, log_std 0 ([64, 3] with use_sde).  Drawn on the CPU with a
+        generator seeded by `seed`, so they do not depend on the device."""
         gen = torch.Generator().manual_seed(int(seed))
         w = {}
         for name, shape, gain in (("w0", (128, 13), math.sqrt(2)), ("w1", (64, 128), math.sqrt(2)), ("w2", (3, 64), 0.01),
@@ -56,21 +66,22 @@ class ActorCriticParams:
             t = torch.empty(shape, dtype=torch.float32)
             torch.nn.init.orthogonal_(t, gain=gain, generator=gen)
             w[name] = t.reshape(-1)
-        return cls._from(w, device)
+        return cls._from(w, device, LAYOUT_SDE if use_sde else LAYOUT)
 
     @classmethod
     def from_weights(cls, w: Dict[str, np.ndarray], device="cuda") -> "ActorCriticParams":
-        """From `policy.load_sb3_zip` / `policy.load_npz` output (the critic head and log_std must be present)."""
+        """From `policy.load_sb3_zip` / `policy.load_npz` output (the critic head and log_std must be present); a
+        [64, 3] log_std gives the gSDE layout."""
         missing = [k for k, _ in LAYOUT if w.get(k) is None]
         if missing:
             raise ValueError(f"weights lack {missing}: training needs the critic head and log_std")
-        return cls._from(w, device)
+        return cls._from(w, device, LAYOUT_SDE if np.asarray(w["log_std"]).size == 64 * 3 else LAYOUT)
 
     @classmethod
-    def _from(cls, w, device) -> "ActorCriticParams":
-        flat = torch.zeros(NPARAMS, dtype=torch.float32)
+    def _from(cls, w, device, layout) -> "ActorCriticParams":
+        flat = torch.zeros(sum(int(np.prod(shape)) for _, shape in layout), dtype=torch.float32)
         o = 0
-        for name, shape in LAYOUT:
+        for name, shape in layout:
             size = int(np.prod(shape))
             if name in w:
                 flat[o:o + size] = torch.as_tensor(np.asarray(w[name], np.float32).reshape(-1))
@@ -79,7 +90,7 @@ class ActorCriticParams:
 
     def mlp(self) -> Dict[str, torch.Tensor]:
         """The weight dict `collect_rollout`, `step_policy`, `policy_forward` and `montecarlo` accept."""
-        return {name: getattr(self, name) for name, _ in LAYOUT}
+        return {name: getattr(self, name) for name, _ in self.layout}
 
     def save_npz(self, path: str):
         """Writes `mlp_w0` ... `mlp_log_std`: what `policy.load_npz` and the Monte-Carlo CLI read."""
@@ -113,6 +124,20 @@ class PPOConfig:
     max_grad_norm: float = 0.5
     target_kl: Optional[float] = None
     tensor_cores: int = 3          # policy kernel of the collection (r6_policy: 3 = tcgen05 3xTF32, float32-faithful)
+    use_sde: bool = False          # gSDE exploration (the params must have the gSDE layout)
+    sde_sample_freq: int = -1      # gSDE: redraw the noise every this many steps; -1 = once per rollout
+    # SB3 gSDE options this trainer has no kernels for: only SB3's PPO defaults are accepted
+    full_std: bool = True
+    use_expln: bool = False
+    squash_output: bool = False
+    learn_features: bool = False
+
+    def __post_init__(self):
+        bad = [k for k, ok in (("full_std", self.full_std), ("use_expln", not self.use_expln),
+                                ("squash_output", not self.squash_output), ("learn_features", not self.learn_features)) if not ok]
+        if bad:
+            raise ValueError(f"gSDE options {bad} are not implemented (only full_std=True, use_expln=False, "
+                             "squash_output=False, learn_features=False)")
 
 
 def _check_cuda(name, t, dtype, dev):
@@ -129,8 +154,10 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     `rollout` is `collect_rollout`'s dict (obs [T, N, 13] with any strides, actions [T, N, 3], log_probs, advantages,
     returns [T, N]).  Indices outside [0, T N) are skipped and counted in terms[4] (checking them here would
     synchronise).  The minibatch's advantage mean and 1 / (std + 1e-8) are computed on the device (no synchronise).
-    Returns (grad_sum float32 [R6_PPO_NPARAMS], terms float64 [5])."""
+    Returns (grad_sum float32 [R6_PPO_NPARAMS], terms float64 [5]); for gSDE params (r6_ppo_grad_sde) grad_sum
+    [R6_PPO_NPARAMS_SDE] and terms [6], the last the sum of the per-sample entropies."""
     dev = params.flat.device
+    P, NT = params.flat.numel(), (_lib.PPO_NTERMS_SDE if params.use_sde else _lib.PPO_NTERMS)
     obs, act = rollout["obs"], rollout["actions"]
     lp, adv, ret = rollout["log_probs"], rollout["advantages"], rollout["returns"]
     for name, t in (("obs", obs), ("actions", act), ("log_probs", lp), ("advantages", adv), ("returns", ret)):
@@ -147,15 +174,15 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
         raise ValueError("idx must be a contiguous 1-D int64 tensor")
     B = idx.numel()
     if grad_sum is None:
-        grad_sum = torch.empty(NPARAMS, dtype=torch.float32, device=dev)
+        grad_sum = torch.empty(P, dtype=torch.float32, device=dev)
     if terms is None:
-        terms = torch.empty(_lib.PPO_NTERMS, dtype=torch.float64, device=dev)
+        terms = torch.empty(NT, dtype=torch.float64, device=dev)
     _check_cuda("grad_sum", grad_sum, torch.float32, dev)
     _check_cuda("terms", terms, torch.float64, dev)
-    if grad_sum.shape != (NPARAMS,) or terms.shape != (_lib.PPO_NTERMS,) or not grad_sum.is_contiguous():
+    if grad_sum.shape != (P,) or terms.shape != (NT,) or not grad_sum.is_contiguous():
         raise ValueError("grad_sum / terms have the wrong shape")
     L = _lib.load()
-    need = int(L.r6_ppo_work_bytes(B))
+    need = int(L.r6_ppo_sde_work_bytes(B) if params.use_sde else L.r6_ppo_work_bytes(B))
     if work is None or work.numel() < need:
         work = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
     stats = None
@@ -169,8 +196,14 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     coef = _lib.R6PpoCoef(float(clip_range), float(vf_coef), float(ent_coef), None if stats is None else stats.data_ptr())
     m = _lib.make_mlp(params.mlp())
     with torch.cuda.device(dev):
-        _lib.check(L.r6_ppo_grad(C.byref(m), C.byref(ro), idx.data_ptr(), B, C.byref(coef), grad_sum.data_ptr(),
-                                 terms.data_ptr(), work.data_ptr(), torch.cuda.current_stream(dev).cuda_stream), L)
+        if params.use_sde:
+            sde = _lib.R6Sde(params.log_std.data_ptr(), None)
+            _lib.check(L.r6_ppo_grad_sde(C.byref(m), C.byref(sde), C.byref(ro), idx.data_ptr(), B, C.byref(coef),
+                                         grad_sum.data_ptr(), terms.data_ptr(), work.data_ptr(),
+                                         torch.cuda.current_stream(dev).cuda_stream), L)
+        else:
+            _lib.check(L.r6_ppo_grad(C.byref(m), C.byref(ro), idx.data_ptr(), B, C.byref(coef), grad_sum.data_ptr(),
+                                     terms.data_ptr(), work.data_ptr(), torch.cuda.current_stream(dev).cuda_stream), L)
     return grad_sum, terms
 
 
@@ -200,6 +233,10 @@ class PPOTrainer:
 
     def __init__(self, batch, params: ActorCriticParams, cfg: Optional[PPOConfig] = None, seed: int = 0):
         self.batch, self.params, self.cfg = batch, params, cfg or PPOConfig()
+        if params.use_sde != self.cfg.use_sde:
+            raise ValueError(f"PPOConfig(use_sde={self.cfg.use_sde}) needs params with the "
+                             f"{'gSDE' if self.cfg.use_sde else 'diagonal Gaussian'} layout "
+                             f"(ActorCriticParams.sb3_init(use_sde={self.cfg.use_sde}))")
         dev = params.flat.device
         self.m = torch.zeros_like(params.flat)
         self.v = torch.zeros_like(params.flat)
@@ -209,7 +246,7 @@ class PPOTrainer:
         self.adam_steps = 0
         self.num_timesteps = 0
         self.progress_remaining = 1.0
-        self._grad = torch.empty(NPARAMS, dtype=torch.float32, device=dev)
+        self._grad = torch.empty(params.flat.numel(), dtype=torch.float32, device=dev)
         self._work = None
 
     def batch_size(self, total: int) -> int:
@@ -220,19 +257,22 @@ class PPOTrainer:
 
         As SB3 1.6 logs them [memory]: policy_gradient_loss, value_loss, clip_fraction and entropy_loss are means over
         every minibatch that ran (the one `target_kl` stops at included), approx_kl is the mean over the minibatches of
-        the last epoch that ran, entropy_loss and loss use each minibatch's log_std before its Adam step, and loss is the
-        last minibatch's.  The learning rate is `learning_rate(progress_remaining)`."""
+        the last epoch that ran, entropy_loss and loss use each minibatch's log_std before its Adam step (gSDE: the mean
+        per-sample entropy of the minibatch, from the kernel's entropy term), and loss is the last minibatch's.  The
+        learning rate is `learning_rate(progress_remaining)`."""
         cfg, dev = self.cfg, self.params.flat.device
         T, n = rollout["advantages"].shape
         total = T * n
         bs = self.batch_size(total)
         lr = _progress_lr(cfg.learning_rate, self.progress_remaining)
         nmb = -(-total // bs)
-        terms = torch.zeros(cfg.n_epochs * nmb, _lib.PPO_NTERMS, dtype=torch.float64, device=dev)
+        sde = self.params.use_sde
+        terms = torch.zeros(cfg.n_epochs * nmb, _lib.PPO_NTERMS_SDE if sde else _lib.PPO_NTERMS, dtype=torch.float64,
+                            device=dev)
         log_std_sums = torch.zeros(cfg.n_epochs * nmb, dtype=torch.float64, device=dev)
         sizes = []
         L = _lib.load()
-        need = int(L.r6_ppo_work_bytes(min(bs, total)))
+        need = int((L.r6_ppo_sde_work_bytes if sde else L.r6_ppo_work_bytes)(min(bs, total)))
         if self._work is None or self._work.numel() < need:
             self._work = torch.empty(need, dtype=torch.uint8, device=dev)
         done = False
@@ -245,10 +285,11 @@ class PPOTrainer:
                 loss_and_grad(self.params, rollout, idx, clip_range=cfg.clip_range, vf_coef=cfg.vf_coef,
                               ent_coef=cfg.ent_coef, normalize_advantage=cfg.normalize_advantage, grad_sum=self._grad,
                               terms=terms[k], work=self._work)
-                log_std_sums[k] = self.params.log_std.sum(dtype=torch.float64)    # this minibatch's entropy (no sync)
+                if not sde:
+                    log_std_sums[k] = self.params.log_std.sum(dtype=torch.float64)    # this minibatch's entropy (no sync)
                 sizes.append(idx.numel())
                 if cfg.target_kl is not None:
-                    kl = float(terms[k, _lib.PPO_NTERMS - 2]) / idx.numel()      # the one host read per minibatch
+                    kl = float(terms[k, 3]) / idx.numel()      # approx-kl sum: the one host read per minibatch
                     if kl > 1.5 * cfg.target_kl:
                         done = True
                         break
@@ -262,7 +303,10 @@ class PPOTrainer:
         if t[:, 4].sum() != 0:
             raise ValueError("a minibatch index was outside the rollout")
         means = t[:, :4] / np.asarray(sizes, np.float64)[:, None]
-        entropy = log_std_sums[:len(sizes)].cpu().numpy() + 3 * (0.5 + _LOG_SQRT_2PI)     # per minibatch
+        if sde:                                  # mean per-sample entropy of each minibatch
+            entropy = t[:, 5] / np.asarray(sizes, np.float64)
+        else:
+            entropy = log_std_sums[:len(sizes)].cpu().numpy() + 3 * (0.5 + _LOG_SQRT_2PI)     # per minibatch
         log_std = self.params.log_std.detach().double().cpu().numpy()
         v, r = rollout["values"].reshape(-1).double(), rollout["returns"].reshape(-1).double()
         var_r = float(r.var())
@@ -286,7 +330,8 @@ class PPOTrainer:
         while self.num_timesteps < total_timesteps:
             b.reset_stats()
             ro = b.collect_rollout(cfg.n_steps, self.params.mlp(), gamma=cfg.gamma, gae_lambda=cfg.gae_lambda,
-                                   tensor_cores=cfg.tensor_cores, bootstrap_truncated=True)
+                                   tensor_cores=cfg.tensor_cores, bootstrap_truncated=True,
+                                   sde_sample_freq=cfg.sde_sample_freq)
             self.num_timesteps += cfg.n_steps * b.num_envs
             self.progress_remaining = 1.0 - self.num_timesteps / total_timesteps
             log = {"rollout/" + k: v for k, v in b.stats_dict().items()}
