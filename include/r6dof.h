@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 19
+#define R6_ABI_VERSION 20
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -162,13 +162,22 @@ typedef struct R6Buffers {
                                to be the largest root, otherwise the cold start runs */
 } R6Buffers;
 
-/* Weights of the SB3 MlpPolicy actor (net_arch [128, 64], tanh), float32 row-major [out][in]. */
+/*
+ * Weights of the SB3 MlpPolicy actor (net_arch [128, 64], tanh), float32 row-major [out][in].
+ * With the value tower set (vf_w0 != NULL) the network is instead SB3 1.6's default separate towers,
+ * net_arch [dict(pi=[64, 64], vf=[64, 64])]: w0 [64][13], b0 [64], w1 [64][64], b1 [64] are the policy tower
+ * (mlp_extractor.policy_net), vf_* the value tower (mlp_extractor.value_net); w2, b2 read the policy latent and
+ * wv, bv the value latent.  Entry points without a separate-tower kernel return R6_EINVAL for such a network:
+ * r6_policy* with tensor_cores = 1, r6_rollout with R6_ACT_MLP / R6_ACT_MLP_TC, r6_policy_sde_range, r6_ppo_grad_sde.
+ */
 typedef struct R6Mlp {
-    const float *w0, *b0;   /* [128][13], [128] */
-    const float *w1, *b1;   /* [64][128], [64]  */
+    const float *w0, *b0;   /* [128][13], [128]   (separate towers: [64][13], [64]) */
+    const float *w1, *b1;   /* [64][128], [64]    (separate towers: [64][64], [64]) */
     const float *w2, *b2;   /* [3][64],  [3]    action_net */
     const float *wv, *bv;   /* [64], [1] nullable: value_net on the same latent (the critic of the shared-trunk policy) */
     const float *log_std;   /* [3] nullable: state-independent log standard deviation of the Gaussian policy */
+    const float *vf_w0, *vf_b0;   /* [64][13], [64] nullable: value tower layer 0 (all four set, or none) */
+    const float *vf_w1, *vf_b1;   /* [64][64], [64] nullable: value tower layer 1 */
 } R6Mlp;
 
 int r6_abi_version(void);
@@ -261,7 +270,7 @@ int r6_tgo(const double *c2, const double *c3, const double *c4, double c0, int6
  * tensor memory, single pass (fast mode, |d action| ~2e-3 vs mode 0); 3: the same kernel with 3xTF32 compensation
  * chained into one TMEM accumulator and a float32-accurate tanh (faithful mode, |d action| <= 3e-6 vs mode 0 and vs
  * the reference's recorded actions; the mode the closed-loop and PPO-collection paths use by default).  Modes 2 and 3
- * need mlp->w1 16-byte aligned.
+ * need mlp->w1 (and with the separate towers mlp->vf_w1) 16-byte aligned.  The separate towers run in modes 0, 2, 3.
  */
 int r6_policy(const R6Mlp *mlp, const float *obs, int64_t n, int32_t tensor_cores, float *actions, void *stream);
 
@@ -368,8 +377,16 @@ int r6_trunc_bootstrap(float *rew, int32_t T, int64_t n, int32_t slots, const in
  *     wv [64] @10243, bv [1] @10307, log_std [3] @10308
  * (w1 starts at float 1792 so that an R6Mlp pointing into a 16-byte aligned buffer keeps w1 16-byte aligned, as
  * r6_policy tensor_cores = 2 / 3 need).
+ *
+ * The separate-tower layout (R6Mlp with the value tower), R6_PPO_NPARAMS_SEP float32:
+ *     w0 [64][13] @0, vf_w0 [64][13] @832, b0 [64] @1664, vf_b0 [64] @1728, w1 [64][64] @1792, b1 [64] @5888,
+ *     vf_w1 [64][64] @5952, vf_b1 [64] @10048, w2 [3][64] @10112, b2 [3] @10304, wv [64] @10307, bv [1] @10371,
+ *     log_std [3] @10372
+ * (the two layer-0 blocks stacked are the shared layout's [128][13] + [128]; w1 and vf_w1 are 16-byte aligned).
+ * r6_ppo_grad takes the layout of its mlp: grad_sum has R6_PPO_NPARAMS_SEP elements when the value tower is set.
  */
 #define R6_PPO_NPARAMS 10311
+#define R6_PPO_NPARAMS_SEP 10375
 #define R6_PPO_NTERMS 5
 /* terms[] slots of r6_ppo_grad (float64 sums over the minibatch) */
 enum { R6_PPO_T_PG = 0, R6_PPO_T_VLOSS, R6_PPO_T_CLIPPED, R6_PPO_T_APPROX_KL, R6_PPO_T_BAD_INDEX };
@@ -403,7 +420,7 @@ int r6_ppo_rollout_size(void);
 int r6_ppo_coef_size(void);
 int r6_adam_coef_size(void);
 
-/* Size of r6_ppo_grad's work buffer for a minibatch of B samples (DEVICE bytes, no initialisation needed). */
+/* Size of r6_ppo_grad's work buffer for a minibatch of B samples, either layout (DEVICE bytes, no initialisation needed). */
 int64_t r6_ppo_work_bytes(int64_t B);
 
 /*

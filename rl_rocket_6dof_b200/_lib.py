@@ -12,7 +12,7 @@ from .params import R6Params
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libr6dof.so")
-ABI_VERSION = 19
+ABI_VERSION = 20
 
 u8p = C.c_void_p
 
@@ -38,7 +38,8 @@ class R6Buffers(C.Structure):
 class R6Mlp(C.Structure):
     _fields_ = [("w0", C.c_void_p), ("b0", C.c_void_p), ("w1", C.c_void_p), ("b1", C.c_void_p),
                 ("w2", C.c_void_p), ("b2", C.c_void_p),
-                ("wv", C.c_void_p), ("bv", C.c_void_p), ("log_std", C.c_void_p)]     # nullable: critic head, Gaussian log-std
+                ("wv", C.c_void_p), ("bv", C.c_void_p), ("log_std", C.c_void_p),    # nullable: critic head, Gaussian log-std
+                ("vf_w0", C.c_void_p), ("vf_b0", C.c_void_p), ("vf_w1", C.c_void_p), ("vf_b1", C.c_void_p)]  # nullable: value tower
 
 
 class R6PpoRollout(C.Structure):
@@ -63,12 +64,14 @@ class R6Sde(C.Structure):
 PPO_NPARAMS = 10311
 PPO_NTERMS = 5
 PPO_NPARAMS_SDE = 10500
+PPO_NPARAMS_SEP = 10375
 PPO_NTERMS_SDE = 6
 SDE_NXI = 192
 
 
 def make_mlp(weights: dict) -> "R6Mlp":
-    """R6Mlp from a dict of tensors / arrays exposing data_ptr() or ctypes.data (optional keys: wv, bv, log_std)."""
+    """R6Mlp from a dict of tensors / arrays exposing data_ptr() or ctypes.data (optional keys: wv, bv, log_std, and
+    the separate value tower vf_w0, vf_b0, vf_w1, vf_b1)."""
     def ptr(x):
         if x is None:
             return None
@@ -78,6 +81,8 @@ def make_mlp(weights: dict) -> "R6Mlp":
     if ls is not None and len(ls.shape) == 2:          # gSDE [64, 3]: passed through R6Sde, never as the Gaussian [3]
         ls = None
     m.wv, m.bv, m.log_std = ptr(weights.get("wv")), ptr(weights.get("bv")), ptr(ls)
+    m.vf_w0, m.vf_b0 = ptr(weights.get("vf_w0")), ptr(weights.get("vf_b0"))
+    m.vf_w1, m.vf_b1 = ptr(weights.get("vf_w1")), ptr(weights.get("vf_b1"))
     return m
 
 

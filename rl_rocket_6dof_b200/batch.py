@@ -28,6 +28,17 @@ MULTIPASS_MIN_ENVS = 1 << 18   # smallest batch the multi-pass integrator is the
 STAT_NAMES = ["episodes", "return_sum", "length_sum", "landed", "ground", "out_of_bounds", "truncated", "steps"]
 
 
+def _check_separate(mlp: dict, tensor_cores):
+    """Refuses, before anything is launched, what the kernels do not run for SB3 1.6's separate policy / value towers."""
+    if mlp.get("vf_w0") is None:
+        return
+    if int(tensor_cores) == 1:
+        raise ValueError("the separate policy / value towers have no mma.sync policy kernel (tensor_cores=1): use 0, 2 or 3")
+    ls = mlp.get("log_std")
+    if ls is not None and ls.dim() == 2:
+        raise ValueError("gSDE is not implemented for the separate policy / value towers")
+
+
 class Rocket6DOFBatch:
     """Batched env.  All tensors are CUDA tensors on `device`; nothing is computed on the host."""
 
@@ -382,6 +393,9 @@ class Rocket6DOFBatch:
         values, all without a host synchronise.  Needs auto-reset (ValueError otherwise).  The default False leaves the
         rewards as the env returned them.
 
+        `mlp` may hold SB3 1.6's separate policy / value towers (vf_w0 ... vf_b1, `ActorCriticParams.LAYOUT_SEP`): the
+        values are then the value tower's.  That network has no mma.sync kernel: tensor_cores=1 raises ValueError.
+
         A [64, 3] log_std in `mlp` collects with gSDE, as SB3's collect_rollouts with use_sde=True: `reset_noise` at the
         start of the rollout, and with sde_sample_freq > 0 every lane redraws the noise of its env range before step j
         whenever j % sde_sample_freq == 0, keyed by steps_done + j (step 0 reuses the start draw, which has that key).
@@ -394,6 +408,7 @@ class Rocket6DOFBatch:
         from .gae import compute_gae
         k = int(k)
         n, dev = self.num_envs, self.device
+        _check_separate(mlp, tensor_cores)
         if bootstrap_truncated and not self.auto_reset:
             raise ValueError("bootstrap_truncated needs auto_reset=True (a frozen one-episode env keeps its flags)")
         self.join()
@@ -469,7 +484,9 @@ class Rocket6DOFBatch:
         the actions, the step kernel consumes them — VecEnv semantics (auto-reset as configured).  Faster than the
         single fused rollout kernel for large batches; `rollout(k, ACT_MLP)` remains for one-episode semantics.
         With stream lanes every lane runs its own policy -> step chain (r6_policy_range, r6_step_range) for the k
-        steps and the lanes are joined at the end (join=False leaves them running, as in `step`)."""
+        steps and the lanes are joined at the end (join=False leaves them running, as in `step`).  SB3 1.6's separate
+        policy / value towers run in modes 0, 2 and 3; tensor_cores=1 raises ValueError for them."""
+        _check_separate(mlp, tensor_cores)
         act = getattr(self, "_policy_act", None)
         if act is None:
             act = self._policy_act = torch.empty(self.num_envs, 3, dtype=torch.float32, device=self.device)

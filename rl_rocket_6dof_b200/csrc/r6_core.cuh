@@ -1589,6 +1589,87 @@ R6_HD void mlp_policy(const float *W, const float *x, float &a0, float &a1, floa
     a2 = fminf(fmaxf(out[2], -1.0f), 1.0f);
 }
 
+// ------------------------------------------------------------------------------------------------
+// SB3 1.6's default MlpPolicy without policy_kwargs: separate tanh towers net_arch [dict(pi=[64, 64], vf=[64, 64])],
+// action_net on the policy latent, value_net on the value latent (R6Mlp with vf_w0 set).  The packed block keeps the
+// shared layout's offsets with the two towers stacked, plus the value tower's second bias:
+//     [0, 2048)        W0 rows: j < 64 the policy tower's w0[j], j >= 64 the value tower's vf_w0[j - 64] (with b0 / vf_b0)
+//     [2048, 10240)    W1 transposed [in j][out k]: j < 64 w1[k][j] (policy), j >= 64 vf_w1[k][j - 64] (value)
+//     [10240, 10304)   b1 (policy)   [10304, 10560) W2 [4][64]: rows 0..2 action_net, row 3 value_net   [10560, 10564) b2, bv
+//     [10564, 10628)   vf_b1
+// The same multiply-adds as the shared trunk (13 x 128 + 2 x 64 x 64 = 13 x 128 + 128 x 64), 256 tanh instead of 192.
+constexpr int kMlpOffVb1 = kMlpFloats, kMlpFloatsSep = kMlpOffVb1 + kMlpH1;
+static_assert(2 * kMlpH1 == kMlpH0, "the two towers stack into the shared trunk's layer 0");
+
+R6_HD bool mlp_separate(const R6Mlp &m) { return m.vf_w0 != nullptr; }
+
+R6_HD float mlp_pack_element_sep(const R6Mlp &m, int idx)
+{
+    if (idx < kMlpOffW1) {
+        const int j = idx >> 4, i = idx & 15;
+        const float *w0 = j < kMlpH1 ? m.w0 + j * kMlpIn : m.vf_w0 + (j - kMlpH1) * kMlpIn;
+        const float b0 = j < kMlpH1 ? m.b0[j] : m.vf_b0[j - kMlpH1];
+        return i < kMlpIn ? w0[i] : (i == kMlpIn ? b0 : 0.0f);
+    }
+    if (idx < kMlpOffB1) {
+        const int r = idx - kMlpOffW1, j = r / kMlpH1, k = r % kMlpH1;
+        return j < kMlpH1 ? m.w1[k * kMlpH1 + j] : m.vf_w1[k * kMlpH1 + j - kMlpH1];
+    }
+    if (idx < kMlpOffVb1) return mlp_pack_element(m, idx);      // b1, W2 rows, b2 / bv: as the shared layout
+    return m.vf_b1[idx - kMlpOffVb1];
+}
+
+// acc[k] = sum over the 64 layer-0 units j0 .. j0 + 63 of W1T[j][k] tanh(W0[j] x + b0[j]): one tower's layer 1 before
+// its bias (mlp_forward_latent's loop over half of the stacked units).  unit0(j, h) sees every layer-0 activation.
+template <int j0, class Unit0>
+R6_HD void mlp_tower_acc(const float *W, const float *x, float (&acc)[kMlpH1], Unit0 &&unit0)
+{
+#pragma unroll
+    for (int k = 0; k < kMlpH1; k++) acc[k] = 0.0f;
+#pragma unroll 2
+    for (int j = j0; j < j0 + kMlpH1; j++) {
+        const F4 wa = ld4(W + j * 16), wb = ld4(W + j * 16 + 4), wc = ld4(W + j * 16 + 8), wd = ld4(W + j * 16 + 12);
+        float s = wa.x * x[0];
+        s = f32_fma(wa.y, x[1], s); s = f32_fma(wa.z, x[2], s); s = f32_fma(wa.w, x[3], s);
+        s = f32_fma(wb.x, x[4], s); s = f32_fma(wb.y, x[5], s); s = f32_fma(wb.z, x[6], s); s = f32_fma(wb.w, x[7], s);
+        s = f32_fma(wc.x, x[8], s); s = f32_fma(wc.y, x[9], s); s = f32_fma(wc.z, x[10], s); s = f32_fma(wc.w, x[11], s);
+        s = f32_fma(wd.x, x[12], s);
+        const float h = tanhf(s + wd.y);
+        unit0(j, h);
+        const float *w1 = W + kMlpOffW1 + j * kMlpH1;
+#pragma unroll
+        for (int k = 0; k < kMlpH1; k += 4) {
+            const F4 w = ld4(w1 + k);
+            acc[k] = f32_fma(w.x, h, acc[k]); acc[k + 1] = f32_fma(w.y, h, acc[k + 1]);
+            acc[k + 2] = f32_fma(w.z, h, acc[k + 2]); acc[k + 3] = f32_fma(w.w, h, acc[k + 3]);
+        }
+    }
+}
+
+// mlp_forward over the separate towers (packed by mlp_pack_element_sep): the value tower first, reduced to the value
+// as its latent is formed, then the policy tower in the same 64 accumulators.  out as mlp_forward.
+R6_HD void mlp_forward_sep(const float *W, const float *x, float (&out)[4])
+{
+    float acc[kMlpH1];
+    mlp_tower_acc<kMlpH1>(W, x, acc, [](int, float) {});
+    float o3 = 0.0f;
+#pragma unroll
+    for (int k = 0; k < kMlpH1; k++) o3 = f32_fma(W[kMlpOffW2 + 3 * kMlpH1 + k], tanhf(acc[k] + W[kMlpOffVb1 + k]), o3);
+    mlp_tower_acc<0>(W, x, acc, [](int, float) {});
+    float o0 = 0.0f, o1 = 0.0f, o2 = 0.0f;
+#pragma unroll
+    for (int k = 0; k < kMlpH1; k++) {
+        const float h = tanhf(acc[k] + W[kMlpOffB1 + k]);
+        o0 = f32_fma(W[kMlpOffW2 + k], h, o0);
+        o1 = f32_fma(W[kMlpOffW2 + kMlpH1 + k], h, o1);
+        o2 = f32_fma(W[kMlpOffW2 + 2 * kMlpH1 + k], h, o2);
+    }
+    out[0] = o0 + W[kMlpOffB2];
+    out[1] = o1 + W[kMlpOffB2 + 1];
+    out[2] = o2 + W[kMlpOffB2 + 2];
+    out[3] = o3 + W[kMlpOffB2 + 3];
+}
+
 // sin(pi x), cos(pi x): exact argument reduction, 1 ulp (CUDA math library); the host build in double precision
 R6_HD void sincospi_f32(float x, float &s, float &c)
 {

@@ -11,6 +11,7 @@
 //   policy_kernel, policy_tc5_kernel   the policy MLP alone: float32 FMAs, mma.sync 3xTF32 tiles, or tcgen05.mma with
 //                                    accumulators and activations in TMEM (r6_mlp_tc.cuh, r6_mlp_tcgen05.cuh)
 //   ppo_grad_kernel | ppo_reduce_kernel, adam_kernel   the PPO update: minibatch loss gradient, Adam step
+//   (policy_sep_kernel, policy_tc5_sep_kernel, ppo_grad_sep_kernel: the same for SB3 1.6's separate policy / value towers)
 //   trunc_record_kernel, trunc_bootstrap_kernel   time-limit truncations filed per step, bootstrapped with the critic
 //   reset_kernel, sim_raw_kernel, tgo_kernel, gae_kernel, peak_fma_kernel
 //
@@ -943,6 +944,172 @@ policy_tc5_kernel(const R6Mlp mlp, const float *__restrict__ obs, int64_t n, con
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
 }
 
+// policy_kernel<false> for SB3 1.6's separate towers (R6Mlp with the value tower): mlp_forward_sep.  At the shared
+// kernel's four CTAs per SM (128 registers) ptxas spills 276 B of it (the shared kernel: 24 B); it asks for 255
+// registers unbounded, so fewer CTAs per SM do not remove the spill (three: 168 registers, 220 B).
+__global__ void __launch_bounds__(kThreads, 4)
+policy_sep_kernel(const R6Mlp mlp, const float *__restrict__ obs, int64_t n, const PolicyOut po)
+{
+    extern __shared__ __align__(16) double r6_smem[];
+    float *Ws = reinterpret_cast<float *>(r6_smem);
+    for (int idx = threadIdx.x; idx < kMlpFloatsSep; idx += kThreads) Ws[idx] = mlp_pack_element_sep(mlp, idx);
+    __syncthreads();
+    const int64_t i1 = po.i1;
+    const int64_t tiles = (i1 - po.i0 + kThreads - 1) / kThreads;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        const int64_t i = po.i0 + tile * kThreads + threadIdx.x;
+        float x[kMlpIn], out[4];
+#pragma unroll
+        for (int c = 0; c < kMlpIn; c++) x[c] = i < i1 ? obs[(int64_t)c * n + i] : 0.0f;
+        mlp_forward_sep(Ws, x, out);
+        if (i < i1) policy_epilogue(po, mlp.log_std, i, out);
+    }
+}
+constexpr int kSmemPolicySep = r6::kMlpFloatsSep * (int)sizeof(float);
+
+// policy_tc5_kernel for the separate towers (r6_policy tensor_cores = 2 / 3 with the value tower set): stacked layer 0,
+// then the value chain (reduced to the value in its epilogue), then the policy chain and the action head.  Schedule and
+// TMEM use: r6_mlp_tcgen05.cuh.  A copy of policy_tc5_kernel rather than a template flag of it, so that the shared-trunk
+// kernel keeps its register allocation.
+template <bool kFaithful>
+__global__ void __launch_bounds__(tc5::kThreads, 1)
+policy_tc5_sep_kernel(const R6Mlp mlp, const float *__restrict__ obs, int64_t n, const PolicyOut po)
+{
+    using namespace tc5;
+    extern __shared__ __align__(16) double r6_smem[];
+    char *S = reinterpret_cast<char *>(r6_smem);
+    const int tid = threadIdx.x, group = tid >> 8, lt = tid & 127, half = (tid >> 7) & 1, warp = tid >> 5;
+    grid_dependency_wait();
+    // ---- one-time per CTA: [w0; vf_w0] and [w1 | vf_w1] split into TF32 hi / lo parts in canonical K-major tiles ----
+    for (int idx = tid; idx < 128 * 16; idx += tc5::kThreads) {
+        const int r = idx >> 4, k = idx & 15;
+        const float *w0 = r < kMlpH1 ? mlp.w0 + r * kMlpIn : mlp.vf_w0 + (r - kMlpH1) * kMlpIn;
+        float hi, lo;
+        split_tf32(k < kMlpIn ? w0[k] : 0.0f, hi, lo);
+        *reinterpret_cast<float *>(S + kOffW0h + tile_off(r, k, 16)) = hi;
+        *reinterpret_cast<float *>(S + kOffW0l + tile_off(r, k, 16)) = lo;
+    }
+    for (int idx = tid; idx < 64 * 32; idx += tc5::kThreads) {
+        const int r = idx >> 5, k = (idx & 31) * 4;
+        const float *src = k < kMlpH1 ? mlp.w1 + r * kMlpH1 + k : mlp.vf_w1 + r * kMlpH1 + (k - kMlpH1);
+        const float4 w = *reinterpret_cast<const float4 *>(src);
+        float4 h, l;
+        split_tf32(w.x, h.x, l.x); split_tf32(w.y, h.y, l.y); split_tf32(w.z, h.z, l.z); split_tf32(w.w, h.w, l.w);
+        *reinterpret_cast<float4 *>(S + kOffW1h + tile_off(r, k, 128)) = h;
+        *reinterpret_cast<float4 *>(S + kOffW1l + tile_off(r, k, 128)) = l;
+    }
+    for (int idx = tid; idx < 16 * 16; idx += tc5::kThreads) {        // action_net rows 0..2; row 3 (value) stays zero
+        const int r = idx >> 4, k = (idx & 15) * 4;
+        float4 h, l;
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k] : 0.0f, h.x, l.x);
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k + 1] : 0.0f, h.y, l.y);
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k + 2] : 0.0f, h.z, l.z);
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k + 3] : 0.0f, h.w, l.w);
+        *reinterpret_cast<float4 *>(S + kOffW2h + tile_off(r, k, 64)) = h;
+        *reinterpret_cast<float4 *>(S + kOffW2l + tile_off(r, k, 64)) = l;
+    }
+    float *bias = reinterpret_cast<float *>(S + kOffBias);
+    float *vb1 = reinterpret_cast<float *>(S + kOffSep), *wv = reinterpret_cast<float *>(S + kOffSepWv);
+    float *vpart = reinterpret_cast<float *>(S + kOffSepPart) + group * kTile;
+    const float bscale = kFaithful ? kTwoLog2e : 1.0f;
+    if (tid < 64) bias[tid] = bscale * mlp.b0[tid];
+    else if (tid < 128) bias[tid] = bscale * mlp.vf_b0[tid - 64];
+    if (tid < 64) {
+        bias[128 + tid] = bscale * mlp.b1[tid];
+        vb1[tid] = bscale * mlp.vf_b1[tid];
+        wv[tid] = mlp.wv != nullptr ? mlp.wv[tid] : 0.0f;
+    }
+    if (tid < 4) bias[192 + tid] = mlp_b2_row(mlp, tid);
+    if (tid == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(S + kOffBar)) : "memory");
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(S + kOffBar + 8)) : "memory");
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(S + kOffTmemPtr)), "n"(kTmemCols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    fence_async_smem();
+    fence_before();
+    __syncthreads();
+    fence_after();
+    const int warp_u = __shfl_sync(0xffffffffu, warp, 0);
+    const uint32_t tmem_base = __shfl_sync(0xffffffffu, *reinterpret_cast<volatile uint32_t *>(S + kOffTmemPtr), 0);
+    const uint32_t tmem_g = tmem_base + (uint32_t)(warp_u >> 3) * kGroupCols;
+    const uint32_t tmem_row = tmem_g + ((uint32_t)((warp & 3) * 32) << 16);
+    const uint32_t sbase = __shfl_sync(0xffffffffu, smem_u32(S), 0);
+    const uint32_t aW0h = sbase + kOffW0h, aW0l = sbase + kOffW0l, aW1h = sbase + kOffW1h;
+    const uint32_t aW1l = sbase + kOffW1l, aW2h = sbase + kOffW2h, aW2l = sbase + kOffW2l;
+    const uint32_t bar = sbase + kOffBar + 8 * (uint32_t)(warp_u >> 3);
+    const bool issuer = (warp_u & 7) == 0;
+    uint32_t phase = 0;
+    const int64_t i1 = po.i1;
+    const int64_t tiles = (i1 - po.i0 + kTile - 1) / kTile;
+    const int64_t slots = (tiles + 2 * (int64_t)gridDim.x - 1) / (2 * (int64_t)gridDim.x);
+    float xo[8];
+    auto load_obs = [&](int64_t tile) {
+        const int64_t i = po.i0 + tile * kTile + lt;
+#pragma unroll
+        for (int q = 0; q < 8; q++) {
+            const int k = 8 * half + q;
+            xo[q] = (k < kMlpIn && i < i1) ? __ldg(obs + (int64_t)k * n + i) : 0.0f;
+        }
+    };
+    load_obs(2 * (int64_t)blockIdx.x + group);
+    float outv[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+    int64_t out_i = i1;
+    if (group == 1) token_pass(0);
+    for (int64_t slot = 0; slot < slots; slot++) {
+        const int64_t tile = 2 * ((int64_t)blockIdx.x + slot * gridDim.x) + group;
+        const int64_t i = po.i0 + tile * kTile + lt;
+        {
+            float h[8], l[8];
+#pragma unroll
+            for (int q = 0; q < 8; q++) split_tf32(xo[q], h[q], l[q]);
+            tmem_st8(tmem_row + kColD1 + 8 * half, h);
+            if (kFaithful) tmem_st8(tmem_row + kColL + 8 * half, l);
+            tmem_st_wait();
+        }
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD0, tmem_g + kColD1, tmem_g + kColL, aW0h, aW0l, 512, 2, 128, false); if (elect_one()) mma_commit(bar); }
+        load_obs(tile + 2 * (int64_t)gridDim.x);
+        if (half == 0 && out_i < i1) policy_epilogue(po, mlp.log_std, out_i, outv);
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- value tower: layer 0 units 64..127 -> its layer 1 (W1 columns 64..127 = vf_w1) ----
+        epilogue_in_tmem<kFaithful>(tmem_row, kColD0 + 64, bias + 64, half, group);
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD1, tmem_g + kColD0 + 64, tmem_g + kColL, aW1h + 2048, aW1l + 2048, 4096, 8, 64, false); if (elect_one()) mma_commit(bar); }
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- value = value_net(tanh(D1 + vf_b1)) on the CUDA cores; the second half's sum goes through shared memory ----
+        const float vs = epilogue_value<kFaithful>(tmem_row, kColD1, vb1, wv, half, group);
+        if (half == 1) vpart[lt] = vs;
+        // ---- policy tower: layer 0 units 0..63 -> its layer 1 (W1 columns 0..63 = w1), over the value chain's D1 ----
+        epilogue_in_tmem<kFaithful>(tmem_row, kColD0, bias, half, group);
+        fence_before(); group_sync(group);       // also publishes vpart to the first half
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD1, tmem_g + kColD0, tmem_g + kColL, aW1h, aW1l, 4096, 8, 64, false); if (elect_one()) mma_commit(bar); }
+        const float value = half == 0 ? vs + vpart[lt] : 0.0f;
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- policy latent -> action_net ----
+        epilogue_in_tmem<kFaithful>(tmem_row, kColD1, bias + 128, half, group);
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD0, tmem_g + kColD1, tmem_g + kColL, aW2h, aW2l, 2048, 8, 16, false); if (elect_one()) mma_commit(bar); }
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        out_i = i1;
+        if (half == 0) {
+            tmem_ld4(tmem_row + kColD0, outv);
+#pragma unroll
+            for (int q = 0; q < 3; q++) outv[q] += bias[192 + q];
+            outv[3] = value + bias[195];
+            out_i = i;
+        }
+    }
+    if (half == 0 && out_i < i1) policy_epilogue(po, mlp.log_std, out_i, outv);
+    if (group == 0) token_take(0);
+    fence_before();
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
+}
+
 // policy_tc5_kernel with the gSDE head (r6_policy_sde_range tensor_cores = 2 / 3): the sums h E and h^2 sigma^2 are
 // formed in the last hidden layer's epilogue (epilogue_in_tmem_sde), where each of the two threads of an env row holds
 // 32 of the 64 activations; the second half hands its sums to the first through shared memory (kOffSdePart), and the
@@ -1389,6 +1556,212 @@ ppo_grad_sde_kernel(const R6Mlp mlp, const float *__restrict__ log_std, const R6
     ppo_grad_body<true>(mlp, log_std, ro, idx, B, clip, vf, ent, adv_stats, part_terms, part);
 }
 
+// r6_ppo_grad for SB3 1.6's separate towers (ppo_grad_sep_kernel).  The same tiles, CTA count, accumulators and
+// reduction as ppo_grad_kernel; the [unit][sample] tile keeps its 284 rows by giving the latent rows to the deltas in
+// place: rows 128..191 hold the policy latent h1p, rows 192..255 the value latent h1v, both overwritten by their
+// delta1 once the head gradients (dW2 from h1p, dwv from h1v) have been accumulated.  The 8 x 8 dW1 block of a thread
+// covers dW1p[k][j] for its columns j < 64 and dW1v[k][j - 64] for j >= 64 (the stacked layer-0 units), and delta0 of
+// unit j comes from its own tower's delta1.  225,232 B of shared memory (vf_b1 joins the packed weights).
+constexpr int kPpoRowHP = 128, kPpoRowHV = 192;
+constexpr int kSmemPpoSep = (kMlpFloatsSep + kPpoRows * kPpoTS + kPpoAccW1) * (int)sizeof(float);
+static_assert(kMlpFloatsSep % 4 == 0 && kPpoRowHP == kPpoRowH1 && kPpoRowHV == kPpoRowD1 && kSmemPpoSep <= 232448,
+              "PPO separate-tower tile layout");
+
+__global__ void __launch_bounds__(kThreads, 1)
+ppo_grad_sep_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restrict__ idx, int64_t B, float clip, float vf,
+                    float ent, const double *__restrict__ adv_stats, double *__restrict__ part_terms, float *__restrict__ part)
+{
+    extern __shared__ __align__(16) double r6_smem[];
+    float *Ws = reinterpret_cast<float *>(r6_smem);
+    float *S = Ws + kMlpFloatsSep;
+    float *A1 = S + kPpoRows * kPpoTS;
+    const int tid = threadIdx.x, kq = tid & 7, jq = tid >> 3;
+    for (int i = tid; i < kMlpFloatsSep; i += kThreads) Ws[i] = mlp_pack_element_sep(mlp, i);
+    for (int i = tid; i < kPpoAccW1; i += kThreads) A1[i] = 0.0f;
+    const int64_t nsamp = ro.T * ro.n;
+    float aW0[14], aHd[6];                   // dW0 / dvf_w0 row tid, its bias; dW2[0..2][tid], dwv, db1, dvf_b1
+    double aS = 0.0;
+#pragma unroll
+    for (int c = 0; c < 14; c++) aW0[c] = 0.0f;
+#pragma unroll
+    for (int c = 0; c < 6; c++) aHd[c] = 0.0f;
+    __syncthreads();
+    const int64_t tiles = (B + kThreads - 1) / kThreads;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        PpoHead hd = {};
+        {   // this thread's sample: forward and loss head
+            const int64_t s = tile * kThreads + tid;
+            const int64_t q = s < B ? idx[s] : -1;
+            const bool ok = q >= 0 && q < nsamp;
+            float x[kMlpIn], out[4];
+            if (ok) {
+                const int64_t t = q / ro.n, i = q - t * ro.n;
+                const float *o = ro.obs + t * ro.obs_stride_step + i * ro.obs_stride_env;
+#pragma unroll
+                for (int c = 0; c < kMlpIn; c++) x[c] = o[c * ro.obs_stride_comp];
+            } else {
+#pragma unroll
+                for (int c = 0; c < kMlpIn; c++) x[c] = 0.0f;
+            }
+#pragma unroll
+            for (int c = 0; c < kMlpIn; c++) S[(kPpoRowX + c) * kPpoTS + tid] = x[c];
+            ppo_forward_sep(Ws, x, S + kPpoRowH0 * kPpoTS + tid, S + kPpoRowHP * kPpoTS + tid, S + kPpoRowHV * kPpoTS + tid,
+                            kPpoTS, out);
+            if (ok) {
+                const float a[3] = {ro.actions[3 * q], ro.actions[3 * q + 1], ro.actions[3 * q + 2]};
+                ppo_head(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], mlp.log_std, clip,
+                         vf, ent, hd);
+            }
+#pragma unroll
+            for (int r = 0; r < 7; r++) S[(kPpoRowG + r) * kPpoTS + tid] = hd.g[r];
+            S[(kPpoRowG + 7) * kPpoTS + tid] = (s < B && !ok) ? 1.0f : 0.0f;
+            S[(kPpoRowT + 0) * kPpoTS + tid] = hd.pg;
+            S[(kPpoRowT + 1) * kPpoTS + tid] = hd.vloss;
+            S[(kPpoRowT + 2) * kPpoTS + tid] = hd.clipped;
+            S[(kPpoRowT + 3) * kPpoTS + tid] = hd.kl;
+        }
+        __syncthreads();
+        // heads from the latents (dW2 on h1p, dwv on h1v) and the scalar sums, before the latent rows become deltas
+        if (tid < kMlpH1) {
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                const F4 hp = ld4(S + (kPpoRowHP + tid) * kPpoTS + s4), hv = ld4(S + (kPpoRowHV + tid) * kPpoTS + s4);
+#pragma unroll
+                for (int c = 0; c < 4; c++) {
+                    const F4 g = ld4(S + (kPpoRowG + c) * kPpoTS + s4);
+                    const F4 h = c < 3 ? hp : hv;
+                    float a = aHd[c];
+                    a = __fmaf_rn(g.x, h.x, a); a = __fmaf_rn(g.y, h.y, a);
+                    a = __fmaf_rn(g.z, h.z, a); a = __fmaf_rn(g.w, h.w, a);
+                    aHd[c] = a;
+                }
+            }
+        } else if (tid < kMlpH1 + 12) {
+            const float *row = S + (kPpoRowG + tid - kMlpH1) * kPpoTS;
+#pragma unroll 4
+            for (int s = 0; s < kThreads; s++) aS += (double)row[s];
+        }
+        __syncthreads();
+        ppo_delta1_sep(Ws, hd, S + kPpoRowHP * kPpoTS + tid, S + kPpoRowHV * kPpoTS + tid, kPpoTS);
+        __syncthreads();
+        // dW1p / dW1v += delta1^T h0 (columns jq + 16 c: c < 4 policy units, c >= 4 value units), db1 / dvf_b1
+#pragma unroll 1
+        for (int r0 = 0; r0 < 8; r0 += 4) {
+            float aW1[4][8];
+#pragma unroll
+            for (int r = 0; r < 4; r++)
+#pragma unroll
+                for (int c = 0; c < 8; c++) aW1[r][c] = A1[((r0 + r) * 8 + c) * kThreads + tid];
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                F4 h[8];
+#pragma unroll
+                for (int c = 0; c < 8; c++) h[c] = ld4(S + (kPpoRowH0 + jq + 16 * c) * kPpoTS + s4);
+#pragma unroll
+                for (int r = 0; r < 4; r++) {
+                    const F4 dp = ld4(S + (kPpoRowHP + kq + 8 * (r0 + r)) * kPpoTS + s4);
+                    const F4 dv = ld4(S + (kPpoRowHV + kq + 8 * (r0 + r)) * kPpoTS + s4);
+#pragma unroll
+                    for (int c = 0; c < 8; c++) {
+                        const F4 d = c < 4 ? dp : dv;
+                        float a = aW1[r][c];
+                        a = __fmaf_rn(d.x, h[c].x, a); a = __fmaf_rn(d.y, h[c].y, a);
+                        a = __fmaf_rn(d.z, h[c].z, a); a = __fmaf_rn(d.w, h[c].w, a);
+                        aW1[r][c] = a;
+                    }
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < 4; r++)
+#pragma unroll
+                for (int c = 0; c < 8; c++) A1[((r0 + r) * 8 + c) * kThreads + tid] = aW1[r][c];
+        }
+        if (tid < kMlpH1) {
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                const F4 dp = ld4(S + (kPpoRowHP + tid) * kPpoTS + s4), dv = ld4(S + (kPpoRowHV + tid) * kPpoTS + s4);
+                aHd[4] = (((aHd[4] + dp.x) + dp.y) + dp.z) + dp.w;
+                aHd[5] = (((aHd[5] + dv.x) + dv.y) + dv.z) + dv.w;
+            }
+        }
+        __syncthreads();
+        {   // delta0 over h0, in place, each tower's units from its own delta1: this thread's column only
+            float d1[kMlpH1];
+#pragma unroll 1
+            for (int t = 0; t < 2; t++) {
+                const int row = t == 0 ? kPpoRowHP : kPpoRowHV;
+#pragma unroll
+                for (int k = 0; k < kMlpH1; k++) d1[k] = S[(row + k) * kPpoTS + tid];
+#pragma unroll 1
+                for (int j = t * kMlpH1; j < (t + 1) * kMlpH1; j++) {
+                    float *p = S + (kPpoRowH0 + j) * kPpoTS + tid;
+                    *p = ppo_delta0(Ws, j, d1, *p);
+                }
+            }
+        }
+        __syncthreads();
+        // dW0[tid] += delta0_tid [x, 1]   (rows 0..63 the policy tower's w0, 64..127 the value tower's: stacked in P)
+#pragma unroll 1
+        for (int s4 = 0; s4 < kThreads; s4 += 4) {
+            const F4 d = ld4(S + (kPpoRowH0 + tid) * kPpoTS + s4);
+#pragma unroll
+            for (int c = 0; c < kMlpIn; c++) {
+                const F4 xv = ld4(S + (kPpoRowX + c) * kPpoTS + s4);
+                float a = aW0[c];
+                a = __fmaf_rn(d.x, xv.x, a); a = __fmaf_rn(d.y, xv.y, a);
+                a = __fmaf_rn(d.z, xv.z, a); a = __fmaf_rn(d.w, xv.w, a);
+                aW0[c] = a;
+            }
+            aW0[13] = (((aW0[13] + d.x) + d.y) + d.z) + d.w;
+        }
+        __syncthreads();
+    }
+    float *P = part + (int64_t)blockIdx.x * kPpoParamsSep;
+#pragma unroll
+    for (int r = 0; r < 8; r++)
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            const int k = kq + 8 * r, j = jq + 16 * c;
+            P[(c < 4 ? kSepOffW1 + k * kMlpH1 + j : kSepOffVw1 + k * kMlpH1 + j - kMlpH1)] = A1[(r * 8 + c) * kThreads + tid];
+        }
+#pragma unroll
+    for (int c = 0; c < kMlpIn; c++) P[kSepOffW0 + tid * kMlpIn + c] = aW0[c];
+    P[kSepOffB0 + tid] = aW0[13];
+    if (tid < kMlpH1) {
+#pragma unroll
+        for (int c = 0; c < 3; c++) P[kSepOffW2 + c * kMlpH1 + tid] = aHd[c];
+        P[kSepOffWv + tid] = aHd[3];
+        P[kSepOffB1 + tid] = aHd[4];
+        P[kSepOffVb1 + tid] = aHd[5];
+    } else if (tid < kMlpH1 + 12) {
+        const int r = tid - kMlpH1;          // rows: g0..g2 (db2), g3 (dbv), g4..g6 (dlog_std), bad index, 4 loss terms
+        double *T = part_terms + (int64_t)blockIdx.x * R6_PPO_NTERMS;
+        if (r < 3) P[kSepOffB2 + r] = (float)aS;
+        else if (r == 3) P[kSepOffBv] = (float)aS;
+        else if (r < 7) P[kSepOffLogStd + r - 4] = (float)aS;
+        else if (r == 7) T[R6_PPO_T_BAD_INDEX] = aS;
+        else T[r - 8] = aS;
+    }
+}
+
+// ppo_reduce_kernel over the separate-tower layout
+__global__ void __launch_bounds__(256)
+ppo_reduce_sep_kernel(const double *__restrict__ part_terms, const float *__restrict__ part, int G, float *__restrict__ grad,
+                      double *__restrict__ terms)
+{
+    const int p = blockIdx.x * 256 + threadIdx.x;
+    if (p < kPpoParamsSep) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += (double)part[(int64_t)g * kPpoParamsSep + p];
+        grad[p] = (float)s;
+    }
+    if (blockIdx.x == 0 && threadIdx.x < R6_PPO_NTERMS) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += part_terms[g * R6_PPO_NTERMS + threadIdx.x];
+        terms[threadIdx.x] = s;
+    }
+}
+
 // grad[p] = sum of the CTA partials in CTA order (float64, rounded once); terms likewise
 __global__ void __launch_bounds__(256)
 ppo_reduce_kernel(const double *__restrict__ part_terms, const float *__restrict__ part, int G, float *__restrict__ grad,
@@ -1522,6 +1895,10 @@ int ensure_attributes()
     rc |= enable_smem(policy_sde_kernel, kSmemPolicySde);
     rc |= enable_smem(policy_tc5_sde_kernel<true>, tc5::kSmemBytesSde);
     rc |= enable_smem(policy_tc5_sde_kernel<false>, tc5::kSmemBytesSde);
+    rc |= enable_smem(policy_sep_kernel, kSmemPolicySep);
+    rc |= enable_smem(policy_tc5_sep_kernel<true>, tc5::kSmemBytesSep);
+    rc |= enable_smem(policy_tc5_sep_kernel<false>, tc5::kSmemBytesSep);
+    rc |= enable_smem(ppo_grad_sep_kernel, kSmemPpoSep);
     rc |= enable_smem(sim_raw_kernel<false>);
     rc |= enable_smem(sim_raw_kernel<true>);
     if (rc) return R6_ECUDA;
@@ -1582,6 +1959,15 @@ int check_mlp(const R6Mlp *mlp)
 {
     if (!mlp || !mlp->w0 || !mlp->b0 || !mlp->w1 || !mlp->b1 || !mlp->w2 || !mlp->b2)
         return fail(R6_EINVAL, "policy weights are null%s");
+    const int vf = (mlp->vf_w0 != nullptr) + (mlp->vf_b0 != nullptr) + (mlp->vf_w1 != nullptr) + (mlp->vf_b1 != nullptr);
+    if (vf != 0 && vf != 4) return fail(R6_EINVAL, "the value tower needs all of vf_w0, vf_b0, vf_w1, vf_b1 (or none)%s");
+    return R6_OK;
+}
+// the entry points without a separate-tower kernel refuse such a network rather than run the shared trunk on it
+int reject_separate(const R6Mlp *mlp, const char *what)
+{
+    if (mlp && mlp_separate(*mlp))
+        return fail(R6_EINVAL, "%s does not support the separate policy / value towers (R6Mlp.vf_w0 set)", what);
     return R6_OK;
 }
 
@@ -1711,6 +2097,8 @@ int r6_rollout(const R6Params *p, const R6Buffers *b, int64_t n, int64_t env_off
                const R6Mlp *mlp, const float *act_buf, uint64_t seed, int64_t step_base, float *traj_obs,
                float *traj_act, float *traj_rew, uint8_t *traj_done, void *stream)
 {
+    if (mode == R6_ACT_MLP || mode == R6_ACT_MLP_TC)
+        if (int rc = reject_separate(mlp, "r6_rollout with R6_ACT_MLP / R6_ACT_MLP_TC")) return rc;
     int rc = validate_step(p, b, n);
     if (rc) return rc;
     if (k < 0) return fail(R6_EINVAL, "k < 0%s");
@@ -1759,6 +2147,10 @@ int r6_policy_range(const R6Mlp *mlp, const float *obs, int64_t n, int64_t first
     if (n < 0) return fail(R6_EINVAL, "n < 0%s");
     if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
     if (tensor_cores < 0 || tensor_cores > 3) return fail(R6_EINVAL, "tensor_cores must be 0, 1, 2 or 3%s");
+    const bool sep = mlp_separate(*mlp);
+    if (sep && tensor_cores == 1) return reject_separate(mlp, "r6_policy with tensor_cores = 1 (mma.sync)");
+    if (sep && tensor_cores >= 2 && (reinterpret_cast<uintptr_t>(mlp->vf_w1) & 15u) != 0)
+        return fail(R6_EINVAL, "tensor_cores = 2 / 3 need vf_w1 16-byte aligned%s");
     if (count == 0) return R6_OK;
     int rc = ensure_attributes();
     if (rc) return rc;
@@ -1776,9 +2168,12 @@ int r6_policy_range(const R6Mlp *mlp, const float *obs, int64_t n, int64_t first
         if ((reinterpret_cast<uintptr_t>(mlp->w1) & 15u) != 0) return fail(R6_EINVAL, "tensor_cores = 2 / 3 need w1 16-byte aligned%s");
         const int64_t pairs = (blocks_for(count) + 1) / 2;                 // one CTA per SM, two tile groups per CTA
         const unsigned g5 = (unsigned)(pairs < sm_count ? pairs : sm_count);
-        if (tensor_cores == 3) launch_pdl(policy_tc5_kernel<true>, g5, tc5::kThreads, tc5::kSmemBytes, (cudaStream_t)stream, *mlp, obs, n, po);
+        if (sep && tensor_cores == 3) launch_pdl(policy_tc5_sep_kernel<true>, g5, tc5::kThreads, tc5::kSmemBytesSep, (cudaStream_t)stream, *mlp, obs, n, po);
+        else if (sep) launch_pdl(policy_tc5_sep_kernel<false>, g5, tc5::kThreads, tc5::kSmemBytesSep, (cudaStream_t)stream, *mlp, obs, n, po);
+        else if (tensor_cores == 3) launch_pdl(policy_tc5_kernel<true>, g5, tc5::kThreads, tc5::kSmemBytes, (cudaStream_t)stream, *mlp, obs, n, po);
         else launch_pdl(policy_tc5_kernel<false>, g5, tc5::kThreads, tc5::kSmemBytes, (cudaStream_t)stream, *mlp, obs, n, po);
     }
+    else if (sep) policy_sep_kernel<<<g, kThreads, kSmemPolicySep, (cudaStream_t)stream>>>(*mlp, obs, n, po);
     else if (tensor_cores) policy_kernel<true><<<g, kThreads, kSmemPolicyTc, (cudaStream_t)stream>>>(*mlp, obs, n, po);
     else policy_kernel<false><<<g, kThreads, kSmemPolicy, (cudaStream_t)stream>>>(*mlp, obs, n, po);
     return check_launch("r6_policy");
@@ -1803,6 +2198,7 @@ int r6_policy_sde_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, in
                         float *log_prob, void *stream)
 {
     if (int rc = check_mlp(mlp)) return rc;
+    if (int rc = reject_separate(mlp, "r6_policy_sde_range (gSDE)")) return rc;
     if (!sde || !sde->log_std || !sde->xi || !obs || !actions) return fail(R6_EINVAL, "null pointer%s");
     if (n < 0) return fail(R6_EINVAL, "n < 0%s");
     if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
@@ -1886,7 +2282,7 @@ int r6_adam_coef_size(void) { return (int)sizeof(R6AdamCoef); }
 
 int64_t r6_ppo_work_bytes(int64_t B)
 {
-    return B > 0 ? ppo_ctas(B) * (int64_t)(R6_PPO_NTERMS * sizeof(double) + kPpoParams * sizeof(float)) : 0;
+    return B > 0 ? ppo_ctas(B) * (int64_t)(R6_PPO_NTERMS * sizeof(double) + kPpoParamsSep * sizeof(float)) : 0;
 }
 
 }  // extern "C"
@@ -1897,7 +2293,9 @@ template <bool kSde>
 int ppo_grad_launch(const R6Mlp *mlp, const float *sde_log_std, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
                     const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream)
 {
-    constexpr int kP = kSde ? kPpoParamsSde : kPpoParams, kNT = kSde ? R6_PPO_NTERMS_SDE : R6_PPO_NTERMS;
+    const bool sep = !kSde && mlp_separate(*mlp);
+    const int kP = kSde ? kPpoParamsSde : (sep ? kPpoParamsSep : kPpoParams);
+    constexpr int kNT = kSde ? R6_PPO_NTERMS_SDE : R6_PPO_NTERMS;
     if (!rollout || !rollout->obs || !rollout->actions || !rollout->log_probs || !rollout->advantages || !rollout->returns)
         return fail(R6_EINVAL, "null rollout buffer%s");
     if (rollout->T < 0 || rollout->n < 0 || B < 0) return fail(R6_EINVAL, "negative size%s");
@@ -1921,6 +2319,12 @@ int ppo_grad_launch(const R6Mlp *mlp, const float *sde_log_std, const R6PpoRollo
         if (rc) return rc;
         ppo_reduce_sde_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
         return check_launch("r6_ppo_grad_sde (reduce)");
+    } else if (sep) {
+        ppo_grad_sep_kernel<<<G, kThreads, kSmemPpoSep, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, coef->adv_stats, pt, pp);
+        rc = check_launch("r6_ppo_grad (separate towers)");
+        if (rc) return rc;
+        ppo_reduce_sep_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
+        return check_launch("r6_ppo_grad (separate towers, reduce)");
     } else {
         ppo_grad_kernel<<<G, kThreads, kSmemPpo, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, coef->adv_stats, pt, pp);
         rc = check_launch("r6_ppo_grad");
@@ -1950,6 +2354,7 @@ int r6_ppo_grad_sde(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *roll
                     const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream)
 {
     if (int rc = check_mlp(mlp)) return rc;
+    if (int rc = reject_separate(mlp, "r6_ppo_grad_sde (gSDE)")) return rc;
     if (!mlp->wv || !mlp->bv || !sde || !sde->log_std) return fail(R6_EINVAL, "r6_ppo_grad_sde needs the critic head and log_std%s");
     return ppo_grad_launch<true>(mlp, sde->log_std, rollout, idx, B, coef, grad_sum, terms, work, stream);
 }

@@ -36,6 +36,18 @@
 // Measured (profiles/r02_policy_tcgen05_tmem.md): 2^20 envs in 0.175 ms faithful (XU pipe 57 % busy, tensor pipe
 // 38 %); the shared-memory-operand version it replaces took 0.30 ms.
 //
+// Separate towers (SB3 1.6's net_arch [dict(pi=[64, 64], vf=[64, 64])], policy_tc5_sep_kernel).  Layer 0 is the shared
+// kernel's once the two towers' w0 are stacked ([pi; vf], 128 rows), and W1's [64][128] tile holds [w1 | vf_w1] side by
+// side, so the two layer-1 chains are the shared kernel's 1a / 1b with their own accumulators.  TMEM is what binds:
+// D0, D1 and L take a group's 256 columns and a third 64-column accumulator does not fit with both groups resident.
+// So the value chain runs first and is reduced on the CUDA cores:
+//     layer 1v: A = H0v hi D0[64:128) lo L[0:64) -> D1     then  value = wv . tanh(D1 + vf_b1) in the epilogue, from the
+//               float32 accumulator (32 FMAs per column half; the second half's sum handed over through shared memory)
+//     layer 1p: A = H0p hi D0[0:64)  lo L[0:64) -> D1     (overwrites the value chain's accumulator, read by then)
+//     layer 2 : as above, W2 row 3 zero (the value is not an MMA output)
+// Per tile that is one more epilogue (four: H0v, value, H0p, H1p) and the same four MMA commits; the value never
+// needs a TF32 split.  Extra shared memory: vf_b1, wv and per group the second half's value sums (kOffSep..).
+//
 // Shared-memory operand layout of the weights (K-major, SWIZZLE_NONE "interleaved" canonical layout): element (row r,
 // k) of a tile with K_tot columns lives at byte (r % 8) * 16 + (r / 8) * SBO + (k / 4) * 128 + (k % 4) * 4,
 // SBO = (K_tot / 4) * 128: 8-row x 16-byte core matrices, consecutive K chunks 128 B apart (LBO), 8-row groups SBO
@@ -62,6 +74,9 @@ constexpr int kSmemBytes = kOffTmemPtr + 16;
 // gSDE kernels only: sigma [192], sigma^2 [192], and per group the second column half's partial sums [128 rows][6]
 constexpr int kOffSde = kSmemBytes, kOffSdePart = kOffSde + 2 * 192 * 4;
 constexpr int kSmemBytesSde = kOffSdePart + 2 * kTile * 6 * 4;
+// separate-tower kernels only: vf_b1 [64] (pre-scaled like b1), wv [64], per group the second half's value sums [128]
+constexpr int kOffSep = kSmemBytes, kOffSepWv = kOffSep + 64 * 4, kOffSepPart = kOffSepWv + 64 * 4;
+constexpr int kSmemBytesSep = kOffSepPart + 2 * kTile * 4;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ int tile_off(int r, int k, int ktot) { return (r & 7) * 16 + (r >> 3) * (ktot * 32) + (k >> 2) * 128 + (k & 3) * 4; }
@@ -219,6 +234,26 @@ __device__ __forceinline__ void epilogue_in_tmem(uint32_t tmem_row, uint32_t src
         tmem_st32(tmem_row + src + cc, v);
     }
     tmem_st_wait();
+}
+
+// The value tower's last hidden layer (separate towers): sum over this thread's 32 units k = cc .. cc + 31 of
+// wv_k tanh(D[:, src + k] + vf_b1_k), from the float32 accumulator.  Nothing is stored back: the value latent feeds no MMA.
+template <bool kFaithful>
+__device__ __forceinline__ float epilogue_value(uint32_t tmem_row, uint32_t src, const float *bias, const float *wv, int half,
+                                                int group)
+{
+    const int cc = 32 * half;
+    float v[32];
+    tmem_ld32(tmem_row + src + cc, v);
+    token_take(group);
+    float s = 0.0f;
+#pragma unroll
+    for (int q = 0; q < 32; q++) {
+        const float h = kFaithful ? tanh_exact_scaled(fmaf(v[q], kTwoLog2e, bias[cc + q])) : tanh_fast(v[q] + bias[cc + q]);
+        s = fmaf(wv[cc + q], h, s);
+    }
+    token_pass(group ^ 1);
+    return s;
 }
 
 // epilogue_in_tmem of the last hidden layer with the gSDE sums over this thread's 32 units k = cc .. cc + 31 of its env row

@@ -1,7 +1,8 @@
 // r6_ppo.cuh — per-sample math of the PPO update (stable-baselines3 1.6.0 `PPO.train`, main_6DOF.py:136): one
 // sample's forward pass, its contribution to the clipped-surrogate + value + entropy loss, and the backward pass
 // through the shared-trunk actor-critic (13 -> 128 -> 64 tanh, action_net 64 -> 3, value_net 64 -> 1, state-independent
-// log_std).  Compiled for the device (r6_ppo_grad) and, for tests/ppo_hostsim only, for the host.
+// log_std) or SB3 1.6's separate towers (13 -> 64 -> 64 tanh twice, action_net on the policy latent, value_net on the
+// value latent; ppo_forward_sep / ppo_delta1_sep, then ppo_delta0 on either tower's units).  Compiled for the device (r6_ppo_grad) and, for tests/ppo_hostsim only, for the host.
 //
 // The loss, from memory of SB3 1.6.0 PPO.train [memory]:
 //     logp   = sum_j -(a_j - mean_j)^2 / (2 sigma_j^2) - log sigma_j - log sqrt(2 pi),  sigma = exp(log_std),
@@ -29,6 +30,19 @@ static_assert(kPpoParamsSde == R6_PPO_NPARAMS_SDE, "flat layout (gSDE)");
 static_assert(kPpoOffB0 == kMlpH0 * kMlpIn && kPpoOffW1 == kPpoOffB0 + kMlpH0 && kPpoOffB1 == kPpoOffW1 + kMlpH1 * kMlpH0 &&
               kPpoOffW2 == kPpoOffB1 + kMlpH1 && kPpoOffB2 == kPpoOffW2 + 3 * kMlpH1 && kPpoOffWv == kPpoOffB2 + 3 &&
               kPpoOffBv == kPpoOffWv + kMlpH1 && kPpoOffLogStd == kPpoOffBv + 1 && kPpoOffW1 % 4 == 0, "flat layout");
+
+// the separate-tower layout (R6_PPO_NPARAMS_SEP): policy and value layer 0 stacked, then each tower's layer 1, the heads
+constexpr int kSepOffW0 = 0, kSepOffVw0 = 832, kSepOffB0 = 1664, kSepOffVb0 = 1728, kSepOffW1 = 1792, kSepOffB1 = 5888,
+              kSepOffVw1 = 5952, kSepOffVb1 = 10048, kSepOffW2 = 10112, kSepOffB2 = 10304, kSepOffWv = 10307,
+              kSepOffBv = 10371, kSepOffLogStd = 10372, kPpoParamsSep = 10375;
+static_assert(kPpoParamsSep == R6_PPO_NPARAMS_SEP, "flat layout (separate towers)");
+static_assert(kSepOffVw0 == kMlpH1 * kMlpIn && kSepOffB0 == kSepOffVw0 + kMlpH1 * kMlpIn && kSepOffVb0 == kSepOffB0 + kMlpH1 &&
+              kSepOffW1 == kSepOffVb0 + kMlpH1 && kSepOffB1 == kSepOffW1 + kMlpH1 * kMlpH1 && kSepOffVw1 == kSepOffB1 + kMlpH1 &&
+              kSepOffVb1 == kSepOffVw1 + kMlpH1 * kMlpH1 && kSepOffW2 == kSepOffVb1 + kMlpH1 &&
+              kSepOffB2 == kSepOffW2 + 3 * kMlpH1 && kSepOffWv == kSepOffB2 + 3 && kSepOffBv == kSepOffWv + kMlpH1 &&
+              kSepOffLogStd == kSepOffBv + 1, "flat layout (separate towers)");
+// the stacked layer 0 is the shared layout's [128][13] + [128]; w1 and vf_w1 keep the 16-byte alignment of tensor_cores 2 / 3
+static_assert(kSepOffB0 == kPpoOffB0 && kSepOffW1 == kPpoOffW1 && kSepOffW1 % 4 == 0 && kSepOffVw1 % 4 == 0, "flat layout (separate towers)");
 
 // per-sample gradient w.r.t. the network outputs: g[0..2] = d/d mean, g[3] = d/d value, g[4..6] = d/d log_std
 struct PpoHead {
@@ -74,6 +88,40 @@ R6_HD void ppo_forward(const float *W, const float *x, float *h0, float *h1s, in
         o1 = f32_fma(W[kMlpOffW2 + kMlpH1 + k], h, o1);
         o2 = f32_fma(W[kMlpOffW2 + 2 * kMlpH1 + k], h, o2);
         o3 = f32_fma(W[kMlpOffW2 + 3 * kMlpH1 + k], h, o3);
+    }
+    out[0] = o0 + W[kMlpOffB2];
+    out[1] = o1 + W[kMlpOffB2 + 1];
+    out[2] = o2 + W[kMlpOffB2 + 2];
+    out[3] = o3 + W[kMlpOffB2 + 3];
+}
+
+// ppo_forward over the separate towers (mlp_forward_sep's operation order, packed by mlp_pack_element_sep): the layer-0
+// activations h0[j * st] (policy units 0..63, value units 64..127) and the two latents h1p[k * st], h1v[k * st]
+R6_HD void ppo_forward_sep(const float *W, const float *x, float *h0, float *h1p, float *h1v, int st, float (&out)[4])
+{
+    float acc[kMlpH1];
+    const auto keep = [&](int j, float h) { h0[j * st] = h; };
+    mlp_tower_acc<kMlpH1>(W, x, acc, keep);
+#pragma unroll
+    for (int k = 0; k < kMlpH1; k++) h1v[k * st] = acc[k];
+    float o3 = 0.0f;
+#pragma unroll 4
+    for (int k = 0; k < kMlpH1; k++) {
+        const float h = tanhf(h1v[k * st] + W[kMlpOffVb1 + k]);
+        h1v[k * st] = h;
+        o3 = f32_fma(W[kMlpOffW2 + 3 * kMlpH1 + k], h, o3);
+    }
+    mlp_tower_acc<0>(W, x, acc, keep);
+#pragma unroll
+    for (int k = 0; k < kMlpH1; k++) h1p[k * st] = acc[k];
+    float o0 = 0.0f, o1 = 0.0f, o2 = 0.0f;
+#pragma unroll 4
+    for (int k = 0; k < kMlpH1; k++) {
+        const float h = tanhf(h1p[k * st] + W[kMlpOffB1 + k]);
+        h1p[k * st] = h;
+        o0 = f32_fma(W[kMlpOffW2 + k], h, o0);
+        o1 = f32_fma(W[kMlpOffW2 + kMlpH1 + k], h, o1);
+        o2 = f32_fma(W[kMlpOffW2 + 2 * kMlpH1 + k], h, o2);
     }
     out[0] = o0 + W[kMlpOffB2];
     out[1] = o1 + W[kMlpOffB2 + 1];
@@ -191,6 +239,21 @@ R6_HD void ppo_delta1(const float *W, const PpoHead &h, const float *h1, float *
         s = f32_fma(W[kMlpOffW2 + 3 * kMlpH1 + k], h.g[3], s);
         const float hk = h1[k * st];
         d1[k * st] = s * f32_fma(-hk, hk, 1.0f);
+    }
+}
+
+// the separate towers' delta1, in place over the latents: policy (sum_c W2[c][k] g_c) (1 - h1p_k^2), value
+// wv_k g_v (1 - h1v_k^2)
+R6_HD void ppo_delta1_sep(const float *W, const PpoHead &h, float *h1p, float *h1v, int st)
+{
+#pragma unroll 4
+    for (int k = 0; k < kMlpH1; k++) {
+        float s = W[kMlpOffW2 + k] * h.g[0];
+        s = f32_fma(W[kMlpOffW2 + kMlpH1 + k], h.g[1], s);
+        s = f32_fma(W[kMlpOffW2 + 2 * kMlpH1 + k], h.g[2], s);
+        const float hp = h1p[k * st], hv = h1v[k * st];
+        h1p[k * st] = s * f32_fma(-hp, hp, 1.0f);
+        h1v[k * st] = (W[kMlpOffW2 + 3 * kMlpH1 + k] * h.g[3]) * f32_fma(-hv, hv, 1.0f);
     }
 }
 

@@ -45,7 +45,13 @@ def run_montecarlo(n_episodes: int, weights: Dict[str, np.ndarray], env_config: 
     tensor_cores=True evaluates the policy on the tensor cores at float32 accuracy instead of with float32 FMAs.
     two_kernel (default: batches above 65536 episodes): the closed loop as policy kernel + env-step kernels per step
     (`step_policy`: tcgen05 3xTF32 policy when tensor_cores, multi-pass integrator, stream `lanes`) instead of the one
-    fused rollout kernel — about twice the throughput for large dispersions, same one-episode semantics."""
+    fused rollout kernel — about twice the throughput for large dispersions, same one-episode semantics.  SB3 1.6's
+    separate policy / value towers (weights with vf_w0 ...) always take the two-kernel path: the fused rollout kernel
+    does not run that network."""
+    if _policy.is_separate(weights):
+        if two_kernel is False:
+            raise ValueError("the separate policy / value towers have no fused rollout kernel: two_kernel must be True")
+        two_kernel = True
     if two_kernel is None:
         two_kernel = n_episodes > SPLIT_MIN_ENVS
     env = Rocket6DOFBatch(n_episodes, env_config, sb3_config, device=device, seed=seed, auto_reset=False,

@@ -11,7 +11,9 @@ over rollouts collected by `Rocket6DOFBatch.collect_rollout`, with the loss grad
 The network is SB3's default `MlpPolicy` of SB3 1.6: a shared tanh trunk 13 -> 128 -> 64, `action_net` 64 -> 3,
 `value_net` 64 -> 1 and a state-independent `log_std` [3], or with `PPOConfig(use_sde=True)` SB3's generalised
 state-dependent exploration (gSDE: log_std [64, 3], noise h (exp(log_std) * xi) held between `reset_noise` draws;
-params from `ActorCriticParams.sb3_init(use_sde=True)`).  No `clip_range_vf`.
+params from `ActorCriticParams.sb3_init(use_sde=True)`), or SB3 1.6's default without policy_kwargs: separate tanh
+towers 13 -> 64 -> 64 for the policy and the value (`ActorCriticParams.sb3_init(net_arch=[dict(pi=[64, 64],
+vf=[64, 64])])`, no gSDE).  No `clip_range_vf`.
 """
 from __future__ import annotations
 
@@ -32,21 +34,30 @@ NPARAMS = _lib.PPO_NPARAMS
 # the gSDE layout (R6_PPO_NPARAMS_SDE): the same prefix, log_std [64][3]
 LAYOUT_SDE = LAYOUT[:-1] + (("log_std", (64, 3)),)
 NPARAMS_SDE = _lib.PPO_NPARAMS_SDE
+# SB3 1.6's default separate towers (R6_PPO_NPARAMS_SEP): the two layer-0 blocks stacked (as the shared [128][13] + [128]),
+# then each tower's layer 1, the heads and log_std
+LAYOUT_SEP = (("w0", (64, 13)), ("vf_w0", (64, 13)), ("b0", (64,)), ("vf_b0", (64,)), ("w1", (64, 64)), ("b1", (64,)),
+              ("vf_w1", (64, 64)), ("vf_b1", (64,)), ("w2", (3, 64)), ("b2", (3,)), ("wv", (64,)), ("bv", (1,)),
+              ("log_std", (3,)))
+NPARAMS_SEP = _lib.PPO_NPARAMS_SEP
+NET_ARCH_SEP = [dict(pi=[64, 64], vf=[64, 64])]
 _LOG_SQRT_2PI = 0.5 * math.log(2.0 * math.pi)
 
 
 class ActorCriticParams:
     """The actor-critic as one flat float32 CUDA tensor `flat` with views w0 ... log_std into it: [R6_PPO_NPARAMS]
-    with log_std [3], or [R6_PPO_NPARAMS_SDE] with the gSDE log_std [64, 3] (`use_sde`)."""
+    with log_std [3], [R6_PPO_NPARAMS_SDE] with the gSDE log_std [64, 3] (`use_sde`), or [R6_PPO_NPARAMS_SEP] for SB3
+    1.6's separate policy / value towers (`separate`, LAYOUT_SEP)."""
 
     def __init__(self, flat: torch.Tensor):
-        if (flat.dtype != torch.float32 or not flat.is_cuda or flat.shape not in ((NPARAMS,), (NPARAMS_SDE,))
+        if (flat.dtype != torch.float32 or not flat.is_cuda or flat.shape not in ((NPARAMS,), (NPARAMS_SDE,), (NPARAMS_SEP,))
                 or not flat.is_contiguous()):
-            raise ValueError(f"flat parameters must be a contiguous float32 CUDA tensor of {NPARAMS} or {NPARAMS_SDE} "
-                             "(gSDE) elements")
+            raise ValueError(f"flat parameters must be a contiguous float32 CUDA tensor of {NPARAMS}, {NPARAMS_SDE} "
+                             f"(gSDE) or {NPARAMS_SEP} (separate towers) elements")
         self.flat = flat
         self.use_sde = flat.numel() == NPARAMS_SDE
-        self.layout = LAYOUT_SDE if self.use_sde else LAYOUT
+        self.separate = flat.numel() == NPARAMS_SEP
+        self.layout = LAYOUT_SDE if self.use_sde else (LAYOUT_SEP if self.separate else LAYOUT)
         o = 0
         for name, shape in self.layout:
             size = int(np.prod(shape))
@@ -55,27 +66,56 @@ class ActorCriticParams:
         assert o == flat.numel()
 
     @classmethod
-    def sb3_init(cls, seed: int = 0, device="cuda", use_sde: bool = False) -> "ActorCriticParams":
+    def sb3_init(cls, seed: int = 0, device="cuda", use_sde: bool = False, net_arch=None) -> "ActorCriticParams":
         """SB3's construction-time weights (ortho_init): `torch.nn.init.orthogonal_` with gain sqrt(2) on the trunk,
         0.01 on action_net and 1 on value_net, zero biases, log_std 0 ([64, 3] with use_sde).  Drawn on the CPU with a
-        generator seeded by `seed`, so they do not depend on the device."""
+        generator seeded by `seed`, so they do not depend on the device.
+
+        net_arch: [128, 64] (the default: the shared trunk of the reference's policy_kwargs) or
+        [dict(pi=[64, 64], vf=[64, 64])] (SB3 1.6's default without policy_kwargs: separate towers, both at gain
+        sqrt(2)).  The matrices are drawn in the order w0, w1 (shared trunk or policy tower), then vf_w0, vf_w1 (value
+        tower), then action_net, value_net.  No other architecture has kernels: anything else raises ValueError."""
+        sep = cls._separate_arch(net_arch)
+        if sep and use_sde:
+            raise ValueError("gSDE is not implemented for the separate policy / value towers")
+        w = cls.sb3_init_weights(seed, net_arch)
+        return cls._from(w, device, LAYOUT_SEP if sep else (LAYOUT_SDE if use_sde else LAYOUT))
+
+    @classmethod
+    def sb3_init_weights(cls, seed: int = 0, net_arch=None) -> Dict[str, torch.Tensor]:
+        """The weight matrices of `sb3_init` as flat float32 CPU tensors (biases and log_std are zero and not listed)."""
+        sep = cls._separate_arch(net_arch)
         gen = torch.Generator().manual_seed(int(seed))
         w = {}
-        for name, shape, gain in (("w0", (128, 13), math.sqrt(2)), ("w1", (64, 128), math.sqrt(2)), ("w2", (3, 64), 0.01),
-                                  ("wv", (1, 64), 1.0)):
+        trunk = ((("w0", (64, 13), math.sqrt(2)), ("w1", (64, 64), math.sqrt(2)), ("vf_w0", (64, 13), math.sqrt(2)),
+                  ("vf_w1", (64, 64), math.sqrt(2))) if sep else
+                 (("w0", (128, 13), math.sqrt(2)), ("w1", (64, 128), math.sqrt(2))))
+        for name, shape, gain in trunk + (("w2", (3, 64), 0.01), ("wv", (1, 64), 1.0)):
             t = torch.empty(shape, dtype=torch.float32)
             torch.nn.init.orthogonal_(t, gain=gain, generator=gen)
             w[name] = t.reshape(-1)
-        return cls._from(w, device, LAYOUT_SDE if use_sde else LAYOUT)
+        return w
+
+    @staticmethod
+    def _separate_arch(net_arch) -> bool:
+        if net_arch is None or list(net_arch) == [128, 64]:
+            return False
+        if list(net_arch) == NET_ARCH_SEP:
+            return True
+        raise ValueError(f"net_arch {net_arch!r} has no kernels: use [128, 64] or [dict(pi=[64, 64], vf=[64, 64])]")
 
     @classmethod
     def from_weights(cls, w: Dict[str, np.ndarray], device="cuda") -> "ActorCriticParams":
         """From `policy.load_sb3_zip` / `policy.load_npz` output (the critic head and log_std must be present); a
-        [64, 3] log_std gives the gSDE layout."""
-        missing = [k for k, _ in LAYOUT if w.get(k) is None]
+        [64, 3] log_std gives the gSDE layout, a value tower (vf_w0 ...) the separate-tower layout."""
+        sep = w.get("vf_w0") is not None
+        missing = [k for k, _ in (LAYOUT_SEP if sep else LAYOUT) if w.get(k) is None]
         if missing:
             raise ValueError(f"weights lack {missing}: training needs the critic head and log_std")
-        return cls._from(w, device, LAYOUT_SDE if np.asarray(w["log_std"]).size == 64 * 3 else LAYOUT)
+        sde = np.asarray(w["log_std"]).size == 64 * 3
+        if sep and sde:
+            raise ValueError("gSDE is not implemented for the separate policy / value towers")
+        return cls._from(w, device, LAYOUT_SEP if sep else (LAYOUT_SDE if sde else LAYOUT))
 
     @classmethod
     def _from(cls, w, device, layout) -> "ActorCriticParams":
@@ -154,7 +194,8 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     `rollout` is `collect_rollout`'s dict (obs [T, N, 13] with any strides, actions [T, N, 3], log_probs, advantages,
     returns [T, N]).  Indices outside [0, T N) are skipped and counted in terms[4] (checking them here would
     synchronise).  The minibatch's advantage mean and 1 / (std + 1e-8) are computed on the device (no synchronise).
-    Returns (grad_sum float32 [R6_PPO_NPARAMS], terms float64 [5]); for gSDE params (r6_ppo_grad_sde) grad_sum
+    Returns (grad_sum float32 [params.flat.numel()]: R6_PPO_NPARAMS, or R6_PPO_NPARAMS_SEP for the separate towers,
+    terms float64 [5]); for gSDE params (r6_ppo_grad_sde) grad_sum
     [R6_PPO_NPARAMS_SDE] and terms [6], the last the sum of the per-sample entropies."""
     dev = params.flat.device
     P, NT = params.flat.numel(), (_lib.PPO_NTERMS_SDE if params.use_sde else _lib.PPO_NTERMS)
@@ -233,6 +274,10 @@ class PPOTrainer:
 
     def __init__(self, batch, params: ActorCriticParams, cfg: Optional[PPOConfig] = None, seed: int = 0):
         self.batch, self.params, self.cfg = batch, params, cfg or PPOConfig()
+        if params.separate and self.cfg.use_sde:
+            raise ValueError("gSDE (use_sde=True) is not implemented for the separate policy / value towers")
+        if params.separate and int(self.cfg.tensor_cores) == 1:
+            raise ValueError("the separate policy / value towers have no mma.sync policy kernel (tensor_cores=1)")
         if params.use_sde != self.cfg.use_sde:
             raise ValueError(f"PPOConfig(use_sde={self.cfg.use_sde}) needs params with the "
                              f"{'gSDE' if self.cfg.use_sde else 'diagonal Gaussian'} layout "
