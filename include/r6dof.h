@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 20
+#define R6_ABI_VERSION 21
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -402,12 +402,16 @@ typedef struct R6PpoRollout {
     const float *advantages; /* [T][n] */
     const float *returns;    /* [T][n] */
     int64_t T, n;
+    const float *old_values; /* [T][n] the critic's values at collection (collect_rollout's `values`, before any
+                                truncation bootstrap); read only when R6PpoCoef.clip_range_vf > 0, nullable otherwise */
 } R6PpoRollout;
 
 typedef struct R6PpoCoef {
     double clip_range, vf_coef, ent_coef;
     const double *adv_stats; /* DEVICE [2] = (mean, 1 / (std + 1e-8)) of the minibatch's advantages, or NULL = no
                                 normalisation.  A device pointer, so that no minibatch has to synchronise */
+    double clip_range_vf;    /* SB3's clip_range_vf: > 0 clips the value prediction to old_values +- clip_range_vf
+                                (rollout->old_values required); 0 = off.  Negative or non-finite: R6_EINVAL */
 } R6PpoCoef;
 
 typedef struct R6AdamCoef {
@@ -432,6 +436,13 @@ int64_t r6_ppo_work_bytes(int64_t B);
  * (R - V)^2, the number of samples with |ratio - 1| > clip_range, (ratio - 1) - log ratio, and the number of indices
  * outside [0, T n) (those samples are skipped).  mlp must carry wv, bv and log_std.  Sums, not means: the caller scales.
  * The launch shape depends on B only, so the result is bit-reproducible on any device.
+ *
+ * Value clipping (coef->clip_range_vf = c > 0, SB3's clip_range_vf): per sample, in float32 and torch's order,
+ *     d = V - V_old,  vp = V_old + clamp(d, -fl32(c), fl32(c)),  value loss (R - vp)^2,
+ * V_old = rollout->old_values; d loss / d V = 2 vf_coef (vp - R) for -c <= d <= c, else 0 (the sample adds nothing to
+ * the value head or, with separate towers, to the value tower).  terms[R6_PPO_T_VLOSS] is then the sum of the clipped
+ * (R - vp)^2.  Returns R6_EINVAL, before any CUDA call and writing nothing, for c < 0 or not finite, and for c > 0 with
+ * old_values NULL and B > 0.  c = 0 is the unclipped loss above, bit for bit.
  */
 int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *idx, int64_t B, const R6PpoCoef *coef,
                 float *grad_sum, double *terms, void *work, void *stream);
@@ -444,6 +455,7 @@ int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *id
  *     d loss / d log_std[k][a] = exp(2 log_std[k][a]) sum_s h_{s,k}^2 (w_s (z_{s,a}^2 - 1) - ent_coef) / std_a(s)^2,
  * w = d pg / d logp, z = (a - mean) / std.  terms [R6_PPO_NTERMS_SDE]: those of r6_ppo_grad plus the sum of the per-sample
  * entropies (R6_PPO_T_ENTROPY).  sde->log_std is the [64][3] matrix (sde->xi is not read; mlp->log_std is not read).
+ * Value clipping (coef->clip_range_vf) and its R6_EINVAL cases as r6_ppo_grad.
  */
 #define R6_PPO_NPARAMS_SDE 10500
 #define R6_PPO_NTERMS_SDE 6

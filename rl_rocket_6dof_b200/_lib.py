@@ -12,7 +12,7 @@ from .params import R6Params
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libr6dof.so")
-ABI_VERSION = 20
+ABI_VERSION = 21
 
 u8p = C.c_void_p
 
@@ -45,11 +45,13 @@ class R6Mlp(C.Structure):
 class R6PpoRollout(C.Structure):
     _fields_ = [("obs", C.c_void_p), ("obs_stride_step", C.c_int64), ("obs_stride_comp", C.c_int64),
                 ("obs_stride_env", C.c_int64), ("actions", C.c_void_p), ("log_probs", C.c_void_p),
-                ("advantages", C.c_void_p), ("returns", C.c_void_p), ("T", C.c_int64), ("n", C.c_int64)]
+                ("advantages", C.c_void_p), ("returns", C.c_void_p), ("T", C.c_int64), ("n", C.c_int64),
+                ("old_values", C.c_void_p)]                  # nullable: read only with R6PpoCoef.clip_range_vf > 0
 
 
 class R6PpoCoef(C.Structure):
-    _fields_ = [("clip_range", C.c_double), ("vf_coef", C.c_double), ("ent_coef", C.c_double), ("adv_stats", C.c_void_p)]
+    _fields_ = [("clip_range", C.c_double), ("vf_coef", C.c_double), ("ent_coef", C.c_double), ("adv_stats", C.c_void_p),
+                ("clip_range_vf", C.c_double)]               # 0 = no value clipping
 
 
 class R6AdamCoef(C.Structure):

@@ -1353,10 +1353,12 @@ int64_t ppo_ctas(int64_t B)
     return tiles < kPpoMaxCtas ? tiles : kPpoMaxCtas;
 }
 
-template <bool kSde>
+// kVfClip: SB3's clip_range_vf = vfc > 0 (ppo_value_clip on every sample, reading ro.old_values); the false
+// instantiations are the kernels without it, unchanged
+template <bool kSde, bool kVfClip>
 __device__ __forceinline__ void ppo_grad_body(const R6Mlp mlp, const float *sde_log_std, const R6PpoRollout ro,
                                               const int64_t *__restrict__ idx, int64_t B, float clip, float vf, float ent,
-                                              const double *__restrict__ adv_stats, double *__restrict__ part_terms,
+                                              float vfc, const double *__restrict__ adv_stats, double *__restrict__ part_terms,
                                               float *__restrict__ part)
 {
     constexpr int kP = kSde ? kPpoParamsSde : kPpoParams, kNT = kSde ? R6_PPO_NTERMS_SDE : R6_PPO_NTERMS;
@@ -1414,6 +1416,7 @@ __device__ __forceinline__ void ppo_grad_body(const R6Mlp mlp, const float *sde_
                 } else
                     ppo_head(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], mlp.log_std,
                              clip, vf, ent, hd);
+                if constexpr (kVfClip) ppo_value_clip(out[3], ro.old_values[q], ro.returns[q], vfc, vf, hd);
             }
             ppo_delta1(Ws, hd, S + kPpoRowH1 * kPpoTS + tid, S + kPpoRowD1 * kPpoTS + tid, kPpoTS);
 #pragma unroll
@@ -1542,18 +1545,21 @@ __device__ __forceinline__ void ppo_grad_body(const R6Mlp mlp, const float *sde_
         else T[R6_PPO_T_ENTROPY] = aS;
     }
 }
+template <bool kVfClip>
 __global__ void __launch_bounds__(kThreads, 1)
 ppo_grad_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restrict__ idx, int64_t B, float clip, float vf,
-                float ent, const double *__restrict__ adv_stats, double *__restrict__ part_terms, float *__restrict__ part)
+                float ent, float vfc, const double *__restrict__ adv_stats, double *__restrict__ part_terms,
+                float *__restrict__ part)
 {
-    ppo_grad_body<false>(mlp, nullptr, ro, idx, B, clip, vf, ent, adv_stats, part_terms, part);
+    ppo_grad_body<false, kVfClip>(mlp, nullptr, ro, idx, B, clip, vf, ent, vfc, adv_stats, part_terms, part);
 }
+template <bool kVfClip>
 __global__ void __launch_bounds__(kThreads, 1)
 ppo_grad_sde_kernel(const R6Mlp mlp, const float *__restrict__ log_std, const R6PpoRollout ro, const int64_t *__restrict__ idx,
-                    int64_t B, float clip, float vf, float ent, const double *__restrict__ adv_stats,
+                    int64_t B, float clip, float vf, float ent, float vfc, const double *__restrict__ adv_stats,
                     double *__restrict__ part_terms, float *__restrict__ part)
 {
-    ppo_grad_body<true>(mlp, log_std, ro, idx, B, clip, vf, ent, adv_stats, part_terms, part);
+    ppo_grad_body<true, kVfClip>(mlp, log_std, ro, idx, B, clip, vf, ent, vfc, adv_stats, part_terms, part);
 }
 
 // r6_ppo_grad for SB3 1.6's separate towers (ppo_grad_sep_kernel).  The same tiles, CTA count, accumulators and
@@ -1567,9 +1573,12 @@ constexpr int kSmemPpoSep = (kMlpFloatsSep + kPpoRows * kPpoTS + kPpoAccW1) * (i
 static_assert(kMlpFloatsSep % 4 == 0 && kPpoRowHP == kPpoRowH1 && kPpoRowHV == kPpoRowD1 && kSmemPpoSep <= 232448,
               "PPO separate-tower tile layout");
 
+// kVfClip as ppo_grad_body: a clipped sample's g[3] = 0 gives its value tower zero deltas through ppo_delta1_sep
+template <bool kVfClip>
 __global__ void __launch_bounds__(kThreads, 1)
 ppo_grad_sep_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__restrict__ idx, int64_t B, float clip, float vf,
-                    float ent, const double *__restrict__ adv_stats, double *__restrict__ part_terms, float *__restrict__ part)
+                    float ent, float vfc, const double *__restrict__ adv_stats, double *__restrict__ part_terms,
+                    float *__restrict__ part)
 {
     extern __shared__ __align__(16) double r6_smem[];
     float *Ws = reinterpret_cast<float *>(r6_smem);
@@ -1611,6 +1620,7 @@ ppo_grad_sep_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__res
                 const float a[3] = {ro.actions[3 * q], ro.actions[3 * q + 1], ro.actions[3 * q + 2]};
                 ppo_head(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], mlp.log_std, clip,
                          vf, ent, hd);
+                if constexpr (kVfClip) ppo_value_clip(out[3], ro.old_values[q], ro.returns[q], vfc, vf, hd);
             }
 #pragma unroll
             for (int r = 0; r < 7; r++) S[(kPpoRowG + r) * kPpoTS + tid] = hd.g[r];
@@ -1890,15 +1900,18 @@ int ensure_attributes()
     rc |= enable_smem(policy_kernel<false>, kSmemPolicy);
     rc |= enable_smem(policy_tc5_kernel<true>, tc5::kSmemBytes);
     rc |= enable_smem(policy_tc5_kernel<false>, tc5::kSmemBytes);
-    rc |= enable_smem(ppo_grad_kernel, kSmemPpo);
-    rc |= enable_smem(ppo_grad_sde_kernel, kSmemPpoSde);
+    rc |= enable_smem(ppo_grad_kernel<false>, kSmemPpo);
+    rc |= enable_smem(ppo_grad_kernel<true>, kSmemPpo);
+    rc |= enable_smem(ppo_grad_sde_kernel<false>, kSmemPpoSde);
+    rc |= enable_smem(ppo_grad_sde_kernel<true>, kSmemPpoSde);
     rc |= enable_smem(policy_sde_kernel, kSmemPolicySde);
     rc |= enable_smem(policy_tc5_sde_kernel<true>, tc5::kSmemBytesSde);
     rc |= enable_smem(policy_tc5_sde_kernel<false>, tc5::kSmemBytesSde);
     rc |= enable_smem(policy_sep_kernel, kSmemPolicySep);
     rc |= enable_smem(policy_tc5_sep_kernel<true>, tc5::kSmemBytesSep);
     rc |= enable_smem(policy_tc5_sep_kernel<false>, tc5::kSmemBytesSep);
-    rc |= enable_smem(ppo_grad_sep_kernel, kSmemPpoSep);
+    rc |= enable_smem(ppo_grad_sep_kernel<false>, kSmemPpoSep);
+    rc |= enable_smem(ppo_grad_sep_kernel<true>, kSmemPpoSep);
     rc |= enable_smem(sim_raw_kernel<false>);
     rc |= enable_smem(sim_raw_kernel<true>);
     if (rc) return R6_ECUDA;
@@ -2300,6 +2313,10 @@ int ppo_grad_launch(const R6Mlp *mlp, const float *sde_log_std, const R6PpoRollo
         return fail(R6_EINVAL, "null rollout buffer%s");
     if (rollout->T < 0 || rollout->n < 0 || B < 0) return fail(R6_EINVAL, "negative size%s");
     if (!coef || !grad_sum || !terms || (B > 0 && (!idx || !work))) return fail(R6_EINVAL, "null pointer%s");
+    if (!(coef->clip_range_vf >= 0.0) || !isfinite(coef->clip_range_vf))
+        return fail(R6_EINVAL, "clip_range_vf must be finite and >= 0 (0 = no value clipping)%s");
+    const bool vclip = coef->clip_range_vf > 0.0;
+    if (vclip && B > 0 && !rollout->old_values) return fail(R6_EINVAL, "clip_range_vf > 0 needs rollout->old_values%s");
     cudaStream_t s = (cudaStream_t)stream;
     if (B == 0) {
         cudaError_t e = cudaMemsetAsync(grad_sum, 0, sizeof(float) * kP, s);
@@ -2313,20 +2330,34 @@ int ppo_grad_launch(const R6Mlp *mlp, const float *sde_log_std, const R6PpoRollo
     double *pt = static_cast<double *>(work);
     float *pp = reinterpret_cast<float *>(pt + (int64_t)G * kNT);
     const float clip = (float)coef->clip_range, vf = (float)coef->vf_coef, ent = (float)coef->ent_coef;
+    const float vfc = (float)coef->clip_range_vf;
     if constexpr (kSde) {
-        ppo_grad_sde_kernel<<<G, kThreads, kSmemPpoSde, s>>>(*mlp, sde_log_std, *rollout, idx, B, clip, vf, ent, coef->adv_stats, pt, pp);
+        if (vclip)
+            ppo_grad_sde_kernel<true><<<G, kThreads, kSmemPpoSde, s>>>(*mlp, sde_log_std, *rollout, idx, B, clip, vf, ent, vfc,
+                                                                      coef->adv_stats, pt, pp);
+        else
+            ppo_grad_sde_kernel<false><<<G, kThreads, kSmemPpoSde, s>>>(*mlp, sde_log_std, *rollout, idx, B, clip, vf, ent, vfc,
+                                                                       coef->adv_stats, pt, pp);
         rc = check_launch("r6_ppo_grad_sde");
         if (rc) return rc;
         ppo_reduce_sde_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
         return check_launch("r6_ppo_grad_sde (reduce)");
     } else if (sep) {
-        ppo_grad_sep_kernel<<<G, kThreads, kSmemPpoSep, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, coef->adv_stats, pt, pp);
+        if (vclip)
+            ppo_grad_sep_kernel<true><<<G, kThreads, kSmemPpoSep, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, vfc, coef->adv_stats,
+                                                                      pt, pp);
+        else
+            ppo_grad_sep_kernel<false><<<G, kThreads, kSmemPpoSep, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, vfc, coef->adv_stats,
+                                                                       pt, pp);
         rc = check_launch("r6_ppo_grad (separate towers)");
         if (rc) return rc;
         ppo_reduce_sep_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
         return check_launch("r6_ppo_grad (separate towers, reduce)");
     } else {
-        ppo_grad_kernel<<<G, kThreads, kSmemPpo, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, coef->adv_stats, pt, pp);
+        if (vclip)
+            ppo_grad_kernel<true><<<G, kThreads, kSmemPpo, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, vfc, coef->adv_stats, pt, pp);
+        else
+            ppo_grad_kernel<false><<<G, kThreads, kSmemPpo, s>>>(*mlp, *rollout, idx, B, clip, vf, ent, vfc, coef->adv_stats, pt, pp);
         rc = check_launch("r6_ppo_grad");
         if (rc) return rc;
         ppo_reduce_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);

@@ -9,7 +9,7 @@
 //              on the stored UNclipped action
 //     ratio  = exp(logp - old_logp),   A' = (A - mu_B) * inv_std_B when the advantages are normalised
 //     pg     = -min(A' ratio, A' clip(ratio, 1 - eps, 1 + eps))
-//     vloss  = (R - v)^2
+//     vloss  = (R - v)^2,  or with clip_range_vf = c:  (R - (v_old + clamp(v - v_old, -c, c)))^2   (ppo_value_clip)
 //     loss   = pg + vf_coef vloss - ent_coef entropy,   entropy = sum_j (log sigma_j + 1/2 + log sqrt(2 pi))
 // Gradient (torch.min / clamp semantics): d pg / d logp = -A' ratio when the unclipped branch is the minimum (always so
 // for ratio inside [1 - eps, 1 + eps]), else 0; d logp / d mean_j = (a_j - mean_j) / sigma_j^2,
@@ -164,6 +164,20 @@ R6_HD void ppo_head(const float (&out)[4], const float *a, float old_logp, float
     h.vloss = e * e;
     h.clipped = fabsf(ratio - 1.0f) > clip ? 1.0f : 0.0f;
     h.kl = (ratio - 1.0f) - lr;
+}
+
+// SB3's value clipping (PPO(clip_range_vf=c), c > 0) on a head ppo_head / ppo_head_sde has filled: overwrites g[3] and
+// vloss from v = V, v_old = the rollout's value at collection, ret = R, in torch's float32 order [memory]
+//     d = V - V_old;  vp = V_old + clamp(d, -c, c);  vloss = (vp - R)^2
+// (vp is formed inside the band too: it need not round to V).  d loss / d V = 2 vf_coef (vp - R) for -c <= d <= c (clamp's
+// gradient mask takes both bounds), else 0.
+R6_HD void ppo_value_clip(float v, float v_old, float ret, float c, float vf_coef, PpoHead &h)
+{
+    const float d = v - v_old;
+    const float vp = v_old + fminf(fmaxf(d, -c), c);
+    const float e = vp - ret;
+    h.g[3] = d >= -c && d <= c ? 2.0f * vf_coef * e : 0.0f;
+    h.vloss = e * e;
 }
 
 // 1 / sqrt(v), rounded once (the device form has no slow path, unlike a division)

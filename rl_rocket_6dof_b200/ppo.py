@@ -13,7 +13,8 @@ The network is SB3's default `MlpPolicy` of SB3 1.6: a shared tanh trunk 13 -> 1
 state-dependent exploration (gSDE: log_std [64, 3], noise h (exp(log_std) * xi) held between `reset_noise` draws;
 params from `ActorCriticParams.sb3_init(use_sde=True)`), or SB3 1.6's default without policy_kwargs: separate tanh
 towers 13 -> 64 -> 64 for the policy and the value (`ActorCriticParams.sb3_init(net_arch=[dict(pi=[64, 64],
-vf=[64, 64])])`, no gSDE).  No `clip_range_vf`.
+vf=[64, 64])])`, no gSDE).  SB3's value clipping (`PPOConfig(clip_range_vf=...)`) and clip-range schedules are
+supported on every network.
 """
 from __future__ import annotations
 
@@ -138,6 +139,7 @@ class ActorCriticParams:
 
 
 def _progress_lr(lr, progress_remaining: float) -> float:
+    """SB3's get_schedule_fn: a callable is called with progress_remaining, a number is a constant schedule."""
     return float(lr(progress_remaining)) if callable(lr) else float(lr)
 
 
@@ -149,15 +151,17 @@ class PPOConfig:
     would mean 2^27-sample rollouts in 2^21 minibatches of 64.  Here a rollout is `n_steps` (default 32) steps of every
     env, and `batch_size` defaults to a quarter of it (4 minibatches per epoch).  As in SB3 the last minibatch of an
     epoch may be short.  A minibatch of one sample is not normalised (its std is undefined: SB3 1.6 yields NaN there
-    [memory]; later SB3 releases add the same guard).  A callable learning_rate is SB3's schedule: it is called once per
-    update with progress_remaining (see `PPOTrainer.learn`)."""
+    [memory]; later SB3 releases add the same guard).  A callable learning_rate, clip_range or clip_range_vf is SB3's
+    schedule: it is called once per update with progress_remaining (see `PPOTrainer.learn`).  clip_range_vf (None: off)
+    clips the value prediction to the rollout's values +- clip_range_vf in the value loss, as SB3's; a number must be
+    > 0, as SB3 asserts."""
     learning_rate: Union[float, Callable[[float], float]] = 3e-4
     n_steps: int = 32
     batch_size: Optional[int] = None
     n_epochs: int = 10
     gamma: float = 0.99
     gae_lambda: float = 0.95
-    clip_range: float = 0.2
+    clip_range: Union[float, Callable[[float], float]] = 0.2
     normalize_advantage: bool = True
     ent_coef: float = 0.0
     vf_coef: float = 0.5
@@ -171,8 +175,11 @@ class PPOConfig:
     use_expln: bool = False
     squash_output: bool = False
     learn_features: bool = False
+    clip_range_vf: Union[None, float, Callable[[float], float]] = None
 
     def __post_init__(self):
+        if self.clip_range_vf is not None and not callable(self.clip_range_vf) and not float(self.clip_range_vf) > 0:
+            raise ValueError(f"clip_range_vf must be > 0 (or None for no value clipping), got {self.clip_range_vf!r}")
         bad = [k for k, ok in (("full_std", self.full_std), ("use_expln", not self.use_expln),
                                 ("squash_output", not self.squash_output), ("learn_features", not self.learn_features)) if not ok]
         if bad:
@@ -188,7 +195,7 @@ def _check_cuda(name, t, dtype, dev):
 def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *, clip_range: float = 0.2,
                   vf_coef: float = 0.5, ent_coef: float = 0.0, normalize_advantage: bool = True,
                   grad_sum: Optional[torch.Tensor] = None, terms: Optional[torch.Tensor] = None,
-                  work: Optional[torch.Tensor] = None):
+                  work: Optional[torch.Tensor] = None, clip_range_vf: Optional[float] = None):
     """SUM over the minibatch `idx` (int64 sample indices t * N + i into the [T, N] rollout) of the per-sample PPO loss
     gradient, and the float64 term sums (policy-gradient loss, (R - V)^2, clipped count, approx-kl, bad indices).
     `rollout` is `collect_rollout`'s dict (obs [T, N, 13] with any strides, actions [T, N, 3], log_probs, advantages,
@@ -196,7 +203,11 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     synchronise).  The minibatch's advantage mean and 1 / (std + 1e-8) are computed on the device (no synchronise).
     Returns (grad_sum float32 [params.flat.numel()]: R6_PPO_NPARAMS, or R6_PPO_NPARAMS_SEP for the separate towers,
     terms float64 [5]); for gSDE params (r6_ppo_grad_sde) grad_sum
-    [R6_PPO_NPARAMS_SDE] and terms [6], the last the sum of the per-sample entropies."""
+    [R6_PPO_NPARAMS_SDE] and terms [6], the last the sum of the per-sample entropies.
+
+    clip_range_vf (SB3's, > 0; None = off) clips each sample's value prediction to old_values +- clip_range_vf, where
+    old_values is `rollout["values"]` (float32 [T, N] contiguous, the critic at collection); terms[1] is then the sum
+    of the clipped (R - V_pred)^2."""
     dev = params.flat.device
     P, NT = params.flat.numel(), (_lib.PPO_NTERMS_SDE if params.use_sde else _lib.PPO_NTERMS)
     obs, act = rollout["obs"], rollout["actions"]
@@ -214,6 +225,14 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     if idx.dim() != 1 or not idx.is_contiguous():
         raise ValueError("idx must be a contiguous 1-D int64 tensor")
     B = idx.numel()
+    vals = None
+    if clip_range_vf is not None:
+        if not float(clip_range_vf) > 0 or not math.isfinite(float(clip_range_vf)):
+            raise ValueError(f"clip_range_vf must be finite and > 0 (None for no value clipping), got {clip_range_vf!r}")
+        vals = rollout.get("values")
+        _check_cuda("values", vals, torch.float32, dev)
+        if vals.shape != (T, n) or not vals.is_contiguous():
+            raise ValueError("values (the old values of clip_range_vf) must be a contiguous [T, N] tensor")
     if grad_sum is None:
         grad_sum = torch.empty(P, dtype=torch.float32, device=dev)
     if terms is None:
@@ -235,6 +254,8 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     ro = _lib.R6PpoRollout(obs.data_ptr(), obs.stride(0), obs.stride(2), obs.stride(1), act.data_ptr(), lp.data_ptr(),
                            adv.data_ptr(), ret.data_ptr(), T, n)
     coef = _lib.R6PpoCoef(float(clip_range), float(vf_coef), float(ent_coef), None if stats is None else stats.data_ptr())
+    if vals is not None:
+        ro.old_values, coef.clip_range_vf = vals.data_ptr(), float(clip_range_vf)
     m = _lib.make_mlp(params.mlp())
     with torch.cuda.device(dev):
         if params.use_sde:
@@ -304,12 +325,18 @@ class PPOTrainer:
         every minibatch that ran (the one `target_kl` stops at included), approx_kl is the mean over the minibatches of
         the last epoch that ran, entropy_loss and loss use each minibatch's log_std before its Adam step (gSDE: the mean
         per-sample entropy of the minibatch, from the kernel's entropy term), and loss is the last minibatch's.  The
-        learning rate is `learning_rate(progress_remaining)`."""
+        learning rate, clip_range and clip_range_vf are their schedules at progress_remaining, evaluated once per update;
+        with clip_range_vf, value_loss is the clipped loss and train/clip_range_vf is logged."""
         cfg, dev = self.cfg, self.params.flat.device
         T, n = rollout["advantages"].shape
         total = T * n
         bs = self.batch_size(total)
         lr = _progress_lr(cfg.learning_rate, self.progress_remaining)
+        clip = _progress_lr(cfg.clip_range, self.progress_remaining)
+        vfc = None if cfg.clip_range_vf is None else _progress_lr(cfg.clip_range_vf, self.progress_remaining)
+        if vfc is not None and not (vfc > 0 and math.isfinite(vfc)):
+            raise ValueError(f"clip_range_vf({self.progress_remaining}) = {vfc}: the schedule must stay finite and > 0")
+        vkw = {} if vfc is None else dict(clip_range_vf=vfc)
         nmb = -(-total // bs)
         sde = self.params.use_sde
         terms = torch.zeros(cfg.n_epochs * nmb, _lib.PPO_NTERMS_SDE if sde else _lib.PPO_NTERMS, dtype=torch.float64,
@@ -327,9 +354,9 @@ class PPOTrainer:
             for start in range(0, total, bs):
                 idx = perm[start:start + bs]
                 k = len(sizes)
-                loss_and_grad(self.params, rollout, idx, clip_range=cfg.clip_range, vf_coef=cfg.vf_coef,
+                loss_and_grad(self.params, rollout, idx, clip_range=clip, vf_coef=cfg.vf_coef,
                               ent_coef=cfg.ent_coef, normalize_advantage=cfg.normalize_advantage, grad_sum=self._grad,
-                              terms=terms[k], work=self._work)
+                              terms=terms[k], work=self._work, **vkw)
                 if not sde:
                     log_std_sums[k] = self.params.log_std.sum(dtype=torch.float64)    # this minibatch's entropy (no sync)
                 sizes.append(idx.numel())
@@ -356,12 +383,15 @@ class PPOTrainer:
         v, r = rollout["values"].reshape(-1).double(), rollout["returns"].reshape(-1).double()
         var_r = float(r.var())
         ev = float("nan") if var_r == 0 else 1.0 - float((r - v).var()) / var_r
-        return {"train/policy_gradient_loss": float(means[:, 0].mean()), "train/value_loss": float(means[:, 1].mean()),
+        logs = {"train/policy_gradient_loss": float(means[:, 0].mean()), "train/value_loss": float(means[:, 1].mean()),
                 "train/entropy_loss": float(-entropy.mean()), "train/approx_kl": float(means[epoch_start:, 3].mean()),
                 "train/clip_fraction": float(means[:, 2].mean()),
                 "train/loss": float(means[-1, 0] - cfg.ent_coef * entropy[-1] + cfg.vf_coef * means[-1, 1]),
                 "train/explained_variance": ev, "train/std": float(np.exp(log_std).mean()),
-                "train/n_updates": self.n_updates, "train/learning_rate": lr, "train/clip_range": cfg.clip_range}
+                "train/n_updates": self.n_updates, "train/learning_rate": lr, "train/clip_range": clip}
+        if vfc is not None:
+            logs["train/clip_range_vf"] = vfc
+        return logs
 
     def learn(self, total_timesteps: int, callback: Optional[Callable[[dict], None]] = None) -> list:
         """Alternates collect_rollout (n_steps of every env) and train until total_timesteps env-steps; returns one log
