@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 21
+#define R6_ABI_VERSION 22
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -168,7 +168,8 @@ typedef struct R6Buffers {
  * net_arch [dict(pi=[64, 64], vf=[64, 64])]: w0 [64][13], b0 [64], w1 [64][64], b1 [64] are the policy tower
  * (mlp_extractor.policy_net), vf_* the value tower (mlp_extractor.value_net); w2, b2 read the policy latent and
  * wv, bv the value latent.  Entry points without a separate-tower kernel return R6_EINVAL for such a network:
- * r6_policy* with tensor_cores = 1, r6_rollout with R6_ACT_MLP / R6_ACT_MLP_TC, r6_policy_sde_range, r6_ppo_grad_sde.
+ * r6_policy* with tensor_cores = 1, r6_rollout with R6_ACT_MLP / R6_ACT_MLP_TC, r6_policy_sde_range and r6_ppo_grad_sde
+ * (gSDE on the separate towers has its own entry points, r6_policy_sde_sep_range and r6_ppo_grad_sde_sep).
  */
 typedef struct R6Mlp {
     const float *w0, *b0;   /* [128][13], [128]   (separate towers: [64][13], [64]) */
@@ -333,6 +334,18 @@ int r6_policy_sde_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, in
                         float *log_prob, void *stream);
 
 /*
+ * r6_policy_sde_range for SB3 1.6's separate towers (R6Mlp with the value tower set; PPO("MlpPolicy", env, use_sde=True)
+ * without policy_kwargs): h is the POLICY tower's 64-unit latent, the value comes from the value tower and plays no part
+ * in the distribution.  Same arguments and outputs as r6_policy_sde_range; deterministic actions and the values are
+ * bit-identical to r6_policy_range's on the same towers.  tensor_cores = 0, 2 or 3.  Returns R6_EINVAL, before any CUDA
+ * call and writing nothing, for tensor_cores = 1, for a shared trunk (its gSDE policy is r6_policy_sde_range), and in
+ * modes 2 / 3 for w1 or vf_w1 not 16-byte aligned.
+ */
+int r6_policy_sde_sep_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, int64_t n, int64_t first, int64_t count,
+                            int32_t tensor_cores, int32_t stochastic, float *actions, float *actions_raw, float *values,
+                            float *log_prob, void *stream);
+
+/*
  * Generalised advantage estimation over a recorded rollout, on the device, so that the PPO update of
  * main_6DOF.py:136 (`model.learn`) can consume r6_rollout's trajectory buffers without a host round trip.
  * Restates stable-baselines3 1.6.0 `RolloutBuffer.compute_returns_and_advantage` (common/buffers.py; SB3 is a
@@ -460,16 +473,28 @@ int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *id
 #define R6_PPO_NPARAMS_SDE 10500
 #define R6_PPO_NTERMS_SDE 6
 #define R6_PPO_T_ENTROPY 5
+/* Size of the work buffer of r6_ppo_grad_sde and r6_ppo_grad_sde_sep for a minibatch of B samples (either layout). */
 int64_t r6_ppo_sde_work_bytes(int64_t B);
 int r6_ppo_grad_sde(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
                     const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream);
+
+/*
+ * r6_ppo_grad_sde for SB3 1.6's separate towers with gSDE (mlp with the value tower set; a shared trunk is R6_EINVAL).
+ * Flat layout R6_PPO_NPARAMS_SEP_SDE: the prefix of R6_PPO_NPARAMS_SEP through bv (10372 floats), then
+ * log_std [64][3] @10372 (16-byte aligned).  h above is the policy tower's latent, detached: no gradient flows through
+ * std into either tower, whose deltas are those of r6_ppo_grad on the separate towers.  grad_sum [R6_PPO_NPARAMS_SEP_SDE],
+ * terms [R6_PPO_NTERMS_SDE]; value clipping and its R6_EINVAL cases as r6_ppo_grad.
+ */
+#define R6_PPO_NPARAMS_SEP_SDE 10564
+int r6_ppo_grad_sde_sep(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
+                        const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream);
 
 /*
  * One torch.optim.Adam step (no weight decay, no amsgrad) on the flat parameters, after clip_grad_norm_:
  *     g = scale * grad_sum;  norm = ||g||_2 (accumulated in float64);  g *= min(1, max_grad_norm / (norm + 1e-6));
  *     m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g^2;
  *     p -= lr / (1 - beta1^step) * m / (sqrt(v) / sqrt(1 - beta2^step) + eps)
- * params, grad_sum, m, v: float32 [P] DEVICE (any P: R6_PPO_NPARAMS, R6_PPO_NPARAMS_SDE); step >= 1 counts the updates including this one; grad_norm_out
+ * params, grad_sum, m, v: float32 [P] DEVICE (any P: R6_PPO_NPARAMS, R6_PPO_NPARAMS_SDE, ...); step >= 1 counts the updates including this one; grad_norm_out
  * (nullable DEVICE double) receives the norm before clipping.
  */
 int r6_adam_step(float *params, const float *grad_sum, float *m, float *v, int64_t P, const R6AdamCoef *coef,

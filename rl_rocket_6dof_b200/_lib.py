@@ -12,7 +12,7 @@ from .params import R6Params
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libr6dof.so")
-ABI_VERSION = 21
+ABI_VERSION = 22
 
 u8p = C.c_void_p
 
@@ -67,6 +67,7 @@ PPO_NPARAMS = 10311
 PPO_NTERMS = 5
 PPO_NPARAMS_SDE = 10500
 PPO_NPARAMS_SEP = 10375
+PPO_NPARAMS_SEP_SDE = 10564
 PPO_NTERMS_SDE = 6
 SDE_NXI = 192
 
@@ -92,7 +93,7 @@ EXPORTS = ["r6_abi_version", "r6_last_error", "r6_params_size", "r6_buffers_size
            "r6_rollout", "r6_sim_step_raw", "r6_tgo", "r6_stats_reset", "r6_peak_fma", "r6_gae", "r6_policy", "r6_policy_ex", "r6_step_random", "r6_step_range", "r6_policy_range", "r6_work_bytes",
            "r6_ppo_rollout_size", "r6_ppo_coef_size", "r6_adam_coef_size", "r6_ppo_work_bytes", "r6_ppo_grad", "r6_adam_step",
            "r6_trunc_record", "r6_trunc_bootstrap", "r6_sde_size", "r6_sde_noise", "r6_policy_sde_range",
-           "r6_ppo_sde_work_bytes", "r6_ppo_grad_sde"]
+           "r6_ppo_sde_work_bytes", "r6_ppo_grad_sde", "r6_policy_sde_sep_range", "r6_ppo_grad_sde_sep"]
 
 
 class R6Error(RuntimeError):
@@ -164,10 +165,12 @@ def load(path: str | None = None):
     L.r6_sde_noise.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]
     L.r6_policy_sde_range.argtypes = [C.POINTER(R6Mlp), C.POINTER(R6Sde), C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32,
                                       C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_policy_sde_sep_range.argtypes = L.r6_policy_sde_range.argtypes
     L.r6_ppo_sde_work_bytes.argtypes = [C.c_int64]
     L.r6_ppo_sde_work_bytes.restype = C.c_int64
     L.r6_ppo_grad_sde.argtypes = [C.POINTER(R6Mlp), C.POINTER(R6Sde), C.POINTER(R6PpoRollout), C.c_void_p, C.c_int64,
                                   C.POINTER(R6PpoCoef), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_ppo_grad_sde_sep.argtypes = L.r6_ppo_grad_sde.argtypes
     L.r6_peak_fma.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
     _lib = L
     return L

@@ -29,14 +29,12 @@ STAT_NAMES = ["episodes", "return_sum", "length_sum", "landed", "ground", "out_o
 
 
 def _check_separate(mlp: dict, tensor_cores):
-    """Refuses, before anything is launched, what the kernels do not run for SB3 1.6's separate policy / value towers."""
+    """Refuses, before anything is launched, what the kernels do not run for SB3 1.6's separate policy / value towers
+    (with or without gSDE): the mma.sync mode."""
     if mlp.get("vf_w0") is None:
         return
     if int(tensor_cores) == 1:
         raise ValueError("the separate policy / value towers have no mma.sync policy kernel (tensor_cores=1): use 0, 2 or 3")
-    ls = mlp.get("log_std")
-    if ls is not None and ls.dim() == 2:
-        raise ValueError("gSDE is not implemented for the separate policy / value towers")
 
 
 class Rocket6DOFBatch:
@@ -209,11 +207,12 @@ class Rocket6DOFBatch:
                 act: int, raw: Optional[int], val: Optional[int], logp: Optional[int], stream: torch.cuda.Stream,
                 sde: Optional[_lib.R6Sde] = None):
         """The policy network over envs [first, first + count) of the component-major observations at device pointer
-        `obs` (r6_policy_range, or r6_policy_sde_range with gSDE inputs `sde`); the output pointers raw / val / logp may be
-        None (not written)."""
+        `obs` (r6_policy_range, or with gSDE inputs `sde` r6_policy_sde_range, r6_policy_sde_sep_range for the separate
+        towers); the output pointers raw / val / logp may be None (not written)."""
         if sde is not None:
-            _lib.check(self.lib.r6_policy_sde_range(C.byref(m), C.byref(sde), obs, self.num_envs, first, count, int(tensor_cores),
-                                                    int(bool(stochastic)), act, raw, val, logp, stream.cuda_stream), self.lib)
+            fn = self.lib.r6_policy_sde_sep_range if m.vf_w0 else self.lib.r6_policy_sde_range
+            _lib.check(fn(C.byref(m), C.byref(sde), obs, self.num_envs, first, count, int(tensor_cores), int(bool(stochastic)),
+                          act, raw, val, logp, stream.cuda_stream), self.lib)
             return
         _lib.check(self.lib.r6_policy_range(C.byref(m), obs, self.num_envs, first, count, int(tensor_cores),
                                             int(bool(stochastic)), self.seed_value, self.env_offset, step_index, act, raw,
@@ -393,8 +392,9 @@ class Rocket6DOFBatch:
         values, all without a host synchronise.  Needs auto-reset (ValueError otherwise).  The default False leaves the
         rewards as the env returned them.
 
-        `mlp` may hold SB3 1.6's separate policy / value towers (vf_w0 ... vf_b1, `ActorCriticParams.LAYOUT_SEP`): the
-        values are then the value tower's.  That network has no mma.sync kernel: tensor_cores=1 raises ValueError.
+        `mlp` may hold SB3 1.6's separate policy / value towers (vf_w0 ... vf_b1, `ActorCriticParams.LAYOUT_SEP`, or
+        LAYOUT_SEP_SDE with gSDE, whose h is the policy tower's latent): the values are then the value tower's.  That
+        network has no mma.sync kernel: tensor_cores=1 raises ValueError.
 
         A [64, 3] log_std in `mlp` collects with gSDE, as SB3's collect_rollouts with use_sde=True: `reset_noise` at the
         start of the rollout, and with sde_sample_freq > 0 every lane redraws the noise of its env range before step j

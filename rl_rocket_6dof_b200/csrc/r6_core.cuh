@@ -1670,6 +1670,33 @@ R6_HD void mlp_forward_sep(const float *W, const float *x, float (&out)[4])
     out[3] = o3 + W[kMlpOffB2 + 3];
 }
 
+// mlp_forward_sep with latent(k, h) called on every unit of the POLICY tower's latent (the gSDE head of the separate
+// towers reads it): the same operations in the same order, so out is bit-identical to mlp_forward_sep's.  A copy rather
+// than a callback added to mlp_forward_sep, so that the kernels built on that keep their register allocation.
+template <class Latent>
+R6_HD void mlp_forward_sep_latent(const float *W, const float *x, float (&out)[4], Latent &&latent)
+{
+    float acc[kMlpH1];
+    mlp_tower_acc<kMlpH1>(W, x, acc, [](int, float) {});
+    float o3 = 0.0f;
+#pragma unroll
+    for (int k = 0; k < kMlpH1; k++) o3 = f32_fma(W[kMlpOffW2 + 3 * kMlpH1 + k], tanhf(acc[k] + W[kMlpOffVb1 + k]), o3);
+    mlp_tower_acc<0>(W, x, acc, [](int, float) {});
+    float o0 = 0.0f, o1 = 0.0f, o2 = 0.0f;
+#pragma unroll
+    for (int k = 0; k < kMlpH1; k++) {
+        const float h = tanhf(acc[k] + W[kMlpOffB1 + k]);
+        latent(k, h);
+        o0 = f32_fma(W[kMlpOffW2 + k], h, o0);
+        o1 = f32_fma(W[kMlpOffW2 + kMlpH1 + k], h, o1);
+        o2 = f32_fma(W[kMlpOffW2 + 2 * kMlpH1 + k], h, o2);
+    }
+    out[0] = o0 + W[kMlpOffB2];
+    out[1] = o1 + W[kMlpOffB2 + 1];
+    out[2] = o2 + W[kMlpOffB2 + 2];
+    out[3] = o3 + W[kMlpOffB2 + 3];
+}
+
 // sin(pi x), cos(pi x): exact argument reduction, 1 ulp (CUDA math library); the host build in double precision
 R6_HD void sincospi_f32(float x, float &s, float &c)
 {

@@ -1264,6 +1264,195 @@ policy_tc5_sde_kernel(const R6Mlp mlp, const SdeIn sde, const float *__restrict_
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
 }
 
+// policy_sep_kernel with the gSDE head (r6_policy_sde_sep_range tensor_cores = 0): the sums of policy_sde_kernel over the
+// POLICY tower's latent (mlp_forward_sep_latent), sigma and sigma^2 staged after the packed weights
+__global__ void __launch_bounds__(kThreads, 4)
+policy_sep_sde_kernel(const R6Mlp mlp, const SdeIn sde, const float *__restrict__ obs, int64_t n, const PolicyOut po)
+{
+    extern __shared__ __align__(16) double r6_smem[];
+    float *Ws = reinterpret_cast<float *>(r6_smem);
+    float *sig = Ws + kMlpFloatsSep, *sig2 = sig + kSdeXi;
+    for (int idx = threadIdx.x; idx < kMlpFloatsSep; idx += kThreads) Ws[idx] = mlp_pack_element_sep(mlp, idx);
+    sde_stage(sde.log_std, sig, sig2, threadIdx.x, kThreads);
+    __syncthreads();
+    const int64_t i1 = po.i1;
+    const int64_t tiles = (i1 - po.i0 + kThreads - 1) / kThreads;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        const int64_t i = po.i0 + tile * kThreads + threadIdx.x;
+        const bool in = i < i1, draw = in && po.stochastic != 0;
+        float x[kMlpIn], out[4], nz[3] = {0.0f, 0.0f, 0.0f}, var[3] = {0.0f, 0.0f, 0.0f};
+#pragma unroll
+        for (int c = 0; c < kMlpIn; c++) x[c] = in ? obs[(int64_t)c * n + i] : 0.0f;
+        mlp_forward_sep_latent(Ws, x, out, [&](int k, float h) {
+            const float hh = h * h;
+#pragma unroll
+            for (int a = 0; a < 3; a++) {
+                const int c = 3 * k + a;
+                if (draw) nz[a] = f32_fma(h, sig[c] * __ldg(sde.xi + (int64_t)c * n + i), nz[a]);
+                var[a] = f32_fma(hh, sig2[c], var[a]);
+            }
+        });
+        if (in) sde_epilogue(po, i, out, nz, var);
+    }
+}
+constexpr int kSmemPolicySepSde = kSmemPolicySep + 2 * kSdeXi * (int)sizeof(float);
+
+// policy_tc5_sep_kernel with the gSDE head (r6_policy_sde_sep_range tensor_cores = 2 / 3): the policy latent's epilogue
+// (the last hidden-layer epilogue, on D1 after the policy chain) is epilogue_in_tmem_sde, and the second column half hands
+// its sums to the first through shared memory as in policy_tc5_sde_kernel.  The value chain is policy_tc5_sep_kernel's.
+// Shared memory: the separate-tower region (kOffSep..) and then the gSDE region (kOffSepSde..).
+template <bool kFaithful>
+__global__ void __launch_bounds__(tc5::kThreads, 1)
+policy_tc5_sep_sde_kernel(const R6Mlp mlp, const SdeIn sde, const float *__restrict__ obs, int64_t n, const PolicyOut po)
+{
+    using namespace tc5;
+    extern __shared__ __align__(16) double r6_smem[];
+    char *S = reinterpret_cast<char *>(r6_smem);
+    const int tid = threadIdx.x, group = tid >> 8, lt = tid & 127, half = (tid >> 7) & 1, warp = tid >> 5;
+    grid_dependency_wait();
+    // ---- one-time per CTA: [w0; vf_w0] and [w1 | vf_w1] split into TF32 hi / lo parts in canonical K-major tiles ----
+    for (int idx = tid; idx < 128 * 16; idx += tc5::kThreads) {
+        const int r = idx >> 4, k = idx & 15;
+        const float *w0 = r < kMlpH1 ? mlp.w0 + r * kMlpIn : mlp.vf_w0 + (r - kMlpH1) * kMlpIn;
+        float hi, lo;
+        split_tf32(k < kMlpIn ? w0[k] : 0.0f, hi, lo);
+        *reinterpret_cast<float *>(S + kOffW0h + tile_off(r, k, 16)) = hi;
+        *reinterpret_cast<float *>(S + kOffW0l + tile_off(r, k, 16)) = lo;
+    }
+    for (int idx = tid; idx < 64 * 32; idx += tc5::kThreads) {
+        const int r = idx >> 5, k = (idx & 31) * 4;
+        const float *src = k < kMlpH1 ? mlp.w1 + r * kMlpH1 + k : mlp.vf_w1 + r * kMlpH1 + (k - kMlpH1);
+        const float4 w = *reinterpret_cast<const float4 *>(src);
+        float4 h, l;
+        split_tf32(w.x, h.x, l.x); split_tf32(w.y, h.y, l.y); split_tf32(w.z, h.z, l.z); split_tf32(w.w, h.w, l.w);
+        *reinterpret_cast<float4 *>(S + kOffW1h + tile_off(r, k, 128)) = h;
+        *reinterpret_cast<float4 *>(S + kOffW1l + tile_off(r, k, 128)) = l;
+    }
+    for (int idx = tid; idx < 16 * 16; idx += tc5::kThreads) {        // action_net rows 0..2; row 3 (value) stays zero
+        const int r = idx >> 4, k = (idx & 15) * 4;
+        float4 h, l;
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k] : 0.0f, h.x, l.x);
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k + 1] : 0.0f, h.y, l.y);
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k + 2] : 0.0f, h.z, l.z);
+        split_tf32(r < kMlpOut ? mlp.w2[r * kMlpH1 + k + 3] : 0.0f, h.w, l.w);
+        *reinterpret_cast<float4 *>(S + kOffW2h + tile_off(r, k, 64)) = h;
+        *reinterpret_cast<float4 *>(S + kOffW2l + tile_off(r, k, 64)) = l;
+    }
+    float *bias = reinterpret_cast<float *>(S + kOffBias);
+    float *vb1 = reinterpret_cast<float *>(S + kOffSep), *wv = reinterpret_cast<float *>(S + kOffSepWv);
+    float *vpart = reinterpret_cast<float *>(S + kOffSepPart) + group * kTile;
+    const float bscale = kFaithful ? kTwoLog2e : 1.0f;
+    if (tid < 64) bias[tid] = bscale * mlp.b0[tid];
+    else if (tid < 128) bias[tid] = bscale * mlp.vf_b0[tid - 64];
+    if (tid < 64) {
+        bias[128 + tid] = bscale * mlp.b1[tid];
+        vb1[tid] = bscale * mlp.vf_b1[tid];
+        wv[tid] = mlp.wv != nullptr ? mlp.wv[tid] : 0.0f;
+    }
+    if (tid < 4) bias[192 + tid] = mlp_b2_row(mlp, tid);
+    sde_stage(sde.log_std, reinterpret_cast<float *>(S + kOffSepSde), reinterpret_cast<float *>(S + kOffSepSde) + kSdeXi, tid,
+              tc5::kThreads);
+    if (tid == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(S + kOffBar)) : "memory");
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(S + kOffBar + 8)) : "memory");
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(S + kOffTmemPtr)), "n"(kTmemCols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    fence_async_smem();
+    fence_before();
+    __syncthreads();
+    fence_after();
+    const int warp_u = __shfl_sync(0xffffffffu, warp, 0);
+    const uint32_t tmem_base = __shfl_sync(0xffffffffu, *reinterpret_cast<volatile uint32_t *>(S + kOffTmemPtr), 0);
+    const uint32_t tmem_g = tmem_base + (uint32_t)(warp_u >> 3) * kGroupCols;
+    const uint32_t tmem_row = tmem_g + ((uint32_t)((warp & 3) * 32) << 16);
+    const uint32_t sbase = __shfl_sync(0xffffffffu, smem_u32(S), 0);
+    const uint32_t aW0h = sbase + kOffW0h, aW0l = sbase + kOffW0l, aW1h = sbase + kOffW1h;
+    const uint32_t aW1l = sbase + kOffW1l, aW2h = sbase + kOffW2h, aW2l = sbase + kOffW2l;
+    const uint32_t bar = sbase + kOffBar + 8 * (uint32_t)(warp_u >> 3);
+    const bool issuer = (warp_u & 7) == 0;
+    uint32_t phase = 0;
+    const int64_t i1 = po.i1;
+    const int64_t tiles = (i1 - po.i0 + kTile - 1) / kTile;
+    const int64_t slots = (tiles + 2 * (int64_t)gridDim.x - 1) / (2 * (int64_t)gridDim.x);
+    float xo[8];
+    auto load_obs = [&](int64_t tile) {
+        const int64_t i = po.i0 + tile * kTile + lt;
+#pragma unroll
+        for (int q = 0; q < 8; q++) {
+            const int k = 8 * half + q;
+            xo[q] = (k < kMlpIn && i < i1) ? __ldg(obs + (int64_t)k * n + i) : 0.0f;
+        }
+    };
+    load_obs(2 * (int64_t)blockIdx.x + group);
+    float outv[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+    float nzv[3] = {0.0f, 0.0f, 0.0f}, varv[3] = {0.0f, 0.0f, 0.0f};
+    int64_t out_i = i1;
+    if (group == 1) token_pass(0);
+    for (int64_t slot = 0; slot < slots; slot++) {
+        const int64_t tile = 2 * ((int64_t)blockIdx.x + slot * gridDim.x) + group;
+        const int64_t i = po.i0 + tile * kTile + lt;
+        {
+            float h[8], l[8];
+#pragma unroll
+            for (int q = 0; q < 8; q++) split_tf32(xo[q], h[q], l[q]);
+            tmem_st8(tmem_row + kColD1 + 8 * half, h);
+            if (kFaithful) tmem_st8(tmem_row + kColL + 8 * half, l);
+            tmem_st_wait();
+        }
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD0, tmem_g + kColD1, tmem_g + kColL, aW0h, aW0l, 512, 2, 128, false); if (elect_one()) mma_commit(bar); }
+        load_obs(tile + 2 * (int64_t)gridDim.x);
+        if (half == 0 && out_i < i1) sde_epilogue(po, out_i, outv, nzv, varv);
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- value tower: layer 0 units 64..127 -> its layer 1 (W1 columns 64..127 = vf_w1) ----
+        epilogue_in_tmem<kFaithful>(tmem_row, kColD0 + 64, bias + 64, half, group);
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD1, tmem_g + kColD0 + 64, tmem_g + kColL, aW1h + 2048, aW1l + 2048, 4096, 8, 64, false); if (elect_one()) mma_commit(bar); }
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- value = value_net(tanh(D1 + vf_b1)) on the CUDA cores; the second half's sum goes through shared memory ----
+        const float vs = epilogue_value<kFaithful>(tmem_row, kColD1, vb1, wv, half, group);
+        if (half == 1) vpart[lt] = vs;
+        // ---- policy tower: layer 0 units 0..63 -> its layer 1 (W1 columns 0..63 = w1), over the value chain's D1 ----
+        epilogue_in_tmem<kFaithful>(tmem_row, kColD0, bias, half, group);
+        fence_before(); group_sync(group);       // also publishes vpart to the first half
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD1, tmem_g + kColD0, tmem_g + kColL, aW1h, aW1l, 4096, 8, 64, false); if (elect_one()) mma_commit(bar); }
+        const float value = half == 0 ? vs + vpart[lt] : 0.0f;
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        // ---- policy latent -> action_net, with the gSDE sums over this thread's 32 latent units ----
+        float pnz[3], pvar[3];
+        float *const sig = reinterpret_cast<float *>(S + kOffSepSde), *const sig2 = sig + kSdeXi;
+        float *const part = reinterpret_cast<float *>(S + kOffSepSdePart) + (group * kTile + lt) * 6;   // this row's exchange slot
+        epilogue_in_tmem_sde<kFaithful>(tmem_row, kColD1, bias + 128, half, group, sig, sig2, sde.xi, n, i,
+                                        po.stochastic != 0 && i < i1, pnz, pvar);
+        if (half == 1) {                 // read by the row's first half after the group barrier below
+#pragma unroll
+            for (int a = 0; a < 3; a++) { part[a] = pnz[a]; part[3 + a] = pvar[a]; }
+        }
+        fence_before(); group_sync(group);
+        if (issuer) { fence_after(); issue_mmas<kFaithful>(tmem_g + kColD0, tmem_g + kColD1, tmem_g + kColL, aW2h, aW2l, 2048, 8, 16, false); if (elect_one()) mma_commit(bar); }
+        bar_wait(bar, phase); phase ^= 1; fence_after();
+        out_i = i1;
+        if (half == 0) {
+            tmem_ld4(tmem_row + kColD0, outv);
+#pragma unroll
+            for (int q = 0; q < 3; q++) outv[q] += bias[192 + q];
+            outv[3] = value + bias[195];
+#pragma unroll
+            for (int a = 0; a < 3; a++) { nzv[a] = pnz[a] + part[a]; varv[a] = pvar[a] + part[3 + a]; }
+            out_i = i;
+        }
+    }
+    if (half == 0 && out_i < i1) sde_epilogue(po, out_i, outv, nzv, varv);
+    if (group == 0) token_take(0);
+    fence_before();
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
+}
+
 // GAE scan: one thread per env walks its column of the [T][n] trajectory backwards (every access coalesced over
 // envs).  HBM-bound: 17 B per (t, env).  No FMA contraction: the float32 roundings are NumPy's.
 __global__ void __launch_bounds__(256)
@@ -1754,6 +1943,233 @@ ppo_grad_sep_kernel(const R6Mlp mlp, const R6PpoRollout ro, const int64_t *__res
     }
 }
 
+// r6_ppo_grad_sde_sep: ppo_grad_sep_kernel with the gSDE head of ppo_grad_sde_kernel.  var comes from sde_latent_var over
+// the POLICY latent rows (kPpoRowHP), rows G + 4 .. G + 6 carry r_a, one more row (kPpoRowE) the per-sample entropy, and
+// sigma^2 [64][3] follows the dW1 accumulators.  The log_std accumulators (threads 0..63, sum_s r_a h_p^2) read the policy
+// latent in the head pass, before ppo_delta1_sep overwrites its rows; the tower deltas are ppo_delta1_sep's (the latent is
+// detached: no gradient through std).  226,528 B of shared memory: one CTA per SM.
+constexpr int kSmemPpoSepSde = (kMlpFloatsSep + kPpoRowsSde * kPpoTS + kPpoAccW1 + kSdeXi) * (int)sizeof(float);
+static_assert(kSmemPpoSepSde <= 232448 && kPpoRowE == kPpoRowG + 12, "PPO separate-tower gSDE tile layout");
+
+template <bool kVfClip>
+__global__ void __launch_bounds__(kThreads, 1)
+ppo_grad_sep_sde_kernel(const R6Mlp mlp, const float *__restrict__ log_std, const R6PpoRollout ro,
+                        const int64_t *__restrict__ idx, int64_t B, float clip, float vf, float ent, float vfc,
+                        const double *__restrict__ adv_stats, double *__restrict__ part_terms, float *__restrict__ part)
+{
+    extern __shared__ __align__(16) double r6_smem[];
+    float *Ws = reinterpret_cast<float *>(r6_smem);
+    float *S = Ws + kMlpFloatsSep;
+    float *A1 = S + kPpoRowsSde * kPpoTS;
+    float *sig2 = A1 + kPpoAccW1;
+    const int tid = threadIdx.x, kq = tid & 7, jq = tid >> 3;
+    for (int i = tid; i < kMlpFloatsSep; i += kThreads) Ws[i] = mlp_pack_element_sep(mlp, i);
+    for (int i = tid; i < kPpoAccW1; i += kThreads) A1[i] = 0.0f;
+    for (int c = tid; c < kSdeXi; c += kThreads) {
+        const float sg = expf(log_std[c]);
+        sig2[c] = sg * sg;
+    }
+    const int64_t nsamp = ro.T * ro.n;
+    float aW0[14], aHd[6];                   // dW0 / dvf_w0 row tid, its bias; dW2[0..2][tid], dwv, db1, dvf_b1
+    float aLs[3] = {0.0f, 0.0f, 0.0f};       // sum_s r_a h_p,tid^2 (threads 0..63)
+    double aS = 0.0;
+#pragma unroll
+    for (int c = 0; c < 14; c++) aW0[c] = 0.0f;
+#pragma unroll
+    for (int c = 0; c < 6; c++) aHd[c] = 0.0f;
+    __syncthreads();
+    const int64_t tiles = (B + kThreads - 1) / kThreads;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        PpoHeadSde hd = {};
+        {   // this thread's sample: forward and loss head
+            const int64_t s = tile * kThreads + tid;
+            const int64_t q = s < B ? idx[s] : -1;
+            const bool ok = q >= 0 && q < nsamp;
+            float x[kMlpIn], out[4];
+            if (ok) {
+                const int64_t t = q / ro.n, i = q - t * ro.n;
+                const float *o = ro.obs + t * ro.obs_stride_step + i * ro.obs_stride_env;
+#pragma unroll
+                for (int c = 0; c < kMlpIn; c++) x[c] = o[c * ro.obs_stride_comp];
+            } else {
+#pragma unroll
+                for (int c = 0; c < kMlpIn; c++) x[c] = 0.0f;
+            }
+#pragma unroll
+            for (int c = 0; c < kMlpIn; c++) S[(kPpoRowX + c) * kPpoTS + tid] = x[c];
+            ppo_forward_sep(Ws, x, S + kPpoRowH0 * kPpoTS + tid, S + kPpoRowHP * kPpoTS + tid, S + kPpoRowHV * kPpoTS + tid,
+                            kPpoTS, out);
+            if (ok) {
+                const float a[3] = {ro.actions[3 * q], ro.actions[3 * q + 1], ro.actions[3 * q + 2]};
+                float var[3];
+                sde_latent_var(S + kPpoRowHP * kPpoTS + tid, kPpoTS, sig2, var);
+                ppo_head_sde(out, a, ro.log_probs[q], ppo_advantage(ro.advantages[q], adv_stats), ro.returns[q], var, clip, vf,
+                             ent, hd);
+                if constexpr (kVfClip) ppo_value_clip(out[3], ro.old_values[q], ro.returns[q], vfc, vf, hd);
+            }
+#pragma unroll
+            for (int r = 0; r < 7; r++) S[(kPpoRowG + r) * kPpoTS + tid] = hd.g[r];
+            S[(kPpoRowG + 7) * kPpoTS + tid] = (s < B && !ok) ? 1.0f : 0.0f;
+            S[(kPpoRowT + 0) * kPpoTS + tid] = hd.pg;
+            S[(kPpoRowT + 1) * kPpoTS + tid] = hd.vloss;
+            S[(kPpoRowT + 2) * kPpoTS + tid] = hd.clipped;
+            S[(kPpoRowT + 3) * kPpoTS + tid] = hd.kl;
+            S[kPpoRowE * kPpoTS + tid] = hd.ent;
+        }
+        __syncthreads();
+        // heads from the latents (dW2 on h1p, dwv on h1v), log_std from h1p^2, and the scalar sums, before the latent rows
+        // become deltas
+        if (tid < kMlpH1) {
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                const F4 hp = ld4(S + (kPpoRowHP + tid) * kPpoTS + s4), hv = ld4(S + (kPpoRowHV + tid) * kPpoTS + s4);
+#pragma unroll
+                for (int c = 0; c < 4; c++) {
+                    const F4 g = ld4(S + (kPpoRowG + c) * kPpoTS + s4);
+                    const F4 h = c < 3 ? hp : hv;
+                    float a = aHd[c];
+                    a = __fmaf_rn(g.x, h.x, a); a = __fmaf_rn(g.y, h.y, a);
+                    a = __fmaf_rn(g.z, h.z, a); a = __fmaf_rn(g.w, h.w, a);
+                    aHd[c] = a;
+                }
+                const F4 hh = {hp.x * hp.x, hp.y * hp.y, hp.z * hp.z, hp.w * hp.w};
+#pragma unroll
+                for (int c = 0; c < 3; c++) {
+                    const F4 r = ld4(S + (kPpoRowG + 4 + c) * kPpoTS + s4);
+                    float a = aLs[c];
+                    a = __fmaf_rn(r.x, hh.x, a); a = __fmaf_rn(r.y, hh.y, a);
+                    a = __fmaf_rn(r.z, hh.z, a); a = __fmaf_rn(r.w, hh.w, a);
+                    aLs[c] = a;
+                }
+            }
+        } else if (tid < kMlpH1 + 13) {
+            const float *row = S + (kPpoRowG + tid - kMlpH1) * kPpoTS;
+#pragma unroll 4
+            for (int s = 0; s < kThreads; s++) aS += (double)row[s];
+        }
+        __syncthreads();
+        ppo_delta1_sep(Ws, hd, S + kPpoRowHP * kPpoTS + tid, S + kPpoRowHV * kPpoTS + tid, kPpoTS);
+        __syncthreads();
+        // dW1p / dW1v += delta1^T h0 (columns jq + 16 c: c < 4 policy units, c >= 4 value units), db1 / dvf_b1
+#pragma unroll 1
+        for (int r0 = 0; r0 < 8; r0 += 4) {
+            float aW1[4][8];
+#pragma unroll
+            for (int r = 0; r < 4; r++)
+#pragma unroll
+                for (int c = 0; c < 8; c++) aW1[r][c] = A1[((r0 + r) * 8 + c) * kThreads + tid];
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                F4 h[8];
+#pragma unroll
+                for (int c = 0; c < 8; c++) h[c] = ld4(S + (kPpoRowH0 + jq + 16 * c) * kPpoTS + s4);
+#pragma unroll
+                for (int r = 0; r < 4; r++) {
+                    const F4 dp = ld4(S + (kPpoRowHP + kq + 8 * (r0 + r)) * kPpoTS + s4);
+                    const F4 dv = ld4(S + (kPpoRowHV + kq + 8 * (r0 + r)) * kPpoTS + s4);
+#pragma unroll
+                    for (int c = 0; c < 8; c++) {
+                        const F4 d = c < 4 ? dp : dv;
+                        float a = aW1[r][c];
+                        a = __fmaf_rn(d.x, h[c].x, a); a = __fmaf_rn(d.y, h[c].y, a);
+                        a = __fmaf_rn(d.z, h[c].z, a); a = __fmaf_rn(d.w, h[c].w, a);
+                        aW1[r][c] = a;
+                    }
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < 4; r++)
+#pragma unroll
+                for (int c = 0; c < 8; c++) A1[((r0 + r) * 8 + c) * kThreads + tid] = aW1[r][c];
+        }
+        if (tid < kMlpH1) {
+#pragma unroll 1
+            for (int s4 = 0; s4 < kThreads; s4 += 4) {
+                const F4 dp = ld4(S + (kPpoRowHP + tid) * kPpoTS + s4), dv = ld4(S + (kPpoRowHV + tid) * kPpoTS + s4);
+                aHd[4] = (((aHd[4] + dp.x) + dp.y) + dp.z) + dp.w;
+                aHd[5] = (((aHd[5] + dv.x) + dv.y) + dv.z) + dv.w;
+            }
+        }
+        __syncthreads();
+        {   // delta0 over h0, in place, each tower's units from its own delta1: this thread's column only
+            float d1[kMlpH1];
+#pragma unroll 1
+            for (int t = 0; t < 2; t++) {
+                const int row = t == 0 ? kPpoRowHP : kPpoRowHV;
+#pragma unroll
+                for (int k = 0; k < kMlpH1; k++) d1[k] = S[(row + k) * kPpoTS + tid];
+#pragma unroll 1
+                for (int j = t * kMlpH1; j < (t + 1) * kMlpH1; j++) {
+                    float *p = S + (kPpoRowH0 + j) * kPpoTS + tid;
+                    *p = ppo_delta0(Ws, j, d1, *p);
+                }
+            }
+        }
+        __syncthreads();
+        // dW0[tid] += delta0_tid [x, 1]   (rows 0..63 the policy tower's w0, 64..127 the value tower's: stacked in P)
+#pragma unroll 1
+        for (int s4 = 0; s4 < kThreads; s4 += 4) {
+            const F4 d = ld4(S + (kPpoRowH0 + tid) * kPpoTS + s4);
+#pragma unroll
+            for (int c = 0; c < kMlpIn; c++) {
+                const F4 xv = ld4(S + (kPpoRowX + c) * kPpoTS + s4);
+                float a = aW0[c];
+                a = __fmaf_rn(d.x, xv.x, a); a = __fmaf_rn(d.y, xv.y, a);
+                a = __fmaf_rn(d.z, xv.z, a); a = __fmaf_rn(d.w, xv.w, a);
+                aW0[c] = a;
+            }
+            aW0[13] = (((aW0[13] + d.x) + d.y) + d.z) + d.w;
+        }
+        __syncthreads();
+    }
+    float *P = part + (int64_t)blockIdx.x * kPpoParamsSepSde;
+#pragma unroll
+    for (int r = 0; r < 8; r++)
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            const int k = kq + 8 * r, j = jq + 16 * c;
+            P[(c < 4 ? kSepOffW1 + k * kMlpH1 + j : kSepOffVw1 + k * kMlpH1 + j - kMlpH1)] = A1[(r * 8 + c) * kThreads + tid];
+        }
+#pragma unroll
+    for (int c = 0; c < kMlpIn; c++) P[kSepOffW0 + tid * kMlpIn + c] = aW0[c];
+    P[kSepOffB0 + tid] = aW0[13];
+    if (tid < kMlpH1) {
+#pragma unroll
+        for (int c = 0; c < 3; c++) P[kSepOffW2 + c * kMlpH1 + tid] = aHd[c];
+        P[kSepOffWv + tid] = aHd[3];
+        P[kSepOffB1 + tid] = aHd[4];
+        P[kSepOffVb1 + tid] = aHd[5];
+#pragma unroll
+        for (int c = 0; c < 3; c++) P[kSepOffLogStd + 3 * tid + c] = aLs[c] * sig2[3 * tid + c];
+    } else if (tid < kMlpH1 + 13) {
+        const int r = tid - kMlpH1;          // rows: g0..g2 (db2), g3 (dbv), g4..g6 (r_a sums, unused), bad index, 4 loss
+        double *T = part_terms + (int64_t)blockIdx.x * R6_PPO_NTERMS_SDE;   // terms, entropy
+        if (r < 3) P[kSepOffB2 + r] = (float)aS;
+        else if (r == 3) P[kSepOffBv] = (float)aS;
+        else if (r == 7) T[R6_PPO_T_BAD_INDEX] = aS;
+        else if (r >= 8 && r < 12) T[r - 8] = aS;
+        else if (r == 12) T[R6_PPO_T_ENTROPY] = aS;
+    }
+}
+
+// ppo_reduce_kernel over the separate-tower gSDE layout
+__global__ void __launch_bounds__(256)
+ppo_reduce_sep_sde_kernel(const double *__restrict__ part_terms, const float *__restrict__ part, int G, float *__restrict__ grad,
+                          double *__restrict__ terms)
+{
+    const int p = blockIdx.x * 256 + threadIdx.x;
+    if (p < kPpoParamsSepSde) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += (double)part[(int64_t)g * kPpoParamsSepSde + p];
+        grad[p] = (float)s;
+    }
+    if (blockIdx.x == 0 && threadIdx.x < R6_PPO_NTERMS_SDE) {
+        double s = 0.0;
+        for (int g = 0; g < G; g++) s += part_terms[g * R6_PPO_NTERMS_SDE + threadIdx.x];
+        terms[threadIdx.x] = s;
+    }
+}
+
 // ppo_reduce_kernel over the separate-tower layout
 __global__ void __launch_bounds__(256)
 ppo_reduce_sep_kernel(const double *__restrict__ part_terms, const float *__restrict__ part, int G, float *__restrict__ grad,
@@ -1912,6 +2328,11 @@ int ensure_attributes()
     rc |= enable_smem(policy_tc5_sep_kernel<false>, tc5::kSmemBytesSep);
     rc |= enable_smem(ppo_grad_sep_kernel<false>, kSmemPpoSep);
     rc |= enable_smem(ppo_grad_sep_kernel<true>, kSmemPpoSep);
+    rc |= enable_smem(policy_sep_sde_kernel, kSmemPolicySepSde);
+    rc |= enable_smem(policy_tc5_sep_sde_kernel<true>, tc5::kSmemBytesSepSde);
+    rc |= enable_smem(policy_tc5_sep_sde_kernel<false>, tc5::kSmemBytesSepSde);
+    rc |= enable_smem(ppo_grad_sep_sde_kernel<false>, kSmemPpoSepSde);
+    rc |= enable_smem(ppo_grad_sep_sde_kernel<true>, kSmemPpoSepSde);
     rc |= enable_smem(sim_raw_kernel<false>);
     rc |= enable_smem(sim_raw_kernel<true>);
     if (rc) return R6_ECUDA;
@@ -2211,7 +2632,7 @@ int r6_policy_sde_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, in
                         float *log_prob, void *stream)
 {
     if (int rc = check_mlp(mlp)) return rc;
-    if (int rc = reject_separate(mlp, "r6_policy_sde_range (gSDE)")) return rc;
+    if (int rc = reject_separate(mlp, "r6_policy_sde_range (gSDE; r6_policy_sde_sep_range runs the separate towers)")) return rc;
     if (!sde || !sde->log_std || !sde->xi || !obs || !actions) return fail(R6_EINVAL, "null pointer%s");
     if (n < 0) return fail(R6_EINVAL, "n < 0%s");
     if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
@@ -2238,6 +2659,43 @@ int r6_policy_sde_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, in
         policy_sde_kernel<<<g, kThreads, kSmemPolicySde, s>>>(*mlp, si, obs, n, po);
     }
     return check_launch("r6_policy_sde_range");
+}
+
+int r6_policy_sde_sep_range(const R6Mlp *mlp, const R6Sde *sde, const float *obs, int64_t n, int64_t first, int64_t count,
+                            int32_t tensor_cores, int32_t stochastic, float *actions, float *actions_raw, float *values,
+                            float *log_prob, void *stream)
+{
+    if (int rc = check_mlp(mlp)) return rc;
+    if (!mlp_separate(*mlp))
+        return fail(R6_EINVAL, "r6_policy_sde_sep_range needs the separate towers (R6Mlp.vf_w0 set): the shared trunk's gSDE "
+                               "policy is r6_policy_sde_range%s");
+    if (!sde || !sde->log_std || !sde->xi || !obs || !actions) return fail(R6_EINVAL, "null pointer%s");
+    if (n < 0) return fail(R6_EINVAL, "n < 0%s");
+    if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
+    if (tensor_cores == 1) return fail(R6_EINVAL, "gSDE has no mma.sync policy kernel (tensor_cores = 1): use 0, 2 or 3%s");
+    if (tensor_cores < 0 || tensor_cores > 3) return fail(R6_EINVAL, "tensor_cores must be 0, 2 or 3%s");
+    if (tensor_cores >= 2 && ((reinterpret_cast<uintptr_t>(mlp->w1) | reinterpret_cast<uintptr_t>(mlp->vf_w1)) & 15u) != 0)
+        return fail(R6_EINVAL, "tensor_cores = 2 / 3 need w1 and vf_w1 16-byte aligned%s");
+    if (count == 0) return R6_OK;
+    int rc = ensure_attributes();
+    if (rc) return rc;
+    int dev = 0, sm_count = 0;
+    cudaGetDevice(&dev);
+    if (cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sm_count <= 0) sm_count = 148;
+    const PolicyOut po = {actions, actions_raw, values, log_prob, stochastic, 0, 0, 0, first, first + count};
+    const SdeIn si = {sde->log_std, sde->xi};
+    cudaStream_t s = (cudaStream_t)stream;
+    if (tensor_cores >= 2) {
+        const int64_t pairs = (blocks_for(count) + 1) / 2;
+        const unsigned g5 = (unsigned)(pairs < sm_count ? pairs : sm_count);
+        if (tensor_cores == 3) launch_pdl(policy_tc5_sep_sde_kernel<true>, g5, tc5::kThreads, tc5::kSmemBytesSepSde, s, *mlp, si, obs, n, po);
+        else launch_pdl(policy_tc5_sep_sde_kernel<false>, g5, tc5::kThreads, tc5::kSmemBytesSepSde, s, *mlp, si, obs, n, po);
+    } else {
+        const int64_t wave = (int64_t)sm_count * 4;
+        const unsigned g = (unsigned)(blocks_for(count) < wave ? blocks_for(count) : wave);
+        policy_sep_sde_kernel<<<g, kThreads, kSmemPolicySepSde, s>>>(*mlp, si, obs, n, po);
+    }
+    return check_launch("r6_policy_sde_sep_range");
 }
 
 int r6_policy_ex(const R6Mlp *mlp, const float *obs, int64_t n, int32_t tensor_cores, int32_t stochastic, uint64_t seed,
@@ -2301,13 +2759,14 @@ int64_t r6_ppo_work_bytes(int64_t B)
 }  // extern "C"
 
 namespace {
-// r6_ppo_grad / r6_ppo_grad_sde (sde_log_std != NULL): the gradient kernel, then the reduction of its CTA partials
+// r6_ppo_grad / r6_ppo_grad_sde / r6_ppo_grad_sde_sep (kSde: sde_log_std != NULL; the layout follows the mlp): the
+// gradient kernel, then the reduction of its CTA partials
 template <bool kSde>
 int ppo_grad_launch(const R6Mlp *mlp, const float *sde_log_std, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
                     const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream)
 {
-    const bool sep = !kSde && mlp_separate(*mlp);
-    const int kP = kSde ? kPpoParamsSde : (sep ? kPpoParamsSep : kPpoParams);
+    const bool sep = mlp_separate(*mlp);
+    const int kP = kSde ? (sep ? kPpoParamsSepSde : kPpoParamsSde) : (sep ? kPpoParamsSep : kPpoParams);
     constexpr int kNT = kSde ? R6_PPO_NTERMS_SDE : R6_PPO_NTERMS;
     if (!rollout || !rollout->obs || !rollout->actions || !rollout->log_probs || !rollout->advantages || !rollout->returns)
         return fail(R6_EINVAL, "null rollout buffer%s");
@@ -2332,6 +2791,18 @@ int ppo_grad_launch(const R6Mlp *mlp, const float *sde_log_std, const R6PpoRollo
     const float clip = (float)coef->clip_range, vf = (float)coef->vf_coef, ent = (float)coef->ent_coef;
     const float vfc = (float)coef->clip_range_vf;
     if constexpr (kSde) {
+        if (sep) {
+            if (vclip)
+                ppo_grad_sep_sde_kernel<true><<<G, kThreads, kSmemPpoSepSde, s>>>(*mlp, sde_log_std, *rollout, idx, B, clip, vf, ent,
+                                                                                 vfc, coef->adv_stats, pt, pp);
+            else
+                ppo_grad_sep_sde_kernel<false><<<G, kThreads, kSmemPpoSepSde, s>>>(*mlp, sde_log_std, *rollout, idx, B, clip, vf,
+                                                                                  ent, vfc, coef->adv_stats, pt, pp);
+            rc = check_launch("r6_ppo_grad_sde_sep");
+            if (rc) return rc;
+            ppo_reduce_sep_sde_kernel<<<(kP + 255) / 256, 256, 0, s>>>(pt, pp, G, grad_sum, terms);
+            return check_launch("r6_ppo_grad_sde_sep (reduce)");
+        }
         if (vclip)
             ppo_grad_sde_kernel<true><<<G, kThreads, kSmemPpoSde, s>>>(*mlp, sde_log_std, *rollout, idx, B, clip, vf, ent, vfc,
                                                                       coef->adv_stats, pt, pp);
@@ -2378,15 +2849,29 @@ int r6_ppo_grad(const R6Mlp *mlp, const R6PpoRollout *rollout, const int64_t *id
 
 int64_t r6_ppo_sde_work_bytes(int64_t B)
 {
-    return B > 0 ? ppo_ctas(B) * (int64_t)(R6_PPO_NTERMS_SDE * sizeof(double) + kPpoParamsSde * sizeof(float)) : 0;
+    // both gSDE layouts (shared trunk and separate towers): sized for the larger
+    static_assert(kPpoParamsSepSde >= kPpoParamsSde, "gSDE work buffer");
+    return B > 0 ? ppo_ctas(B) * (int64_t)(R6_PPO_NTERMS_SDE * sizeof(double) + kPpoParamsSepSde * sizeof(float)) : 0;
 }
 
 int r6_ppo_grad_sde(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
                     const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream)
 {
     if (int rc = check_mlp(mlp)) return rc;
-    if (int rc = reject_separate(mlp, "r6_ppo_grad_sde (gSDE)")) return rc;
+    if (int rc = reject_separate(mlp, "r6_ppo_grad_sde (gSDE; r6_ppo_grad_sde_sep trains the separate towers)")) return rc;
     if (!mlp->wv || !mlp->bv || !sde || !sde->log_std) return fail(R6_EINVAL, "r6_ppo_grad_sde needs the critic head and log_std%s");
+    return ppo_grad_launch<true>(mlp, sde->log_std, rollout, idx, B, coef, grad_sum, terms, work, stream);
+}
+
+int r6_ppo_grad_sde_sep(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
+                        const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream)
+{
+    if (int rc = check_mlp(mlp)) return rc;
+    if (!mlp_separate(*mlp))
+        return fail(R6_EINVAL, "r6_ppo_grad_sde_sep needs the separate towers (R6Mlp.vf_w0 set): the shared trunk's gSDE "
+                               "gradient is r6_ppo_grad_sde%s");
+    if (!mlp->wv || !mlp->bv || !sde || !sde->log_std)
+        return fail(R6_EINVAL, "r6_ppo_grad_sde_sep needs the critic head and log_std%s");
     return ppo_grad_launch<true>(mlp, sde->log_std, rollout, idx, B, coef, grad_sum, terms, work, stream);
 }
 

@@ -47,6 +47,8 @@
 //     layer 2 : as above, W2 row 3 zero (the value is not an MMA output)
 // Per tile that is one more epilogue (four: H0v, value, H0p, H1p) and the same four MMA commits; the value never
 // needs a TF32 split.  Extra shared memory: vf_b1, wv and per group the second half's value sums (kOffSep..).
+// With gSDE (policy_tc5_sep_sde_kernel) the H1p epilogue is epilogue_in_tmem_sde, which forms h E and h^2 sigma^2 over the
+// policy latent; sigma, sigma^2 and the second half's sums follow the separate-tower region (kOffSepSde.., ~100 KB in all).
 //
 // Shared-memory operand layout of the weights (K-major, SWIZZLE_NONE "interleaved" canonical layout): element (row r,
 // k) of a tile with K_tot columns lives at byte (r % 8) * 16 + (r / 8) * SBO + (k / 4) * 128 + (k % 4) * 4,
@@ -77,6 +79,9 @@ constexpr int kSmemBytesSde = kOffSdePart + 2 * kTile * 6 * 4;
 // separate-tower kernels only: vf_b1 [64] (pre-scaled like b1), wv [64], per group the second half's value sums [128]
 constexpr int kOffSep = kSmemBytes, kOffSepWv = kOffSep + 64 * 4, kOffSepPart = kOffSepWv + 64 * 4;
 constexpr int kSmemBytesSep = kOffSepPart + 2 * kTile * 4;
+// separate towers with gSDE (policy_tc5_sep_sde_kernel): the separate-tower region, then the gSDE region after it
+constexpr int kOffSepSde = kSmemBytesSep, kOffSepSdePart = kOffSepSde + 2 * 192 * 4;
+constexpr int kSmemBytesSepSde = kOffSepSdePart + 2 * kTile * 6 * 4;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ int tile_off(int r, int k, int ktot) { return (r & 7) * 16 + (r >> 3) * (ktot * 32) + (k >> 2) * 128 + (k & 3) * 4; }

@@ -43,6 +43,9 @@ static_assert(kSepOffVw0 == kMlpH1 * kMlpIn && kSepOffB0 == kSepOffVw0 + kMlpH1 
               kSepOffLogStd == kSepOffBv + 1, "flat layout (separate towers)");
 // the stacked layer 0 is the shared layout's [128][13] + [128]; w1 and vf_w1 keep the 16-byte alignment of tensor_cores 2 / 3
 static_assert(kSepOffB0 == kPpoOffB0 && kSepOffW1 == kPpoOffW1 && kSepOffW1 % 4 == 0 && kSepOffVw1 % 4 == 0, "flat layout (separate towers)");
+// the separate towers with gSDE (R6_PPO_NPARAMS_SEP_SDE): the same prefix through bv, then log_std [64][3] (SB3 order)
+constexpr int kPpoParamsSepSde = kSepOffLogStd + kSdeXi;
+static_assert(kPpoParamsSepSde == R6_PPO_NPARAMS_SEP_SDE && kSepOffLogStd % 4 == 0, "flat layout (separate towers, gSDE)");
 
 // per-sample gradient w.r.t. the network outputs: g[0..2] = d/d mean, g[3] = d/d value, g[4..6] = d/d log_std
 struct PpoHead {

@@ -13,8 +13,9 @@ The network is SB3's default `MlpPolicy` of SB3 1.6: a shared tanh trunk 13 -> 1
 state-dependent exploration (gSDE: log_std [64, 3], noise h (exp(log_std) * xi) held between `reset_noise` draws;
 params from `ActorCriticParams.sb3_init(use_sde=True)`), or SB3 1.6's default without policy_kwargs: separate tanh
 towers 13 -> 64 -> 64 for the policy and the value (`ActorCriticParams.sb3_init(net_arch=[dict(pi=[64, 64],
-vf=[64, 64])])`, no gSDE).  SB3's value clipping (`PPOConfig(clip_range_vf=...)`) and clip-range schedules are
-supported on every network.
+vf=[64, 64])])`), with or without gSDE (with it, h is the policy tower's latent: `sb3_init(use_sde=True,
+net_arch=...)`, layout LAYOUT_SEP_SDE).  SB3's value clipping (`PPOConfig(clip_range_vf=...)`) and clip-range schedules
+are supported on every network.
 """
 from __future__ import annotations
 
@@ -41,24 +42,28 @@ LAYOUT_SEP = (("w0", (64, 13)), ("vf_w0", (64, 13)), ("b0", (64,)), ("vf_b0", (6
               ("vf_w1", (64, 64)), ("vf_b1", (64,)), ("w2", (3, 64)), ("b2", (3,)), ("wv", (64,)), ("bv", (1,)),
               ("log_std", (3,)))
 NPARAMS_SEP = _lib.PPO_NPARAMS_SEP
+# the separate towers with gSDE (R6_PPO_NPARAMS_SEP_SDE): LAYOUT_SEP through bv, then log_std [64, 3]
+LAYOUT_SEP_SDE = LAYOUT_SEP[:-1] + (("log_std", (64, 3)),)
+NPARAMS_SEP_SDE = _lib.PPO_NPARAMS_SEP_SDE
 NET_ARCH_SEP = [dict(pi=[64, 64], vf=[64, 64])]
 _LOG_SQRT_2PI = 0.5 * math.log(2.0 * math.pi)
 
 
 class ActorCriticParams:
     """The actor-critic as one flat float32 CUDA tensor `flat` with views w0 ... log_std into it: [R6_PPO_NPARAMS]
-    with log_std [3], [R6_PPO_NPARAMS_SDE] with the gSDE log_std [64, 3] (`use_sde`), or [R6_PPO_NPARAMS_SEP] for SB3
-    1.6's separate policy / value towers (`separate`, LAYOUT_SEP)."""
+    with log_std [3], [R6_PPO_NPARAMS_SDE] with the gSDE log_std [64, 3] (`use_sde`), [R6_PPO_NPARAMS_SEP] for SB3
+    1.6's separate policy / value towers (`separate`, LAYOUT_SEP), or [R6_PPO_NPARAMS_SEP_SDE] for the separate towers
+    with gSDE (both `separate` and `use_sde`, LAYOUT_SEP_SDE)."""
 
     def __init__(self, flat: torch.Tensor):
-        if (flat.dtype != torch.float32 or not flat.is_cuda or flat.shape not in ((NPARAMS,), (NPARAMS_SDE,), (NPARAMS_SEP,))
-                or not flat.is_contiguous()):
+        if (flat.dtype != torch.float32 or not flat.is_cuda
+                or flat.shape not in ((NPARAMS,), (NPARAMS_SDE,), (NPARAMS_SEP,), (NPARAMS_SEP_SDE,)) or not flat.is_contiguous()):
             raise ValueError(f"flat parameters must be a contiguous float32 CUDA tensor of {NPARAMS}, {NPARAMS_SDE} "
-                             f"(gSDE) or {NPARAMS_SEP} (separate towers) elements")
+                             f"(gSDE), {NPARAMS_SEP} (separate towers) or {NPARAMS_SEP_SDE} (separate towers, gSDE) elements")
         self.flat = flat
-        self.use_sde = flat.numel() == NPARAMS_SDE
-        self.separate = flat.numel() == NPARAMS_SEP
-        self.layout = LAYOUT_SDE if self.use_sde else (LAYOUT_SEP if self.separate else LAYOUT)
+        self.use_sde = flat.numel() in (NPARAMS_SDE, NPARAMS_SEP_SDE)
+        self.separate = flat.numel() in (NPARAMS_SEP, NPARAMS_SEP_SDE)
+        self.layout = _layout(self.separate, self.use_sde)
         o = 0
         for name, shape in self.layout:
             size = int(np.prod(shape))
@@ -75,12 +80,11 @@ class ActorCriticParams:
         net_arch: [128, 64] (the default: the shared trunk of the reference's policy_kwargs) or
         [dict(pi=[64, 64], vf=[64, 64])] (SB3 1.6's default without policy_kwargs: separate towers, both at gain
         sqrt(2)).  The matrices are drawn in the order w0, w1 (shared trunk or policy tower), then vf_w0, vf_w1 (value
-        tower), then action_net, value_net.  No other architecture has kernels: anything else raises ValueError."""
+        tower), then action_net, value_net; use_sde changes none of them (log_std [64, 3] is zero).  No other architecture
+        has kernels: anything else raises ValueError."""
         sep = cls._separate_arch(net_arch)
-        if sep and use_sde:
-            raise ValueError("gSDE is not implemented for the separate policy / value towers")
         w = cls.sb3_init_weights(seed, net_arch)
-        return cls._from(w, device, LAYOUT_SEP if sep else (LAYOUT_SDE if use_sde else LAYOUT))
+        return cls._from(w, device, _layout(sep, use_sde))
 
     @classmethod
     def sb3_init_weights(cls, seed: int = 0, net_arch=None) -> Dict[str, torch.Tensor]:
@@ -108,15 +112,13 @@ class ActorCriticParams:
     @classmethod
     def from_weights(cls, w: Dict[str, np.ndarray], device="cuda") -> "ActorCriticParams":
         """From `policy.load_sb3_zip` / `policy.load_npz` output (the critic head and log_std must be present); a
-        [64, 3] log_std gives the gSDE layout, a value tower (vf_w0 ...) the separate-tower layout."""
+        [64, 3] log_std gives a gSDE layout, a value tower (vf_w0 ...) a separate-tower layout."""
         sep = w.get("vf_w0") is not None
         missing = [k for k, _ in (LAYOUT_SEP if sep else LAYOUT) if w.get(k) is None]
         if missing:
             raise ValueError(f"weights lack {missing}: training needs the critic head and log_std")
         sde = np.asarray(w["log_std"]).size == 64 * 3
-        if sep and sde:
-            raise ValueError("gSDE is not implemented for the separate policy / value towers")
-        return cls._from(w, device, LAYOUT_SEP if sep else (LAYOUT_SDE if sde else LAYOUT))
+        return cls._from(w, device, _layout(sep, sde))
 
     @classmethod
     def _from(cls, w, device, layout) -> "ActorCriticParams":
@@ -136,6 +138,10 @@ class ActorCriticParams:
     def save_npz(self, path: str):
         """Writes `mlp_w0` ... `mlp_log_std`: what `policy.load_npz` and the Monte-Carlo CLI read."""
         np.savez(path, **{"mlp_" + k: v.detach().cpu().numpy() for k, v in self.mlp().items()})
+
+
+def _layout(separate: bool, use_sde: bool):
+    return (LAYOUT_SEP_SDE if use_sde else LAYOUT_SEP) if separate else (LAYOUT_SDE if use_sde else LAYOUT)
 
 
 def _progress_lr(lr, progress_remaining: float) -> float:
@@ -202,8 +208,8 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     returns [T, N]).  Indices outside [0, T N) are skipped and counted in terms[4] (checking them here would
     synchronise).  The minibatch's advantage mean and 1 / (std + 1e-8) are computed on the device (no synchronise).
     Returns (grad_sum float32 [params.flat.numel()]: R6_PPO_NPARAMS, or R6_PPO_NPARAMS_SEP for the separate towers,
-    terms float64 [5]); for gSDE params (r6_ppo_grad_sde) grad_sum
-    [R6_PPO_NPARAMS_SDE] and terms [6], the last the sum of the per-sample entropies.
+    terms float64 [5]); for gSDE params (r6_ppo_grad_sde, or r6_ppo_grad_sde_sep for the separate towers) grad_sum
+    [R6_PPO_NPARAMS_SDE] (R6_PPO_NPARAMS_SEP_SDE) and terms [6], the last the sum of the per-sample entropies.
 
     clip_range_vf (SB3's, > 0; None = off) clips each sample's value prediction to old_values +- clip_range_vf, where
     old_values is `rollout["values"]` (float32 [T, N] contiguous, the critic at collection); terms[1] is then the sum
@@ -260,9 +266,9 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     with torch.cuda.device(dev):
         if params.use_sde:
             sde = _lib.R6Sde(params.log_std.data_ptr(), None)
-            _lib.check(L.r6_ppo_grad_sde(C.byref(m), C.byref(sde), C.byref(ro), idx.data_ptr(), B, C.byref(coef),
-                                         grad_sum.data_ptr(), terms.data_ptr(), work.data_ptr(),
-                                         torch.cuda.current_stream(dev).cuda_stream), L)
+            fn = L.r6_ppo_grad_sde_sep if params.separate else L.r6_ppo_grad_sde
+            _lib.check(fn(C.byref(m), C.byref(sde), C.byref(ro), idx.data_ptr(), B, C.byref(coef), grad_sum.data_ptr(),
+                          terms.data_ptr(), work.data_ptr(), torch.cuda.current_stream(dev).cuda_stream), L)
         else:
             _lib.check(L.r6_ppo_grad(C.byref(m), C.byref(ro), idx.data_ptr(), B, C.byref(coef), grad_sum.data_ptr(),
                                      terms.data_ptr(), work.data_ptr(), torch.cuda.current_stream(dev).cuda_stream), L)
@@ -295,8 +301,6 @@ class PPOTrainer:
 
     def __init__(self, batch, params: ActorCriticParams, cfg: Optional[PPOConfig] = None, seed: int = 0):
         self.batch, self.params, self.cfg = batch, params, cfg or PPOConfig()
-        if params.separate and self.cfg.use_sde:
-            raise ValueError("gSDE (use_sde=True) is not implemented for the separate policy / value towers")
         if params.separate and int(self.cfg.tensor_cores) == 1:
             raise ValueError("the separate policy / value towers have no mma.sync policy kernel (tensor_cores=1)")
         if params.use_sde != self.cfg.use_sde:
