@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 22
+#define R6_ABI_VERSION 23
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -488,6 +488,21 @@ int r6_ppo_grad_sde(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *roll
 #define R6_PPO_NPARAMS_SEP_SDE 10564
 int r6_ppo_grad_sde_sep(const R6Mlp *mlp, const R6Sde *sde, const R6PpoRollout *rollout, const int64_t *idx, int64_t B,
                         const R6PpoCoef *coef, float *grad_sum, double *terms, void *work, void *stream);
+
+/*
+ * Data-parallel training: the rank-ordered sum of the W ranks' r6_ppo_grad* outputs, gathered by any transport.
+ * grads [world][P] float32 and terms [world][nterms] float64 (DEVICE, rows in rank order, row g of grads at element g * P:
+ * rows need not be 16-byte aligned).  For every entry j, in this order and in float64 without FMA:
+ *     acc = 0;  for g = 0, 1, ..., world - 1:  acc += (double)grads[g * P + j];   grad_out[j] = (float)acc
+ * (one rounding to float32), and the same rank-order float64 sum of terms into terms_out [nterms] (no rounding to
+ * float32).  The order is the contract: every rank that sums the same rows gets the same bits, whatever gathered them
+ * and on whichever GPU it runs.  The outputs must not overlap the inputs.  Returns R6_EINVAL, before any CUDA call and
+ * writing nothing, for world < 1, P < 1, nterms < 0, world * P beyond int64, a NULL pointer (terms and terms_out may
+ * be NULL only with nterms = 0), and a base pointer not aligned to its element (4 bytes for grads / grad_out, 8 for
+ * terms / terms_out).
+ */
+int r6_rank_sum(const float *grads, const double *terms, int world, int64_t P, int nterms, float *grad_out,
+                double *terms_out, void *stream);
 
 /*
  * One torch.optim.Adam step (no weight decay, no amsgrad) on the flat parameters, after clip_grad_norm_:

@@ -11,6 +11,7 @@
 //   policy_kernel, policy_tc5_kernel   the policy MLP alone: float32 FMAs, mma.sync 3xTF32 tiles, or tcgen05.mma with
 //                                    accumulators and activations in TMEM (r6_mlp_tc.cuh, r6_mlp_tcgen05.cuh)
 //   ppo_grad_kernel | ppo_reduce_kernel, adam_kernel   the PPO update: minibatch loss gradient, Adam step
+//   rank_sum_kernel                  data-parallel PPO: the rank-ordered float64 sum of the ranks' gathered gradients
 //   (policy_sep_kernel, policy_tc5_sep_kernel, ppo_grad_sep_kernel: the same for SB3 1.6's separate policy / value towers)
 //   trunc_record_kernel, trunc_bootstrap_kernel   time-limit truncations filed per step, bootstrapped with the critic
 //   reset_kernel, sim_raw_kernel, tgo_kernel, gae_kernel, peak_fma_kernel
@@ -2263,6 +2264,29 @@ adam_kernel(float *__restrict__ p, const float *__restrict__ gs, float *__restri
     }
 }
 
+// r6_rank_sum: one thread per entry j of grad_out (and of terms_out), the W rows read at j: a warp's loads of one row
+// are 32 consecutive floats, whatever the row's alignment.  The float64 accumulation runs in rank order with explicit
+// round-to-nearest adds (no contraction), so the bits are the header's rank-order sum.
+constexpr int kRankSumThreads = 256;
+__global__ void __launch_bounds__(kRankSumThreads)
+rank_sum_kernel(const float *__restrict__ grads, const double *__restrict__ terms, int world, int64_t P, int nterms,
+                float *__restrict__ grad_out, double *__restrict__ terms_out)
+{
+    const int64_t stride = (int64_t)gridDim.x * kRankSumThreads;
+    for (int64_t j = (int64_t)blockIdx.x * kRankSumThreads + threadIdx.x; j < P; j += stride) {
+        double acc = 0.0;
+#pragma unroll 8
+        for (int g = 0; g < world; g++) acc = __dadd_rn(acc, (double)grads[(int64_t)g * P + j]);
+        grad_out[j] = (float)acc;
+    }
+    if (blockIdx.x == 0)
+        for (int j = threadIdx.x; j < nterms; j += kRankSumThreads) {
+            double acc = 0.0;
+            for (int g = 0; g < world; g++) acc = __dadd_rn(acc, terms[(int64_t)g * nterms + j]);
+            terms_out[j] = acc;
+        }
+}
+
 // FMA-pipe micro-benchmark: 8 independent chains per thread
 template <typename T>
 __global__ void __launch_bounds__(256) peak_fma_kernel(int iters, double *sink)
@@ -2888,6 +2912,23 @@ int r6_adam_step(float *params, const float *grad_sum, float *m, float *v, int64
     adam_coefs(*coef, step, a.c);
     adam_kernel<<<1, kAdamThreads, 0, (cudaStream_t)stream>>>(params, grad_sum, m, v, (int)P, a, grad_norm_out);
     return check_launch("r6_adam_step");
+}
+
+int r6_rank_sum(const float *grads, const double *terms, int world, int64_t P, int nterms, float *grad_out,
+                double *terms_out, void *stream)
+{
+    if (world < 1 || P < 1 || nterms < 0) return fail(R6_EINVAL, "need world >= 1, P >= 1 and nterms >= 0%s");
+    if (P > INT64_MAX / world) return fail(R6_EINVAL, "world * P overflows int64%s");
+    if (!grads || !grad_out || (nterms > 0 && (!terms || !terms_out))) return fail(R6_EINVAL, "null pointer%s");
+    if ((reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(grad_out)) & 3u)
+        return fail(R6_EINVAL, "grads / grad_out must be 4-byte aligned%s");
+    if ((reinterpret_cast<uintptr_t>(terms) | reinterpret_cast<uintptr_t>(terms_out)) & 7u)
+        return fail(R6_EINVAL, "terms / terms_out must be 8-byte aligned%s");
+    const int64_t need = (P > nterms ? P : (int64_t)nterms);
+    const int64_t blocks = (need + kRankSumThreads - 1) / kRankSumThreads;
+    rank_sum_kernel<<<(unsigned)(blocks < 4096 ? blocks : 4096), kRankSumThreads, 0, (cudaStream_t)stream>>>(
+        grads, terms, world, P, nterms, grad_out, terms_out);
+    return check_launch("r6_rank_sum");
 }
 
 int r6_stats_reset(double *stats, void *stream)

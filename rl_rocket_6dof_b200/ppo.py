@@ -16,6 +16,20 @@ towers 13 -> 64 -> 64 for the policy and the value (`ActorCriticParams.sb3_init(
 vf=[64, 64])])`), with or without gSDE (with it, h is the policy tower's latent: `sb3_init(use_sde=True,
 net_arch=...)`, layout LAYOUT_SEP_SDE).  SB3's value clipping (`PPOConfig(clip_range_vf=...)`) and clip-range schedules
 are supported on every network.
+
+Data-parallel training (`PPOTrainer(..., group=process_group)`, one process per GPU under torchrun): rank r of W holds
+the env shard [r n, (r + 1) n) of W n envs (`sharding.shard_batch_kwargs`), collects it as a single GPU would (every
+Philox stream is keyed by global env id, so the W rollouts side by side are the W n-env rollout), and draws its own
+permutation; a global minibatch of `batch_size` samples is batch_size / W consecutive entries of every rank's
+permutation (a stratified draw, not SB3's one permutation of the whole rollout).  Per minibatch the ranks exchange two
+things with `all_gather` (bytes only, no arithmetic in the transport): the float64 (count, mean, M2) of their advantages,
+combined in rank order into the global minibatch's mean and unbiased std, and their gradient sums and loss terms, which
+`r6_rank_sum` adds in float64 in rank order.  Every rank then takes the same Adam step on bit-identical inputs, so the
+replicas stay bit-identical without a parameter broadcast after construction:
+
+    dist.init_process_group("nccl", device_id=dev)                 # torchrun --nproc-per-node W
+    batch = Rocket6DOFBatch(n, device=dev, **sharding.shard_batch_kwargs(n, rank, W))
+    trainer = PPOTrainer(batch, ActorCriticParams.sb3_init(seed=0, device=dev), PPOConfig(), seed=0, group=dist.group.WORLD)
 """
 from __future__ import annotations
 
@@ -201,7 +215,8 @@ def _check_cuda(name, t, dtype, dev):
 def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *, clip_range: float = 0.2,
                   vf_coef: float = 0.5, ent_coef: float = 0.0, normalize_advantage: bool = True,
                   grad_sum: Optional[torch.Tensor] = None, terms: Optional[torch.Tensor] = None,
-                  work: Optional[torch.Tensor] = None, clip_range_vf: Optional[float] = None):
+                  work: Optional[torch.Tensor] = None, clip_range_vf: Optional[float] = None,
+                  adv_stats: Optional[torch.Tensor] = None):
     """SUM over the minibatch `idx` (int64 sample indices t * N + i into the [T, N] rollout) of the per-sample PPO loss
     gradient, and the float64 term sums (policy-gradient loss, (R - V)^2, clipped count, approx-kl, bad indices).
     `rollout` is `collect_rollout`'s dict (obs [T, N, 13] with any strides, actions [T, N, 3], log_probs, advantages,
@@ -213,7 +228,10 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
 
     clip_range_vf (SB3's, > 0; None = off) clips each sample's value prediction to old_values +- clip_range_vf, where
     old_values is `rollout["values"]` (float32 [T, N] contiguous, the critic at collection); terms[1] is then the sum
-    of the clipped (R - V_pred)^2."""
+    of the clipped (R - V_pred)^2.
+
+    adv_stats (float64 [2] on the device: mean, 1 / (std + 1e-8)) replaces the minibatch's own advantage statistics
+    when normalize_advantage is set: a data-parallel rank passes those of the global minibatch its `idx` is part of."""
     dev = params.flat.device
     P, NT = params.flat.numel(), (_lib.PPO_NTERMS_SDE if params.use_sde else _lib.PPO_NTERMS)
     obs, act = rollout["obs"], rollout["actions"]
@@ -252,7 +270,12 @@ def loss_and_grad(params: ActorCriticParams, rollout: dict, idx: torch.Tensor, *
     if work is None or work.numel() < need:
         work = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
     stats = None
-    if normalize_advantage and B > 1:
+    if adv_stats is not None:
+        _check_cuda("adv_stats", adv_stats, torch.float64, dev)
+        if adv_stats.shape != (2,) or not adv_stats.is_contiguous():
+            raise ValueError("adv_stats must be a contiguous float64 [2] tensor (mean, 1 / (std + 1e-8))")
+        stats = adv_stats if normalize_advantage else None
+    elif normalize_advantage and B > 1:
         # clamped: an index outside the rollout must not reach torch's gather (a device-side assert); the kernel skips
         # and counts such indices (terms[4]), and a caller that sees a non-zero count discards the result
         a = adv.reshape(-1)[idx.clamp(0, max(T * n - 1, 0))].double()
@@ -296,31 +319,232 @@ def adam_step(params: torch.Tensor, grad_sum: torch.Tensor, m: torch.Tensor, v: 
                                   torch.cuda.current_stream(dev).cuda_stream), L)
 
 
-class PPOTrainer:
-    """SB3 1.6 `PPO.learn` over a `Rocket6DOFBatch`: collection by `collect_rollout`, update by `train`."""
+def rank_sum(grads: torch.Tensor, terms: torch.Tensor, grad_out: Optional[torch.Tensor] = None,
+             terms_out: Optional[torch.Tensor] = None):
+    """`r6_rank_sum`: grad_out [P] = fl32(sum over rows g = 0, 1, ... of grads [W, P] float32, accumulated in float64
+    in that order) and terms_out [NT] = the same rank-order float64 sum of terms [W, NT].  The order is fixed, so the
+    result does not depend on the transport that gathered the rows or on the device.  Returns (grad_out, terms_out)."""
+    dev = grads.device
+    _check_cuda("grads", grads, torch.float32, dev)
+    _check_cuda("terms", terms, torch.float64, dev)
+    if grads.dim() != 2 or terms.dim() != 2 or not grads.is_contiguous() or not terms.is_contiguous():
+        raise ValueError("grads [W, P] and terms [W, NT] must be contiguous 2-D tensors")
+    W, P = grads.shape
+    NT = terms.shape[1]
+    if terms.shape[0] != W or W < 1 or P < 1:
+        raise ValueError("grads and terms must have the same W >= 1 rows, and P >= 1")
+    if grad_out is None:
+        grad_out = torch.empty(P, dtype=torch.float32, device=dev)
+    if terms_out is None:
+        terms_out = torch.empty(NT, dtype=torch.float64, device=dev)
+    for name, t, dt, size in (("grad_out", grad_out, torch.float32, P), ("terms_out", terms_out, torch.float64, NT)):
+        _check_cuda(name, t, dt, dev)
+        if t.dim() != 1 or not t.is_contiguous() or t.numel() != size:
+            raise ValueError(f"{name} must be contiguous 1-D with {size} elements")
+    L = _lib.load()
+    with torch.cuda.device(dev):
+        _lib.check(L.r6_rank_sum(grads.data_ptr(), terms.data_ptr(), W, P, NT, grad_out.data_ptr(),
+                                 terms_out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream), L)
+    return grad_out, terms_out
 
-    def __init__(self, batch, params: ActorCriticParams, cfg: Optional[PPOConfig] = None, seed: int = 0):
+
+def local_moments(x: torch.Tensor) -> torch.Tensor:
+    """(count, mean, M2) [3] float64 of the float64 tensor x, M2 the sum of squared deviations from the mean, on x's
+    device (no host read)."""
+    mean = x.mean()
+    return torch.stack([torch.full((), float(x.numel()), dtype=torch.float64, device=x.device), mean,
+                        ((x - mean) ** 2).sum()])
+
+
+def combine_moments(rows: torch.Tensor) -> torch.Tensor:
+    """(count, mean, M2) [3] of the union of the sets whose float64 (count, mean, M2) are rows [W, 3], combined by
+    Chan, Golub and LeVeque's pairwise formula in row (rank) order:
+        n = n_a + n_b,  d = mean_b - mean_a,  mean = mean_a + d n_b / n,  M2 = M2_a + M2_b + d^2 n_a n_b / n.
+    Every rank that holds the same rows gets the same bits.  The unbiased variance is M2 / (n - 1)."""
+    n, mean, m2 = rows[0, 0], rows[0, 1], rows[0, 2]
+    for r in range(1, rows.shape[0]):
+        nb, mb, m2b = rows[r, 0], rows[r, 1], rows[r, 2]
+        tot = n + nb
+        d = mb - mean
+        mean = mean + d * (nb / tot)
+        m2 = m2 + m2b + d * d * (n * nb / tot)
+        n = tot
+    return torch.stack([n, mean, m2])
+
+
+def minibatch_slices(total_local: int, batch_size: int, world: int):
+    """[(start, stop)] into each rank's permutation of its total_local samples: a global minibatch of batch_size
+    (a multiple of world) takes batch_size / world consecutive entries of every rank's permutation.  As in SB3 the last
+    minibatch of an epoch may be short, and it is equally short on every rank."""
+    if world < 1 or batch_size < 1 or batch_size % world:
+        raise ValueError(f"batch_size {batch_size} must be a positive multiple of the world size {world}")
+    b = batch_size // world
+    return [(s, min(s + b, total_local)) for s in range(0, total_local, b)]
+
+
+# PPOTrainer's construction-time consistency row: what must agree across the ranks of a data-parallel group
+_DP_FIELDS = ("num_envs", "env_offset", "num_envs_global", "nparams", "use_sde", "separate", "env_seed_hi",
+              "env_seed_lo", "local_error", "learning_rate", "n_steps", "batch_size", "n_epochs", "gamma", "gae_lambda",
+              "clip_range", "normalize_advantage", "ent_coef", "vf_coef", "max_grad_norm", "target_kl",
+              "tensor_cores", "cfg_use_sde", "sde_sample_freq", "clip_range_vf")
+_DP_PER_RANK = ("env_offset", "local_error")        # checked against the rank's index, not against rank 0
+_LOCAL_ERRORS = {1: "the separate policy / value towers have no mma.sync policy kernel (tensor_cores=1)",
+                 2: "PPOConfig(use_sde=...) does not match the params' layout (ActorCriticParams.sb3_init(use_sde=...))"}
+
+
+def _scalar(x) -> float:
+    """A config value as a float64 that compares across ranks: None -> +inf, a schedule (callable) -> -inf (schedules
+    cannot be compared; each rank must pass the same one)."""
+    return math.inf if x is None else (-math.inf if callable(x) else float(x))
+
+
+def _group_errors(rows: np.ndarray, world: int) -> list:
+    """What is inconsistent in the gathered _DP_FIELDS rows [W, F]: a function of the rows only, so every rank finds the
+    same list."""
+    col = {k: rows[:, i] for i, k in enumerate(_DP_FIELDS)}
+    n = int(col["num_envs"][0])
+    errors = [f"rank {r}: {_LOCAL_ERRORS.get(int(e), 'local check failed')}"
+              for r, e in enumerate(col["local_error"]) if e != 0]
+    errors += [f"{k} differs across ranks ({col[k].tolist()})" for k in _DP_FIELDS
+               if k not in _DP_PER_RANK and not np.all(col[k] == col[k][0])]
+    errors += [f"rank {r} has env_offset {int(o)}, its shard starts at {r * n}"
+               for r, o in enumerate(col["env_offset"]) if o != r * n]
+    if col["num_envs_global"][0] != world * n:
+        errors.append(f"num_envs_global {int(col['num_envs_global'][0])} is not world {world} x num_envs {n}")
+    bs = col["batch_size"][0]
+    if math.isfinite(bs) and int(bs) % world:
+        errors.append(f"batch_size {int(bs)} (the global minibatch) is not a multiple of the world size {world}")
+    return errors
+
+
+class PPOTrainer:
+    """SB3 1.6 `PPO.learn` over a `Rocket6DOFBatch`: collection by `collect_rollout`, update by `train`.
+
+    group (a `torch.distributed` process group, default None) trains data-parallel, one env shard per rank: rank r of
+    W holds a batch with num_envs = n, env_offset = r n and num_envs_global = W n (`sharding.shard_batch_kwargs`).
+      - Construction: one all_gather of every rank's shard, parameter count, layout, env seed and PPOConfig scalars;
+        anything inconsistent makes every rank raise the same ValueError (no rank is left in a later collective).  The
+        parameters are then broadcast from the group's first rank; Adam's m and v start at zero everywhere.
+      - Collection is each rank's own collect_rollout; because every stream is keyed by global env id, the W rollouts
+        side by side along N are the rollout one GPU collects for W n envs.
+      - Minibatches: cfg.batch_size is the global minibatch size, a multiple of W (default W ceil(n_steps n / 4)).
+        Each rank permutes its own n_steps n samples with a generator seeded from (seed, rank) (rank 0: `seed`, as
+        without a group) and takes batch_size / W consecutive entries per minibatch (`minibatch_slices`): a stratified
+        draw, not SB3's single permutation of the concatenated rollout.  The last minibatch may be short, equally on
+        every rank.
+      - Advantages are normalised with the global minibatch's mean and unbiased std: each rank's float64
+        (count, mean, M2), all_gathered and combined in rank order (`combine_moments`).
+      - Gradient: each rank's r6_ppo_grad* sum over its part and its float64 terms are all_gathered into [W, P] /
+        [W, NT] and added in rank order by `r6_rank_sum`; every rank then takes the Adam step with scale 1 / B_global on
+        bit-identical inputs, so the replicas stay bit-identical.  Gathers move bytes and do no arithmetic, so the
+        result does not depend on the backend or on the GPUs.
+      - target_kl, the train/ logs, explained_variance (global variances, rank-order moments) and rollout/ (episode
+        statistics summed by r6_rank_sum) are global, hence the same on every rank; num_timesteps counts W n n_steps
+        env-steps per iteration.
+    A group of size 1 trains exactly as group=None (there is nothing to exchange); train() must be called on every rank
+    with that rank's rollout of the same shape.  With group=None the trainer issues the same launches as before."""
+
+    def __init__(self, batch, params: ActorCriticParams, cfg: Optional[PPOConfig] = None, seed: int = 0, group=None):
         self.batch, self.params, self.cfg = batch, params, cfg or PPOConfig()
+        self.group = group
+        self.world, self.rank = 1, 0
+        local_error = 0
         if params.separate and int(self.cfg.tensor_cores) == 1:
-            raise ValueError("the separate policy / value towers have no mma.sync policy kernel (tensor_cores=1)")
-        if params.use_sde != self.cfg.use_sde:
-            raise ValueError(f"PPOConfig(use_sde={self.cfg.use_sde}) needs params with the "
-                             f"{'gSDE' if self.cfg.use_sde else 'diagonal Gaussian'} layout "
-                             f"(ActorCriticParams.sb3_init(use_sde={self.cfg.use_sde}))")
+            local_error = 1
+        elif params.use_sde != self.cfg.use_sde:
+            local_error = 2
+        if group is None:
+            if local_error == 1:
+                raise ValueError(_LOCAL_ERRORS[1])
+            if local_error == 2:
+                raise ValueError(f"PPOConfig(use_sde={self.cfg.use_sde}) needs params with the "
+                                 f"{'gSDE' if self.cfg.use_sde else 'diagonal Gaussian'} layout "
+                                 f"(ActorCriticParams.sb3_init(use_sde={self.cfg.use_sde}))")
+        else:
+            self._join_group(group, local_error)
         dev = params.flat.device
         self.m = torch.zeros_like(params.flat)
         self.v = torch.zeros_like(params.flat)
         self.gen = torch.Generator(device=dev)
-        self.gen.manual_seed(int(seed))
+        # rank 0 keeps `seed`, so a one-rank group draws the permutations of group=None
+        self.gen.manual_seed((int(seed) + self.rank * 0x9E3779B97F4A7C15) % (1 << 64))
         self.n_updates = 0            # SB3's _n_updates (epochs run)
         self.adam_steps = 0
         self.num_timesteps = 0
         self.progress_remaining = 1.0
         self._grad = torch.empty(params.flat.numel(), dtype=torch.float32, device=dev)
         self._work = None
+        if self.world > 1:            # the exchange buffers: rows [W] of what each rank contributes
+            W, P = self.world, params.flat.numel()
+            NT = _lib.PPO_NTERMS_SDE if params.use_sde else _lib.PPO_NTERMS
+            f32, f64 = torch.float32, torch.float64
+            self._moments, self._moments_all = torch.empty(3, dtype=f64, device=dev), torch.empty(W, 3, dtype=f64, device=dev)
+            self._terms, self._terms_all = torch.empty(NT, dtype=f64, device=dev), torch.empty(W, NT, dtype=f64, device=dev)
+            self._grads_all = torch.empty(W, P, dtype=f32, device=dev)
+            self._adv_stats = torch.empty(2, dtype=f64, device=dev)
+            self._stats_all = torch.empty(W, 8, dtype=f64, device=dev)
+            self._one_all = torch.zeros(W, 1, dtype=f32, device=dev)    # r6_rank_sum's float32 half, unused for stats
+            self._one = torch.empty(1, dtype=f32, device=dev)
+
+    def _join_group(self, group, local_error: int):
+        """The construction-time exchange: one all_gather of every rank's _DP_FIELDS row, the same verdict on every rank
+        (ValueError), then the parameter broadcast from the group's first rank."""
+        import torch.distributed as dist
+        self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
+        b, cfg, p = self.batch, self.cfg, self.params
+        seed = int(b.seed_value) % (1 << 64)
+        vals = dict(num_envs=b.num_envs, env_offset=b.env_offset, num_envs_global=b.num_envs_global,
+                    nparams=p.flat.numel(), use_sde=p.use_sde, separate=p.separate, env_seed_hi=seed >> 32,
+                    env_seed_lo=seed & 0xFFFFFFFF, local_error=local_error, learning_rate=_scalar(cfg.learning_rate),
+                    n_steps=cfg.n_steps, batch_size=_scalar(cfg.batch_size or None), n_epochs=cfg.n_epochs,
+                    gamma=cfg.gamma, gae_lambda=cfg.gae_lambda, clip_range=_scalar(cfg.clip_range),
+                    normalize_advantage=cfg.normalize_advantage, ent_coef=cfg.ent_coef, vf_coef=cfg.vf_coef,
+                    max_grad_norm=cfg.max_grad_norm, target_kl=_scalar(cfg.target_kl), tensor_cores=cfg.tensor_cores,
+                    cfg_use_sde=cfg.use_sde, sde_sample_freq=cfg.sde_sample_freq, clip_range_vf=_scalar(cfg.clip_range_vf))
+        dev = p.flat.device
+        row = torch.tensor([float(vals[k]) for k in _DP_FIELDS], dtype=torch.float64, device=dev)
+        rows = torch.empty(self.world, len(_DP_FIELDS), dtype=torch.float64, device=dev)
+        dist.all_gather(list(rows.unbind(0)), row, group=group)
+        errors = _group_errors(rows.cpu().numpy(), self.world)
+        if errors:
+            raise ValueError("data-parallel PPOTrainer: " + "; ".join(errors))
+        dist.broadcast(p.flat, src=dist.get_global_rank(group, 0), group=group)
 
     def batch_size(self, total: int) -> int:
-        return int(self.cfg.batch_size) if self.cfg.batch_size else max(1, -(-total // 4))
+        """The global minibatch size for a rollout of `total` samples per rank (without a group, the rollout's)."""
+        return int(self.cfg.batch_size) if self.cfg.batch_size else self.world * max(1, -(-total // 4))
+
+    def _gather_moments(self, local: torch.Tensor) -> torch.Tensor:
+        """[W, ...] float64: every rank's `local` in rank order."""
+        import torch.distributed as dist
+        out = torch.empty((self.world,) + tuple(local.shape), dtype=torch.float64, device=local.device)
+        dist.all_gather(list(out.unbind(0)), local.contiguous(), group=self.group)
+        return out
+
+    def _exchange_moments(self, rollout: dict, idx: torch.Tensor) -> torch.Tensor:
+        """The first exchange of a minibatch: this rank's advantage (count, mean, M2) out, the global minibatch's
+        (mean, 1 / (std + 1e-8)) back, on the device (std unbiased, as torch's and SB3's)."""
+        import torch.distributed as dist
+        self._moments.copy_(local_moments(rollout["advantages"].reshape(-1)[idx].double()))
+        dist.all_gather(list(self._moments_all.unbind(0)), self._moments, group=self.group)
+        n, mean, m2 = combine_moments(self._moments_all).unbind(0)
+        torch.stack([mean, 1.0 / (torch.sqrt(m2 / (n - 1)) + 1e-8)], out=self._adv_stats)
+        return self._adv_stats
+
+    def _exchange_grad(self, terms_out: torch.Tensor):
+        """The second exchange: every rank's gradient sum and terms gathered, then added in rank order by r6_rank_sum
+        into self._grad and terms_out."""
+        import torch.distributed as dist
+        dist.all_gather(list(self._grads_all.unbind(0)), self._grad, group=self.group)
+        dist.all_gather(list(self._terms_all.unbind(0)), self._terms, group=self.group)
+        rank_sum(self._grads_all, self._terms_all, grad_out=self._grad, terms_out=terms_out)
+
+    def _global_stats(self) -> torch.Tensor:
+        """The group's episode statistics: every rank's 8 slots, summed in rank order by r6_rank_sum's float64 half."""
+        import torch.distributed as dist
+        self.batch.join()
+        dist.all_gather(list(self._stats_all.unbind(0)), self.batch.stats, group=self.group)
+        return rank_sum(self._one_all, self._stats_all, grad_out=self._one)[1]
 
     def train(self, rollout: dict) -> dict:
         """n_epochs passes over the rollout in minibatches of a seeded on-device permutation; returns SB3's train/ logs.
@@ -330,48 +554,59 @@ class PPOTrainer:
         the last epoch that ran, entropy_loss and loss use each minibatch's log_std before its Adam step (gSDE: the mean
         per-sample entropy of the minibatch, from the kernel's entropy term), and loss is the last minibatch's.  The
         learning rate, clip_range and clip_range_vf are their schedules at progress_remaining, evaluated once per update;
-        with clip_range_vf, value_loss is the clipped loss and train/clip_range_vf is logged."""
+        with clip_range_vf, value_loss is the clipped loss and train/clip_range_vf is logged.  With a group of W > 1
+        ranks, `rollout` is this rank's and the minibatches, statistics and logs are the global ones (class docstring)."""
         cfg, dev = self.cfg, self.params.flat.device
         T, n = rollout["advantages"].shape
         total = T * n
+        dp = self.world > 1
         bs = self.batch_size(total)
+        slices = minibatch_slices(total, bs, self.world) if dp else [(s, s + bs) for s in range(0, total, bs)]
         lr = _progress_lr(cfg.learning_rate, self.progress_remaining)
         clip = _progress_lr(cfg.clip_range, self.progress_remaining)
         vfc = None if cfg.clip_range_vf is None else _progress_lr(cfg.clip_range_vf, self.progress_remaining)
         if vfc is not None and not (vfc > 0 and math.isfinite(vfc)):
             raise ValueError(f"clip_range_vf({self.progress_remaining}) = {vfc}: the schedule must stay finite and > 0")
         vkw = {} if vfc is None else dict(clip_range_vf=vfc)
-        nmb = -(-total // bs)
+        nmb = len(slices)
         sde = self.params.use_sde
         terms = torch.zeros(cfg.n_epochs * nmb, _lib.PPO_NTERMS_SDE if sde else _lib.PPO_NTERMS, dtype=torch.float64,
                             device=dev)
         log_std_sums = torch.zeros(cfg.n_epochs * nmb, dtype=torch.float64, device=dev)
         sizes = []
         L = _lib.load()
-        need = int((L.r6_ppo_sde_work_bytes if sde else L.r6_ppo_work_bytes)(min(bs, total)))
+        need = int((L.r6_ppo_sde_work_bytes if sde else L.r6_ppo_work_bytes)(min(slices[0][1], total)))
         if self._work is None or self._work.numel() < need:
             self._work = torch.empty(need, dtype=torch.uint8, device=dev)
         done = False
         for epoch in range(cfg.n_epochs):
             perm = torch.randperm(total, generator=self.gen, device=dev)
             epoch_start = len(sizes)
-            for start in range(0, total, bs):
-                idx = perm[start:start + bs]
+            for start, stop in slices:
+                idx = perm[start:stop]
                 k = len(sizes)
-                loss_and_grad(self.params, rollout, idx, clip_range=clip, vf_coef=cfg.vf_coef,
-                              ent_coef=cfg.ent_coef, normalize_advantage=cfg.normalize_advantage, grad_sum=self._grad,
-                              terms=terms[k], work=self._work, **vkw)
+                B = idx.numel() * self.world                  # the global minibatch (every rank's part is as long)
+                if dp:
+                    stats = self._exchange_moments(rollout, idx) if cfg.normalize_advantage else None
+                    loss_and_grad(self.params, rollout, idx, clip_range=clip, vf_coef=cfg.vf_coef,
+                                  ent_coef=cfg.ent_coef, normalize_advantage=cfg.normalize_advantage,
+                                  grad_sum=self._grad, terms=self._terms, work=self._work, adv_stats=stats, **vkw)
+                    self._exchange_grad(terms[k])
+                else:
+                    loss_and_grad(self.params, rollout, idx, clip_range=clip, vf_coef=cfg.vf_coef,
+                                  ent_coef=cfg.ent_coef, normalize_advantage=cfg.normalize_advantage,
+                                  grad_sum=self._grad, terms=terms[k], work=self._work, **vkw)
                 if not sde:
                     log_std_sums[k] = self.params.log_std.sum(dtype=torch.float64)    # this minibatch's entropy (no sync)
-                sizes.append(idx.numel())
+                sizes.append(B)
                 if cfg.target_kl is not None:
-                    kl = float(terms[k, 3]) / idx.numel()      # approx-kl sum: the one host read per minibatch
+                    kl = float(terms[k, 3]) / B      # approx-kl sum (global): the one host read per minibatch
                     if kl > 1.5 * cfg.target_kl:
                         done = True
                         break
                 self.adam_steps += 1
                 adam_step(self.params.flat, self._grad, self.m, self.v, lr=lr, step=self.adam_steps,
-                          scale=1.0 / idx.numel(), max_grad_norm=cfg.max_grad_norm)
+                          scale=1.0 / B, max_grad_norm=cfg.max_grad_norm)
             if done:
                 break
         self.n_updates += cfg.n_epochs
@@ -385,8 +620,13 @@ class PPOTrainer:
             entropy = log_std_sums[:len(sizes)].cpu().numpy() + 3 * (0.5 + _LOG_SQRT_2PI)     # per minibatch
         log_std = self.params.log_std.detach().double().cpu().numpy()
         v, r = rollout["values"].reshape(-1).double(), rollout["returns"].reshape(-1).double()
-        var_r = float(r.var())
-        ev = float("nan") if var_r == 0 else 1.0 - float((r - v).var()) / var_r
+        if dp:     # global variances: 1 - var(r - v) / var(r) = 1 - M2(r - v) / M2(r)
+            m2 = self._gather_moments(torch.stack([local_moments(r), local_moments(r - v)]))
+            m2_r, m2_res = (float(combine_moments(m2[:, j])[2]) for j in (0, 1))
+            ev = float("nan") if m2_r == 0 else 1.0 - m2_res / m2_r
+        else:
+            var_r = float(r.var())
+            ev = float("nan") if var_r == 0 else 1.0 - float((r - v).var()) / var_r
         logs = {"train/policy_gradient_loss": float(means[:, 0].mean()), "train/value_loss": float(means[:, 1].mean()),
                 "train/entropy_loss": float(-entropy.mean()), "train/approx_kl": float(means[epoch_start:, 3].mean()),
                 "train/clip_fraction": float(means[:, 2].mean()),
@@ -401,7 +641,8 @@ class PPOTrainer:
         """Alternates collect_rollout (n_steps of every env) and train until total_timesteps env-steps; returns one log
         dict per iteration (train/ logs plus the env's episode statistics of that collection under rollout/).  As in
         SB3, progress_remaining is updated after the collection, so update i of a run from 0 uses
-        1 - i n_steps N / total_timesteps (the last one 0 when total_timesteps is a multiple of n_steps N)."""
+        1 - i n_steps N / total_timesteps (the last one 0 when total_timesteps is a multiple of n_steps N).  With a group,
+        N is the global env count W n and rollout/ holds the group's statistics."""
         b, cfg = self.batch, self.cfg
         if self.num_timesteps == 0:
             b.reset()
@@ -411,9 +652,10 @@ class PPOTrainer:
             ro = b.collect_rollout(cfg.n_steps, self.params.mlp(), gamma=cfg.gamma, gae_lambda=cfg.gae_lambda,
                                    tensor_cores=cfg.tensor_cores, bootstrap_truncated=True,
                                    sde_sample_freq=cfg.sde_sample_freq)
-            self.num_timesteps += cfg.n_steps * b.num_envs
+            self.num_timesteps += cfg.n_steps * b.num_envs * self.world
             self.progress_remaining = 1.0 - self.num_timesteps / total_timesteps
-            log = {"rollout/" + k: v for k, v in b.stats_dict().items()}
+            stats = self._global_stats() if self.world > 1 else None
+            log = {"rollout/" + k: v for k, v in b.stats_dict(stats).items()}
             log.update(self.train(ro))
             log["time/total_timesteps"] = self.num_timesteps
             logs.append(log)

@@ -25,6 +25,14 @@ def shard_range(n_global: int, world: int, rank: int) -> Tuple[int, int]:
     return offset, count
 
 
+def shard_batch_kwargs(n_local: int, rank: int, world: int) -> dict:
+    """`Rocket6DOFBatch` keyword arguments of rank's shard when every one of `world` ranks holds n_local envs (what the
+    data-parallel `ppo.PPOTrainer` expects): env_offset = rank n_local, num_envs_global = world n_local."""
+    if n_local < 1 or world < 1 or not (0 <= rank < world):
+        raise ValueError("bad shard request")
+    return dict(env_offset=rank * n_local, num_envs_global=world * n_local)
+
+
 def env_world() -> Tuple[int, int, int]:
     """(rank, local_rank, world_size) from the torchrun environment (1 process = 1 GPU)."""
     return (int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0")),
