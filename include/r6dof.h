@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define R6_ABI_VERSION 23
+#define R6_ABI_VERSION 24
 #define R6_MAX_LANES 32
 #define R6_NSTATE 14
 #define R6_NTERMS 7
@@ -381,6 +381,60 @@ int r6_trunc_record(const uint8_t *flags, const float *terminal_obs, int64_t n, 
                     int32_t slots, int32_t *slot_step, float *slot_obs, void *stream);
 int r6_trunc_bootstrap(float *rew, int32_t T, int64_t n, int32_t slots, const int32_t *slot_step, const float *slot_values,
                        double gamma, void *stream);
+
+/*
+ * VecNormalize: SB3 1.6's running statistics of the observations and of the discounted return (VecNormalize with
+ * RunningMeanStd(epsilon=1e-4)).  Running statistics rms are float64 [mean[dim], var[dim], count] (DEVICE); moments are
+ * float64 (count, mean, M2) per row, M2 the sum of squared deviations (the batch variance is M2 / count, ddof = 0).
+ * Every entry point returns R6_EINVAL, before any CUDA call and writing nothing, for a NULL pointer, a bad size or range,
+ * clip <= 0 (or NaN) and eps < 0 (or not finite).
+ *
+ * r6_vn_moments: out[r] = moments of x[r][first .. first + count) for rows r < rows of the component-major float32
+ * block x [rows][n], count >= 1.  Computed in float64 (SB3 reduces its float32 observation array in float32; this is a
+ * deliberate deviation).  ceil(count / 2048) CTAs of 256 threads each combine their columns' moments; the CTA results are
+ * combined in CTA order (Chan's formula, as ppo.combine_moments).  The grid and the order depend on count only: the bits do
+ * not depend on the device, the stream or the lanes.  work: r6_vn_moments_work_bytes(count, rows) DEVICE bytes.
+ */
+int64_t r6_vn_moments_work_bytes(int64_t count, int32_t rows);
+int r6_vn_moments(const float *x, int64_t n, int32_t rows, int64_t first, int64_t count, double *out, void *work,
+                  void *stream);
+
+/*
+ * r6_vn_update: `steps` successive RunningMeanStd.update_from_moments of rms [2 dim + 1] with moments [steps][dim][3]
+ * (the batch count is that of row 0), in float64 without FMA and in numpy's order:
+ *     delta = bm - mean;  tot = count + bc;  mean' = mean + (delta bc) / tot;
+ *     M2 = (var count + bv bc) + ((delta^2 count) bc) / (count + bc);  var' = M2 / (count + bc);  count' = bc + count.
+ * hist (nullable) [steps + 1][2][dim]: row 0 (mean, sqrt(var + eps)) before the first update, row s + 1 after update s
+ * (IEEE division and square root).  steps = 0 with hist writes the current statistics' row.  1 <= dim <= 1024.
+ */
+int r6_vn_update(double *rms, int32_t dim, const double *moments, int32_t steps, double eps, double *hist, void *stream);
+
+/*
+ * r6_vn_normalize: out[c][i] = fl32(clip((fl64(in[c][i]) - mean[c]) / std[c], -clip, clip)) for the 13 observation rows
+ * c < 13 and envs i in [first, first + count) of in / out (row stride n; in == out allowed; other rows untouched).
+ * (mean, std) are row hist_row of hist [hist_rows][2][13] (r6_vn_update's history), or, with step (int32 [n], nullable),
+ * row step[i] + 1 for each env: columns with step[i] < 0 or step[i] + 1 >= hist_rows are not written (a truncation slot
+ * layer of r6_trunc_record, normalized with the statistics of the step it truncated at).
+ */
+int r6_vn_normalize(const float *in, float *out, int64_t n, int64_t first, int64_t count, const double *hist,
+                    int32_t hist_row, const int32_t *step, int32_t hist_rows, double clip, void *stream);
+
+/*
+ * r6_vn_ret_moments: VecNormalize's return scan over a collected rollout, rew float32 [T][n] (the raw rewards), done
+ * uint8 [T][n].  Per env and step t: returns[i] = returns[i] gamma + fl64(rew[t][i]) (float64, no FMA); out[t] = the
+ * moments over envs of those returns, taken before returns[i] = 0 where done[t][i].  returns [n] float64 carries over
+ * rollouts.  One thread per env, ceil(n / 256) CTAs of 8 warps; per step the warps' moments are combined in warp order,
+ * as r6_vn_moments combines its CTAs'.  work: r6_vn_ret_work_bytes(T, n) DEVICE bytes.  1 <= T <= 65535, gamma finite and >= 0.
+ */
+int64_t r6_vn_ret_work_bytes(int32_t T, int64_t n);
+int r6_vn_ret_moments(const float *rew, const uint8_t *done, int32_t T, int64_t n, double *returns, double gamma,
+                      double *out, void *work, void *stream);
+
+/*
+ * r6_vn_scale_rewards: rew[t][i] = fl32(clip(fl64(rew[t][i]) / hist[t + 1][1], -clip, clip)) in place, hist [T + 1][2][1]
+ * the history r6_vn_update wrote for the T updates of ret_rms (std_t = sqrt(var_t + eps) after update t).
+ */
+int r6_vn_scale_rewards(float *rew, int32_t T, int64_t n, const double *hist, double clip, void *stream);
 
 /*
  * PPO update (stable-baselines3 1.6.0 `PPO.train`, the optimiser of main_6DOF.py:136).

@@ -12,7 +12,7 @@ from .params import R6Params
 
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libr6dof.so")
-ABI_VERSION = 23
+ABI_VERSION = 24
 
 u8p = C.c_void_p
 
@@ -93,7 +93,9 @@ EXPORTS = ["r6_abi_version", "r6_last_error", "r6_params_size", "r6_buffers_size
            "r6_rollout", "r6_sim_step_raw", "r6_tgo", "r6_stats_reset", "r6_peak_fma", "r6_gae", "r6_policy", "r6_policy_ex", "r6_step_random", "r6_step_range", "r6_policy_range", "r6_work_bytes",
            "r6_ppo_rollout_size", "r6_ppo_coef_size", "r6_adam_coef_size", "r6_ppo_work_bytes", "r6_ppo_grad", "r6_adam_step",
            "r6_trunc_record", "r6_trunc_bootstrap", "r6_sde_size", "r6_sde_noise", "r6_policy_sde_range",
-           "r6_ppo_sde_work_bytes", "r6_ppo_grad_sde", "r6_policy_sde_sep_range", "r6_ppo_grad_sde_sep", "r6_rank_sum"]
+           "r6_ppo_sde_work_bytes", "r6_ppo_grad_sde", "r6_policy_sde_sep_range", "r6_ppo_grad_sde_sep", "r6_rank_sum",
+           "r6_vn_moments_work_bytes", "r6_vn_moments", "r6_vn_update", "r6_vn_normalize", "r6_vn_ret_work_bytes",
+           "r6_vn_ret_moments", "r6_vn_scale_rewards"]
 
 
 class R6Error(RuntimeError):
@@ -172,6 +174,17 @@ def load(path: str | None = None):
                                   C.POINTER(R6PpoCoef), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.r6_ppo_grad_sde_sep.argtypes = L.r6_ppo_grad_sde.argtypes
     L.r6_rank_sum.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_vn_moments_work_bytes.argtypes = [C.c_int64, C.c_int32]
+    L.r6_vn_moments_work_bytes.restype = C.c_int64
+    L.r6_vn_moments.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.r6_vn_update.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_double, C.c_void_p, C.c_void_p]
+    L.r6_vn_normalize.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p,
+                                  C.c_int32, C.c_double, C.c_void_p]
+    L.r6_vn_ret_work_bytes.argtypes = [C.c_int32, C.c_int64]
+    L.r6_vn_ret_work_bytes.restype = C.c_int64
+    L.r6_vn_ret_moments.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_double, C.c_void_p,
+                                    C.c_void_p, C.c_void_p]
+    L.r6_vn_scale_rewards.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_double, C.c_void_p]
     L.r6_peak_fma.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
     _lib = L
     return L

@@ -379,7 +379,7 @@ class Rocket6DOFBatch:
 
     def collect_rollout(self, k: int, mlp: dict, *, gamma: float = 0.99, gae_lambda: float = 0.95,
                         stochastic: bool = True, tensor_cores=3, bootstrap_truncated: bool = False,
-                        sde_sample_freq: int = -1) -> dict:
+                        sde_sample_freq: int = -1, vec_normalize=None) -> dict:
         """What SB3's `PPO.collect_rollouts` + `RolloutBuffer.compute_returns_and_advantage` produce for k steps of
         this VecEnv, entirely on the device: per step one policy launch (action, value, log-prob; by default the
         faithful tcgen05 3xTF32 kernel, tensor_cores=3) and one env step, then the GAE scan.  Returns tensors shaped
@@ -404,13 +404,29 @@ class Rocket6DOFBatch:
         a component-major buffer [k + 1, 14, N] (the layout the kernels read and write), its reward and done flags into
         row j of `rewards` / `dones`, and the policy of step j + 1 reads that slice — no per-step copies (with auto-reset,
         the training configuration; one-episode batches keep the copies).  `obs` is therefore a strided [k, N, 13] view of
-        that buffer (`.contiguous()` gives dense rows if a consumer needs them)."""
+        that buffer (`.contiguous()` gives dense rows if a consumer needs them).
+
+        vec_normalize (a `vec_normalize.VecNormalize` of this batch) collects as SB3's PPO inside VecNormalize: after
+        every step the lanes join, one r6_vn_moments launch over the batch and r6_vn_update update obs_rms (when training
+        and norm_obs), and each lane normalizes its range of the step's observations in place before the next policy
+        launch.  obs[0] is the batch's obs normalized with the current statistics (SB3's _last_obs), truncation slots are
+        normalized with the statistics of their step before the slot values, last_values come from the normalized last
+        observations, and the reward pass (return scan, ret_rms updates, normalized rewards) runs before the bootstrap and
+        the GAE.  The batch's obs, reward_f32 and episode statistics stay raw; `obs` and `rewards` of the result are the
+        normalized ones.  Needs auto-reset (ValueError otherwise)."""
         from .gae import compute_gae
         k = int(k)
         n, dev = self.num_envs, self.device
         _check_separate(mlp, tensor_cores)
         if bootstrap_truncated and not self.auto_reset:
             raise ValueError("bootstrap_truncated needs auto_reset=True (a frozen one-episode env keeps its flags)")
+        vn = vec_normalize
+        if vn is not None:
+            if not self.auto_reset:
+                raise ValueError("vec_normalize needs auto_reset=True")
+            if vn.batch is not self:
+                raise ValueError("vec_normalize belongs to another batch")
+        norm_obs = vn is not None and vn.norm_obs
         self.join()
         # one slot per truncation an env can have in k steps: two of them are at least max_episode_steps apart
         limit = int(self._p.max_episode_steps)
@@ -420,6 +436,12 @@ class Rocket6DOFBatch:
             slot_obs = torch.empty(slots, 13, n, dtype=torch.float32, device=dev)
         obs_cm = torch.empty(k + 1, 14, n, dtype=torch.float32, device=dev)
         obs_cm[0].copy_(self.obs)
+        if norm_obs:          # hist[j]: (mean, sqrt(var + eps)) of obs_rms after j steps; last: obs[k] normalized
+            hist = vn.obs_hist(k + 1) if not vn.training else torch.empty(k + 1, 2, 13, dtype=torch.float64, device=dev)
+            if vn.training:
+                vn.update(vn.obs_rms, None, 0, hist[:1])
+            vn.normalize(obs_cm[0], obs_cm[0], hist, 0)
+            last_norm = torch.zeros(14, n, dtype=torch.float32, device=dev)
         acts = torch.empty(k, n, 3, dtype=torch.float32, device=dev)
         vals = torch.empty(k, n, dtype=torch.float32, device=dev)
         logp = torch.empty(k, n, dtype=torch.float32, device=dev)
@@ -458,6 +480,8 @@ class Rocket6DOFBatch:
                             with torch.cuda.stream(st):
                                 rews[j, first:first + count] = self.reward_f32[first:first + count]
                                 dones[j, first:first + count] = self.done[first:first + count]
+                    if norm_obs:
+                        self._vn_step(vn, lanes, obs_cm[j + 1], last_norm if j == k - 1 else obs_cm[j + 1], hist, j)
         finally:
             self._b.obs, self._b.reward_f32, self._b.done = saved
         self._advance(k)
@@ -465,12 +489,22 @@ class Rocket6DOFBatch:
             self.obs.copy_(obs_cm[k])
             self.reward_f32.copy_(rews[k - 1])
             self.done.copy_(dones[k - 1])
-        _, _, last_v, _ = self.policy_forward(mlp, stochastic=False, tensor_cores=tensor_cores)
+        if norm_obs:
+            last_v = torch.empty(n, dtype=torch.float32, device=dev)
+            with torch.cuda.device(dev):
+                self._policy(m, last_norm.data_ptr(), 0, n, tensor_cores, False, self.steps_done, a_env.data_ptr(),
+                             None, last_v.data_ptr(), None, torch.cuda.current_stream(dev), sde)
+        else:
+            _, _, last_v, _ = self.policy_forward(mlp, stochastic=False, tensor_cores=tensor_cores)
+        if vn is not None and k > 0:
+            vn.reward_pass(rews, dones)
         if slots:
             cur = torch.cuda.current_stream(dev)
             slot_v = torch.empty(slots, n, dtype=torch.float32, device=dev)
             with torch.cuda.device(dev):
                 for s in range(slots):
+                    if norm_obs:
+                        vn.normalize(slot_obs[s], slot_obs[s], hist, step=slot_step[s])
                     self._policy(m, slot_obs[s].data_ptr(), 0, n, tensor_cores, False, 0, a_env.data_ptr(), None,
                                  slot_v[s].data_ptr(), None, cur)
                 _lib.check(self.lib.r6_trunc_bootstrap(rews.data_ptr(), k, n, slots, slot_step.data_ptr(), slot_v.data_ptr(),
@@ -479,23 +513,58 @@ class Rocket6DOFBatch:
         return dict(obs=obs_cm[:k, :13].permute(0, 2, 1), actions=acts, values=vals, log_probs=logp, rewards=rews, dones=dones,
                     advantages=adv, returns=ret, last_values=last_v)
 
-    def step_policy(self, k: int, mlp: dict, *, tensor_cores=3, join: bool = True):
+    def _vn_step(self, vn, lanes: list, obs: torch.Tensor, out: torch.Tensor, hist: torch.Tensor, j: int):
+        """Step j of a collection with VecNormalize: the lanes join, obs_rms is updated with the step's observations
+        (training only; hist rows j, j + 1), and each lane normalizes its range of obs into out with hist row j + 1."""
+        if vn.training:
+            cur = torch.cuda.current_stream(self.device)
+            if self.lanes > 1:
+                for st in self._lane_streams:
+                    cur.wait_stream(st)
+            vn.observe(obs, hist[j:j + 2])
+            if self.lanes > 1:
+                self._lane_fork.record(cur)
+                for st in self._lane_streams:
+                    st.wait_event(self._lane_fork)
+        for _, first, count, st in lanes:
+            vn.normalize(obs, out, hist, j + 1, first, count, stream=st)
+
+    def step_policy(self, k: int, mlp: dict, *, tensor_cores=3, join: bool = True, vec_normalize=None):
         """k closed-loop env-steps as 2k launches: the policy kernel (a uniform GEMM chain at high occupancy) writes
         the actions, the step kernel consumes them — VecEnv semantics (auto-reset as configured).  Faster than the
         single fused rollout kernel for large batches; `rollout(k, ACT_MLP)` remains for one-episode semantics.
         With stream lanes every lane runs its own policy -> step chain (r6_policy_range, r6_step_range) for the k
         steps and the lanes are joined at the end (join=False leaves them running, as in `step`).  SB3 1.6's separate
-        policy / value towers run in modes 0, 2 and 3; tensor_cores=1 raises ValueError for them."""
+        policy / value towers run in modes 0, 2 and 3; tensor_cores=1 raises ValueError for them.
+
+        vec_normalize (a `vec_normalize.VecNormalize` with norm_obs) applies its frozen statistics, as SB3's
+        VecNormalize with training=False: before each policy launch every lane normalizes its range of obs into a
+        scratch [14, N] that the policy reads.  The statistics are never updated."""
         _check_separate(mlp, tensor_cores)
         act = getattr(self, "_policy_act", None)
         if act is None:
             act = self._policy_act = torch.empty(self.num_envs, 3, dtype=torch.float32, device=self.device)
         k, m = int(k), _lib.make_mlp(mlp)
+        vn = vec_normalize if vec_normalize is not None and vec_normalize.norm_obs else None
+        src = self.obs
+        if vn is not None:
+            self.join()
+            if vn.device != self.device:
+                raise ValueError("vec_normalize lives on another device")
+            hist = vn.obs_hist()
+            src = getattr(self, "_vn_obs", None)
+            if src is None:
+                src = self._vn_obs = torch.empty(14, self.num_envs, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
             lanes = self._fork(mlp=mlp)
+            if vn is not None:
+                for st in (self._lane_streams if self.lanes > 1 else ()):
+                    hist.record_stream(st)
             for j in range(k):
                 for ln, first, count, st in lanes:
-                    self._policy(m, self.obs.data_ptr(), first, count, tensor_cores, False, self.steps_done + j,
+                    if vn is not None:
+                        vn.normalize(self.obs, src, hist, 0, first, count, stream=st)
+                    self._policy(m, src.data_ptr(), first, count, tensor_cores, False, self.steps_done + j,
                                  act.data_ptr(), None, None, None, st)
                     self._env_step(ln, first, count, act.data_ptr(), self.steps_done + j, st)
         self._advance(k, join)

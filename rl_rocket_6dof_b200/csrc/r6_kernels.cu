@@ -14,6 +14,8 @@
 //   rank_sum_kernel                  data-parallel PPO: the rank-ordered float64 sum of the ranks' gathered gradients
 //   (policy_sep_kernel, policy_tc5_sep_kernel, ppo_grad_sep_kernel: the same for SB3 1.6's separate policy / value towers)
 //   trunc_record_kernel, trunc_bootstrap_kernel   time-limit truncations filed per step, bootstrapped with the critic
+//   vn_moments_partial_kernel | vn_moments_final_kernel, vn_update_kernel, vn_normalize_kernel, vn_ret_scan_kernel,
+//   vn_scale_rewards_kernel   VecNormalize: batch moments, running statistics, observation and reward normalization
 //   reset_kernel, sim_raw_kernel, tgo_kernel, gae_kernel, peak_fma_kernel
 //
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo (see build.py).
@@ -1516,6 +1518,213 @@ trunc_bootstrap_kernel(float *__restrict__ rew, int T, int64_t n, int slots, con
     }
 }
 
+// VecNormalize (SB3 1.6's running observation / return statistics, r6_vn_*).  Batch moments are float64
+// (count, mean, M2).  A warp sums (x - K) and (x - K)^2 over its elements, K the value of its first element, in a fixed
+// shuffle tree; its (count, mean, M2) then enter Chan's pairwise combination, in warp order within a CTA and in CTA
+// order across CTAs (vn_moments_final_kernel).  Every grid and order is a function of the element count only, so the
+// moments are bit-reproducible on any device and whatever the stream lanes did before.
+struct VnMom {
+    double c, m, m2;
+};
+constexpr int kVnThreads = 256;
+constexpr int kVnColsPerCta = 2048;       // observation moments: 8 columns per thread
+
+// Chan, Golub and LeVeque in (a, b) order, the arithmetic of ppo.combine_moments; an empty side gives the other back
+__device__ __forceinline__ VnMom vn_chan(VnMom a, VnMom b)
+{
+    if (b.c == 0.0) return a;
+    if (a.c == 0.0) return b;
+    const double tot = __dadd_rn(a.c, b.c), d = __dsub_rn(b.m, a.m);
+    return VnMom{tot, __dadd_rn(a.m, __dmul_rn(d, __ddiv_rn(b.c, tot))),
+                 __dadd_rn(__dadd_rn(a.m2, b.m2), __dmul_rn(__dmul_rn(d, d), __ddiv_rn(__dmul_rn(a.c, b.c), tot)))};
+}
+
+// The warp's moments from each lane's (count, sum (x - K), sum (x - K)^2), K shared by the warp; valid in lane 0.
+__device__ __forceinline__ VnMom vn_warp_moments(double c, double s1, double s2, double K)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        c = __dadd_rn(c, __shfl_down_sync(0xffffffffu, c, o));
+        s1 = __dadd_rn(s1, __shfl_down_sync(0xffffffffu, s1, o));
+        s2 = __dadd_rn(s2, __shfl_down_sync(0xffffffffu, s2, o));
+    }
+    if (c == 0.0) return VnMom{0.0, 0.0, 0.0};
+    const double m2 = __dsub_rn(s2, __ddiv_rn(__dmul_rn(s1, s1), c));
+    return VnMom{c, __dadd_rn(K, __ddiv_rn(s1, c)), m2 > 0.0 ? m2 : 0.0};
+}
+
+__device__ __forceinline__ VnMom vn_shfl_down(VnMom a, int o)
+{
+    return VnMom{__shfl_down_sync(0xffffffffu, a.c, o), __shfl_down_sync(0xffffffffu, a.m, o),
+                 __shfl_down_sync(0xffffffffu, a.m2, o)};
+}
+
+__device__ __forceinline__ void vn_store(double *p, VnMom a)
+{
+    p[0] = a.c;
+    p[1] = a.m;
+    p[2] = a.m2;
+}
+
+// Partial moments of rows [0, gridDim.y) of x [rows][n] over columns [first, first + count): CTA b takes the chunk
+// [b chunk, (b + 1) chunk) of the range, thread t its columns t, t + 256, ... (coalesced), and writes its CTA's moments
+// to part[row][b].
+__global__ void __launch_bounds__(kVnThreads)
+vn_moments_partial_kernel(const float *__restrict__ x, int64_t n, int64_t first, int64_t count, int64_t chunk,
+                          double *__restrict__ part)
+{
+    __shared__ VnMom wm[kVnThreads / 32];
+    const int row = blockIdx.y, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t lo = (int64_t)blockIdx.x * chunk, hi = min(lo + chunk, count);
+    const float *xr = x + (int64_t)row * n + first;
+    const int64_t k0 = lo + 32 * warp;
+    const double K = k0 < hi ? (double)xr[k0] : 0.0;
+    double c = 0.0, s1 = 0.0, s2 = 0.0;
+    for (int64_t k0 = lo + threadIdx.x; k0 < hi; k0 += 8 * kVnThreads) {     // the 8 loads issued before the adds
+        float v[8];
+#pragma unroll
+        for (int u = 0; u < 8; u++) v[u] = k0 + u * kVnThreads < hi ? xr[k0 + u * kVnThreads] : 0.0f;
+#pragma unroll
+        for (int u = 0; u < 8; u++)
+            if (k0 + u * kVnThreads < hi) {
+                const double d = __dsub_rn((double)v[u], K);
+                c = __dadd_rn(c, 1.0);
+                s1 = __dadd_rn(s1, d);
+                s2 = __dadd_rn(s2, __dmul_rn(d, d));
+            }
+    }
+    const VnMom w = vn_warp_moments(c, s1, s2, K);
+    if (lane == 0) wm[warp] = w;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        VnMom a = wm[0];
+        for (int i = 1; i < kVnThreads / 32; i++) a = vn_chan(a, wm[i]);
+        vn_store(part + ((int64_t)row * gridDim.x + blockIdx.x) * 3, a);
+    }
+}
+
+// out[row] = the CTA-order combination of part[row][0 .. parts): thread t combines parts t, t + 256, ... in order, then
+// a fixed shuffle tree and the warps in order.
+__global__ void __launch_bounds__(kVnThreads)
+vn_moments_final_kernel(const double *__restrict__ part, int64_t parts, double *__restrict__ out)
+{
+    __shared__ VnMom wm[kVnThreads / 32];
+    const int row = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const double *p = part + (int64_t)row * parts * 3;
+    VnMom a{0.0, 0.0, 0.0};
+    for (int64_t b = threadIdx.x; b < parts; b += kVnThreads) a = vn_chan(a, VnMom{p[b * 3], p[b * 3 + 1], p[b * 3 + 2]});
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {               // lane l takes lane l + o's combination of the next o lanes
+        const VnMom b = vn_shfl_down(a, o);
+        if ((lane & (2 * o - 1)) == 0) a = vn_chan(a, b);
+    }
+    if (lane == 0) wm[warp] = a;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        VnMom r = wm[0];
+        for (int i = 1; i < kVnThreads / 32; i++) r = vn_chan(r, wm[i]);
+        vn_store(out + (int64_t)row * 3, r);
+    }
+}
+
+// SB3's RunningMeanStd.update_from_moments, `steps` times in sequence, on rms = [mean[dim], var[dim], count]; the
+// batch variance is M2 / count (ddof = 0).  hist [steps + 1][2][dim] (nullable): row 0 the (mean, sqrt(var + eps)) before
+// the first update, row s + 1 after update s.  One thread per component; every thread carries the shared count.
+__global__ void __launch_bounds__(1024)
+vn_update_kernel(double *__restrict__ rms, int dim, const double *__restrict__ mom, int steps, double eps,
+                 double *__restrict__ hist)
+{
+    const int d = threadIdx.x;
+    double count = rms[2 * dim];
+    double mean = d < dim ? rms[d] : 0.0, var = d < dim ? rms[dim + d] : 1.0;
+    if (hist && d < dim) {
+        hist[d] = mean;
+        hist[dim + d] = __dsqrt_rn(__dadd_rn(var, eps));
+    }
+    for (int s = 0; s < steps; s++) {
+        const double *ms = mom + (int64_t)s * dim * 3;
+        const double bc = ms[0];
+        if (bc > 0.0 && d < dim) {
+            const double bm = ms[d * 3 + 1], bv = __ddiv_rn(ms[d * 3 + 2], bc);
+            const double delta = __dsub_rn(bm, mean), tot = __dadd_rn(count, bc);
+            mean = __dadd_rn(mean, __ddiv_rn(__dmul_rn(delta, bc), tot));
+            const double m2 = __dadd_rn(__dadd_rn(__dmul_rn(var, count), __dmul_rn(bv, bc)),
+                                        __ddiv_rn(__dmul_rn(__dmul_rn(__dmul_rn(delta, delta), count), bc), __dadd_rn(count, bc)));
+            var = __ddiv_rn(m2, __dadd_rn(count, bc));
+        }
+        if (bc > 0.0) count = __dadd_rn(bc, count);
+        if (hist && d < dim) {
+            double *h = hist + (int64_t)(s + 1) * 2 * dim;
+            h[d] = mean;
+            h[dim + d] = __dsqrt_rn(__dadd_rn(var, eps));
+        }
+    }
+    if (d < dim) {
+        rms[d] = mean;
+        rms[dim + d] = var;
+    }
+    __syncthreads();                                  // every thread has read the old count
+    if (d == 0) rms[2 * dim] = count;
+}
+
+__device__ __forceinline__ double vn_clip(double x, double c) { return x < -c ? -c : (x > c ? c : x); }
+
+// out[c][i] = fl32(clip((fl64(in[c][i]) - mean[c]) / std[c], +-clip)) for rows c < 13 of env range [i0, i1), (mean, std)
+// the history row `hrow`, or with `step` the row step[i] + 1 of each column (columns with step[i] < 0 or a row outside
+// the history are not written).  in and out may be the same block.
+__global__ void __launch_bounds__(kVnThreads)
+vn_normalize_kernel(const float *in, float *out, int64_t n, int64_t i0, int64_t i1, const double *__restrict__ hist,
+                    int hrow, const int32_t *__restrict__ step, int hrows, double clip)
+{
+    const int64_t i = i0 + (int64_t)blockIdx.x * kVnThreads + threadIdx.x;
+    if (i >= i1) return;
+    int r = hrow;
+    if (step) {
+        r = step[i];
+        if (r < 0 || r + 1 >= hrows) return;
+        r += 1;
+    }
+    const double *h = hist + (int64_t)r * 2 * 13;
+#pragma unroll
+    for (int c = 0; c < 13; c++)
+        out[(int64_t)c * n + i] = (float)vn_clip(__ddiv_rn(__dsub_rn((double)in[(int64_t)c * n + i], h[c]), h[13 + c]), clip);
+}
+
+// The discounted-return scan of a rollout, one thread per env: ret = ret gamma + r (float64, no FMA) at every step, the
+// per-step warp moments of ret into part[t][global warp] (before the reset), ret = 0 where done; ret carries over
+// rollouts.  No barrier: the warps' moments are combined in warp order by vn_moments_final_kernel.
+__global__ void __launch_bounds__(kVnThreads)
+vn_ret_scan_kernel(const float *__restrict__ rew, const uint8_t *__restrict__ done, int T, int64_t n,
+                   double *__restrict__ returns, double gamma, double *__restrict__ part)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t i = (int64_t)blockIdx.x * kVnThreads + threadIdx.x, wg = i >> 5, nw = (int64_t)gridDim.x * (kVnThreads / 32);
+    const bool live = i < n;
+    double ret = live ? returns[i] : 0.0;
+    for (int t = 0; t < T; t++) {
+        const int64_t o = (int64_t)t * n + i;
+        if (live) ret = __dadd_rn(__dmul_rn(ret, gamma), (double)rew[o]);
+        const double K = __shfl_sync(0xffffffffu, ret, 0);
+        const double d = __dsub_rn(ret, K);
+        const VnMom w = vn_warp_moments(live ? 1.0 : 0.0, live ? d : 0.0, live ? __dmul_rn(d, d) : 0.0, K);
+        if (lane == 0) vn_store(part + ((int64_t)t * nw + wg) * 3, w);
+        if (live && done[o]) ret = 0.0;
+    }
+    if (live) returns[i] = ret;
+}
+
+// rew[t][i] = fl32(clip(fl64(rew[t][i]) / std_t, +-clip)), std_t = hist[t + 1][1] (r6_vn_update's history of ret_rms).
+__global__ void __launch_bounds__(kVnThreads)
+vn_scale_rewards_kernel(float *__restrict__ rew, int T, int64_t n, const double *__restrict__ hist, double clip)
+{
+    const int64_t i = (int64_t)blockIdx.x * kVnThreads + threadIdx.x;
+    if (i >= n) return;
+    for (int t = 0; t < T; t++) {
+        float *r = rew + (int64_t)t * n + i;
+        *r = (float)vn_clip(__ddiv_rn((double)*r, hist[(int64_t)(t + 1) * 2 + 1]), clip);
+    }
+}
+
 // PPO minibatch gradient (r6_ppo_grad).  A grid of ppo_ctas(B) CTAs (a function of B only, so the summation order and
 // the result do not depend on the device) walks tiles of 128 samples.  Each thread runs the forward pass, loss head
 // and deltas of its sample (r6_ppo.cuh) and stages its inputs, activations and deltas in shared memory unit-major,
@@ -2769,6 +2978,85 @@ int r6_trunc_bootstrap(float *rew, int32_t T, int64_t n, int32_t slots, const in
     trunc_bootstrap_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rew, T, n, slots, slot_step, slot_values,
                                                                                        (float)gamma);
     return check_launch("r6_trunc_bootstrap");
+}
+
+static int64_t vn_obs_parts(int64_t count) { return (count + kVnColsPerCta - 1) / kVnColsPerCta; }
+static int64_t vn_ret_ctas(int64_t n) { return (n + kVnThreads - 1) / kVnThreads; }
+static int64_t vn_ret_parts(int64_t n) { return vn_ret_ctas(n) * (kVnThreads / 32); }
+
+int64_t r6_vn_moments_work_bytes(int64_t count, int32_t rows)
+{
+    if (count < 1 || rows < 1) return 0;
+    return vn_obs_parts(count) * rows * 3 * (int64_t)sizeof(double);
+}
+
+int64_t r6_vn_ret_work_bytes(int32_t T, int64_t n)
+{
+    if (T < 1 || n < 1) return 0;
+    return vn_ret_parts(n) * T * 3 * (int64_t)sizeof(double);
+}
+
+int r6_vn_moments(const float *x, int64_t n, int32_t rows, int64_t first, int64_t count, double *out, void *work,
+                  void *stream)
+{
+    if (!x || !out || !work) return fail(R6_EINVAL, "null pointer%s");
+    if (n < 1 || rows < 1 || rows > 65535) return fail(R6_EINVAL, "need n >= 1 and 1 <= rows <= 65535%s");
+    if (first < 0 || count < 1 || first + count > n) return fail(R6_EINVAL, "column range empty or outside [0, n)%s");
+    const int64_t parts = vn_obs_parts(count);
+    if (parts > INT32_MAX) return fail(R6_EINVAL, "count too large%s");
+    double *part = static_cast<double *>(work);
+    vn_moments_partial_kernel<<<dim3((unsigned)parts, (unsigned)rows), kVnThreads, 0, (cudaStream_t)stream>>>(
+        x, n, first, count, kVnColsPerCta, part);
+    vn_moments_final_kernel<<<(unsigned)rows, kVnThreads, 0, (cudaStream_t)stream>>>(part, parts, out);
+    return check_launch("r6_vn_moments");
+}
+
+int r6_vn_update(double *rms, int32_t dim, const double *moments, int32_t steps, double eps, double *hist, void *stream)
+{
+    if (!rms || (steps > 0 && !moments)) return fail(R6_EINVAL, "null pointer%s");
+    if (dim < 1 || dim > 1024 || steps < 0) return fail(R6_EINVAL, "need 1 <= dim <= 1024 and steps >= 0%s");
+    if (!(eps >= 0.0) || eps == INFINITY) return fail(R6_EINVAL, "eps must be finite and >= 0%s");
+    if (steps == 0 && !hist) return R6_OK;
+    vn_update_kernel<<<1, dim, 0, (cudaStream_t)stream>>>(rms, dim, moments, steps, eps, hist);
+    return check_launch("r6_vn_update");
+}
+
+int r6_vn_normalize(const float *in, float *out, int64_t n, int64_t first, int64_t count, const double *hist,
+                    int32_t hist_row, const int32_t *step, int32_t hist_rows, double clip, void *stream)
+{
+    if (!in || !out || !hist) return fail(R6_EINVAL, "null pointer%s");
+    if (n < 0) return fail(R6_EINVAL, "n < 0%s");
+    if (first < 0 || count < 0 || first + count > n) return fail(R6_EINVAL, "env sub-range outside [0, n)%s");
+    if (hist_rows < 1 || (!step && (hist_row < 0 || hist_row >= hist_rows)))
+        return fail(R6_EINVAL, "need hist_rows >= 1 and, without step, 0 <= hist_row < hist_rows%s");
+    if (!(clip > 0.0)) return fail(R6_EINVAL, "clip must be > 0%s");
+    if (count == 0) return R6_OK;
+    vn_normalize_kernel<<<(unsigned)((count + kVnThreads - 1) / kVnThreads), kVnThreads, 0, (cudaStream_t)stream>>>(
+        in, out, n, first, first + count, hist, hist_row, step, hist_rows, clip);
+    return check_launch("r6_vn_normalize");
+}
+
+int r6_vn_ret_moments(const float *rew, const uint8_t *done, int32_t T, int64_t n, double *returns, double gamma,
+                      double *out, void *work, void *stream)
+{
+    if (!rew || !done || !returns || !out || !work) return fail(R6_EINVAL, "null pointer%s");
+    if (T < 1 || T > 65535 || n < 1) return fail(R6_EINVAL, "need 1 <= T <= 65535 and n >= 1%s");
+    if (!(gamma >= 0.0) || gamma == INFINITY) return fail(R6_EINVAL, "gamma must be finite and >= 0%s");
+    const int64_t parts = vn_ret_parts(n);
+    if (vn_ret_ctas(n) > INT32_MAX) return fail(R6_EINVAL, "n too large%s");
+    double *part = static_cast<double *>(work);
+    vn_ret_scan_kernel<<<(unsigned)vn_ret_ctas(n), kVnThreads, 0, (cudaStream_t)stream>>>(rew, done, T, n, returns, gamma, part);
+    vn_moments_final_kernel<<<(unsigned)T, kVnThreads, 0, (cudaStream_t)stream>>>(part, parts, out);
+    return check_launch("r6_vn_ret_moments");
+}
+
+int r6_vn_scale_rewards(float *rew, int32_t T, int64_t n, const double *hist, double clip, void *stream)
+{
+    if (!rew || !hist) return fail(R6_EINVAL, "null pointer%s");
+    if (T < 1 || n < 1) return fail(R6_EINVAL, "need T >= 1 and n >= 1%s");
+    if (!(clip > 0.0)) return fail(R6_EINVAL, "clip must be > 0%s");
+    vn_scale_rewards_kernel<<<(unsigned)vn_ret_ctas(n), kVnThreads, 0, (cudaStream_t)stream>>>(rew, T, n, hist, clip);
+    return check_launch("r6_vn_scale_rewards");
 }
 
 int r6_ppo_rollout_size(void) { return (int)sizeof(R6PpoRollout); }

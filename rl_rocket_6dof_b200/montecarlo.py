@@ -39,7 +39,7 @@ def run_montecarlo(n_episodes: int, weights: Dict[str, np.ndarray], env_config: 
                    sb3_config: Optional[dict] = None, *, device="cuda", seed: Optional[int] = None,
                    chunk_steps: int = 128, csv_path: Optional[str] = None, ic_table: Optional[np.ndarray] = None,
                    env_offset: int = 0, num_envs_global: Optional[int] = None, tensor_cores: bool = False,
-                   two_kernel: Optional[bool] = None, lanes: int = 1) -> dict:
+                   two_kernel: Optional[bool] = None, lanes: int = 1, vec_normalize=None) -> dict:
     """Returns {"columns": {name: np.ndarray[n]}, "mean": {...}, "std": {...}, "episode_length", "episode_return",
     "landed", "stats"}.  `std` is the sample standard deviation (pandas' default, ddof=1).
     tensor_cores=True evaluates the policy on the tensor cores at float32 accuracy instead of with float32 FMAs.
@@ -47,7 +47,16 @@ def run_montecarlo(n_episodes: int, weights: Dict[str, np.ndarray], env_config: 
     (`step_policy`: tcgen05 3xTF32 policy when tensor_cores, multi-pass integrator, stream `lanes`) instead of the one
     fused rollout kernel — about twice the throughput for large dispersions, same one-episode semantics.  SB3 1.6's
     separate policy / value towers (weights with vf_w0 ...) always take the two-kernel path: the fused rollout kernel
-    does not run that network."""
+    does not run that network.
+
+    vec_normalize (the path of a `VecNormalize.save` .npz, or a VecNormalize whose statistics are used) runs a policy
+    trained under VecNormalize: its frozen observation statistics normalize the observations before every policy launch
+    (SB3's training=False; they are never updated).  It takes the two-kernel path; two_kernel=False raises ValueError."""
+    if vec_normalize is not None:
+        if two_kernel is False:
+            raise ValueError("vec_normalize runs on the two-kernel path only (the fused rollout kernel has no "
+                             "normalization): two_kernel must be True or None")
+        two_kernel = True
     if _policy.is_separate(weights):
         if two_kernel is False:
             raise ValueError("the separate policy / value towers have no fused rollout kernel: two_kernel must be True")
@@ -59,6 +68,15 @@ def run_montecarlo(n_episodes: int, weights: Dict[str, np.ndarray], env_config: 
                           num_envs_global=num_envs_global, lanes=lanes if two_kernel else 1,
                           split_step=True if two_kernel else None)
     w = _policy.to_device(weights, env.device)
+    vn = None
+    if vec_normalize is not None:
+        from .vec_normalize import VecNormalize
+        vn = VecNormalize(env, training=False)
+        if isinstance(vec_normalize, VecNormalize):
+            vn.obs_rms.copy_(vec_normalize.obs_rms)
+            vn.norm_obs, vn.clip_obs, vn.epsilon = vec_normalize.norm_obs, vec_normalize.clip_obs, vec_normalize.epsilon
+        else:
+            vn.load(vec_normalize)
     env.reset()
     max_steps = int(env.params.max_episode_steps) if env.params.max_episode_steps else 1500
     steps = 0
@@ -66,7 +84,7 @@ def run_montecarlo(n_episodes: int, weights: Dict[str, np.ndarray], env_config: 
         chunk_steps = min(chunk_steps, 64)      # frozen envs still cost a policy launch: look for the end more often
     while steps < max_steps:
         if two_kernel:
-            env.step_policy(chunk_steps, w, tensor_cores=3 if tensor_cores else 0)
+            env.step_policy(chunk_steps, w, tensor_cores=3 if tensor_cores else 0, vec_normalize=vn)
         else:
             env.rollout(chunk_steps, ACT_MLP_TC if tensor_cores else ACT_MLP, mlp=w)
         steps += chunk_steps
@@ -112,11 +130,13 @@ def main(argv=None) -> int:
     ap.add_argument("--seed", type=int, default=None)
     ap.add_argument("--device", default="cuda")
     ap.add_argument("--tensor-cores", action="store_true", help="evaluate the policy with the 3xTF32 MMA tiles")
+    ap.add_argument("--vecnormalize", default=None, metavar="STATS_NPZ",
+                    help="VecNormalize statistics (VecNormalize.save) the policy was trained with")
     a = ap.parse_args(argv)
     w = _policy.load_npz(a.policy) if a.policy.endswith(".npz") else _policy.load_sb3_zip(a.policy)
     sb3_config, env_config = load_config(a.config)
     res = run_montecarlo(a.episodes, w, env_config, sb3_config, device=a.device, seed=a.seed, csv_path=a.csv,
-                         tensor_cores=a.tensor_cores)
+                         tensor_cores=a.tensor_cores, vec_normalize=a.vecnormalize)
     print(format_report(res))
     print(f"episodes: {a.episodes}, landed: {int(res['landed'].sum())}, mean length {res['episode_length'].mean():.1f} steps")
     return 0

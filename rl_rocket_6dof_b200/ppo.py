@@ -442,11 +442,22 @@ class PPOTrainer:
         statistics summed by r6_rank_sum) are global, hence the same on every rank; num_timesteps counts W n n_steps
         env-steps per iteration.
     A group of size 1 trains exactly as group=None (there is nothing to exchange); train() must be called on every rank
-    with that rank's rollout of the same shape.  With group=None the trainer issues the same launches as before."""
+    with that rank's rollout of the same shape.  With group=None the trainer issues the same launches as before.
 
-    def __init__(self, batch, params: ActorCriticParams, cfg: Optional[PPOConfig] = None, seed: int = 0, group=None):
+    vec_normalize (a `vec_normalize.VecNormalize` of `batch`, default None) trains as SB3's PPO inside VecNormalize:
+    `learn` calls its reset() after the batch's and passes it to every collection, so the rollouts hold normalized
+    observations and rewards (train() is unchanged).  With a group, it must have been built with the same group."""
+
+    def __init__(self, batch, params: ActorCriticParams, cfg: Optional[PPOConfig] = None, seed: int = 0, group=None,
+                 vec_normalize=None):
         self.batch, self.params, self.cfg = batch, params, cfg or PPOConfig()
         self.group = group
+        if vec_normalize is not None:
+            if vec_normalize.batch is not batch:
+                raise ValueError("vec_normalize belongs to another batch")
+            if vec_normalize.group is not group:
+                raise ValueError("vec_normalize must have the trainer's process group")
+        self.vec_normalize = vec_normalize
         self.world, self.rank = 1, 0
         local_error = 0
         if params.separate and int(self.cfg.tensor_cores) == 1:
@@ -646,12 +657,14 @@ class PPOTrainer:
         b, cfg = self.batch, self.cfg
         if self.num_timesteps == 0:
             b.reset()
+            if self.vec_normalize is not None:
+                self.vec_normalize.reset()
         logs = []
         while self.num_timesteps < total_timesteps:
             b.reset_stats()
             ro = b.collect_rollout(cfg.n_steps, self.params.mlp(), gamma=cfg.gamma, gae_lambda=cfg.gae_lambda,
                                    tensor_cores=cfg.tensor_cores, bootstrap_truncated=True,
-                                   sde_sample_freq=cfg.sde_sample_freq)
+                                   sde_sample_freq=cfg.sde_sample_freq, vec_normalize=self.vec_normalize)
             self.num_timesteps += cfg.n_steps * b.num_envs * self.world
             self.progress_remaining = 1.0 - self.num_timesteps / total_timesteps
             stats = self._global_stats() if self.world > 1 else None
