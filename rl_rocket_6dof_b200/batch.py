@@ -63,6 +63,7 @@ class Rocket6DOFBatch:
         self.num_envs_global = int(num_envs_global if num_envs_global is not None else env_offset + num_envs)
         self.seed_value = int(params.seed if seed is None else seed)
         self.auto_reset = auto_reset
+        self.time_limit = bool(time_limit)
         if precision not in ("fp64", "fp32"):
             raise ValueError("precision must be 'fp64' (parity path) or 'fp32' (throughput path)")
         self.precision = precision

@@ -35,6 +35,48 @@ def dispersion_columns(terminal_state: torch.Tensor) -> Dict[str, torch.Tensor]:
     }
 
 
+def landed(flags: torch.Tensor) -> torch.Tensor:
+    """The envs whose episode ended in a landing: every landing-condition bit of the episode flags set."""
+    return (flags & 0xF8) == 0xF8
+
+
+def run_episodes(batch: Rocket6DOFBatch, weights: Dict[str, torch.Tensor], *, tensor_cores=0, vec_normalize=None,
+                 chunk_steps: int = 128, fused: bool = False) -> dict:
+    """One deterministic episode of every env of `batch` (auto_reset=False): `batch.reset()`, then the closed loop until
+    every env is done or max_episode_steps have run.  `weights` are device tensors (`policy.to_device`,
+    `ActorCriticParams.mlp()`; a gSDE log_std is ignored, the deterministic action is the mean).  A reused batch draws
+    fresh initial conditions every call: r6_reset keys them by (seed, global env id, episode id) and counts the episode.
+
+    The loop is `step_policy` (policy kernel + env-step kernels per step; tensor_cores is its mode, vec_normalize a
+    frozen `VecNormalize` of the batch applied before every policy launch), or with fused=True the fused rollout kernel
+    (`rollout(..., ACT_MLP / ACT_MLP_TC)`, shared trunk only, no normalization).  The host reads one byte per chunk of
+    steps to see whether every env is done.
+
+    Returns {"episode_return" float64 [n], "episode_length" int64 [n], "flags" uint8 [n], "terminal_state" [14, n],
+    "stats": the batch's episode statistics of this call}; the tensors live on the device, the first, third and fourth
+    are views of the batch's buffers (valid until its next step or reset)."""
+    if batch.auto_reset:
+        raise ValueError("run_episodes needs one-episode semantics: a batch with auto_reset=False")
+    if fused and vec_normalize is not None:
+        raise ValueError("the fused rollout kernel has no observation normalization")
+    batch.reset()
+    batch.reset_stats()
+    max_steps = int(batch.params.max_episode_steps) if batch.params.max_episode_steps else 1500
+    if not fused:
+        chunk_steps = min(chunk_steps, 64)      # frozen envs still cost a policy launch: look for the end more often
+    steps = 0
+    while steps < max_steps:
+        if fused:
+            batch.rollout(chunk_steps, ACT_MLP_TC if tensor_cores else ACT_MLP, mlp=weights)
+        else:
+            batch.step_policy(chunk_steps, weights, tensor_cores=tensor_cores, vec_normalize=vec_normalize)
+        steps += chunk_steps
+        if bool(batch.done.all()):        # one device->host byte per chunk, not per step
+            break
+    return {"episode_return": batch.ep_info[0], "episode_length": batch.ep_info[1].to(torch.int64),
+            "flags": batch.flags, "terminal_state": batch.terminal_state, "stats": batch.stats_dict()}
+
+
 def run_montecarlo(n_episodes: int, weights: Dict[str, np.ndarray], env_config: Optional[dict] = None,
                    sb3_config: Optional[dict] = None, *, device="cuda", seed: Optional[int] = None,
                    chunk_steps: int = 128, csv_path: Optional[str] = None, ic_table: Optional[np.ndarray] = None,
@@ -71,37 +113,21 @@ def run_montecarlo(n_episodes: int, weights: Dict[str, np.ndarray], env_config: 
     vn = None
     if vec_normalize is not None:
         from .vec_normalize import VecNormalize
-        vn = VecNormalize(env, training=False)
-        if isinstance(vec_normalize, VecNormalize):
-            vn.obs_rms.copy_(vec_normalize.obs_rms)
-            vn.norm_obs, vn.clip_obs, vn.epsilon = vec_normalize.norm_obs, vec_normalize.clip_obs, vec_normalize.epsilon
-        else:
-            vn.load(vec_normalize)
-    env.reset()
-    max_steps = int(env.params.max_episode_steps) if env.params.max_episode_steps else 1500
-    steps = 0
-    if two_kernel:
-        chunk_steps = min(chunk_steps, 64)      # frozen envs still cost a policy launch: look for the end more often
-    while steps < max_steps:
-        if two_kernel:
-            env.step_policy(chunk_steps, w, tensor_cores=3 if tensor_cores else 0, vec_normalize=vn)
-        else:
-            env.rollout(chunk_steps, ACT_MLP_TC if tensor_cores else ACT_MLP, mlp=w)
-        steps += chunk_steps
-        if bool(env.done.all()):        # one device->host byte per chunk, not per step
-            break
+        vn = VecNormalize.frozen(env, vec_normalize)
+    ep = run_episodes(env, w, tensor_cores=3 if tensor_cores else 0, vec_normalize=vn, chunk_steps=chunk_steps,
+                      fused=not two_kernel)
     cols = dispersion_columns(env.terminal_state)
     out_cols = {k: v.cpu().numpy() for k, v in cols.items()}
     res = {
         "columns": out_cols,
         "mean": {k: float(np.mean(v)) for k, v in out_cols.items()},
         "std": {k: float(np.std(v, ddof=1)) if len(v) > 1 else 0.0 for k, v in out_cols.items()},
-        "episode_return": env.ep_info[0].cpu().numpy(),
-        "episode_length": env.ep_info[1].cpu().numpy().astype(np.int64),
-        "landed": ((env.flags & 0xF8) == 0xF8).cpu().numpy(),
-        "flags": env.flags.cpu().numpy(),
-        "terminal_state": env.terminal_state.t().cpu().numpy(),
-        "stats": env.stats_dict(),
+        "episode_return": ep["episode_return"].cpu().numpy(),
+        "episode_length": ep["episode_length"].cpu().numpy(),
+        "landed": landed(ep["flags"]).cpu().numpy(),
+        "flags": ep["flags"].cpu().numpy(),
+        "terminal_state": ep["terminal_state"].t().cpu().numpy(),
+        "stats": ep["stats"],
     }
     if csv_path:
         with open(csv_path, "w", newline="") as f:

@@ -648,12 +648,17 @@ class PPOTrainer:
             logs["train/clip_range_vf"] = vfc
         return logs
 
-    def learn(self, total_timesteps: int, callback: Optional[Callable[[dict], None]] = None) -> list:
+    def learn(self, total_timesteps: int, callback: Optional[Callable[[dict], None]] = None,
+              eval_callback=None) -> list:
         """Alternates collect_rollout (n_steps of every env) and train until total_timesteps env-steps; returns one log
         dict per iteration (train/ logs plus the env's episode statistics of that collection under rollout/).  As in
         SB3, progress_remaining is updated after the collection, so update i of a run from 0 uses
         1 - i n_steps N / total_timesteps (the last one 0 when total_timesteps is a multiple of n_steps N).  With a group,
-        N is the global env count W n and rollout/ holds the group's statistics."""
+        N is the global env count W n and rollout/ holds the group's statistics.
+
+        eval_callback (an `evaluation.EvalCallback`, default None) is called after each collection and before its
+        train(), with the parameters that collected it; the eval/ logs it returns join that iteration's log.  It
+        touches nothing the training reads, so the parameters and the other logs are those of a run without it."""
         b, cfg = self.batch, self.cfg
         if self.num_timesteps == 0:
             b.reset()
@@ -669,6 +674,8 @@ class PPOTrainer:
             self.progress_remaining = 1.0 - self.num_timesteps / total_timesteps
             stats = self._global_stats() if self.world > 1 else None
             log = {"rollout/" + k: v for k, v in b.stats_dict(stats).items()}
+            if eval_callback is not None:
+                log.update(eval_callback.on_rollout_end(self))
             log.update(self.train(ro))
             log["time/total_timesteps"] = self.num_timesteps
             logs.append(log)

@@ -216,6 +216,20 @@ class VecNormalize:
                           "norm_obs": self.norm_obs, "norm_reward": self.norm_reward, "gamma": self.gamma,
                           "epsilon": self.epsilon, "training": self.training})
 
+    @classmethod
+    def frozen(cls, batch, source, into: Optional["VecNormalize"] = None) -> "VecNormalize":
+        """A `VecNormalize(batch, training=False)` holding frozen observation statistics for a deterministic evaluation:
+        `source` is the path of a `save` .npz (everything `load` restores), or a VecNormalize whose obs_rms, norm_obs,
+        clip_obs and epsilon are copied (SB3's sync_envs_normalization; rewards are not normalized by an evaluation).
+        `into` (a VecNormalize of `batch`) is refreshed instead of building a new one."""
+        vn = into if into is not None else cls(batch, training=False)
+        if isinstance(source, VecNormalize):
+            vn.obs_rms.copy_(source.obs_rms)
+            vn.norm_obs, vn.clip_obs, vn.epsilon = source.norm_obs, source.clip_obs, source.epsilon
+        else:
+            vn.load(source)
+        return vn
+
     def load(self, path: str) -> "VecNormalize":
         """Restores what `save` wrote (statistics and settings, as unpickling SB3's object does); `returns` is left as
         it is.  Returns self."""
